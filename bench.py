@@ -19,6 +19,8 @@ verify  : at N = 1, config 2 (or with --verify; --no-verify skips it), outside e
           over a <= 10 M-read file of the same generator is compared with the oracle, every row of every column
           (oracle/verify.py); the result goes into the line's "verify" key.
 --config: 2 (default) full projection | 3 fixed-width projection | 4 BAI region query chr1:50M-150M | 5 long reads
+--dump-outputs DIR: after the timed steps, <= 64 MB of what the last end-to-end step handed its caller, as float .npy files
+          (column_arrays): 16 windows of 1024 rows at seeded offsets, so two builds can be compared output for output
 """
 import argparse
 import json
@@ -30,6 +32,10 @@ import sys
 import threading
 import time
 from pathlib import Path
+
+import numpy as np
+import pyarrow as pa
+import pyarrow.compute as pc
 
 ROOT = Path(__file__).resolve().parent
 PKG = ROOT / "datafusion-bio-formats_b200"
@@ -51,10 +57,10 @@ def ensure_bam(reads: int, seed: int, want_bai: bool, mode: str = "short") -> tu
     meta = path.with_suffix(".json")
     if path.exists() and meta.exists() and (not want_bai or Path(str(path) + ".bai").exists()):
         return path, json.loads(meta.read_text())
-    exe = ROOT / "tools" / "_build" / "bamgen"
+    exe = ROOT / "tools" / "_build" / "bamgen"          # built by __graft_entry__.build()
     src = ROOT / "tools" / "bamgen.cpp"
     if not exe.exists() or exe.stat().st_mtime < src.stat().st_mtime:
-        exe.parent.mkdir(exist_ok=True)
+        exe = base / "bamgen"                            # the source tree may be read-only: build beside the data
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-pthread", "-o", str(exe), str(src), "-lz"])
     t0 = time.time()
     out = subprocess.check_output([str(exe), "--mode", mode, "--reads", str(reads), "--seed", str(seed), "--out", str(path),
@@ -64,6 +70,85 @@ def ensure_bam(reads: int, seed: int, want_bai: bool, mode: str = "short") -> tu
     meta.write_text(json.dumps(info))
     log(f"[bench] generated {path} in {info['generate_s']} s: {info}")
     return path, info
+
+
+DUMP_BYTES = 64 << 20
+DUMP_WINDOWS, DUMP_WINDOW_ROWS = 16, 1024
+
+
+def dump_windows(rows: int, seed: int = 0):
+    """Row windows [lo, hi) of one step's output to dump, in row order: DUMP_WINDOW_ROWS rows at a seeded offset inside
+    each of DUMP_WINDOWS equal strata, or the whole output when it is smaller."""
+    if rows <= DUMP_WINDOWS * DUMP_WINDOW_ROWS:
+        return [(0, rows)]
+    rng = np.random.default_rng(seed)
+    stratum = rows // DUMP_WINDOWS
+    starts = [k * stratum + int(rng.integers(0, stratum - DUMP_WINDOW_ROWS + 1)) for k in range(DUMP_WINDOWS)]
+    return [(lo, lo + DUMP_WINDOW_ROWS) for lo in starts]
+
+
+def keep_window_rows(batch, first_row: int, windows, kept: list):
+    """Appends (row index, copy of the rows) to `kept` for the rows of `batch` that fall in `windows`; `first_row` is the
+    index of the batch's first row in the step's output.  Only the copies outlive the batch."""
+    for lo, hi in windows:
+        lo, hi = max(lo, first_row), min(hi, first_row + batch.num_rows)
+        if lo < hi:
+            kept.append((lo, batch.take(pa.array(np.arange(lo - first_row, hi - first_row)))))
+
+
+def _is_bytes(t):
+    return pa.types.is_string(t) or pa.types.is_binary(t)
+
+
+def column_arrays(name, col):
+    """One Arrow column as float arrays: numbers as float64 with NaN for null; strings and binaries as their UTF-8 / raw
+    bytes (float32) plus per-row byte lengths (float64, NaN for null); lists as their flattened values plus lengths."""
+    f64 = lambda a: np.asarray(a.to_numpy(zero_copy_only=False), dtype=np.float64)
+    t = col.type
+    if _is_bytes(t):
+        data = b"".join(v.encode() if isinstance(v, str) else v for v in col.to_pylist() if v is not None)
+        return {f"{name}.bytes": np.frombuffer(data, np.uint8).astype(np.float32), f"{name}.lengths": f64(pc.binary_length(col))}
+    if pa.types.is_list(t) and not _is_bytes(t.value_type):
+        return {f"{name}.values": f64(pc.cast(pc.list_flatten(col), pa.float64())), f"{name}.lengths": f64(pc.list_value_length(col))}
+    if pa.types.is_integer(t) or pa.types.is_floating(t):
+        return {name: f64(pc.cast(col, pa.float64()))}
+    raise TypeError(f"column {name}: no float form for {t}")
+
+
+def dump_outputs(out_dir: Path, kept, windows, prefix: str, budget: int) -> dict:
+    """Writes the rows in `kept` (keep_window_rows, row order) as out_dir/<prefix><name>.npy: row_index.npy plus one file
+    per column_arrays entry.  When they would exceed `budget` bytes, every window keeps the same number of leading rows."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    if not kept:
+        np.save(out_dir / f"{prefix}row_index.npy", np.zeros(0, np.float64))
+        return {"dir": str(out_dir), "rows": 0, "bytes": 0}
+    t = pa.Table.from_batches([b for _, b in kept]).combine_chunks()
+    index = np.concatenate([np.arange(lo, lo + b.num_rows) for lo, b in kept])
+    lengths = lambda a: np.nan_to_num(np.asarray(a.to_numpy(zero_copy_only=False), dtype=np.float64))
+    cost, files = np.full(t.num_rows, 8.0), 1       # bytes each row adds to the files: row_index, then per column
+    for col in t.columns:
+        cost += 8.0                                  # the value, or the length
+        if _is_bytes(col.type):
+            cost += 4.0 * lengths(pc.binary_length(col)); files += 2
+        elif pa.types.is_list(col.type):
+            cost += 8.0 * lengths(pc.list_value_length(col)); files += 2
+        else:
+            files += 1
+    starts = np.array([lo for lo, _ in windows])
+    offset = index - starts[np.searchsorted(starts, index, side="right") - 1]          # a row's place in its window
+    cost_upto = np.cumsum(np.bincount(offset, weights=cost))
+    per_window = int(np.searchsorted(cost_upto, budget - 128 * files, side="right"))   # 128: an .npy header
+    sel = np.flatnonzero(offset < per_window)
+    t = t.take(pa.array(sel))
+    arrays = {"row_index": index[sel].astype(np.float64)}
+    for name, col in zip(t.column_names, t.columns):
+        arrays.update(column_arrays(name, col))
+    total = 0
+    for name, arr in arrays.items():
+        path = out_dir / f"{prefix}{name}.npy"
+        np.save(path, arr)
+        total += path.stat().st_size
+    return {"dir": str(out_dir), "rows": len(sel), "bytes": total}
 
 
 def bai_linear_offsets(bai_path: Path):
@@ -278,6 +363,8 @@ def main():
     ap.add_argument("--verify", action="store_true", help="(default at N = 1, config 2) compare the product path with the oracle outside the timed regions")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-replicas", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write a fixed, seeded row sample of the last timed end-to-end step's RecordBatches to DIR/<name>.npy")
     args = ap.parse_args()
     if args.config == 3:
         args.projection = "fixed"
@@ -385,23 +472,32 @@ def main():
                        "first_record_uoff": st.get("first_record_uoff", 0), "end_chain_uoff": st.get("end_chain_uoff", 0)})
 
     # ---------------- end to end through the provider API ----------------
-    def e2e_step():
+    def e2e_step(windows=None, kept=None):
         n = 0
         for p in my_parts:
             for b in plan.execute(p):
+                if windows:
+                    keep_window_rows(b, n, windows, kept)    # a batch is a whole inflate wave (GBs): copy the rows, not it
                 n += b.num_rows
                 del b
         return n
 
     for _ in range(max(1, args.warmup)):   # warm-up: the pinned arena pool settles after a few scans
-        e2e_step()
+        step_rows = e2e_step()
+    windows = dump_windows(step_rows) if args.dump_outputs else None
+    kept = []
     barrier()
     t0 = time.perf_counter()
     e2e_rows = 0
-    for _ in range(args.steps):
-        e2e_rows += e2e_step()
+    for i in range(args.steps):
+        e2e_rows += e2e_step(windows if i == args.steps - 1 else None, kept)
     barrier()
     e2e_s = all_max(time.perf_counter() - t0)
+    dumped = None
+    if args.dump_outputs:
+        prefix = f"rank{rank}." if world > 1 else ""
+        dumped = dump_outputs(args.dump_outputs, kept, windows, prefix, DUMP_BYTES // world)
+        log(f"[bench r{rank}] wrote {dumped['rows']} sampled rows of {step_rows} ({dumped['bytes']} bytes) to {args.dump_outputs}")
     est = plan.last_stats if my_parts else {"h2d_bytes": 0, "d2h_bytes": 0}
     e2e_value = all_sum(e2e_rows) / e2e_s
     h2d_all, d2h_all = all_sum(est["h2d_bytes"]), all_sum(est["d2h_bytes"])
@@ -469,6 +565,8 @@ def main():
     }
     if replicas:
         line["replicas"] = replicas
+    if dumped:
+        line["dump_outputs"] = dumped
     if world == 1 and args.config == 2:
         # CPU baseline beside it (bounded samples): the oracle port on all host threads, on one thread, and inflate alone
         from oracle.bam_oracle import OracleBam
