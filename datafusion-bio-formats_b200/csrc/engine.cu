@@ -251,19 +251,14 @@ namespace bamscan {
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 static double wall_ms() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
 
-#ifndef BAMSCAN_ICTA_NT
-#define BAMSCAN_ICTA_NT 256
-#endif
-constexpr int ICTA_NT = BAMSCAN_ICTA_NT;                      // threads of the CTA-per-member inflate kernel
-using IctaCfg = icta::Cfg<ICTA_NT>;
 static bool g_crc_init[64] = {};
 static uint32_t* g_crc_tabs[64] = {};
 static unsigned long long* g_icta_prof = nullptr;   // bamscan_bench_inflate with BAMSCAN_ICTA_PROF=1: per-phase cycle counters             // per device: tables of the in-window CRC stage (kernels_inflate_cta.cuh)
 static int init_device_constants(int dev) {
   if (dev >= 64) { set_error("device id %d out of range", dev); return BAMSCAN_ERR_CUDA; }
   if (g_crc_init[dev]) return BAMSCAN_OK;
-  CU_TRY(cudaMalloc((void**)&g_crc_tabs[dev], icta::CrcTabs<ICTA_NT>::WORDS * 4));
-  icta::crc_tables_init_kernel<ICTA_NT><<<1, 256>>>(g_crc_tabs[dev]);
+  CU_TRY(cudaMalloc((void**)&g_crc_tabs[dev], icta::CrcTabs<icta::NT_C>::WORDS * 4));
+  icta::crc_tables_init_kernel<icta::NT_C><<<1, 256>>>(g_crc_tabs[dev]);
   CU_TRY(cudaDeviceSynchronize());
   // x^(8 * 2^j) mod P in the reflected domain
   auto mulmod = [](uint32_t a, uint32_t b) { uint32_t p = 0; for (int i = 0; i < 32; i++) { if (b & 0x80000000u) p ^= a; a = (a >> 1) ^ ((a & 1u) ? 0xEDB88320u : 0u); b <<= 1; } return p; };
@@ -276,7 +271,7 @@ static int init_device_constants(int dev) {
 }
 
 // ---- inflate: three kernels, one picked per launch ----
-//   inflate_cta_kernel   one CTA per member, parallel INSIDE the member (kernels_inflate_cta.cuh): 296 members in flight, a member
+//   inflate_cta_kernel   parallel INSIDE the member, two members per CTA (kernels_inflate_cta.cuh): 592 members in flight, a member
 //                        is done in ~0.3 ms.  Members it refuses (INF_RETRY) are redone by inflate_kernel.  Picked for every
 //                        launch of up to ICTA_MAX_MEMBERS members: region queries, tail chunks, small and long-read files.
 //   inflate_lg_kernel    4 lanes per member, 152 members per SM (22 496 in flight), a member takes ~17 ms: more members per
@@ -321,7 +316,7 @@ static int launch_inflate(const BamFile* f, cudaStream_t cs, const uint8_t* d_co
   }
   {
     const uint32_t grid = std::min<uint32_t>(nb, sms * 2u);
-    icta::inflate_cta_kernel<ICTA_NT><<<grid, ICTA_NT, IctaCfg::SMEM, cs>>>(d_comp, d_blk, nb, U, d_status, d_ticket, d_err, d_aux + 1, g_crc_tabs[f->device], check_crc, g_icta_prof);
+    icta::inflate_cta_kernel<<<grid, icta::NT, icta::Cfg::SMEM, cs>>>(d_comp, d_blk, nb, U, d_status, d_ticket, d_err, d_aux + 1, g_crc_tabs[f->device], check_crc, g_icta_prof);
     *launches += 1;
     // members flagged INF_RETRY (none on ordinary files); the launch finds nothing to do otherwise
     uint32_t rgrid = std::min<uint32_t>((nb + INF_WARPS - 1) / INF_WARPS, sms);
@@ -359,8 +354,8 @@ static int stream_init(BamScanStream* s) {
   CU_TRY(cudaFuncSetAttribute(inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(InflateShared)));
   CU_TRY(cudaFuncSetAttribute(inflate_lg_kernel<LG_G, LG_W, LG_NLIT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LgCfg::SMEM));
   CU_TRY(cudaFuncSetAttribute(crc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CRC_SMEM));
-  CU_TRY(cudaFuncSetAttribute(icta::inflate_cta_kernel<ICTA_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IctaCfg::SMEM));
-  CU_TRY(cudaFuncSetAttribute(icta::inflate_cta_kernel<ICTA_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+  CU_TRY(cudaFuncSetAttribute(icta::inflate_cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)icta::Cfg::SMEM));
+  CU_TRY(cudaFuncSetAttribute(icta::inflate_cta_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
   // reference dictionary: lengths + names blob
   size_t n_ref = f->ref_names.size();
   std::vector<uint32_t> offs(n_ref + 1, 0);
@@ -1536,10 +1531,11 @@ int bamscan_bench_inflate(BamScanPlan* plan, int32_t partition, int32_t repeats,
     cudaFree(g_icta_prof); g_icta_prof = nullptr;
     unsigned long long sum[16] = {};
     for (size_t i = 0; i < prof_n; i++) sum[i % 16] += h[i];
-    static const char* names[] = {"ticket", "payload load", "block header", "tables", "count rounds", "scan+emit", "resolve", "crc", "store+status"};
+    static const char* names[] = {"ticket", "payload load", "block header", "tables", "count rounds", "scan+emit",
+                                  "resolve", "crc", "store+status", "producer waits for window", "consumer waits for member"};
     const double m = (double)std::max<unsigned long long>(1, sum[13]);
-    fprintf(stderr, "[icta prof] members %llu, count rounds/member %.2f; cycles per member:", sum[13], sum[12] / m);
-    for (int k = 0; k < 9; k++) fprintf(stderr, " %s %.0f |", names[k], sum[k] / m);
+    fprintf(stderr, "[icta prof] members %llu, count rounds/member %.2f, resolve batches/member %.2f; cycles per member:", sum[13], sum[12] / m, sum[11] / m);
+    for (int k = 0; k < 11; k++) fprintf(stderr, " %s%s %.0f |", k < 6 || k == 9 ? "P " : "C ", names[k], sum[k] / m);
     fprintf(stderr, "\n");
   }
   cudaEventDestroy(e0); cudaEventDestroy(e1);

@@ -3,18 +3,23 @@
 // Replaces: noodles-bgzf 0.49.0 io::Reader block inflate + libdeflate `deflate_decompress` / `crc32`
 // (reference call sites: datafusion/bio-format-bam/src/storage.rs:161-169, physical_exec.rs:409).
 //
-// One CTA (NT threads, two CTAs per SM) owns one BGZF member at a time (persistent grid, atomic ticket):
+// One CTA of two teams (two CTAs per SM) holds two BGZF members at a time (persistent grid, atomic ticket).
+// PRODUCER team (warps 0-7, NT_P threads), member k+1:
 //   1. the deflate payload is brought into shared memory by ONE cp.async.bulk (TMA) + mbarrier;
 //   2. per deflate block: warp 0 reads the block header, warps 0/1 build two-level Huffman LUTs in shared memory;
-//   3. the block's symbol stream is cut into NT sub-streams which all lanes decode speculatively and then re-anchor on
+//   3. the block's symbol stream is cut into NT_P sub-streams which all lanes decode speculatively and then re-anchor on
 //      their predecessor's end until nothing changes (inflate_cta_core.h explains why that converges in ~2 rounds);
-//   4. a CTA scan of the per-lane byte counts gives output offsets; the lanes decode again and EMIT literals and parked
-//      matches into the member's 64 KB OUTPUT WINDOW, which lives in shared memory;
-//   5. all warps RESOLVE the parked matches in output order, each warp over its own part of the window, ordered by
-//      per-warp frontiers (every LZ77 source read is a shared-memory read);
+//   4. a team scan of the per-lane byte counts gives output offsets; the lanes decode again and EMIT literals and parked
+//      matches into the member's 64 KB OUTPUT WINDOW, which lives in shared memory.
+// CONSUMER team (warps 8-11, NT_C threads), member k:
+//   5. RESOLVE the parked matches in output order, in batches of at most LIST_CAP matches, each warp over its own part of
+//      the window, ordered by per-piece map bits (every LZ77 source read is a shared-memory read);
 //   6. CRC-32 is computed from the window (no second pass over HBM), ISIZE is checked, and the window leaves the SM once:
 //      cp.async.bulk shared -> global for the 16-byte aligned body, byte stores for the ragged ends.
-// HBM traffic is therefore the algorithmic minimum: payload read once, inflated bytes written once.
+// Steps 1-3 never touch the window or its head bitmap and steps 5-6 never touch the payload or the LUTs, so the producer's
+// header / tables / count of member k+1 run while the consumer resolves member k.  The window (with the head bitmap) is
+// handed over by two named barriers: FULL (producer -> consumer, with a hand-off record) and EMPTY (consumer -> producer).
+// HBM traffic is the algorithmic minimum: payload read once, inflated bytes written once.
 //
 // Members this kernel cannot take (ISIZE > 65536, a Huffman code whose second-level tables exceed the shared-memory budget)
 // are flagged INF_RETRY in status[] and redone by the warp-per-member kernel of kernels_inflate.cuh.
@@ -34,14 +39,6 @@ constexpr uint32_t FRONT_DONE = 0xffffffffu;
 #define BAMSCAN_ICTA_MIN_SUB_BITS 64
 #endif
 constexpr uint32_t MIN_SUB_BITS = BAMSCAN_ICTA_MIN_SUB_BITS;      // shortest sub-stream a lane is given
-#ifndef BAMSCAN_ICTA_RESOLVE_SLOTS
-#define BAMSCAN_ICTA_RESOLVE_SLOTS 1
-#endif
-#ifndef BAMSCAN_ICTA_RESOLVE_WARPS
-#define BAMSCAN_ICTA_RESOLVE_WARPS 0          // 0: every warp of the CTA
-#endif
-constexpr int RESOLVE_SLOTS = BAMSCAN_ICTA_RESOLVE_SLOTS;   // matches per lane the resolver keeps in flight
-constexpr int RESOLVE_WARPS = BAMSCAN_ICTA_RESOLVE_WARPS;   // warps of the resolver
 #ifndef BAMSCAN_ICTA_WARMUP_BITS
 #define BAMSCAN_ICTA_WARMUP_BITS 640
 #endif
@@ -50,52 +47,75 @@ constexpr uint32_t WARMUP_BITS = BAMSCAN_ICTA_WARMUP_BITS;
 #define BAMSCAN_ICTA_WARMUP_MIN_BITS 192
 #endif
 constexpr uint32_t WARMUP_MIN_BITS = BAMSCAN_ICTA_WARMUP_MIN_BITS;
-#ifndef BAMSCAN_ICTA_NSUB
-#define BAMSCAN_ICTA_NSUB 0          // sub-streams per span; 0 = one per thread.  (A CTA of 384 threads with 256 sub-streams keeps the
-#endif                               //  decode passes as they are and gives header / tables / resolve / CRC four more warps.)   // (short sub-streams of a small block: the warm-up may span several predecessors)       // round 0 of the count pass starts this many bits in front of a lane's cut (99.9 % of false starts are on the true chain by then)
+#ifndef BAMSCAN_ICTA_PAY_KB
+#define BAMSCAN_ICTA_PAY_KB 24
+#endif
+
+// the two teams of a CTA
+constexpr int NT_P = 256, NT_C = 128, NT = NT_P + NT_C;
+constexpr int RWARPS = NT_C / 32;                                 // resolver warps = the consumer team
+// named barriers (0 is __syncthreads, used only before the teams split)
+constexpr uint32_t BAR_P = 1, BAR_C = 2, BAR_FULL = 3, BAR_EMPTY = 4;
 
 // global constant tables of the CRC stage, filled once per device by crc_tables_init_kernel:
 //   [0, 1024)     four 256-entry tables of the operator "multiply by x^(32*NT)" (strided slicing-by-4)
 //   [1024, 1024+NT] x^(32*j) mod P for j = 0..NT
 template <int NT> struct CrcTabs { static constexpr uint32_t WORDS = 1024 + NT + 1; };
 
-template <int NT>
 struct Cfg {
-  static constexpr int WARPS = NT / 32;
   static constexpr uint32_t WIN_BYTES = 65536 + 32;
-  static constexpr uint32_t PAY_BYTES = (NT <= 384 ? 29 : 27) * 1024;            // payload buffer (larger payloads are streamed through it)
-  static constexpr uint32_t PAY_SLACK = 64;
   static constexpr uint32_t HB_WORDS = 2052;                  // head bitmap: one bit per window byte
+  static constexpr uint32_t CCTL_BYTES = 256;
+  static constexpr uint32_t CTL_BYTES = 1024;
+  static constexpr uint32_t PAY_BYTES = BAMSCAN_ICTA_PAY_KB * 1024;   // payload buffer (larger payloads are streamed through it)
+  static constexpr uint32_t PAY_SLACK = 64;
   static constexpr uint32_t LUT_LL_WORDS = ROOT_LL + SUB_LL, LUT_D_WORDS = ROOT_D + SUB_D;
+  static constexpr uint32_t SMEM_MAX = 113 * 1024;            // two CTAs per SM
+  // consumer-owned while it holds the window: window, head / unresolved bitmap, consumer control block, match list
   static constexpr uint32_t OFF_WIN = 16;                     // (the resolver gathers up to 3 bytes in front of the window's first word)
   static constexpr uint32_t OFF_HB = OFF_WIN + WIN_BYTES;
-  static constexpr uint32_t OFF_PAY = OFF_HB + HB_WORDS * 4;
+  static constexpr uint32_t OFF_CCTL = OFF_HB + HB_WORDS * 4;
+  static constexpr uint32_t OFF_LIST = OFF_CCTL + CCTL_BYTES;
+  // producer-owned: payload, LUTs, lane arrays, producer control block; the match list takes what is left
+  static constexpr uint32_t PROD_BYTES = PAY_BYTES + PAY_SLACK + (LUT_LL_WORDS + LUT_D_WORDS) * 4 + 2 * NT_P * 4 + CTL_BYTES;
+  static constexpr uint32_t LIST_CAP = ((SMEM_MAX - OFF_LIST - PROD_BYTES) / 2) & ~7u;   // u16 entries, 16-byte multiple
+  static constexpr uint32_t OFF_PAY = OFF_LIST + LIST_CAP * 2;
   static constexpr uint32_t OFF_LUT_LL = OFF_PAY + PAY_BYTES + PAY_SLACK;
   static constexpr uint32_t OFF_LUT_D = OFF_LUT_LL + LUT_LL_WORDS * 4;
   static constexpr uint32_t OFF_LANE_E = OFF_LUT_D + LUT_D_WORDS * 4;
-  static constexpr uint32_t OFF_LANE_N = OFF_LANE_E + NT * 4;
-  static constexpr uint32_t OFF_CTL = OFF_LANE_N + NT * 4;
-  static constexpr uint32_t CTL_BYTES = 1024;
+  static constexpr uint32_t OFF_LANE_N = OFF_LANE_E + NT_P * 4;
+  static constexpr uint32_t OFF_CTL = OFF_LANE_N + NT_P * 4;
   static constexpr uint32_t SMEM = OFF_CTL + CTL_BYTES;
-  // the resolver's in-order list of match heads (u16 each) aliases the payload buffer and the LUTs, which are dead by then
-  static constexpr uint32_t LIST_CAP = (OFF_LANE_E - OFF_PAY) / 2;
-  static_assert(CrcTabs<NT>::WORDS * 4 <= PAY_BYTES, "CRC tables alias the payload buffer");
-  static_assert(SMEM <= 113 * 1024, "two CTAs per SM");
+  static_assert(OFF_PAY % 16 == 0, "cp.async.bulk destination");
+  static_assert(LIST_CAP >= 2048, "match list");
+  static_assert(SMEM <= SMEM_MAX, "two CTAs per SM");
 };
 
+// producer control block
 struct Ctl {
   unsigned long long mbar;
-  unsigned long long psel[8];        // psel[d]: sixteen nibbles k mod d (byte selectors of a period-d piece, resolve stage)
   uint32_t ticket, err, btype, final_block, hdr_end, stored_len, n_ll, n_d;
   uint32_t first_term[2];            // lowest lane whose chain does not hand over (double buffered per round)
   uint32_t last_lane, last_info;
-  uint32_t warp_tot[32];
-  uint32_t n_matches;
-  uint32_t crc_part[32];
+  uint32_t warp_tot[NT_P / 32];
   uint16_t cnt[2][16], first[2][16], nxt[2][16], offs[2][16];
   uint8_t cl[320];
 };
-static_assert(sizeof(Ctl) <= 1024, "Ctl fits its slot");
+static_assert(sizeof(Ctl) <= Cfg::CTL_BYTES, "Ctl fits its slot");
+
+// window hand-off record, producer -> consumer (bi == HANDOFF_END: no more members)
+constexpr uint32_t HANDOFF_END = 0xffffffffu;
+struct Handoff { uint32_t bi, obase, isize, crc, uoff; };
+
+// consumer control block
+struct CCtl {
+  unsigned long long psel[8];        // psel[d]: sixteen nibbles k mod d (byte selectors of a period-d piece, resolve stage)
+  uint32_t err;
+  uint32_t warp_tot[RWARPS];
+  uint32_t crc_part[RWARPS];
+  Handoff h;
+};
+static_assert(sizeof(CCtl) <= Cfg::CCTL_BYTES, "CCtl fits its slot");
 
 // ---- PTX helpers: mbarrier + 1-D bulk copies (TMA) ----
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -126,6 +146,18 @@ __device__ __forceinline__ void bulk_store(void* dst_gmem, const void* src_smem,
 }
 __device__ __forceinline__ void bulk_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// named barriers: a team's own barrier, and the arrive / wait halves of the window hand-off
+template <uint32_t ID, uint32_t N> __device__ __forceinline__ void bar_sync() { asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(N) : "memory"); }
+template <uint32_t ID, uint32_t N> __device__ __forceinline__ void bar_arrive() { asm volatile("bar.arrive %0, %1;" ::"n"(ID), "n"(N) : "memory"); }
+template <uint32_t ID, uint32_t N> __device__ __forceinline__ bool bar_or(bool v) {
+  uint32_t r;
+  asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.or.pred q, %2, %3, p;\n\tselp.u32 %0, 1, 0, q;\n\t}"
+               : "=r"(r) : "r"((uint32_t)v), "n"(ID), "n"(N) : "memory");
+  return r != 0u;
+}
+__device__ __forceinline__ void psync() { bar_sync<BAR_P, NT_P>(); }
+__device__ __forceinline__ void csync() { bar_sync<BAR_C, NT_C>(); }
 
 __device__ __forceinline__ void sts_u32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 __device__ __forceinline__ uint32_t lds_u16(uint32_t a) { uint32_t v; asm volatile("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
@@ -295,7 +327,7 @@ __device__ __noinline__ uint32_t read_precode_warp(SBits& br, uint32_t* plut, Ct
   return INF_OK;
 }
 
-// Part 2, whole CTA: the run-length coded code lengths.  One code-length symbol takes a warp ~300 cycles when it is decoded
+// Part 2, whole producer team (NT threads): the run-length coded code lengths.  One code-length symbol takes a warp ~300 cycles when it is decoded
 // serially (one LUT look-up per symbol on a dependent chain, sharing the issue slots with 15 other warps), and a member has
 // ~500 of them.  Here every thread decodes the symbol that WOULD start at its bit offsets (a table of 16-bit records:
 // bits consumed - 1 [3:0], kind [5:4] = 0 length / 1 repeat previous / 2 zeros / 3 invalid, value or run length [13:6]),
@@ -319,7 +351,7 @@ __device__ __forceinline__ uint32_t read_code_lengths_cta(const uint32_t* pay, u
     else rec = (L + 7u - 1u) | (2u << 4) | ((11u + ((bits >> L) & 127u)) << 6);
     tab[q] = (uint16_t)rec;
   }
-  __syncthreads();
+  bar_sync<BAR_P, NT>();
   if (tid < 32) {
     // Follow the chain of real symbols through the table: warp 0, 32 segments of 64 bit positions at a time.  Every lane walks
     // its segment from the segment's first position (lane 0: from the true entry) and keeps the visited positions as a 64-bit
@@ -389,7 +421,7 @@ __device__ __forceinline__ uint32_t read_code_lengths_cta(const uint32_t* pay, u
     }
     if (lane == 0) { C->last_lane = k_base; C->last_info = q_end; }
   }
-  __syncthreads();
+  bar_sync<BAR_P, NT>();
   const uint32_t k = C->last_lane;
   for (uint32_t j = tid; j < k; j += NT) {
     const uint32_t c = chain[j];
@@ -403,7 +435,7 @@ __device__ __forceinline__ uint32_t read_code_lengths_cta(const uint32_t* pay, u
     }
     for (uint32_t r = 0; r < rep; r++) C->cl[i0 + r] = (uint8_t)val;
   }
-  __syncthreads();
+  bar_sync<BAR_P, NT>();
   if (C->err) return C->err;
   *end_pos = start_pos + C->last_info;
   if (C->cl[256] == 0) return INF_ERR_TABLE;
@@ -411,8 +443,8 @@ __device__ __forceinline__ uint32_t read_code_lengths_cta(const uint32_t* pay, u
 }
 
 
-// RESOLVE stage C: dataflow over the in-order match list.  RESOLVE_WARPS warps x 32 lanes x SLOTS matches are in flight,
-// dealt statically (thread t, slot m takes the matches t + T m, + T SLOTS, ... with T = 32 RESOLVE_WARPS: the lowest
+// RESOLVE stage C: dataflow over the in-order match list.  RWARPS warps x 32 lanes x SLOTS matches are in flight,
+// dealt statically (thread t, slot m takes the matches t + T m, + T SLOTS, ... with T = 32 RWARPS: the lowest
 // unresolved match of the member is therefore always in flight and its sources are final, so the stage always makes
 // progress).  The LZ77 dependency chains of sorted BAM data are 90-190 pieces deep per member (a record copies from the
 // record in front of it): this stage is a latency chain, not a bandwidth problem, and what counts is the length of one
@@ -425,7 +457,7 @@ __device__ __forceinline__ uint32_t read_code_lengths_cta(const uint32_t* pay, u
 __device__ __forceinline__ void sts_u32_if(uint32_t a, uint32_t v, bool on) { asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %2, 0;\n\t@p st.shared.u32 [%0], %1;\n\t}" ::"r"(a), "r"(v), "r"((uint32_t)on) : "memory"); }
 __device__ __forceinline__ void sts_u8_if(uint32_t a, uint32_t v, bool on) { asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %2, 0;\n\t@p st.shared.u8 [%0], %1;\n\t}" ::"r"(a), "r"(v), "r"((uint32_t)on) : "memory"); }
 template <int SLOTS, int RWARPS>
-__device__ __forceinline__ void resolve_dataflow(uint32_t win_s, uint32_t hb_s, uint32_t list_s, uint32_t psel_s, uint32_t obase, uint32_t total, int tid, Ctl* C) {
+__device__ __forceinline__ void resolve_dataflow(uint32_t win_s, uint32_t hb_s, uint32_t list_s, uint32_t psel_s, uint32_t obase, uint32_t total, int tid, uint32_t* err) {
   constexpr uint32_t T = 32u * RWARPS;
   uint32_t o[SLOTS], dist[SLOTS], len[SLOTS], done[SLOTS], no[SLOTS], nv[SLOTS], nr[SLOTS];
   bool pend[SLOTS];
@@ -481,7 +513,7 @@ __device__ __forceinline__ void resolve_dataflow(uint32_t win_s, uint32_t hb_s, 
       anyn |= n[m] != 0u; anywrap |= n[m] > dist[m];
     }
     if (!__any_sync(FULL, anyn)) {                                                 // nothing ready in this warp: another warp's piece comes first
-      if (RWARPS == 1 || ++spins > (1u << 22)) { C->err = INF_ERR_INPUT; break; }  // (one warp: cannot happen; else a safety valve, never taken)
+      if (RWARPS == 1 || ++spins > (1u << 22)) { *err = INF_ERR_INPUT; break; }  // (one warp: cannot happen; else a safety valve, never taken)
       continue;
     }
     if (__any_sync(FULL, anywrap)) {                                               // a piece longer than its period: byte k is src[k mod dist]
@@ -532,59 +564,66 @@ __device__ __forceinline__ void resolve_dataflow(uint32_t win_s, uint32_t hb_s, 
   }
 }
 
-// RESOLVE, whole member, all warps.  `hb` holds one bit per parked match head on entry.
-//   A  every thread ranks the heads of its share of the bitmap words; a CTA scan turns that into an in-order list of
-//      head positions (u16, relative to obase); the bitmap words are zeroed on the way;
-//   B  the bitmap becomes the UNRESOLVED map: every byte of every parked match is flagged;
-//   C  dataflow, warp 0: 32 consecutive matches in flight, one per lane.  A lane copies a piece (<= 16 bytes) of its match
-//      as soon as the map shows that the piece's source bytes are final, then clears the piece's bits.  The lowest
-//      unresolved piece of the member always has final sources, so every iteration makes progress.
-// Returns INF_OK or INF_RETRY (more matches than the list holds).
-template <int NT>
-__device__ __forceinline__ uint32_t resolve_member(uint8_t* win, uint32_t* hb, uint16_t* list, uint32_t list_cap, Ctl* C,
+// RESOLVE, whole member, consumer team (NTC threads).  `hb` holds one bit per parked match head on entry and is all zero
+// on return.  The matches are taken in output-ordered batches of at most `list_cap`; this is exact, because a match's
+// source bytes lie in front of its own bytes and hence in front of every later match.  Per batch:
+//   A  every thread ranks the heads of its share of the bitmap words; a team scan turns the first list_cap of them into an
+//      in-order list of head positions (u16, relative to obase) and clears their bits (later heads stay for the next batch);
+//   B  the bitmap becomes the UNRESOLVED map of the batch: every byte of every listed match is flagged;
+//   C  dataflow (resolve_dataflow above): a lane copies a piece (<= 16 bytes) of its match as soon as the map shows that the
+//      piece's source bytes are final, then clears the piece's bits.  The lowest unresolved piece of the batch always has
+//      final sources (earlier batches are done), so every iteration makes progress.
+// Returns the number of batches.
+template <int NTC>
+__device__ __forceinline__ uint32_t resolve_member(uint8_t* win, uint32_t* hb, uint16_t* list, uint32_t list_cap, CCtl* CC,
                                                    uint32_t obase, uint32_t olimit, int tid) {
-  constexpr int WARPS = NT / 32;
+  constexpr int WARPS = NTC / 32;
   const int lane = tid & 31, warp = tid >> 5;
-  const uint32_t wbeg = obase >> 5, wend = (olimit + 31u) >> 5;
-  const uint32_t WPT = (wend - wbeg + NT - 1) / NT;                 // bitmap words per thread (<= 9)
-  // ---- A: rank + list
-  const uint32_t w0 = wbeg + (uint32_t)tid * WPT, w1 = min(wend, w0 + WPT);
-  uint32_t cnt = 0;
-  for (uint32_t w = w0; w < w1; w++) cnt += __popc(hb[w]);
-  uint32_t incl = cnt;
-  #pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
-  if (lane == 31) C->warp_tot[warp] = incl;
-  __syncthreads();
-  uint32_t base = 0, total = 0;
-  #pragma unroll
-  for (int w = 0; w < WARPS; w++) { const uint32_t t = C->warp_tot[w]; if (w < warp) base += t; total += t; }
-  if (total > list_cap) return INF_RETRY;                           // (uniform; the caller wipes the bitmap)
-  {
-    uint32_t k = base + incl - cnt;
-    for (uint32_t w = w0; w < w1; w++) {
-      uint32_t bits = hb[w];
-      hb[w] = 0;
-      while (bits) { list[k++] = (uint16_t)(w * 32u + (uint32_t)__ffs((int)bits) - 1u - obase); bits &= bits - 1u; }
+  const uint32_t wend = (olimit + 31u) >> 5;
+  uint32_t wbeg = obase >> 5;
+  for (uint32_t batch = 1;; batch++) {
+    const uint32_t WPT = (wend - wbeg + NTC - 1) / NTC;             // bitmap words per thread (<= 17)
+    // ---- A: rank + list
+    const uint32_t w0 = wbeg + (uint32_t)tid * WPT, w1 = min(wend, w0 + WPT);
+    uint32_t cnt = 0;
+    for (uint32_t w = w0; w < w1; w++) cnt += __popc(hb[w]);
+    uint32_t incl = cnt;
+    #pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
+    if (lane == 31) CC->warp_tot[warp] = incl;
+    bar_sync<BAR_C, NTC>();
+    uint32_t base = 0, total = 0;
+    #pragma unroll
+    for (int w = 0; w < WARPS; w++) { const uint32_t t = CC->warp_tot[w]; if (w < warp) base += t; total += t; }
+    const uint32_t n = min(total, list_cap);
+    {
+      uint32_t k = base + incl - cnt;
+      for (uint32_t w = w0; w < w1 && k < n; w++) {
+        uint32_t bits = hb[w];
+        while (bits && k < n) { list[k++] = (uint16_t)(w * 32u + (uint32_t)__ffs((int)bits) - 1u - obase); bits &= bits - 1u; }
+        hb[w] = bits;
+      }
     }
-  }
-  __syncthreads();
-  // ---- B: unresolved map
-  for (uint32_t r = tid; r < total; r += NT) {
-    const uint32_t o = obase + list[r];
-    const uint32_t len = ((((uint32_t)win[o + 1] << 8) | ((uint32_t)win[o + 2] << 16)) >> 15) + 3u;
-    uint32_t w = o >> 5, b = o & 31u, rem = len;
-    while (rem) {
-      const uint32_t n = min(rem, 32u - b);
-      atomicOr(hb + w, (n == 32u ? 0xffffffffu : ((1u << n) - 1u)) << b);
-      rem -= n; w++; b = 0;
+    bar_sync<BAR_C, NTC>();
+    // ---- B: unresolved map
+    for (uint32_t r = tid; r < n; r += NTC) {
+      const uint32_t o = obase + list[r];
+      const uint32_t len = ((((uint32_t)win[o + 1] << 8) | ((uint32_t)win[o + 2] << 16)) >> 15) + 3u;
+      uint32_t w = o >> 5, b = o & 31u, rem = len;
+      while (rem) {
+        const uint32_t m = min(rem, 32u - b);
+        atomicOr(hb + w, (m == 32u ? 0xffffffffu : ((1u << m) - 1u)) << b);
+        rem -= m; w++; b = 0;
+      }
     }
+    bar_sync<BAR_C, NTC>();
+    // ---- C: dataflow
+    resolve_dataflow<1, WARPS>(smem_u32(win), smem_u32(hb), smem_u32(list), smem_u32(CC->psel), obase, n, tid, &CC->err);
+    if (total <= list_cap) return batch;                             // (uniform)
+    bar_sync<BAR_C, NTC>();                                          // the list and the map are free again
+    if (CC->err) return batch;
+    wbeg = (obase + list[n - 1u]) >> 5;                              // the next batch's first head lies in this word or behind it
   }
-  __syncthreads();
-  // ---- C: dataflow (resolve_dataflow above)
-  constexpr int RW = RESOLVE_WARPS ? RESOLVE_WARPS : WARPS;
-  if (warp < RW) resolve_dataflow<RESOLVE_SLOTS, RW>(smem_u32(win), smem_u32(hb), smem_u32(list), smem_u32(C->psel), obase, total, tid, C);
-  return INF_OK;
 }
 
 // CRC tables of the strided CRC (see Cfg / the CRC stage below); one launch per device at init.
@@ -622,23 +661,23 @@ __device__ __forceinline__ uint32_t crc_byte_bitwise(uint32_t st, uint32_t b) {
 }
 
 // =============================================================================================
-template <int NT>
 __global__ void __launch_bounds__(NT, 2)
 inflate_cta_kernel(const uint8_t* __restrict__ comp, const BlockDesc* __restrict__ blocks, uint32_t n_blocks,
                    uint8_t* __restrict__ infl, uint32_t* __restrict__ status, uint32_t* __restrict__ ticket,
                    uint32_t* __restrict__ err_flag, uint32_t* __restrict__ retry_count, const uint32_t* __restrict__ crc_tabs, int check_crc,
                    unsigned long long* __restrict__ prof) {
-  // prof (optional, profiling builds of the bench only): per-phase clock64() sums of thread 0, 16 slots per CTA
-  using K = Cfg<NT>;
-  constexpr int WARPS = K::WARPS;
+  // prof (optional, profiling builds of the bench only): per-phase clock64() sums of producer thread 0 and consumer thread
+  // NT_P, 16 slots per CTA: 0-5 producer phases, 6-8 consumer phases, 9 producer waits for the window, 10 consumer waits for
+  // a member, 11 resolve batches, 12 count rounds, 13 members
+  using K = Cfg;
   extern __shared__ __align__(128) unsigned char smem[];
   uint8_t* const win = smem + K::OFF_WIN;
-  uint32_t* const pay = reinterpret_cast<uint32_t*>(smem + K::OFF_PAY);
   uint32_t* const hb = reinterpret_cast<uint32_t*>(smem + K::OFF_HB);
+  CCtl* const CC = reinterpret_cast<CCtl*>(smem + K::OFF_CCTL);
+  uint32_t* const pay = reinterpret_cast<uint32_t*>(smem + K::OFF_PAY);
   uint32_t* const lut_ll = reinterpret_cast<uint32_t*>(smem + K::OFF_LUT_LL);
   uint32_t* const lut_d = reinterpret_cast<uint32_t*>(smem + K::OFF_LUT_D);
   uint32_t* const laneE = reinterpret_cast<uint32_t*>(smem + K::OFF_LANE_E);
-  uint32_t* const laneN = reinterpret_cast<uint32_t*>(smem + K::OFF_LANE_N);
   Ctl* const C = reinterpret_cast<Ctl*>(smem + K::OFF_CTL);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t win_s = smem_u32(win), pay_s = smem_u32(pay), hb_s = smem_u32(hb), ll_s = smem_u32(lut_ll), d_s = smem_u32(lut_d);
@@ -648,307 +687,337 @@ inflate_cta_kernel(const uint8_t* __restrict__ comp, const BlockDesc* __restrict
   if (tid < 8) {
     unsigned long long m = 0;
     for (uint32_t k = 0; k < 16; k++) m |= (unsigned long long)(tid ? k % (uint32_t)tid : 0u) << (4u * k);
-    C->psel[tid] = m;
+    CC->psel[tid] = m;
   }
-  __syncthreads();
-  uint32_t bar_parity = 0;
-  bool store_pending = false;
+  if (tid == 0) CC->err = INF_OK;
+  __syncthreads();                                                   // (the last CTA-wide barrier: from here on each team has its own)
   long long t_prev = prof ? clock64() : 0;
-#define ICTA_PROF(slot) do { if (prof && tid == 0) { const long long t_now = clock64(); prof[blockIdx.x * 16 + (slot)] += (unsigned long long)(t_now - t_prev); t_prev = t_now; } } while (0)
+#define ICTA_PROF(slot) do { if (prof && (tid == 0 || tid == NT_P)) { const long long t_now = clock64(); prof[blockIdx.x * 16 + (slot)] += (unsigned long long)(t_now - t_prev); t_prev = t_now; } } while (0)
 
-  for (;;) {
-    if (tid == 0) { C->ticket = atomicAdd(ticket, 1u); C->err = INF_OK; }
-    __syncthreads();
-    const uint32_t bi = C->ticket;
-    if (bi >= n_blocks) break;
-    const BlockDesc bd = blocks[bi];
-    const uint8_t* const gpay = comp + bd.cdata_off;
-    const uint32_t isize = bd.isize, clen = bd.cdata_len;
-    const uint32_t obase = bd.uoff & 15u, olimit = obase + isize;
-    uint32_t err = INF_OK;
-    if (isize > 65536u) err = INF_RETRY;
-
-    // ---- payload window: buffer byte 0 <-> payload byte buf_lo (negative: bytes in front of the payload, for 16-byte alignment)
-    int32_t buf_lo = 0; uint32_t loaded = 0;
-    auto load_payload = [&](uint32_t from_byte) {
-      const uintptr_t a = reinterpret_cast<uintptr_t>(gpay + from_byte);
-      const uint32_t ph = (uint32_t)(a & 15u);
-      buf_lo = (int32_t)from_byte - (int32_t)ph;
-      const uint32_t want = (clen - from_byte) + ph + 32u;                  // + slack: the reader looks up to 18 bytes ahead
-      loaded = min((want + 15u) & ~15u, K::PAY_BYTES);
-      __syncthreads();                                                     // everyone is done with the old contents
-      if (tid == 0) {
-        fence_proxy_async();
-        mbar_expect_tx(&C->mbar, loaded);
-        bulk_load(pay, reinterpret_cast<const void*>(a - ph), loaded, &C->mbar);
-      }
-      if (!mbar_wait(&C->mbar, bar_parity)) C->err = INF_ERR_INPUT;
-      bar_parity ^= 1u;
-      __syncthreads();
-      if (C->err) err = C->err;
+  if (warp < NT_P / 32) {
+    // ================= PRODUCER: ticket, payload, headers, tables, count, emit =================
+    uint32_t bar_parity = 0;
+    bool have_win = false;                                           // (uniform over the team)
+    auto acquire_window = [&]() {                                    // before the first window write of a member
+      if (have_win) return;
+      bar_sync<BAR_EMPTY, NT>();
+      have_win = true;
+      ICTA_PROF(9);
     };
-    uint32_t abs_bit = 0;                                                  // position in the payload, in bits
-    const uint32_t end_bit = clen * 8u;
-    ICTA_PROF(0);
-    if (!err) load_payload(0);
-    ICTA_PROF(1);
-    if (store_pending) {                                                   // the previous member's bulk store must have read the window
-      if (tid == 0) bulk_store_wait_read();
-      store_pending = false;
-      __syncthreads();
-    }
-    auto buf_bit = [&](uint32_t abit) { return abit - (uint32_t)(buf_lo * 8); };   // payload bit -> buffer bit (two's complement handles buf_lo < 0)
-    auto has_tail = [&]() { return (int64_t)buf_lo + (int64_t)loaded >= (int64_t)clen + 32; };   // the buffer reaches the end of the payload
-    auto covers = [&](uint32_t abit_end) {                                  // is [.., abit_end) inside the buffer (with look-ahead margin)?
-      return has_tail() ? abit_end <= end_bit : (int64_t)abit_end <= ((int64_t)buf_lo + (int64_t)loaded - 32) * 8;
-    };
+    for (;;) {
+      if (tid == 0) { C->ticket = atomicAdd(ticket, 1u); C->err = INF_OK; }
+      psync();
+      const uint32_t bi = C->ticket;
+      if (bi >= n_blocks) break;
+      const BlockDesc bd = blocks[bi];
+      const uint8_t* const gpay = comp + bd.cdata_off;
+      const uint32_t isize = bd.isize, clen = bd.cdata_len;
+      const uint32_t obase = bd.uoff & 15u, olimit = obase + isize;
+      uint32_t err = INF_OK;
+      if (isize > 65536u) err = INF_RETRY;
 
-    uint32_t outpos = obase;
-    bool final_block = false;
-    while (!final_block && !err) {
-      // ---- block header (warp 0) ----
-      if (abs_bit + 3u > end_bit) { err = INF_ERR_INPUT; break; }
-      if (!covers(min(end_bit, abs_bit + 8u * 1024u))) { load_payload(abs_bit >> 3); if (err) break; }
-      if (warp == 0) {
-        SBits br; br.w = pay; br.pos = buf_bit(abs_bit);
-        const uint32_t hdr = br.take(3);
-        uint32_t e = INF_OK, btype = hdr >> 1, slen = 0;
-        if (btype == 3) e = INF_ERR_BTYPE;
-        else if (btype == 0) {
-          br.pos = (br.pos + 7u) & ~7u;
-          const uint32_t len = br.take(16), nlen = br.take(16);
-          slen = len;
-          if ((len ^ nlen) != 0xffffu) e = INF_ERR_STORED;
-        } else if (btype == 1) {
-          for (int i = lane; i < 288; i += 32) C->cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8;
-          if (lane < 30) C->cl[288 + lane] = 5;
-          if (lane == 0) { C->n_ll = 288; C->n_d = 30; }
-        } else {
-          e = read_precode_warp(br, lut_d + ROOT_D, C, lane);
+      // ---- payload window: buffer byte 0 <-> payload byte buf_lo (negative: bytes in front of the payload, for 16-byte alignment)
+      int32_t buf_lo = 0; uint32_t loaded = 0;
+      auto load_payload = [&](uint32_t from_byte) {
+        const uintptr_t a = reinterpret_cast<uintptr_t>(gpay + from_byte);
+        const uint32_t ph = (uint32_t)(a & 15u);
+        buf_lo = (int32_t)from_byte - (int32_t)ph;
+        const uint32_t want = (clen - from_byte) + ph + 32u;                  // + slack: the reader looks up to 18 bytes ahead
+        loaded = min((want + 15u) & ~15u, K::PAY_BYTES);
+        psync();                                                             // everyone is done with the old contents
+        if (tid == 0) {
+          fence_proxy_async();
+          mbar_expect_tx(&C->mbar, loaded);
+          bulk_load(pay, reinterpret_cast<const void*>(a - ph), loaded, &C->mbar);
         }
-        if (lane == 0) { C->btype = btype; C->final_block = hdr & 1u; C->hdr_end = br.pos + (uint32_t)(buf_lo * 8); C->stored_len = slen; if (e) C->err = e; }
-      }
-      __syncthreads();
-      if (C->btype == 2u && !C->err) {
-        // code lengths, whole CTA; the symbol table aliases the (not yet built) LUTs, the chain records the lane arrays
-        uint32_t endp = 0;
-        const uint32_t e = read_code_lengths_cta<NT>(pay, buf_bit(C->hdr_end), buf_bit(end_bit), lut_d + ROOT_D, reinterpret_cast<uint16_t*>(lut_ll),
-                                                     (K::LUT_LL_WORDS + ROOT_D) * 2u, laneE, C, tid, &endp);
-        if (tid == 0) { if (e) C->err = e; else C->hdr_end = endp + (uint32_t)(buf_lo * 8); }
-      }
-      __syncthreads();
-      ICTA_PROF(2);
-      err = C->err;
-      if (err) break;
-      final_block = C->final_block != 0;
-      abs_bit = C->hdr_end;
-      const uint32_t btype = C->btype;
-      if (btype == 0) {
-        const uint32_t len = C->stored_len, from = abs_bit >> 3;
-        if (from + len > clen || outpos + len > olimit) { err = INF_ERR_STORED; break; }
-        for (uint32_t i = tid; i < len; i += NT) win[outpos + i] = __ldg(gpay + from + i);     // straight from global: any length
-        outpos += len; abs_bit += 8u * len;
-        __syncthreads();
-        continue;
-      }
-      // ---- tables: prepared by warps 0 (litlen) and 1 (distance), root LUTs filled by everyone, second levels by warps 0 / 1 ----
-      {
-        const int n_ll = (int)C->n_ll, n_d = (int)C->n_d;
-        // scratch in the lane arrays (free until the count pass): symbols sorted by (length, symbol) and every symbol's code
-        uint16_t* const sorted_ll = reinterpret_cast<uint16_t*>(laneE), *const codes_ll = sorted_ll + 288, *const sorted_d = codes_ll + 288, *const codes_d = sorted_d + 32;
-        uint32_t e = INF_OK;
-        if (warp == 0) e = lut_prepare_warp<R_LL>(C->cl, n_ll, C, 0, sorted_ll, codes_ll, lane);
-        else if (warp == 1) e = lut_prepare_warp<R_D>(C->cl + n_ll, n_d, C, 1, sorted_d, codes_d, lane);
-        if (e && lane == 0) atomicMax(&C->err, e);
-        __syncthreads();
-        if (!C->err) {
-          lut_fill_root<R_LL, false, NT>(lut_ll, SUB_LL, C, 0, sorted_ll, tid);
-          lut_fill_root<R_D, true, NT>(lut_d, SUB_D, C, 1, sorted_d, tid);
+        if (!mbar_wait(&C->mbar, bar_parity)) C->err = INF_ERR_INPUT;
+        bar_parity ^= 1u;
+        psync();
+        if (C->err) err = C->err;
+      };
+      uint32_t abs_bit = 0;                                                  // position in the payload, in bits
+      const uint32_t end_bit = clen * 8u;
+      ICTA_PROF(0);
+      if (!err) load_payload(0);
+      ICTA_PROF(1);
+      auto buf_bit = [&](uint32_t abit) { return abit - (uint32_t)(buf_lo * 8); };   // payload bit -> buffer bit (two's complement handles buf_lo < 0)
+      auto has_tail = [&]() { return (int64_t)buf_lo + (int64_t)loaded >= (int64_t)clen + 32; };   // the buffer reaches the end of the payload
+      auto covers = [&](uint32_t abit_end) {                                  // is [.., abit_end) inside the buffer (with look-ahead margin)?
+        return has_tail() ? abit_end <= end_bit : (int64_t)abit_end <= ((int64_t)buf_lo + (int64_t)loaded - 32) * 8;
+      };
+
+      uint32_t outpos = obase;
+      bool final_block = false;
+      while (!final_block && !err) {
+        // ---- block header (warp 0) ----
+        if (abs_bit + 3u > end_bit) { err = INF_ERR_INPUT; break; }
+        if (!covers(min(end_bit, abs_bit + 8u * 1024u))) { load_payload(abs_bit >> 3); if (err) break; }
+        if (warp == 0) {
+          SBits br; br.w = pay; br.pos = buf_bit(abs_bit);
+          const uint32_t hdr = br.take(3);
+          uint32_t e = INF_OK, btype = hdr >> 1, slen = 0;
+          if (btype == 3) e = INF_ERR_BTYPE;
+          else if (btype == 0) {
+            br.pos = (br.pos + 7u) & ~7u;
+            const uint32_t len = br.take(16), nlen = br.take(16);
+            slen = len;
+            if ((len ^ nlen) != 0xffffu) e = INF_ERR_STORED;
+          } else if (btype == 1) {
+            for (int i = lane; i < 288; i += 32) C->cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8;
+            if (lane < 30) C->cl[288 + lane] = 5;
+            if (lane == 0) { C->n_ll = 288; C->n_d = 30; }
+          } else {
+            e = read_precode_warp(br, lut_d + ROOT_D, C, lane);
+          }
+          if (lane == 0) { C->btype = btype; C->final_block = hdr & 1u; C->hdr_end = br.pos + (uint32_t)(buf_lo * 8); C->stored_len = slen; if (e) C->err = e; }
         }
-        __syncthreads();
-        if (!C->err) {
-          e = INF_OK;
-          if (warp == 0) e = lut_sub_warp<R_LL, false>(C->cl, n_ll, lut_ll, SUB_LL, C, 0, codes_ll, lane);
-          else if (warp == 1) e = lut_sub_warp<R_D, true>(C->cl + n_ll, n_d, lut_d, SUB_D, C, 1, codes_d, lane);
-          if (e && lane == 0) atomicMax(&C->err, e);        // INF_RETRY (15) wins over a format error of the other table
+        psync();
+        if (C->btype == 2u && !C->err) {
+          // code lengths, whole team; the symbol table aliases the (not yet built) LUTs, the chain records the lane arrays
+          uint32_t endp = 0;
+          const uint32_t e = read_code_lengths_cta<NT_P>(pay, buf_bit(C->hdr_end), buf_bit(end_bit), lut_d + ROOT_D, reinterpret_cast<uint16_t*>(lut_ll),
+                                                         (K::LUT_LL_WORDS + ROOT_D) * 2u, laneE, C, tid, &endp);
+          if (tid == 0) { if (e) C->err = e; else C->hdr_end = endp + (uint32_t)(buf_lo * 8); }
         }
-        __syncthreads();
-        ICTA_PROF(3);
+        psync();
+        ICTA_PROF(2);
         err = C->err;
         if (err) break;
-      }
-      // ---- spans of the symbol stream ----
-      bool block_done = false;
-      while (!block_done && !err) {
-        if (abs_bit >= end_bit) { err = INF_ERR_INPUT; break; }
-        if (!has_tail() && !covers(abs_bit + (K::PAY_BYTES / 2u) * 8u)) { load_payload(abs_bit >> 3); if (err) break; }
-        const uint32_t span_beg = buf_bit(abs_bit);
-        const bool to_end = has_tail();
-        const uint32_t span_end = to_end ? buf_bit(end_bit) : (uint32_t)(((int64_t)loaded - 32) * 8);
-        constexpr uint32_t NSUB = BAMSCAN_ICTA_NSUB ? BAMSCAN_ICTA_NSUB : NT;
-        static_assert(NSUB <= NT && NSUB % 32 == 0, "sub-streams are lanes");
-        uint32_t S = (span_end - span_beg + NSUB - 1) / NSUB;
-        if (S < MIN_SUB_BITS) S = MIN_SUB_BITS;
-        const uint32_t my_p = span_beg + (uint32_t)tid * S;
-        const bool active = (uint32_t)tid < NSUB && my_p < span_end;
-        const uint32_t my_stop = min(my_p + S, span_end);
-        // round 0 starts every lane but the first `ov` bits EARLY and only warms the chain up until the lane's own cut is
-        // reached: by then it is almost always the true chain (self-synchronisation), so most spans need no second round
-        const uint32_t ov = min(WARMUP_BITS, max(S, WARMUP_MIN_BITS));
-        uint32_t my_s = (tid == 0 || my_p - span_beg <= ov) ? span_beg : my_p - ov;
-        bool need = active;
-        uint32_t my_e = 0, my_t = T_CROSS, my_n = 0, F = 0;
-        for (int round = 0;; round++) {
-          if (__any_sync(FULL, need)) {                       // (all lanes of a warp enter together: see decode_sub)
-            const uint32_t from = round == 0 ? (tid == 0 ? span_beg : my_p) : my_s;
-            const SubResult r = decode_sub<false>(need, pay_s, ll_s, d_s, my_s, from, my_stop, 0, 0, 0, 0, 0, nullptr);
-            if (need) {
-              my_e = r.end_bit; my_t = r.term; my_n = r.n_out;
-              if (round == 0) {
-                my_s = r.first_bit;                           // 0xffffffff (chain ended inside the warm-up) never equals a predecessor's end
-                if (r.first_bit == 0xffffffffu) { my_e = my_p; my_t = T_CROSS; my_n = 0; }
+        final_block = C->final_block != 0;
+        abs_bit = C->hdr_end;
+        const uint32_t btype = C->btype;
+        if (btype == 0) {
+          const uint32_t len = C->stored_len, from = abs_bit >> 3;
+          if (from + len > clen || outpos + len > olimit) { err = INF_ERR_STORED; break; }
+          acquire_window();
+          for (uint32_t i = tid; i < len; i += NT_P) win[outpos + i] = __ldg(gpay + from + i);     // straight from global: any length
+          outpos += len; abs_bit += 8u * len;
+          psync();
+          continue;
+        }
+        // ---- tables: prepared by warps 0 (litlen) and 1 (distance), root LUTs filled by everyone, second levels by warps 0 / 1 ----
+        {
+          const int n_ll = (int)C->n_ll, n_d = (int)C->n_d;
+          // scratch in the lane arrays (free until the count pass): symbols sorted by (length, symbol) and every symbol's code
+          uint16_t* const sorted_ll = reinterpret_cast<uint16_t*>(laneE), *const codes_ll = sorted_ll + 288, *const sorted_d = codes_ll + 288, *const codes_d = sorted_d + 32;
+          uint32_t e = INF_OK;
+          if (warp == 0) e = lut_prepare_warp<R_LL>(C->cl, n_ll, C, 0, sorted_ll, codes_ll, lane);
+          else if (warp == 1) e = lut_prepare_warp<R_D>(C->cl + n_ll, n_d, C, 1, sorted_d, codes_d, lane);
+          if (e && lane == 0) atomicMax(&C->err, e);
+          psync();
+          if (!C->err) {
+            lut_fill_root<R_LL, false, NT_P>(lut_ll, SUB_LL, C, 0, sorted_ll, tid);
+            lut_fill_root<R_D, true, NT_P>(lut_d, SUB_D, C, 1, sorted_d, tid);
+          }
+          psync();
+          if (!C->err) {
+            e = INF_OK;
+            if (warp == 0) e = lut_sub_warp<R_LL, false>(C->cl, n_ll, lut_ll, SUB_LL, C, 0, codes_ll, lane);
+            else if (warp == 1) e = lut_sub_warp<R_D, true>(C->cl + n_ll, n_d, lut_d, SUB_D, C, 1, codes_d, lane);
+            if (e && lane == 0) atomicMax(&C->err, e);        // INF_RETRY (15) wins over a format error of the other table
+          }
+          psync();
+          ICTA_PROF(3);
+          err = C->err;
+          if (err) break;
+        }
+        // ---- spans of the symbol stream ----
+        bool block_done = false;
+        while (!block_done && !err) {
+          if (abs_bit >= end_bit) { err = INF_ERR_INPUT; break; }
+          if (!has_tail() && !covers(abs_bit + (K::PAY_BYTES / 2u) * 8u)) { load_payload(abs_bit >> 3); if (err) break; }
+          const uint32_t span_beg = buf_bit(abs_bit);
+          const bool to_end = has_tail();
+          const uint32_t span_end = to_end ? buf_bit(end_bit) : (uint32_t)(((int64_t)loaded - 32) * 8);
+          uint32_t S = (span_end - span_beg + NT_P - 1) / NT_P;
+          if (S < MIN_SUB_BITS) S = MIN_SUB_BITS;
+          const uint32_t my_p = span_beg + (uint32_t)tid * S;
+          const bool active = my_p < span_end;
+          const uint32_t my_stop = min(my_p + S, span_end);
+          // round 0 starts every lane but the first `ov` bits EARLY and only warms the chain up until the lane's own cut is
+          // reached: by then it is almost always the true chain (self-synchronisation), so most spans need no second round
+          const uint32_t ov = min(WARMUP_BITS, max(S, WARMUP_MIN_BITS));
+          uint32_t my_s = (tid == 0 || my_p - span_beg <= ov) ? span_beg : my_p - ov;
+          bool need = active;
+          uint32_t my_e = 0, my_t = T_CROSS, my_n = 0, F = 0;
+          for (int round = 0;; round++) {
+            if (__any_sync(FULL, need)) {                       // (all lanes of a warp enter together: see decode_sub)
+              const uint32_t from = round == 0 ? (tid == 0 ? span_beg : my_p) : my_s;
+              const SubResult r = decode_sub<false>(need, pay_s, ll_s, d_s, my_s, from, my_stop, 0, 0, 0, 0, 0, nullptr);
+              if (need) {
+                my_e = r.end_bit; my_t = r.term; my_n = r.n_out;
+                if (round == 0) {
+                  my_s = r.first_bit;                           // 0xffffffff (chain ended inside the warm-up) never equals a predecessor's end
+                  if (r.first_bit == 0xffffffffu) { my_e = my_p; my_t = T_CROSS; my_n = 0; }
+                }
+                laneE[tid] = my_e;
               }
-              laneE[tid] = my_e;
             }
-          }
-          if (tid == 0) C->first_term[round & 1] = NSUB - 1;
-          __syncthreads();
-          {
-            const uint32_t m = __ballot_sync(FULL, !active || my_t != T_CROSS);
-            if (m && lane == 0) {
-              const int l = __ffs((int)m) - 1;
-              atomicMin(&C->first_term[round & 1], (uint32_t)(warp * 32 + l));
+            if (tid == 0) C->first_term[round & 1] = NT_P - 1;
+            psync();
+            {
+              const uint32_t m = __ballot_sync(FULL, !active || my_t != T_CROSS);
+              if (m && lane == 0) {
+                const int l = __ffs((int)m) - 1;
+                atomicMin(&C->first_term[round & 1], (uint32_t)(warp * 32 + l));
+              }
             }
+            psync();
+            // the lane found above is either inactive (chain ends one before it) or terminates the chain itself
+            F = C->first_term[round & 1];
+            need = false;
+            if (active && tid > 0 && (uint32_t)tid <= F) {
+              const uint32_t pe = laneE[tid - 1];
+              if (pe != my_s) { my_s = pe; need = true; }
+            }
+            if (prof && tid == 0) prof[blockIdx.x * 16 + 12] += 1;
+            if (!bar_or<BAR_P, NT_P>(need)) break;
+            if (round > NT_P + 2) { err = INF_ERR_INPUT; break; }
           }
-          __syncthreads();
-          // the lane found above is either inactive (chain ends one before it) or terminates the chain itself
-          F = C->first_term[round & 1];
-          need = false;
-          if (active && tid > 0 && (uint32_t)tid <= F) {
-            const uint32_t pe = laneE[tid - 1];
-            if (pe != my_s) { my_s = pe; need = true; }
+          ICTA_PROF(4);
+          if (err) break;
+          // F may name the first INACTIVE lane: the chain then ends at F - 1
+          if ((uint32_t)tid == F) C->last_lane = active ? F : F - 1;
+          psync();
+          const uint32_t last = C->last_lane;
+          if ((uint32_t)tid == last) C->last_info = my_t | (my_e << 2);
+          // ---- exclusive scan of the byte counts of lanes 0..last ----
+          const uint32_t cnt_n = ((uint32_t)tid <= last) ? my_n : 0u;
+          uint32_t incl = cnt_n;
+          #pragma unroll
+          for (int o = 1; o < 32; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
+          if (lane == 31) C->warp_tot[warp] = incl;
+          psync();
+          uint32_t wbase = 0, total = 0;
+          #pragma unroll
+          for (int w = 0; w < NT_P / 32; w++) { const uint32_t t = C->warp_tot[w]; if (w < warp) wbase += t; total += t; }
+          const uint32_t last_t = C->last_info & 3u, last_e = C->last_info >> 2;
+          if (last_t == T_BAD) { err = INF_ERR_SYMBOL; break; }
+          if (outpos + total > olimit || total > 65536u) { err = INF_ERR_OVERRUN; break; }
+          // ---- emit ----
+          acquire_window();
+          if ((uint32_t)(warp * 32) <= last) {
+            uint32_t e2 = 0;
+            decode_sub<true>((uint32_t)tid <= last, pay_s, ll_s, d_s, my_s, my_s, my_stop, win_s, hb_s, outpos + wbase + incl - cnt_n, obase, olimit, &e2);
+            if (e2) atomicMax(&C->err, e2);
           }
-          if (prof && tid == 0) prof[blockIdx.x * 16 + 12] += 1;
-          if (!__syncthreads_or(need ? 1 : 0)) break;
-          if (round > (int)NSUB + 2) { err = INF_ERR_INPUT; break; }
+          psync();
+          ICTA_PROF(5);
+          err = C->err;
+          if (err) break;
+          outpos += total;
+          abs_bit = last_e + (uint32_t)(buf_lo * 8);
+          if (last_t == T_EOB) block_done = true;
+          else if (to_end) { err = INF_ERR_INPUT; break; }
         }
-        ICTA_PROF(4);
-        if (err) break;
-        // F may name the first INACTIVE lane: the chain then ends at F - 1
-        if ((uint32_t)tid == F) C->last_lane = active ? F : F - 1;
-        __syncthreads();
-        const uint32_t last = C->last_lane;
-        if ((uint32_t)tid == last) C->last_info = my_t | (my_e << 2);
-        // ---- exclusive scan of the byte counts of lanes 0..last ----
-        const uint32_t cnt_n = ((uint32_t)tid <= last) ? my_n : 0u;
-        uint32_t incl = cnt_n;
-        #pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
-        if (lane == 31) C->warp_tot[warp] = incl;
-        __syncthreads();
-        uint32_t wbase = 0, total = 0;
-        #pragma unroll
-        for (int w = 0; w < WARPS; w++) { const uint32_t t = C->warp_tot[w]; if (w < warp) wbase += t; total += t; }
-        const uint32_t last_t = C->last_info & 3u, last_e = C->last_info >> 2;
-        if (last_t == T_BAD) { err = INF_ERR_SYMBOL; break; }
-        if (outpos + total > olimit || total > 65536u) { err = INF_ERR_OVERRUN; break; }
-        // ---- emit ----
-        if ((uint32_t)(warp * 32) <= last) {
-          uint32_t e2 = 0;
-          decode_sub<true>((uint32_t)tid <= last, pay_s, ll_s, d_s, my_s, my_s, my_stop, win_s, hb_s, outpos + wbase + incl - cnt_n, obase, olimit, &e2);
-          if (e2) atomicMax(&C->err, e2);
-        }
-        __syncthreads();
-        ICTA_PROF(5);
-        err = C->err;
-        if (err) break;
-        outpos += total;
-        abs_bit = last_e + (uint32_t)(buf_lo * 8);
-        if (last_t == T_EOB) block_done = true;
-        else if (to_end) { err = INF_ERR_INPUT; break; }
       }
-    }
-    if (!err && outpos != olimit) err = outpos > olimit ? INF_ERR_OVERRUN : INF_ERR_ISIZE;
+      if (!err && outpos != olimit) err = outpos > olimit ? INF_ERR_OVERRUN : INF_ERR_ISIZE;
 
-    if (!err) {
-      // ---- resolve ----
-      {
-        uint16_t* const list = reinterpret_cast<uint16_t*>(smem + K::OFF_PAY);
-        const uint32_t e = resolve_member<NT>(win, hb, list, K::LIST_CAP, C, obase, olimit, tid);
-        __syncthreads();
-        err = e ? e : C->err;
+      if (!err) {
+        // ---- hand the window over: the consumer resolves, checks and stores this member while the next one is decoded ----
+        acquire_window();                                                    // (an empty member writes nothing, but is handed over all the same)
+        fence_proxy_async();                                                 // window bytes -> the consumer's cp.async.bulk store
+        if (tid == 0) { CC->h.bi = bi; CC->h.obase = obase; CC->h.isize = isize; CC->h.crc = bd.crc; CC->h.uoff = bd.uoff; }
+        bar_arrive<BAR_FULL, NT>();
+        have_win = false;
+      } else {
+        // rejected: leave clean state behind (no head bits); the producer keeps the window
+        psync();
+        if (have_win) for (uint32_t i = tid; i < K::HB_WORDS; i += NT_P) hb[i] = 0;
+        if (tid == 0) {
+          status[bi] = err;
+          if (err == INF_RETRY) atomicAdd(retry_count, 1u);
+          else atomicCAS(err_flag, 0u, (bi << 4) | err | 0x80000000u);
+        }
       }
+      if (prof && tid == 0) prof[blockIdx.x * 16 + 13] += 1;
+      psync();
+    }
+    // end of the ticket stream
+    acquire_window();
+    if (tid == 0) CC->h.bi = HANDOFF_END;
+    bar_arrive<BAR_FULL, NT>();
+  } else {
+    // ================= CONSUMER: resolve, CRC-32, ISIZE, store, status =================
+    const int ct = tid - NT_P, cwarp = ct >> 5;
+    uint16_t* const list = reinterpret_cast<uint16_t*>(smem + K::OFF_LIST);
+    bar_arrive<BAR_EMPTY, NT>();                                             // the window starts empty
+    for (;;) {
+      bar_sync<BAR_FULL, NT>();
+      ICTA_PROF(10);
+      const Handoff h = CC->h;
+      if (h.bi == HANDOFF_END) break;
+      const uint32_t obase = h.obase, isize = h.isize;
+      // ---- resolve ----
+      const uint32_t nbatch = resolve_member<NT_C>(win, hb, list, K::LIST_CAP, CC, obase, obase + isize, ct);
+      csync();
+      uint32_t err = CC->err;
+      if (prof && ct == 0) prof[blockIdx.x * 16 + 11] += nbatch;
       ICTA_PROF(6);
 
-      // ---- CRC-32 from the window (strided slicing-by-4: thread t owns words t, t+NT, ...; tables in the payload buffer) ----
+      // ---- CRC-32 from the window (strided slicing-by-4: thread t owns words t, t+NT_C, ...; tables read through L1) ----
       if (check_crc && !err) {
-        uint32_t* const ctab = pay;
-        for (uint32_t i = tid; i < CrcTabs<NT>::WORDS; i += NT) ctab[i] = __ldg(crc_tabs + i);
-        __syncthreads();
+        const uint32_t* const ctab = crc_tabs;
         const uint32_t head = min(isize, (4u - (obase & 3u)) & 3u);           // bytes in front of the first aligned word
         const uint32_t nw = (isize - head) >> 2, tail = (isize - head) & 3u;
         const uint32_t* const words = reinterpret_cast<const uint32_t*>(win + obase + head);
         uint32_t st = 0;
-        if (tid == 0) { st = 0xffffffffu; for (uint32_t k = 0; k < head; k++) st = crc_byte_bitwise(st, win[obase + k]); }
+        if (ct == 0) { st = 0xffffffffu; for (uint32_t k = 0; k < head; k++) st = crc_byte_bitwise(st, win[obase + k]); }
         uint32_t acc = 0, part = 0;
-        if ((uint32_t)tid < nw) {
-          acc = words[tid] ^ st;                                               // the running state folds into the first word
-          uint32_t k = tid + NT;
-          for (; k < nw; k += NT) {
-            acc = ctab[3 * 256 + (acc & 0xffu)] ^ ctab[2 * 256 + ((acc >> 8) & 0xffu)] ^ ctab[256 + ((acc >> 16) & 0xffu)] ^ ctab[acc >> 24];
+        if ((uint32_t)ct < nw) {
+          acc = words[ct] ^ st;                                                // the running state folds into the first word
+          uint32_t k = ct + NT_C;
+          for (; k < nw; k += NT_C) {
+            acc = __ldg(ctab + 3 * 256 + (acc & 0xffu)) ^ __ldg(ctab + 2 * 256 + ((acc >> 8) & 0xffu)) ^ __ldg(ctab + 256 + ((acc >> 16) & 0xffu)) ^ __ldg(ctab + (acc >> 24));
             acc ^= words[k];
           }
-          // acc sits at word k_last = k - NT; it still has to cross (nw - k_last) words
-          part = crc_mulmod(acc, ctab[1024 + (nw - (k - NT))]);
-        } else if (tid == 0) {
+          // acc sits at word k_last = k - NT_C; it still has to cross (nw - k_last) words
+          part = crc_mulmod(acc, __ldg(ctab + 1024 + (nw - (k - NT_C))));
+        } else if (ct == 0) {
           part = st;                                                           // fewer than one word: only the head bytes
         }
         #pragma unroll
         for (int o = 16; o; o >>= 1) part ^= __shfl_xor_sync(FULL, part, o);
-        if (lane == 0) C->crc_part[warp] = part;
-        __syncthreads();
-        if (tid == 0) {
+        if (lane == 0) CC->crc_part[cwarp] = part;
+        csync();
+        if (ct == 0) {
           uint32_t crc = 0;
-          for (int w = 0; w < WARPS; w++) crc ^= C->crc_part[w];
+          for (int w = 0; w < RWARPS; w++) crc ^= CC->crc_part[w];
           for (uint32_t k = 0; k < tail; k++) crc = crc_byte_bitwise(crc, win[obase + head + 4u * nw + k]);
-          if (~crc != bd.crc) C->err = INF_ERR_CRC;
+          if (~crc != h.crc) CC->err = INF_ERR_CRC;
         }
-        __syncthreads();
-        err = C->err;
+        csync();
+        err = CC->err;
         ICTA_PROF(7);
       }
-    }
-    if (!err) {
-      // ---- the window leaves the SM once: 16-byte aligned body by cp.async.bulk, ragged ends by byte stores ----
-      uint8_t* const gout = infl + bd.uoff;                                    // (gout + k) and (win + obase + k) are congruent mod 16
-      const uint32_t head = min(isize, (16u - obase) & 15u);
-      const uint32_t body = (isize - head) & ~15u, tailb = isize - head - body;
-      if ((uint32_t)tid < head) gout[tid] = win[obase + tid];
-      if ((uint32_t)tid < tailb) gout[head + body + tid] = win[obase + head + body + tid];
-      if (body) {
-        fence_proxy_async();
-        __syncthreads();
-        if (tid == 0) bulk_store(gout + head, win + obase + head, body);
-        store_pending = true;
+      if (!err) {
+        // ---- the window leaves the SM once: 16-byte aligned body by cp.async.bulk, ragged ends by byte stores ----
+        uint8_t* const gout = infl + h.uoff;                                   // (gout + k) and (win + obase + k) are congruent mod 16
+        const uint32_t head = min(isize, (16u - obase) & 15u);
+        const uint32_t body = (isize - head) & ~15u, tailb = isize - head - body;
+        if ((uint32_t)ct < head) gout[ct] = win[obase + ct];
+        if ((uint32_t)ct < tailb) gout[head + body + ct] = win[obase + head + body + ct];
+        if (body) {
+          fence_proxy_async();
+          csync();
+          if (ct == 0) { bulk_store(gout + head, win + obase + head, body); bulk_store_wait_read(); }
+        }
+      } else {
+        // leave clean state behind: no head or map bits
+        for (uint32_t i = ct; i < K::HB_WORDS; i += NT_C) hb[i] = 0;
       }
-    } else {
-      // leave clean state behind: no head bits, no half-done store
-      __syncthreads();
-      for (uint32_t i = tid; i < K::HB_WORDS; i += NT) hb[i] = 0;
+      if (ct == 0) {
+        status[h.bi] = err;
+        if (err) { atomicCAS(err_flag, 0u, (h.bi << 4) | err | 0x80000000u); CC->err = INF_OK; }
+      }
+      csync();                                                               // (the store has read the window)
+      ICTA_PROF(8);
+      bar_arrive<BAR_EMPTY, NT>();
     }
-    if (tid == 0) {
-      status[bi] = err;
-      if (err == INF_RETRY) atomicAdd(retry_count, 1u);
-      else if (err) atomicCAS(err_flag, 0u, (bi << 4) | err | 0x80000000u);
-      if (prof) prof[blockIdx.x * 16 + 13] += 1;
-    }
-    __syncthreads();
-    ICTA_PROF(8);
+    // a bulk store must have finished reading shared memory before the CTA exits; writes complete with the grid
+    if (ct == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
 #undef ICTA_PROF
-  if (store_pending && tid == 0) bulk_store_wait_read();
-  // a bulk store must have finished reading shared memory before the CTA exits; writes complete with the grid
-  if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
 }  // namespace icta

@@ -5,10 +5,11 @@
 // BGZF member of a file with zlib.  Test/verification tool only: nothing in the product links it.
 //
 //   inflate_sim file.bam [--lanes 256] [--max-members N] [--span-bytes B] [--overlap BITS] [--stats]
-//                        [--resolve MODE] [--piece BYTES] [--rlanes N] [--gate G] [--group-sync]
+//                        [--resolve MODE] [--piece BYTES] [--rlanes N] [--gate G] [--group-sync] [--list-cap N]
 // --resolve: 0 the round-2 v3 resolver (eight polling warps, groups of 32), 1 / 2 one warp in order with the frontier rule
 // (groups / rolling), 3 rolling + exact readiness, 4 static lane-strided + exact readiness, 6 the COMMITTED resolver (all warps,
-// static, exact readiness; --gate models the measured-and-dropped gate), 7 list-free dealing by bitmap word (292 rounds: dropped).
+// static, exact readiness; --gate models the measured-and-dropped gate; --list-cap N resolves in output-ordered batches of at most
+// N matches, as the kernel does), 7 list-free dealing by bitmap word (292 rounds: dropped).
 #include <zlib.h>
 
 #include <algorithm>
@@ -71,7 +72,7 @@ static int build_lut(const uint8_t* cl, int n, uint32_t* lut, uint32_t sub_cap) 
   return 0;
 }
 
-struct Stats { long members = 0, blocks = 0, spans = 0, rounds = 0, lane_decodes = 0, lane_slots = 0, resolve_iters = 0, resolve_steps_max = 0, sub_overflow = 0, resolve_batches = 0; };
+struct Stats { long members = 0, blocks = 0, spans = 0, rounds = 0, lane_decodes = 0, lane_slots = 0, resolve_iters = 0, resolve_steps_max = 0, sub_overflow = 0, resolve_batches = 0, matches_max = 0, list_batches = 0; };
 
 
 // Host model of the kernel's resolver (resolve_member in kernels_inflate_cta.cuh): in-order list of match heads, the
@@ -180,12 +181,23 @@ static int resolve_inorder_model(uint8_t* win, uint32_t* hb, uint32_t obase, uin
 // thread t takes matches t, t + 32 W, ...  `group_sync`: a warp adopts its next 32 matches only when all 32 current ones
 // are done, and (gate >= 0) starts polling a group only when the group `gate` groups in front of it is complete.
 // All warps execute one iteration per round (lockstep): rounds ~ latency, polls ~ issued iterations.
-static int g_gate = -1; static bool g_group_sync = false;
+// `list_cap` > 0: the kernel's batched form -- the matches in output order, at most list_cap at a time, each batch's map built
+// only when the batch before it is done (exact: a match's sources lie in front of it, hence in front of every later match).
+static int g_gate = -1; static bool g_group_sync = false; static uint32_t g_list_cap = 0;
+static int resolve_static_batch(uint8_t* win, const uint16_t* list, uint32_t total, uint32_t obase, uint32_t olimit, int W, Stats& S);
 static int resolve_static_model(uint8_t* win, uint32_t* hb, uint32_t obase, uint32_t olimit, int W, Stats& S) {
   const uint32_t wbeg = obase >> 5, wend = (olimit + 31) >> 5;
   std::vector<uint16_t> list;
   for (uint32_t w = wbeg; w < wend; w++) { uint32_t bits = hb[w]; hb[w] = 0; while (bits) { list.push_back((uint16_t)(w * 32 + __builtin_ctz(bits) - obase)); bits &= bits - 1; } }
-  const uint32_t total = (uint32_t)list.size();
+  const uint32_t all = (uint32_t)list.size(), cap = g_list_cap ? g_list_cap : std::max(1u, all);
+  S.matches_max = std::max<long>(S.matches_max, all);
+  for (uint32_t b = 0; b < all; b += cap) {
+    S.list_batches++;
+    if (int rc = resolve_static_batch(win, list.data() + b, std::min(cap, all - b), obase, olimit, W, S)) return rc;
+  }
+  return 0;
+}
+static int resolve_static_batch(uint8_t* win, const uint16_t* list, uint32_t total, uint32_t obase, uint32_t olimit, int W, Stats& S) {
   std::vector<uint8_t> fin(olimit + 64, 1);
   for (uint32_t r = 0; r < total; r++) { uint32_t o = obase + list[r], len = (((win[o + 1] << 8) | (win[o + 2] << 16)) >> 15) + 3; for (uint32_t k = 0; k < len; k++) fin[o + k] = 0; }
   const int T = 32 * W;
@@ -422,7 +434,7 @@ int main(int argc, char** argv) {
   for (int i = 2; i < argc; i++) {
     std::string a = argv[i];
     if (a == "--lanes") NT = atoi(argv[++i]); else if (a == "--max-members") maxm = atol(argv[++i]);
-    else if (a == "--span-bytes") span_bytes = (uint32_t)atol(argv[++i]); else if (a == "--overlap") overlap = (uint32_t)atol(argv[++i]); else if (a == "--stats") stats = true; else if (a == "--resolve") g_rmode = atoi(argv[++i]); else if (a == "--gate") g_gate = atoi(argv[++i]); else if (a == "--group-sync") g_group_sync = true; else if (a == "--rlanes") g_lanes = atoi(argv[++i]); else if (a == "--piece") g_piece = (uint32_t)atol(argv[++i]);
+    else if (a == "--span-bytes") span_bytes = (uint32_t)atol(argv[++i]); else if (a == "--overlap") overlap = (uint32_t)atol(argv[++i]); else if (a == "--stats") stats = true; else if (a == "--resolve") g_rmode = atoi(argv[++i]); else if (a == "--gate") g_gate = atoi(argv[++i]); else if (a == "--group-sync") g_group_sync = true; else if (a == "--rlanes") g_lanes = atoi(argv[++i]); else if (a == "--piece") g_piece = (uint32_t)atol(argv[++i]); else if (a == "--list-cap") g_list_cap = (uint32_t)atol(argv[++i]);
   }
   FILE* f = fopen(argv[1], "rb"); if (!f) { perror("open"); return 2; }
   fseek(f, 0, SEEK_END); long sz = ftell(f); fseek(f, 0, SEEK_SET);
@@ -448,8 +460,10 @@ int main(int argc, char** argv) {
     }
     off += bsize + 1; nm++;
   }
-  printf("%s: members=%ld bad=%ld refused(sub-table)=%ld | deflate blocks=%ld spans=%ld rounds/span=%.2f lane-decodes/span=%.1f (of %d) resolver warp-iterations/member=%.0f groups/member=%.0f\n", argv[1], S.members, bad, S.sub_overflow,
+  printf("%s: members=%ld bad=%ld refused(sub-table)=%ld | deflate blocks=%ld spans=%ld rounds/span=%.2f lane-decodes/span=%.1f (of %d) resolver warp-iterations/member=%.0f groups/member=%.0f", argv[1], S.members, bad, S.sub_overflow,
          S.blocks, S.spans, (double)S.rounds / std::max(1L, S.spans), (double)S.lane_decodes / std::max(1L, S.spans), NT, (double)S.resolve_iters / std::max(1L, S.members), (double)S.resolve_batches / std::max(1L, S.members));
+  if (g_rmode == 6) printf(" matches/member(max)=%ld list-batches=%ld", S.matches_max, S.list_batches);
+  printf("\n");
   (void)stats;
   return bad ? 1 : 0;
 }
