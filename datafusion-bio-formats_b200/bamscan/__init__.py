@@ -78,7 +78,8 @@ class Stats(C.Structure):
                 ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64),
                 ("blocks", C.c_uint64), ("kernel_launches", C.c_uint64), ("boundary_repairs", C.c_uint64),
                 ("ms_total", C.c_double), ("ms_inflate", C.c_double), ("ms_boundary", C.c_double), ("ms_decode", C.c_double),
-                ("boundary_seam_mismatches", C.c_uint64), ("first_record_uoff", C.c_uint64), ("end_chain_uoff", C.c_uint64)]
+                ("boundary_seam_mismatches", C.c_uint64), ("first_record_uoff", C.c_uint64), ("end_chain_uoff", C.c_uint64),
+                ("inflate_retries", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}

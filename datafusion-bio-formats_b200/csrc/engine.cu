@@ -17,6 +17,7 @@
 #include <fcntl.h>
 #include <sys/mman.h>
 #include <unistd.h>
+#include <zlib.h>
 
 #include <algorithm>
 #include <atomic>
@@ -290,9 +291,10 @@ using LgCfg = LgConfig<LG_G, LG_W>;
 static int device_sms(int device) { int sms = 148; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device); return sms; }
 
 // Inflates the nb members described by d_blk (and verifies their CRC-32 unless skip_crc) on stream cs.
-// d_aux: two zeroed words (ticket of the retry launch, retry count).
+// d_retry_ticket, d_retries: zeroed words (ticket of the retry launch; members the CTA kernel refused, counted by it).
 static int launch_inflate(const BamFile* f, cudaStream_t cs, const uint8_t* d_comp, const BlockDesc* d_blk, uint32_t nb, uint8_t* U,
-                          uint32_t* d_status, uint32_t* d_ticket, uint32_t* d_err, uint32_t* d_aux, DeviceBuf* slots, int* launches) {
+                          uint32_t* d_status, uint32_t* d_ticket, uint32_t* d_err, uint32_t* d_retry_ticket, uint32_t* d_retries,
+                          DeviceBuf* slots, int* launches) {
   const uint32_t sms = (uint32_t)device_sms(f->device);
   const int check_crc = f->skip_crc ? 0 : 1;
   if (f->debug_flags & 4) {          // tests: the warp-per-member kernel on everything
@@ -316,11 +318,11 @@ static int launch_inflate(const BamFile* f, cudaStream_t cs, const uint8_t* d_co
   }
   {
     const uint32_t grid = std::min<uint32_t>(nb, sms * 2u);
-    icta::inflate_cta_kernel<<<grid, icta::NT, icta::Cfg::SMEM, cs>>>(d_comp, d_blk, nb, U, d_status, d_ticket, d_err, d_aux + 1, g_crc_tabs[f->device], check_crc, g_icta_prof);
+    icta::inflate_cta_kernel<<<grid, icta::NT, icta::Cfg::SMEM, cs>>>(d_comp, d_blk, nb, U, d_status, d_ticket, d_err, d_retries, g_crc_tabs[f->device], check_crc, g_icta_prof);
     *launches += 1;
     // members flagged INF_RETRY (none on ordinary files); the launch finds nothing to do otherwise
     uint32_t rgrid = std::min<uint32_t>((nb + INF_WARPS - 1) / INF_WARPS, sms);
-    inflate_kernel<<<rgrid, INF_WARPS * 32, sizeof(InflateShared), cs>>>(d_comp, d_blk, nb, U, d_status, d_aux, d_err, check_crc, icta::INF_RETRY);
+    inflate_kernel<<<rgrid, INF_WARPS * 32, sizeof(InflateShared), cs>>>(d_comp, d_blk, nb, U, d_status, d_retry_ticket, d_err, check_crc, icta::INF_RETRY);
     *launches += 1;
   }
   return BAMSCAN_OK;
@@ -450,6 +452,30 @@ static void plan_chunks(const BamFile& f, uint32_t b0, uint32_t b1, bool extensi
   }
 }
 
+// An empty member (ISIZE 0) gives the inflate kernels nothing to do, so it has no descriptor; it is still a member of the
+// file, and zlib and the reference's reader reject it unless its CRC-32 is 0 and its payload inflates to nothing.  It is
+// checked on the host (it is a few bytes; host zlib) when the chunk that holds it is staged: a scan fails on the empty
+// members of the blocks it reads, and a region query never looks at members outside its blocks.
+static int check_empty_member(const BamFile* f, uint32_t b) {
+  const BgzfBlock& B = f->blocks[b];
+  const char* why = nullptr;
+  if (B.crc != 0) why = "CRC32 mismatch";
+  else {
+    z_stream zs; memset(&zs, 0, sizeof zs);
+    uint8_t out = 0;
+    if (inflateInit2(&zs, -15) != Z_OK) { set_error("zlib initialisation failed"); return BAMSCAN_ERR_IO; }
+    zs.next_in = const_cast<Bytef*>(f->data + B.coff + B.cdata_off); zs.avail_in = B.csize - B.cdata_off - 8;
+    zs.next_out = &out; zs.avail_out = 1;
+    const int zr = inflate(&zs, Z_FINISH);
+    if (zs.total_out) why = "ISIZE mismatch";
+    else if (zr != Z_STREAM_END) why = "invalid deflate stream";
+    inflateEnd(&zs);
+  }
+  if (!why) return BAMSCAN_OK;
+  set_error("BAM read error: BGZF member %u (file offset %llu): inflate failed: %s", b, (unsigned long long)B.coff, why);
+  return BAMSCAN_ERR_CRC;
+}
+
 // Builds the chunk's member descriptors in pinned memory and queues them, with the compressed bytes, on the H2D stream.
 // Everything the compute stream needs from the host for this chunk travels here, so the copy engine never makes the
 // kernels of the previous chunk wait (a pageable copy issued on the compute stream would queue behind the big transfer).
@@ -469,6 +495,7 @@ static int issue_h2d(BamScanStream* s, const ChunkPlan& c, int slot) {
   for (uint32_t b = c.b0; b < c.b1; b++) {
     const BgzfBlock& B = f->blocks[b];
     if (B.isize) { BlockDesc d; d.cdata_off = (uint32_t)(B.coff - c.c0) + B.cdata_off; d.cdata_len = B.csize - B.cdata_off - 8; d.isize = B.isize; d.crc = B.crc; d.uoff = uoff; descs[nb++] = d; }
+    else if (int rc = check_empty_member(f, b)) return rc;
     uoff += B.isize;
   }
   s->n_descs[slot] = nb; s->chunk_data_hi[slot] = uoff;
@@ -751,7 +778,10 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   uint32_t* d_seg_count = d_seg_exit + n_seg;
   uint32_t* d_seg_base = d_seg_count + n_seg;
   uint8_t* d_seg_tail = reinterpret_cast<uint8_t*>(d_seg_base + n_seg);
-  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();   // [0..7] boundary flags, [8] inflate ticket, [9] inflate err, [10..11] decode err
+  // [0..7] boundary / filter flags, [8] inflate ticket, [9] inflate error, [10] seams rejected, [11] first disagreeing seam,
+  // [12] retry ticket, [13] first owned record, [14] FASTQ first record line, [15] members the CTA inflate kernel refused:
+  // these 16 words are published to the host.  [16] FASTQ newline count (device only).
+  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
 
   cudaStream_t cs = s->s_chunk[slot];
   const uint8_t* d_comp;
@@ -782,7 +812,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   CU_TRY(cudaEventRecord(s->ev_t[slot][0], cs));
   if (nb) {
     int nl = 0;
-    if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, &s->d_sorted, &nl))) return rc;
+    if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, d_flags + 15, &s->d_sorted, &nl))) return rc;
     s->st.kernel_launches += nl;
   }
   CU_TRY(cudaEventRecord(s->ev_t[slot][1], cs));
@@ -800,11 +830,11 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     const uint32_t line_cap = span / 8 + 4096;                                          // lines[] capacity: FASTQ lines average far more than 8 bytes; beyond that the scan fails loudly
     if ((rc = s->d_recoff[slot].ensure(4ull * line_cap))) return rc;
     fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
-    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + 15);
+    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + 16);
     s->st.kernel_launches += 2;
     fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
     FastqFrame FF{U, lo, data_hi, BP.own_hi, (uint32_t)(s->need_spec ? 1 : 0), (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap};
-    fq_frame_kernel<<<1, 32, 0, cs>>>(FF, d_flags + 15, s->d_recoff[slot].as<uint32_t>(), d_flags);
+    fq_frame_kernel<<<1, 32, 0, cs>>>(FF, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
     s->st.kernel_launches += 2;
     publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
     CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
@@ -847,7 +877,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   }
   if (hf[1] && f->format == 1) { set_error("FASTQ read error: more lines in one chunk than supported (lines shorter than 8 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
   if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - HEADROOM))); return BAMSCAN_ERR_FORMAT; }
-  s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10];
+  s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10]; s->st.inflate_retries += hf[15];
   const uint32_t n_rec = hf[3];
   if (f->format == 1) { if (n_rec > 0) s->need_spec = false; }
   else if (n_rec > 0 || hf[2] != 0xffffffffu) s->need_spec = false;
@@ -1517,7 +1547,7 @@ int bamscan_bench_inflate(BamScanPlan* plan, int32_t partition, int32_t repeats,
     cudaMemsetAsync(flags.p, 0, 64, s->s_compute);
     cudaEventRecord(e0, s->s_compute);
     int nl = 0;
-    launch_inflate(f, s->s_compute, comp.as<uint8_t>(), blk.as<BlockDesc>(), nb, infl.as<uint8_t>(), status.as<uint32_t>(), flags.as<uint32_t>() + 8, flags.as<uint32_t>() + 9, flags.as<uint32_t>() + 12, &s->d_sorted, &nl);
+    launch_inflate(f, s->s_compute, comp.as<uint8_t>(), blk.as<BlockDesc>(), nb, infl.as<uint8_t>(), status.as<uint32_t>(), flags.as<uint32_t>() + 8, flags.as<uint32_t>() + 9, flags.as<uint32_t>() + 12, flags.as<uint32_t>() + 15, &s->d_sorted, &nl);
     cudaEventRecord(e1, s->s_compute);
     cudaEventSynchronize(e1);
     float ms = 0; cudaEventElapsedTime(&ms, e0, e1);

@@ -39,7 +39,8 @@ namespace icta {
 
 constexpr int R_LL = 10, R_D = 8;                       // root LUT index bits (litlen / distance)
 constexpr uint32_t ROOT_LL = 1u << R_LL, ROOT_D = 1u << R_D;
-constexpr uint32_t SUB_LL = 512, SUB_D = 128;           // second-level entries available (a table that needs more is refused)
+constexpr uint32_t SUB_LL = 512, SUB_D = 128;           // second-level entries available (a table that needs more is refused;
+                                                        // a canonical lit/len code over <= 286 symbols never needs 512)
 
 // 32-bit LUT entry (laid out for the fewest instructions in the decode step):
 //   [4:0]   bits this half-token consumes: code length + extra bits (0 = unused code); E_SUB: index bits of the second level
@@ -66,6 +67,13 @@ ICTA_HD uint32_t entry_dist(uint32_t sym, uint32_t len) {
   const uint32_t extra = sym < 4u ? 0u : (sym - 2u) >> 1;
   const uint32_t base = sym < 4u ? 1u + sym : 1u + ((2u + (sym & 1u)) << extra);
   return E_SYM | (len << 5) | (len + extra) | (base << 16);
+}
+// Completeness rule of a lit/len or distance code, as zlib (inftrees.c) and libdeflate apply it.  `left` is the code space
+// the lengths leave unused (0: complete), `n_codes` the number of used symbols, `n_len1` those of length 1.  An incomplete
+// code is rejected unless it is empty (a distance code of a block without matches) or a single code of length 1 (its
+// codeword is the bit 0; the bit 1 is an invalid code).  Over-subscription is checked separately.
+ICTA_HD bool code_complete_ok(uint32_t left, uint32_t n_codes, uint32_t n_len1) {
+  return left == 0u || n_codes == 0u || (n_codes == 1u && n_len1 == 1u);
 }
 ICTA_HD uint32_t entry_sub(uint32_t root_bits, uint32_t sub_bits, uint32_t index) { return E_SUB | (root_bits << 5) | sub_bits | (index << 16); }
 

@@ -25,6 +25,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "inflate_cta_core.h"
+
 namespace bamscan {
 
 struct BlockDesc {        // one BGZF member of the chunk (host-built from the BSIZE chain)
@@ -134,7 +136,7 @@ struct BitReader {
 
 // ---------------------------------------------------------------------------------------------
 // Canonical Huffman table build, warp-cooperative.  cl[0..n) code lengths (0 = unused).
-// Returns false when the code is over-subscribed.
+// Returns false when the code is over-subscribed or incomplete (icta::code_complete_ok; the code-length code must be complete).
 template <int PBITS, int TK>
 __device__ __forceinline__ bool build_table(const uint8_t* cl, int n, uint32_t* lut, uint16_t* sorted,
                                             uint16_t* first, uint16_t* offs, uint16_t* cnt, uint16_t* nxt, int lane) {
@@ -159,6 +161,7 @@ __device__ __forceinline__ bool build_table(const uint8_t* cl, int n, uint32_t* 
     off += c;
   }
   if (over) return false;
+  if (TK == TK_PRECODE ? left != 0u : !icta::code_complete_ok(left, off, cnt[1])) return false;   // incomplete
   __syncwarp();
   const uint32_t lt = (1u << lane) - 1u;
   for (int b = 0; b < n; b += 32) {
@@ -334,10 +337,10 @@ inflate_kernel(const uint8_t* __restrict__ comp, const BlockDesc* __restrict__ b
         continue;
       }
       if (btype == 3) { err = INF_ERR_BTYPE; break; }
-      int n_ll = 288, n_d = 30;
+      int n_ll = 288, n_d = 32;
       if (btype == 1) {
         for (int i = lane; i < 288; i += 32) T.cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8;
-        if (lane < 30) T.cl[288 + lane] = 5;
+        T.cl[288 + lane] = 5;                          // all 32 distance codes: complete, and 30 / 31 decode as invalid
         __syncwarp();
       } else {
         err = read_dynamic_header(br, T, lane, &n_ll, &n_d);
@@ -515,6 +518,7 @@ __device__ __forceinline__ bool build_table16(const uint8_t* cl, int n, uint16_t
     off += c;
   }
   if (over) return false;
+  if (TK == TK_PRECODE ? left != 0u : !icta::code_complete_ok(left, off, S.cnt[1])) return false;   // incomplete
   __syncwarp();
   const uint32_t lt = (1u << lane) - 1u;
   for (int b = 0; b < n; b += 32) {
@@ -712,11 +716,11 @@ inflate_lg_kernel(const uint8_t* __restrict__ comp, const BlockDesc* __restrict_
           continue;
         }
         if (btype == 3) { s_err = INF_ERR_BTYPE; continue; }
-        int n_ll = 288, n_d = 30;
+        int n_ll = 288, n_d = 32;
         __syncwarp();
         if (btype == 1) {
           for (int i = lane; i < 288; i += 32) WS.cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8;
-          if (lane < 30) WS.cl[288 + lane] = 5;
+          WS.cl[288 + lane] = 5;                         // all 32 distance codes: complete, and 30 / 31 decode as invalid
           __syncwarp();
         } else {
           s_err = read_dynamic_header16(br, T, WS, lane, &n_ll, &n_d);

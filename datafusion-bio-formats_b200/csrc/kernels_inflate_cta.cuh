@@ -21,8 +21,9 @@
 // handed over by two named barriers: FULL (producer -> consumer, with a hand-off record) and EMPTY (consumer -> producer).
 // HBM traffic is the algorithmic minimum: payload read once, inflated bytes written once.
 //
-// Members this kernel cannot take (ISIZE > 65536, a Huffman code whose second-level tables exceed the shared-memory budget)
-// are flagged INF_RETRY in status[] and redone by the warp-per-member kernel of kernels_inflate.cuh.
+// Members this kernel cannot take (ISIZE > 65536, a Huffman code whose second-level tables exceed the shared-memory budget:
+// in practice only a distance code, see SUB_D) are flagged INF_RETRY in status[], counted in *retry_count and redone by the
+// warp-per-member kernel of kernels_inflate.cuh.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -172,8 +173,8 @@ __device__ __forceinline__ uint32_t brev_n(uint32_t v, uint32_t bits) { return _
 //   lut_fill_root     ALL threads: root entry idx is decoded canonically (<= RBITS steps) -- perfectly balanced, where a
 //                     symbol-centric fill leaves one lane writing 2^(RBITS - len) entries for the shortest code;
 //   lut_sub_warp      one warp per table: second-level tables for the codes longer than RBITS bits.
-// `S` selects the scratch rows of Ctl.  Error codes: INF_ERR_TABLE for an over-subscribed code, INF_RETRY when the
-// second-level tables do not fit.
+// `S` selects the scratch rows of Ctl.  Error codes: INF_ERR_TABLE for an over-subscribed or incomplete code
+// (code_complete_ok), INF_RETRY when the second-level tables do not fit.
 template <int RBITS>
 __device__ __forceinline__ uint32_t lut_prepare_warp(const uint8_t* cl, int n, Ctl* C, int S, uint16_t* sorted, uint16_t* codes, int lane) {
   uint16_t* cnt = C->cnt[S]; uint16_t* first = C->first[S]; uint16_t* nxt = C->nxt[S]; uint16_t* offs = C->offs[S];
@@ -195,7 +196,7 @@ __device__ __forceinline__ uint32_t lut_prepare_warp(const uint8_t* cl, int n, C
     if (lane == len) { first[len] = (uint16_t)code; offs[len] = (uint16_t)off; }
     off += c;
   }
-  if (over) return INF_ERR_TABLE;
+  if (over || !code_complete_ok(left, off, cnt[1])) return INF_ERR_TABLE;
   __syncwarp();
   const uint32_t lt = (1u << lane) - 1u;
   #pragma unroll
@@ -314,7 +315,7 @@ __device__ __noinline__ uint32_t read_precode_warp(SBits& br, uint32_t* plut, Ct
     left -= c;
     if (lane == len) first[len] = (uint16_t)code;
   }
-  if (over) return INF_ERR_TABLE;
+  if (over || left != 0) return INF_ERR_TABLE;                  // the code-length code must be complete (no exceptions)
   __syncwarp();
   const uint32_t m = __match_any_sync(FULL, L);
   const uint32_t r = __popc(m & ((1u << lane) - 1u));
@@ -764,8 +765,8 @@ inflate_cta_kernel(const uint8_t* __restrict__ comp, const BlockDesc* __restrict
             if ((len ^ nlen) != 0xffffu) e = INF_ERR_STORED;
           } else if (btype == 1) {
             for (int i = lane; i < 288; i += 32) C->cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8;
-            if (lane < 30) C->cl[288 + lane] = 5;
-            if (lane == 0) { C->n_ll = 288; C->n_d = 30; }
+            C->cl[288 + lane] = 5;                                 // all 32 distance codes: complete, and 30 / 31 decode as invalid
+            if (lane == 0) { C->n_ll = 288; C->n_d = 32; }
           } else {
             e = read_precode_warp(br, lut_d + ROOT_D, C, lane);
           }

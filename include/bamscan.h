@@ -111,6 +111,9 @@ typedef struct BamScanStats {
    * whole file is proven exact when end_chain_uoff of partition p - 1 equals first_record_uoff of partition p for every p
    * (bamscan_check_partition_seams; the python mirror and bench.py do this and fail loudly otherwise). */
   uint64_t first_record_uoff, end_chain_uoff;
+  /* BGZF members the CTA-per-member inflate kernel refused (a Huffman code whose second-level tables exceed its shared-memory
+   * budget) and the warp-per-member kernel then inflated. */
+  uint64_t inflate_retries;
 } BamScanStats;
 
 /* Seam check over the stats of the N block-range partitions of one plan, in partition order.  0 = every partition starts

@@ -33,7 +33,7 @@ struct Bits {
 };
 
 // serial canonical build in the kernel's table format: root LUT of RBITS index bits + second-level tables behind it.
-// Returns 0 ok, 1 over-subscribed, 2 second-level space exhausted.
+// Returns 0 ok, 1 over-subscribed or incomplete (code_complete_ok), 2 second-level space exhausted.
 template <int RBITS, bool DIST>
 static int build_lut(const uint8_t* cl, int n, uint32_t* lut, uint32_t sub_cap) {
   const uint32_t ROOT = 1u << RBITS;
@@ -42,6 +42,8 @@ static int build_lut(const uint8_t* cl, int n, uint32_t* lut, uint32_t sub_cap) 
   cnt[0] = 0;
   uint32_t first[17], code = 0; int left = 1;
   for (int L = 1; L <= 15; L++) { code = (code + (L > 1 ? cnt[L - 1] : 0)) << 1; first[L] = code; left <<= 1; left -= cnt[L]; if (left < 0) return 1; }
+  uint32_t n_codes = 0; for (int L = 1; L <= 15; L++) n_codes += cnt[L];
+  if (!code_complete_ok((uint32_t)left, n_codes, (uint32_t)cnt[1])) return 1;
   for (uint32_t i = 0; i < ROOT + sub_cap; i++) lut[i] = E_BAD;
   uint32_t next[16]; for (int L = 1; L <= 15; L++) next[L] = first[L];
   // per root prefix: index bits of its second-level table
@@ -319,8 +321,8 @@ static int inflate_member_sim(const uint8_t* payload, uint32_t clen, uint32_t is
       outpos += len; br.pos += 8 * len;
       continue;
     }
-    uint8_t cl[320] = {0}; int n_ll = 288, n_d = 30;
-    if (btype == 1) { for (int i = 0; i < 288; i++) cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8; for (int i = 0; i < 30; i++) cl[288 + i] = 5; }
+    uint8_t cl[320] = {0}; int n_ll = 288, n_d = 32;   // fixed code: all 32 distance codes (complete; 30 / 31 decode as invalid)
+    if (btype == 1) { for (int i = 0; i < 288; i++) cl[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8; for (int i = 0; i < 32; i++) cl[288 + i] = 5; }
     else {
       uint32_t h = br.take(14); n_ll = (h & 31) + 257; n_d = ((h >> 5) & 31) + 1; int n_clc = (h >> 10) + 4;
       if (n_ll > 286 || n_d > 30) { *why = "hlit/hdist"; return 3; }
@@ -331,6 +333,7 @@ static int inflate_member_sim(const uint8_t* payload, uint32_t clen, uint32_t is
         int cnt[8] = {0}; for (int i = 0; i < 19; i++) cnt[pcl[i]]++; cnt[0] = 0;
         uint32_t code = 0, first[8]; int left = 1;
         for (int L = 1; L <= 7; L++) { code = (code + (L > 1 ? cnt[L - 1] : 0)) << 1; first[L] = code; left <<= 1; left -= cnt[L]; if (left < 0) { *why = "precode oversubscribed"; return 3; } }
+        if (left != 0) { *why = "precode incomplete"; return 3; }
         for (auto& v : plut) v = 0;
         for (int s = 0; s < 19; s++) { int L = pcl[s]; if (!L) continue; uint32_t c = first[L]++; uint32_t r = 0; for (int i = 0; i < L; i++) r |= ((c >> i) & 1u) << (L - 1 - i); for (uint32_t idx = r; idx < 128; idx += 1u << L) plut[idx] = (uint32_t)L | ((uint32_t)s << 16); }
       }
@@ -353,7 +356,7 @@ static int inflate_member_sim(const uint8_t* payload, uint32_t clen, uint32_t is
     int rc = build_lut<R_LL, false>(cl, n_ll, lut_ll.data(), SUB_LL);
     if (!rc) rc = build_lut<R_D, true>(cl + n_ll, n_d, lut_d.data(), SUB_D);
     if (rc == 2) { S.sub_overflow++; *why = "second-level table space exhausted"; return 100; }
-    if (rc) { *why = "oversubscribed"; return 3; }
+    if (rc) { *why = "over-subscribed or incomplete code"; return 3; }
 
     // ---- spans: the symbol stream of this block, NT lanes at a time ----
     uint32_t cur = br.pos;
