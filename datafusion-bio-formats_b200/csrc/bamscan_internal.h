@@ -61,7 +61,8 @@ struct BaiIndex {
 
 // == BamTableProvider (table_provider.rs:314-335)
 struct BamFile {
-  int format = 0;            // 0: BAM; 1: BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index
+  int format = 0;            // 0: BAM; 1: BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index;
+                             // 2: plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index
   std::string path, index_path;
   uint8_t* data = nullptr;   // whole file: read-only mapping (O_RDONLY / PROT_READ, not page-locked); small files: a plain copy
   uint64_t size = 0;
@@ -128,6 +129,9 @@ struct Plan {
 
 // host_file.cpp
 int load_file(BamFile* f);                       // reads the file into pinned memory, walks BGZF, parses header
+bool is_sam_path(const std::string& path);      // BamTableProvider's `is_sam`: the path ends in ".sam", any case
+int load_sam(BamFile* f);                        // format 2: header lines, @SQ references, pseudo-blocks over the text body
+uint64_t sam_record_start_at(const BamFile& f, uint64_t off);   // first line start at or after off (a record belongs to the range holding its first byte)
 int infer_tag_types(const BamFile& f, const std::vector<std::string>& tags, int sample_size,
                     std::map<std::string, std::pair<char, int32_t>>* out, bool all = false);   // table_provider.rs:145-202
 std::string discover_index(const std::string& path);   // index_utils.rs:43-76

@@ -21,6 +21,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <numeric>
 #include <cstdio>
 #include <cstring>
 #include <ctime>
@@ -34,6 +35,7 @@
 #include "kernels_inflate.cuh"
 #include "kernels_inflate_cta.cuh"
 #include "kernels_fastq.cuh"
+#include "kernels_sam.cuh"
 
 namespace bamscan {
 
@@ -230,6 +232,10 @@ struct BamScanStream {
   std::vector<int32_t> out_to_dec;        // projection position -> index into dec_cols
   // device memory
   DeviceBuf d_comp[2], d_blk[2], d_infl[2], d_carry, d_status[2], d_flags[2], d_seg[2], d_recoff[2], d_recoff2[2], d_keep[2], d_tiles, d_totals, d_scratch, d_arena[2], d_refs, d_sorted;
+  // SAM (format 2): per slot the parsed lines, record sizes -> offsets, "QUAL is *" flags, scan tiles and the transcoded BAM records;
+  // the reference names sorted bytewise for RNAME / RNEXT lookups
+  DeviceBuf d_samline[2], d_samsize[2], d_qabs[2], d_samtiles[2], d_bam[2], d_samrefs;
+  cudaEvent_t ev_text_free[2] = {nullptr, nullptr}, ev_ing[2][2] = {};   // the write pass has read a slot's text; ingest copy timing
   bool tail_seen = false, range_stop = false;   // per-reference unmapped tail state (physical_exec.rs:1203-1215)
   const uint8_t* d_comp_all = nullptr; DeviceBuf d_comp_all_buf; uint64_t comp_all_c0 = 0;
   uint32_t* d_hflags = nullptr;           // device alias of h_flags (mapped)
@@ -240,7 +246,7 @@ struct BamScanStream {
   // rows of the current chunk that are not decoded yet: a chunk is one inflate wave, a batch is one slice of its rows
   bool slice_pending = false;    // a decode slice whose time / error word has not been collected (flush_slice)
   int64_t launched_chunk = -1;   // index in `chunks` of a chunk whose inflate + boundary kernels are already queued (run_chunk phase 1)
-  struct { const uint8_t* U = nullptr; const uint32_t* recoff = nullptr; uint32_t n = 0, pos = 0, rows_per_slice = 0; bool long_records = false; uint64_t ubytes = 0; cudaStream_t cs = nullptr; } cur;
+  struct { const uint8_t* U = nullptr; const uint32_t* recoff = nullptr; const uint8_t* qabs = nullptr; uint32_t n = 0, pos = 0, rows_per_slice = 0; bool long_records = false; uint64_t ubytes = 0; cudaStream_t cs = nullptr; } cur;
   PendingBatch pending;
   std::vector<ReadyBatch> ready; size_t ready_pos = 0;
   BamScanStats st{};
@@ -351,6 +357,8 @@ static int stream_init(BamScanStream* s) {
   CU_TRY(cudaEventCreateWithFlags(&s->ev_carry, cudaEventDisableTiming));
   for (auto& row : s->ev_t) for (auto& e : row) CU_TRY(cudaEventCreate(&e));
   for (auto& e : s->ev_dt) CU_TRY(cudaEventCreate(&e));
+  for (auto& e : s->ev_text_free) CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  for (auto& row : s->ev_ing) for (auto& e : row) CU_TRY(cudaEventCreate(&e));
   CU_TRY(cudaHostAlloc((void**)&s->h_flags, 4096, cudaHostAllocPortable | cudaHostAllocMapped));
   CU_TRY(cudaHostGetDevicePointer((void**)&s->d_hflags, s->h_flags, 0));
   CU_TRY(cudaFuncSetAttribute(inflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(InflateShared)));
@@ -370,6 +378,22 @@ static int stream_init(BamScanStream* s) {
   if (n_ref) CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_len, f->ref_lens.data(), 4 * n_ref, cudaMemcpyHostToDevice));
   CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_off, offs.data(), 4 * (n_ref + 1), cudaMemcpyHostToDevice));
   if (!blob.empty()) CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
+  if (f->format == 2) {
+    // SAM: names sorted bytewise + their ids (enc::lookup_ref), laid out as [offsets n_ref + 1][ids n_ref][names]
+    std::vector<int32_t> ids(n_ref);
+    std::iota(ids.begin(), ids.end(), 0);
+    std::sort(ids.begin(), ids.end(), [&](int32_t a, int32_t b) { return f->ref_names[a] < f->ref_names[b]; });
+    std::vector<int32_t> soff(n_ref + 1, 0);
+    std::string sblob;
+    for (size_t i = 0; i < n_ref; i++) { soff[i] = (int32_t)sblob.size(); sblob += f->ref_names[ids[i]]; }
+    soff[n_ref] = (int32_t)sblob.size();
+    const size_t o_ids = align_up(4 * (n_ref + 1), 16), o_names = o_ids + align_up(4 * n_ref + 4, 16);
+    rc = s->d_samrefs.ensure(o_names + sblob.size() + 16);
+    if (rc) return rc;
+    CU_TRY(cudaMemcpy(s->d_samrefs.p, soff.data(), 4 * (n_ref + 1), cudaMemcpyHostToDevice));
+    if (n_ref) CU_TRY(cudaMemcpy(s->d_samrefs.as<uint8_t>() + o_ids, ids.data(), 4 * n_ref, cudaMemcpyHostToDevice));
+    if (!sblob.empty()) CU_TRY(cudaMemcpy(s->d_samrefs.as<uint8_t>() + o_names, sblob.data(), sblob.size(), cudaMemcpyHostToDevice));
+  }
   s->resources_ready = true;
   }
   // unique decode columns
@@ -408,7 +432,8 @@ static void stream_destroy(BamScanStream* s, bool recycle = true) {
     if (s->handle->idle_streams.size() < 2) { s->handle->idle_streams.push_back(s); return; }
   }
   for (auto* b : {&s->d_comp[0], &s->d_comp[1], &s->d_blk[0], &s->d_blk[1], &s->d_infl[0], &s->d_infl[1], &s->d_carry, &s->d_status[0], &s->d_status[1], &s->d_flags[0], &s->d_flags[1], &s->d_seg[0], &s->d_seg[1],
-                  &s->d_recoff[0], &s->d_recoff[1], &s->d_recoff2[0], &s->d_recoff2[1], &s->d_keep[0], &s->d_keep[1], &s->d_tiles, &s->d_totals, &s->d_scratch, &s->d_arena[0], &s->d_arena[1], &s->d_refs, &s->d_comp_all_buf, &s->d_sorted}) b->release();
+                  &s->d_recoff[0], &s->d_recoff[1], &s->d_recoff2[0], &s->d_recoff2[1], &s->d_keep[0], &s->d_keep[1], &s->d_tiles, &s->d_totals, &s->d_scratch, &s->d_arena[0], &s->d_arena[1], &s->d_refs, &s->d_comp_all_buf, &s->d_sorted,
+                  &s->d_samline[0], &s->d_samline[1], &s->d_samsize[0], &s->d_samsize[1], &s->d_qabs[0], &s->d_qabs[1], &s->d_samtiles[0], &s->d_samtiles[1], &s->d_bam[0], &s->d_bam[1], &s->d_samrefs}) b->release();
   if (s->h_flags) cudaFreeHost(s->h_flags);
   for (auto& hd : s->h_descs) if (hd) cudaFreeHost(hd);
   for (auto& hs : s->h_stage) if (hs) cudaFreeHost(hs);
@@ -419,6 +444,8 @@ static void stream_destroy(BamScanStream* s, bool recycle = true) {
   if (s->ev_carry) cudaEventDestroy(s->ev_carry);
   for (auto& row : s->ev_t) for (auto& e : row) if (e) cudaEventDestroy(e);
   for (auto& e : s->ev_dt) if (e) cudaEventDestroy(e);
+  for (auto& e : s->ev_text_free) if (e) cudaEventDestroy(e);
+  for (auto& row : s->ev_ing) for (auto& e : row) if (e) cudaEventDestroy(e);
   for (auto st : s->s_chunk) if (st) cudaStreamDestroy(st);
   if (s->s_h2d) cudaStreamDestroy(s->s_h2d);
   if (s->s_d2h) cudaStreamDestroy(s->s_d2h);
@@ -435,6 +462,7 @@ static uint32_t inflate_wave_members(int device) { return (uint32_t)device_sms(d
 static const uint64_t SLICE_BYTES = 768ull << 20;
 static uint64_t chunk_cap_bytes(const BamFile& f) {
   if (f.chunk_bytes) return f.chunk_bytes;
+  if (f.format == 2) return 512ull << 20;          // SAM: text bytes per chunk (no inflate wave to fill)
   return std::min<uint64_t>((uint64_t)inflate_wave_members(f.device) * 65280ull + 65536ull, 3ull << 30);
 }
 static void plan_chunks(const BamFile& f, uint32_t b0, uint32_t b1, bool extension, std::vector<ChunkPlan>* out) {
@@ -476,12 +504,45 @@ static int check_empty_member(const BamFile* f, uint32_t b) {
   return BAMSCAN_ERR_CRC;
 }
 
+// page cache -> the slot's pinned staging buffer (its previous transfer has long finished)
+static int stage_bytes(BamScanStream* s, uint64_t c0, size_t bytes, int slot) {
+  CU_TRY(cudaEventSynchronize(s->ev_h2d[slot]));
+  if (s->h_stage_cap[slot] < bytes) {
+    if (s->h_stage[slot]) cudaFreeHost(s->h_stage[slot]);
+    const size_t cap = bytes + bytes / 8 + 4096;
+    s->h_stage[slot] = (uint8_t*)pinned_alloc(cap);
+    if (!s->h_stage[slot]) { s->h_stage_cap[slot] = 0; return BAMSCAN_ERR_CUDA; }
+    s->h_stage_cap[slot] = cap;
+  }
+  parallel_copy(s->h_stage[slot], s->f->data + c0, bytes);
+  return BAMSCAN_OK;
+}
+
+// SAM: the chunk's text goes straight into its buffer behind the carry headroom with one copy (H2D from the staging ring, or
+// device to device from the staged partition of a device-resident run).  No descriptors, no inflate.
+static int issue_h2d_text(BamScanStream* s, const ChunkPlan& c, int slot) {
+  const size_t bytes = (size_t)(c.c1 - c.c0);
+  int rc;
+  s->n_descs[slot] = 0; s->chunk_data_hi[slot] = HEADROOM + (uint32_t)bytes;
+  if ((rc = s->d_infl[slot].ensure((size_t)HEADROOM + bytes + INFL_PAD))) return rc;
+  uint8_t* dst = s->d_infl[slot].as<uint8_t>() + HEADROOM;
+  CU_TRY(cudaStreamWaitEvent(s->s_h2d, s->ev_text_free[slot], 0));     // the write pass of the chunk two back has read this buffer
+  if (!s->device_resident && (rc = stage_bytes(s, c.c0, bytes, slot))) return rc;
+  CU_TRY(cudaEventRecord(s->ev_ing[slot][0], s->s_h2d));
+  if (s->device_resident) CU_TRY(cudaMemcpyAsync(dst, s->d_comp_all + (c.c0 - s->comp_all_c0), bytes, cudaMemcpyDeviceToDevice, s->s_h2d));
+  else { CU_TRY(cudaMemcpyAsync(dst, s->h_stage[slot], bytes, cudaMemcpyHostToDevice, s->s_h2d)); s->st.h2d_bytes += bytes; }
+  CU_TRY(cudaEventRecord(s->ev_ing[slot][1], s->s_h2d));
+  CU_TRY(cudaEventRecord(s->ev_h2d[slot], s->s_h2d));
+  return BAMSCAN_OK;
+}
+
 // Builds the chunk's member descriptors in pinned memory and queues them, with the compressed bytes, on the H2D stream.
 // Everything the compute stream needs from the host for this chunk travels here, so the copy engine never makes the
 // kernels of the previous chunk wait (a pageable copy issued on the compute stream would queue behind the big transfer).
 static int issue_h2d(BamScanStream* s, const ChunkPlan& c, int slot) {
   NvtxRange nv("bamscan: stage + H2D of a chunk's compressed members");
   const BamFile* f = s->f;
+  if (f->format == 2) return issue_h2d_text(s, c, slot);
   const uint32_t nb_all = c.b1 - c.b0;
   if (s->h_descs_cap[slot] < nb_all) {
     if (s->h_descs[slot]) cudaFreeHost(s->h_descs[slot]);
@@ -505,16 +566,8 @@ static int issue_h2d(BamScanStream* s, const ChunkPlan& c, int slot) {
   if (!s->device_resident) {
     size_t bytes = (size_t)(c.c1 - c.c0);
     if ((rc = s->d_comp[slot].ensure(bytes + 1024))) return rc;
-    // page cache -> pinned staging buffer of this slot (its previous transfer has long finished) -> one async copy
-    CU_TRY(cudaEventSynchronize(s->ev_h2d[slot]));
-    if (s->h_stage_cap[slot] < bytes) {
-      if (s->h_stage[slot]) cudaFreeHost(s->h_stage[slot]);
-      const size_t cap = bytes + bytes / 8 + 4096;
-      s->h_stage[slot] = (uint8_t*)pinned_alloc(cap);
-      if (!s->h_stage[slot]) { s->h_stage_cap[slot] = 0; return BAMSCAN_ERR_CUDA; }
-      s->h_stage_cap[slot] = cap;
-    }
-    parallel_copy(s->h_stage[slot], s->f->data + c.c0, bytes);
+    // page cache -> pinned staging buffer of this slot -> one async copy
+    if ((rc = stage_bytes(s, c.c0, bytes, slot))) return rc;
     CU_TRY(cudaMemcpyAsync(s->d_comp[slot].p, s->h_stage[slot], bytes, cudaMemcpyHostToDevice, s->s_h2d));
     CU_TRY(cudaMemsetAsync(s->d_comp[slot].as<uint8_t>() + bytes, 0, 1024, s->s_h2d));   // the bit reader may look a few words past the last member
     s->st.h2d_bytes += bytes;
@@ -549,6 +602,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
   const uint8_t* U = s->cur.U;
   const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
   const uint32_t* d_recoff = s->cur.recoff + (size_t)s->cur.pos * (f->format == 1 ? 4 : 1);
+  const uint8_t* d_qabs = s->cur.qabs ? s->cur.qabs + s->cur.pos : nullptr;
   s->cur.pos += n;
   CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
   {
@@ -579,6 +633,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
     memset(&DP, 0, sizeof DP);
     DP.U = U; DP.rec_off = d_recoff; DP.n = n; DP.zero_based = f->zero_based; DP.binary_cigar = f->binary_cigar;
     DP.n_ref = (int32_t)f->ref_names.size();
+    DP.end_zero_span = f->format == 2; DP.qual_absent = d_qabs;
     size_t n_ref = f->ref_names.size();
     DP.ref_name_off = reinterpret_cast<const uint32_t*>(s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16));
     DP.ref_names = s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16) + align_up(4 * (n_ref + 1), 16);
@@ -748,6 +803,64 @@ static int decode_slice(BamScanStream* s, bool* produced) {
   return BAMSCAN_OK;
 }
 
+static int sam_error_to_rc(uint32_t code, unsigned long long rec) {
+  static const char* what[] = {"?", "fewer than 11 fields", "invalid QNAME (1-254 of [!-?A-~])", "invalid FLAG (not an integer in 0..65535)",
+                               "RNAME is not a reference sequence of the header", "invalid POS (not an integer in 0..2^31)",
+                               "invalid MAPQ (not an integer in 0..255)", "invalid CIGAR", "CIGAR with more than 65535 operations is not supported",
+                               "RNEXT is not a reference sequence of the header", "invalid PNEXT (not an integer in 0..2^31)",
+                               "invalid TLEN (not an i32)", "invalid SEQ (not * or [A-Za-z=.]+)", "invalid QUAL (not * or [!-~]+)",
+                               "QUAL length differs from SEQ length", "malformed aux field", "duplicate aux tag", "aux value out of range for its type"};
+  set_error("SAM read error: record %llu of the partition (0-based): %s", rec, code < sizeof what / sizeof *what ? what[code] : "?");
+  return code == sam::SAM_ERR_CIGAR_OPS ? BAMSCAN_ERR_UNSUPPORTED : BAMSCAN_ERR_FORMAT;
+}
+
+// SAM: the chunk's n complete owned lines -> BAM records in the slot's own buffer (kernels_sam.cuh).  One host sync: the first
+// error and the total record bytes (the buffer's size).  *bam / *recoff: the records and their offsets, for the decode stage.
+static int transcode_sam(BamScanStream* s, int slot, cudaStream_t cs, const uint8_t* U, const uint32_t* lines, uint32_t n,
+                         const uint8_t** bam, const uint32_t** recoff) {
+  NvtxRange nv("bamscan: SAM lines -> BAM records");
+  const BamFile* f = s->f;
+  int rc;
+  if ((rc = s->d_samline[slot].ensure(sizeof(sam::SamLine) * (size_t)n)) || (rc = s->d_samsize[slot].ensure(4ull * (n + 1) + 64)) ||
+      (rc = s->d_qabs[slot].ensure((size_t)n + 64))) return rc;
+  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
+  uint32_t* d_err = d_flags + 24;                  // [24] first error, [25] its line, [26..27] total record bytes (u64): device only
+  CU_TRY(cudaMemsetAsync(d_err, 0, 16, cs));
+  const size_t n_ref = f->ref_names.size();
+  const uint8_t* R = s->d_samrefs.as<uint8_t>();
+  const size_t o_ids = align_up(4 * (n_ref + 1), 16), o_names = o_ids + align_up(4 * n_ref + 4, 16);
+  sam::SamSizeArgs A;
+  A.U = U; A.lines = lines; A.n = n;
+  A.R = sam::SamRefs{R + o_names, reinterpret_cast<const int32_t*>(R), reinterpret_cast<const int32_t*>(R + o_ids), (int32_t)n_ref};
+  A.out = s->d_samline[slot].as<sam::SamLine>(); A.sizes = s->d_samsize[slot].as<uint32_t>(); A.qual_absent = s->d_qabs[slot].as<uint8_t>(); A.err = d_err;
+  sam::sam_size_kernel<<<(n + 255) / 256, 256, 0, cs>>>(A);
+  ScanCols SC; memset(&SC, 0, sizeof SC);
+  SC.col[0] = reinterpret_cast<int32_t*>(A.sizes); SC.n_cols = 1; SC.n = n + 1;
+  const uint32_t n_tiles = (SC.n + SCAN_TILE - 1) / SCAN_TILE;
+  if ((rc = s->d_samtiles[slot].ensure(8ull * n_tiles))) return rc;
+  multi_scan_reduce_kernel<<<dim3(n_tiles, 1), SCAN_TPB, 0, cs>>>(SC, s->d_samtiles[slot].as<uint64_t>(), n_tiles);
+  multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_samtiles[slot].as<uint64_t>(), n_tiles, reinterpret_cast<uint64_t*>(d_flags + 26));
+  multi_scan_apply_kernel<<<dim3(n_tiles, 1), SCAN_TPB, 0, cs>>>(SC, s->d_samtiles[slot].as<uint64_t>(), n_tiles);
+  publish_kernel<<<1, 32, 0, cs>>>(d_err, s->d_hflags + 600, 4);     // [600, 604) of the mapped page: nothing else uses it
+  s->st.kernel_launches += 5;
+  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+  CU_TRY(cudaEventSynchronize(s->ev_flags[slot]));
+  CU_TRY(cudaGetLastError());
+  const uint32_t* hf = s->h_flags + 600;
+  if (hf[0]) return sam_error_to_rc(hf[0], (unsigned long long)s->st.rows + hf[1]);
+  const uint64_t total = (uint64_t)hf[2] | ((uint64_t)hf[3] << 32);
+  if (total > 0xffffffffull) { set_error("SAM chunk transcodes to more than 4 GiB of BAM records; lower chunk_inflated_bytes"); return BAMSCAN_ERR_UNSUPPORTED; }
+  if ((rc = s->d_bam[slot].ensure((size_t)total + 64))) return rc;
+  sam::SamWriteArgs W{U, A.out, A.sizes, n, s->d_bam[slot].as<uint8_t>()};
+  // a group of 8 lanes per line (4 lines per warp); 32 when the previous chunk's lines averaged above 2 KiB, as in decode and encode
+  if ((f->debug_flags & 2) || s->mean_record_bytes > 2048) sam::sam_records_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(W);
+  else sam::sam_records_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(W);
+  s->st.kernel_launches++;
+  CU_TRY(cudaEventRecord(s->ev_text_free[slot], cs));
+  *bam = s->d_bam[slot].as<uint8_t>(); *recoff = A.sizes;
+  return BAMSCAN_OK;
+}
+
 // Runs one chunk.  On success *produced tells whether a batch went into s->pending (previous pending must have been consumed).
 // phase 1 queues H2D wait + inflate + record boundaries and returns without waiting (the host can then wait for an older
 // batch's D2H while the GPU works); phase 2 picks the chunk up from there; phase 0 does both.
@@ -839,6 +952,23 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
     CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
     if (phase == 1) return BAMSCAN_OK;
+  } else if (f->format == 2) {
+    // SAM: line starts of the chunk (the FASTQ newline scan), one record per line (kernels_sam.cuh)
+    const uint32_t lo = BP.data_lo, span = data_hi - lo;
+    const uint32_t n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
+    if ((rc = s->d_seg[slot].ensure(8ull * n_tiles + 64))) return rc;
+    uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>(); uint32_t* d_tile_base = d_tile_count + n_tiles;
+    const uint32_t line_cap = span / 8 + 4096;                                          // a SAM record has 11 fields: lines average far more than 8 bytes
+    if ((rc = s->d_recoff[slot].ensure(4ull * line_cap))) return rc;
+    fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
+    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + 16);
+    fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
+    FastqFrame FF{U, lo, data_hi, BP.own_hi, 0u, (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap};
+    sam::sam_frame_kernel<<<1, 32, 0, cs>>>(FF, BP.first_start, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
+    s->st.kernel_launches += 4;
+    publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+    CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+    if (phase == 1) return BAMSCAN_OK;
   } else {
   WalkOut W{d_seg_start, d_seg_exit, d_seg_count, d_seg_tail, d_flags};
   seg_candidates_kernel<<<(n_seg * 32 + 255) / 256, 256, 0, cs>>>(BP, d_seg_start, (f->debug_flags & 1) ? 1 : 0);
@@ -876,6 +1006,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     return BAMSCAN_ERR_CRC;
   }
   if (hf[1] && f->format == 1) { set_error("FASTQ read error: more lines in one chunk than supported (lines shorter than 8 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
+  if (hf[1] && f->format == 2) { set_error("SAM read error: lines shorter than 8 bytes on average (a SAM record has 11 fields)"); return BAMSCAN_ERR_FORMAT; }
   if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - HEADROOM))); return BAMSCAN_ERR_FORMAT; }
   s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10]; s->st.inflate_retries += hf[15];
   const uint32_t n_rec = hf[3];
@@ -885,8 +1016,14 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   if (tail_off > data_hi) tail_off = data_hi;
   *owned_done = tail_off >= BP.own_hi;
   *new_carry = *owned_done ? 0 : data_hi - tail_off;
-  if (*new_carry > HEADROOM) { set_error("BAM record larger than %u bytes is not supported", HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; }
+  if (*new_carry > HEADROOM) { set_error("%s larger than %u bytes is not supported", f->format == 2 ? "SAM line" : "BAM record", HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; }
   if (*new_carry) { CU_TRY(cudaMemcpyAsync(s->d_carry.p, U + tail_off, *new_carry, cudaMemcpyDeviceToDevice, cs)); CU_TRY(cudaEventRecord(s->ev_carry, cs)); }
+  const uint8_t* U_rows = U;               // the bytes the decode stage reads: the inflated chunk, or the SAM chunk's BAM records
+  const uint32_t* sam_recoff = nullptr;
+  if (f->format == 2 && n_rec > 0) {
+    if ((rc = transcode_sam(s, slot, cs, U, s->d_recoff[slot].as<uint32_t>() + hf[14], n_rec, &U_rows, &sam_recoff))) return rc;
+    s->cur.qabs = s->d_qabs[slot].as<uint8_t>();
+  } else s->cur.qabs = nullptr;
   s->st.chunks++; s->st.blocks += nb; s->st.inflated_bytes += c.ubytes; s->st.compressed_bytes += c.c1 - c.c0;
   // seam evidence of block-range partitions (BamScanStats): where the first owned record starts, where the chain lands
   if (n_rec > 0 && s->st.first_record_uoff == ~0ull && hf[13] != 0xffffffffu && hf[13] >= HEADROOM) s->st.first_record_uoff = c.u0 + (hf[13] - HEADROOM);
@@ -897,6 +1034,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     // ---- record offsets
     uint32_t* d_recoff;
     if (f->format == 1) d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14];       // lines[] from the first record's line on: 4 per row
+    else if (f->format == 2) d_recoff = const_cast<uint32_t*>(sam_recoff);
     else {
       if ((rc = s->d_recoff[slot].ensure(4ull * (n_rec + 1)))) return rc;
       d_recoff = s->d_recoff[slot].as<uint32_t>();
@@ -937,7 +1075,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     }
     // ---- hand the rows to decode_slice(): one batch per slice of <= SLICE_BYTES inflated
     const uint32_t n_slices = (uint32_t)std::max<uint64_t>(1, (c.ubytes + SLICE_BYTES - 1) / SLICE_BYTES);
-    s->cur.U = U; s->cur.recoff = d_recoff; s->cur.n = n; s->cur.pos = 0; s->cur.cs = cs;
+    s->cur.U = U_rows; s->cur.recoff = d_recoff; s->cur.n = n; s->cur.pos = 0; s->cur.cs = cs;
     s->cur.rows_per_slice = (n + n_slices - 1) / n_slices;
     s->mean_record_bytes = (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)(data_hi - HEADROOM) / std::max<uint32_t>(n_rec, 1));
     s->cur.long_records = (f->debug_flags & 2) || s->mean_record_bytes > 2048;
@@ -950,6 +1088,7 @@ timing:
   {
     float a = 0, b = 0, d = 0;
     cudaEventElapsedTime(&a, s->ev_t[slot][0], s->ev_t[slot][1]);
+    if (f->format == 2) cudaEventElapsedTime(&a, s->ev_ing[slot][0], s->ev_ing[slot][1]);     // SAM: the ingest copy
     cudaEventElapsedTime(&b, s->ev_t[slot][1], s->ev_t[slot][2]);
     cudaEventElapsedTime(&d, s->ev_t[slot][2], s->ev_t[slot][3]);
     s->st.ms_inflate += a; s->st.ms_boundary += b; s->st.ms_decode += d;
@@ -1015,7 +1154,7 @@ static int advance(BamScanStream* s, bool* produced) {
       uint32_t last = s->chunks.back().b1;
       if (s->carry_len == 0 || last >= f->blocks.size()) {
         if (s->carry_len) {
-          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", f->format == 1 ? "FASTQ" : "BAM", s->carry_len);
+          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", f->format == 1 ? "FASTQ" : f->format == 2 ? "SAM" : "BAM", s->carry_len);
           return BAMSCAN_ERR_FORMAT;
         }
         s->range_open = false; s->range_idx++;
@@ -1170,6 +1309,7 @@ int bamscan_open(const char* path, const char* index_path_or_null, const BamScan
 
 static int bamscan_open_impl(const char* path, const char* index_path_or_null, const BamScanOptions* options, BamScanHandle** out, int format) {
   if (!path || !out) { set_error("bamscan_open: null argument"); return BAMSCAN_ERR_INVALID; }
+  if (format == 0 && is_sam_path(path)) format = 2;
   BamScanOptions opt;
   memset(&opt, 0, sizeof opt);
   opt.coordinate_system_zero_based = 1; opt.infer_tag_types = 1; opt.infer_tag_sample_size = 100;
@@ -1192,7 +1332,7 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
   if (opt.segment_bytes) { f.seg_bytes = std::max<uint32_t>(256, opt.segment_bytes); f.seg_bytes_set = true; }
   f.skip_crc = opt.skip_crc != 0; f.debug_flags = opt.debug_flags; f.decode_all_tags = opt.decode_all_tag_fields != 0;
   int rc = load_file(&f);
-  if (rc == BAMSCAN_ERR_IO || rc == BAMSCAN_ERR_CUDA) { release_file(&f); return rc; }
+  if (rc == BAMSCAN_ERR_IO || rc == BAMSCAN_ERR_CUDA || (format == 2 && rc)) { release_file(&f); return rc; }
   // a file whose header cannot be read still yields a provider with empty metadata (table_provider.rs:423-426);
   // scans on it fail later
   if (format == 1) {
@@ -1203,6 +1343,7 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
     return BAMSCAN_OK;
   }
   if ((rc = build_schema(&f, &opt))) { release_file(&f); return rc; }
+  if (format == 2) { *out = h.release(); return BAMSCAN_OK; }     // SAM: no index (the reference discovers none for SAM paths)
   if (index_path_or_null) f.index_path = index_path_or_null; else f.index_path = discover_index(f.path);   // "" = no index
   if (!f.index_path.empty()) {
     f.bai.reset(new BaiIndex());
@@ -1231,7 +1372,7 @@ int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out) {
 
 static int bamscan_describe_tags_impl(BamScanHandle* h, int32_t sample_size, char* buf, uint64_t cap, uint64_t* needed) {
   if (!h || !needed || (cap && !buf)) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format != 0) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
+  if (h->file.format == 1) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
   if (!h->file.header_ok) { set_error("BAM header could not be read: %s", h->file.path.c_str()); return BAMSCAN_ERR_FORMAT; }
   std::map<std::string, std::pair<char, int32_t>> found;
   infer_tag_types(h->file, {}, sample_size > 0 ? sample_size : 100, &found, true);
@@ -1513,6 +1654,7 @@ int bamscan_bench_inflate(BamScanPlan* plan, int32_t partition, int32_t repeats,
   int rc = make_stream(plan, partition, true, &s);
   if (rc) return rc;
   BamFile* f = s->f;
+  if (f->format == 2) { stream_destroy(s); set_error("a SAM scan has no inflate to benchmark"); return BAMSCAN_ERR_INVALID; }
   if (s->part->ranges.empty()) { stream_destroy(s); set_error("empty partition"); return BAMSCAN_ERR_INVALID; }
   const ScanRange& r = s->part->ranges[0];
   std::vector<ChunkPlan> chunks;

@@ -10,11 +10,13 @@
 // done once per open, exactly where the reference does it (BamTableProvider::new), not the scan path.
 #include <zlib.h>
 
+#include <cctype>
 #include <cstdio>
 #include <cstring>
 #include <sys/stat.h>
 
 #include "bamscan_internal.h"
+#include "f32_parse.h"
 
 namespace bamscan {
 
@@ -87,6 +89,175 @@ static int walk_blocks(BamFile* f) {
   return BAMSCAN_OK;
 }
 
+// ---- plain SAM (format 2) ----
+// The text body is described as pseudo-blocks with csize == isize and coff == uoff == the file offset, so that planning, chunking
+// and the seam evidence of block-range partitions work on it unchanged.
+constexpr uint32_t SAM_BLOCK = 65536;
+
+// @SQ SN / LN -> the reference dictionary (the header's order).  false: the header does not parse (an @SQ line without SN or a
+// positive LN that fits an i32, or a name given twice).
+static bool sam_header_refs(BamFile* f) {
+  size_t pos = 0;
+  const std::string& t = f->text;
+  while (pos < t.size()) {
+    size_t nl = t.find('\n', pos);
+    std::string line = t.substr(pos, nl == std::string::npos ? std::string::npos : nl - pos);
+    pos = nl == std::string::npos ? t.size() : nl + 1;
+    if (!line.empty() && line.back() == '\r') line.pop_back();
+    if (line.compare(0, 4, "@SQ\t") != 0) continue;
+    std::string sn; long long ln = -1; bool has_sn = false;
+    size_t s = 3;
+    while (s != std::string::npos && s < line.size()) {
+      size_t e = line.find('\t', s + 1);
+      std::string tok = line.substr(s + 1, e == std::string::npos ? std::string::npos : e - s - 1);
+      if (tok.compare(0, 3, "SN:") == 0) { sn = tok.substr(3); has_sn = true; }
+      else if (tok.compare(0, 3, "LN:") == 0) {
+        const std::string v = tok.substr(3);
+        ln = -1;
+        if (!v.empty() && v.size() <= 10 && v.find_first_not_of("0123456789") == std::string::npos) ln = std::stoll(v);
+      }
+      s = e;
+    }
+    if (!has_sn || sn.empty() || ln < 1 || ln > 2147483647ll) return false;
+    for (const auto& n : f->ref_names) if (n == sn) return false;
+    f->ref_names.push_back(sn); f->ref_lens.push_back((int32_t)ln);
+  }
+  return true;
+}
+
+int load_sam(BamFile* f) {
+  const uint8_t* d = f->data;
+  const uint64_t n = f->size;
+  if (n >= 2 && d[0] == 0x1f && d[1] == 0x8b) {
+    set_error("%s: gzip / BGZF-compressed SAM is not supported (decompress it, or convert it to BAM)", f->path.c_str());
+    return BAMSCAN_ERR_UNSUPPORTED;
+  }
+  // header: the leading lines that start with '@'
+  uint64_t p = 0;
+  while (p < n && d[p] == '@') { const void* nl = memchr(d + p, '\n', (size_t)(n - p)); p = nl ? (uint64_t)((const uint8_t*)nl - d) + 1 : n; }
+  f->text.assign((const char*)d, (size_t)p);
+  f->first_record_uoff = p;
+  for (uint64_t o = p; o < n; o += SAM_BLOCK) {
+    BgzfBlock b;
+    b.coff = b.uoff = o; b.csize = b.isize = (uint32_t)std::min<uint64_t>(SAM_BLOCK, n - o); b.cdata_off = 0; b.crc = 0;
+    f->blocks.push_back(b);
+  }
+  f->total_inflated = n;
+  // a header that does not parse gives empty metadata and no references, not an error (as for a BAM, table_provider.rs:423-426)
+  f->header_ok = sam_header_refs(f);
+  if (!f->header_ok) { f->ref_names.clear(); f->ref_lens.clear(); }
+  return BAMSCAN_OK;
+}
+
+// BamTableProvider's `is_sam`: a path ending in ".sam", any case (the rule the Python writer uses for its refusal too)
+bool is_sam_path(const std::string& path) {
+  const size_t n = path.size();
+  return n >= 4 && path[n - 4] == '.' && (path[n - 3] | 0x20) == 's' && (path[n - 2] | 0x20) == 'a' && (path[n - 1] | 0x20) == 'm';
+}
+
+uint64_t sam_record_start_at(const BamFile& f, uint64_t off) {
+  if (off <= f.first_record_uoff) return f.first_record_uoff;
+  if (off >= f.size) return f.size;
+  if (f.data[off - 1] == '\n') return off;
+  const void* nl = memchr(f.data + off, '\n', (size_t)(f.size - off));
+  return nl ? (uint64_t)((const uint8_t*)nl - f.data) + 1 : f.size;
+}
+
+// [+-]digits (signed) or [+]digits -> *x, saturated far outside every SAM range; false when not an integer
+static bool sam_int(const char* s, size_t n, bool allow_neg, long long* x) {
+  size_t k = 0; bool neg = false;
+  if (k < n && (s[k] == '+' || (allow_neg && s[k] == '-'))) { neg = s[k] == '-'; k++; }
+  if (k >= n) return false;
+  long long v = 0;
+  for (; k < n; k++) { if (s[k] < '0' || s[k] > '9') return false; if (v < (1ll << 40)) v = v * 10 + (s[k] - '0'); }
+  *x = neg ? -v : v;
+  return true;
+}
+
+// The BAM type of one SAM aux field "TG:T:value", as the BAM walk below would report it for the record the transcoder writes:
+// an `i` value takes the narrowest type (C / S / I when non-negative, c / s / i when negative), so the value decides between
+// Int32 (C, S, c, s, i) and UInt32 (I).  The field is checked by the rules of the device size pass (kernels_sam.cuh::aux_bytes);
+// false: the field is malformed (the walk stops there, as the BAM walk does; the scan refuses the line).
+static bool sam_aux_type(const char* s, size_t n, std::pair<char, int32_t>* v) {
+  auto alpha = [](char c) { return (c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z'); };
+  if (n < 5 || s[2] != ':' || s[4] != ':' || !alpha(s[0]) || !(alpha(s[1]) || (s[1] >= '0' && s[1] <= '9'))) return false;
+  const char* val = s + 5;
+  const size_t vn = n - 5;
+  switch (s[3]) {
+    case 'A': *v = {'A', HK_Utf8}; return vn == 1 && val[0] >= '!' && val[0] <= '~';
+    case 'i': {
+      long long x;
+      if (!sam_int(val, vn, true, &x) || x < -2147483648ll || x > 4294967295ll) return false;
+      *v = x > 65535 ? std::make_pair('I', (int32_t)HK_UInt32) : std::make_pair('i', (int32_t)HK_Int32);
+      return true;
+    }
+    case 'f': { uint32_t b; *v = {'f', HK_Float32}; return f32_parse(val, (uint32_t)vn, &b); }
+    case 'Z':
+      for (size_t k = 0; k < vn; k++) if (val[k] < ' ' || val[k] > '~') return false;
+      *v = {'Z', HK_Utf8}; return true;
+    case 'H':
+      if (vn & 1) return false;
+      for (size_t k = 0; k < vn; k++) if (!isxdigit((unsigned char)val[k])) return false;
+      *v = {'H', HK_Utf8}; return true;
+    case 'B': {
+      if (vn < 1) return false;
+      const char st = val[0];
+      int32_t kind; long long lo = 0, hi = 0;
+      switch (st) { case 'c': kind = HK_ListInt8; lo = -128; hi = 127; break; case 'C': kind = HK_ListUInt8; hi = 255; break;
+                    case 's': kind = HK_ListInt16; lo = -32768; hi = 32767; break; case 'S': kind = HK_ListUInt16; hi = 65535; break;
+                    case 'i': kind = HK_ListInt32; lo = -2147483648ll; hi = 2147483647ll; break; case 'I': kind = HK_ListUInt32; hi = 4294967295ll; break;
+                    case 'f': kind = HK_ListFloat32; break; default: return false; }
+      for (size_t k = 1; k < vn;) {
+        if (val[k] != ',') return false;
+        size_t j = k + 1;
+        while (j < vn && val[j] != ',') j++;
+        if (st == 'f') { uint32_t b; if (!f32_parse(val + k + 1, (uint32_t)(j - k - 1), &b)) return false; }
+        else { long long x; if (!sam_int(val + k + 1, j - k - 1, true, &x) || x < lo || x > hi) return false; }
+        k = j;
+      }
+      *v = {'B', kind};
+      return true;
+    }
+  }
+  return false;
+}
+
+// infer_tag_types on a SAM: the aux fields of the first sample_size lines of the body
+static int infer_tag_types_sam(const BamFile& f, const std::vector<std::string>& tags, int sample_size,
+                               std::map<std::string, std::pair<char, int32_t>>* out, bool all) {
+  uint64_t p = f.first_record_uoff;
+  for (int count = 0; count < sample_size && p < f.size; count++) {
+    const uint8_t* nl = (const uint8_t*)memchr(f.data + p, '\n', (size_t)(f.size - p));
+    uint64_t e = nl ? (uint64_t)(nl - f.data) : f.size;
+    const uint64_t next = nl ? e + 1 : f.size;
+    if (e > p && f.data[e - 1] == '\r') e--;
+    const char* line = (const char*)f.data + p;
+    const size_t n = (size_t)(e - p);
+    p = next;
+    size_t k = 0;
+    int tabs = 0;
+    while (k < n && tabs < 11) { if (line[k] == '\t') tabs++; k++; }
+    if (tabs < 11) continue;
+    std::map<std::string, std::pair<char, int32_t>> seen;
+    while (k < n) {
+      size_t j = k;
+      while (j < n && line[j] != '\t') j++;
+      std::pair<char, int32_t> v;
+      if (!sam_aux_type(line + k, j - k, &v)) break;
+      std::string tag(line + k, 2);
+      if (!seen.count(tag)) seen[tag] = v;
+      if (all && !out->count(tag)) (*out)[tag] = v;
+      k = j + 1;
+    }
+    for (const auto& t : tags) {
+      if (out->count(t) || t.size() != 2) continue;
+      auto it = seen.find(t);
+      if (it != seen.end()) (*out)[t] = it->second;
+    }
+  }
+  return BAMSCAN_OK;
+}
+
 void release_file(BamFile* f) {
   if (!f->data) return;
   if (f->mapped) unmap_file_pinned(f->data, f->size, f->registered); else pinned_free(f->data);
@@ -118,6 +289,7 @@ int load_file(BamFile* f) {
     memset(f->data + f->size, 0, 4096);
   }
   fclose(fp);
+  if (f->format == 2) return load_sam(f);
   int rc = walk_blocks(f);
   if (rc) return rc;
   if (f->format == 1) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ: records start at inflated offset 0
@@ -150,6 +322,7 @@ int load_file(BamFile* f) {
 // `all` (BamTableProvider::describe, table_provider.rs:715-745): every tag met in the sample, first occurrence wins.
 int infer_tag_types(const BamFile& f, const std::vector<std::string>& tags, int sample_size,
                     std::map<std::string, std::pair<char, int32_t>>* out, bool all) {
+  if (f.format == 2) return infer_tag_types_sam(f, tags, sample_size, out, all);
   HostStream hs(f);
   // position on the first record
   while (hs.base_uoff + hs.buf.size() <= f.first_record_uoff) if (!hs.fill()) return BAMSCAN_OK;

@@ -103,7 +103,16 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
       r.exact_start = (p == 0);
       r.first_uoff = (p == 0) ? f->first_record_uoff : (b < n_blocks ? f->blocks[b].uoff : f->total_inflated);
       r.stop_uoff = e < n_blocks ? f->blocks[e].uoff : ~0ull;
-      if (b < e) part.ranges.push_back(r);
+      bool owns = b < e;
+      if (f->format == 2 && owns) {
+        // SAM: a record is a line; the host sees whether the byte in front of the range is '\n', so every range starts exactly
+        // on its first owned line (one that begins in front of the range's end), in the block that holds it
+        r.exact_start = true;
+        r.first_uoff = sam_record_start_at(*f, r.first_uoff);
+        owns = r.first_uoff < std::min<uint64_t>(r.stop_uoff, f->size);
+        if (owns) r.block_begin = block_of_uoff(*f, r.first_uoff);
+      }
+      if (owns) part.ranges.push_back(r);
       part.estimated_bytes = (e > b && b < n_blocks) ? ((e < n_blocks ? f->blocks[e].coff : f->size) - f->blocks[b].coff) : 0;
       plan->partitions.push_back(part);
       b = e;

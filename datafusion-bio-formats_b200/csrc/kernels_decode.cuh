@@ -63,6 +63,11 @@ struct DecodeParams {
   int32_t *l_name, *l_chrom, *l_cigar, *l_mchrom, *l_seq, *l_qual;
   uint8_t *d_name, *d_chrom, *d_cigar, *d_mchrom, *d_seq, *d_qual;
   uint32_t* err;                  // [0] code, [1] row
+  // SAM handles only (kernels_sam.cuh); 0 / null on BAM handles, whose results these leave unchanged.  noodles-sam's RecordBuf
+  // differs from the lazy BAM record in two places:
+  int32_t end_zero_span;          // 1: a placed read whose CIGAR spans no reference base has end = start + 0 - 1 (1-based), not NULL;
+                                  // NULL again at POS 1, where that is 0 (RecordBuf::alignment_end goes through Position::new)
+  const uint8_t* qual_absent;     // [n]: 1 = QUAL was '*' with a non-empty SEQ: the quality string is empty, not 0xFF fill
   TagPlan tags[MAX_TAGS];
 };
 
@@ -182,7 +187,7 @@ decode_fixed_kernel(const DecodeParams P) {
     }
   }
   const bool has_start = sane && pos >= 0;
-  const bool has_end = has_start && span > 0;         // noodles bam::Record::alignment_end: None when the span is 0
+  const bool has_end = has_start && (span > 0 || (P.end_zero_span && pos > 0));     // noodles bam::Record::alignment_end: None when the span is 0
   const bool has_mstart = sane && npos >= 0;
   if (act) {
     if (P.start) P.start[r] = has_start ? (uint32_t)pos + (P.zero_based ? 0u : 1u) : 0u;
@@ -196,7 +201,7 @@ decode_fixed_kernel(const DecodeParams P) {
     if (P.l_mchrom) P.l_mchrom[r] = (sane && nref >= 0) ? (int32_t)(P.ref_name_off[nref + 1] - P.ref_name_off[nref]) : 0;
     if (P.l_cigar) P.l_cigar[r] = sane ? (int32_t)(P.binary_cigar ? 4u * n_cig : cig_txt) : 0;
     if (P.l_seq) P.l_seq[r] = sane ? l_seq : 0;
-    if (P.l_qual) P.l_qual[r] = sane ? l_seq : 0;
+    if (P.l_qual) P.l_qual[r] = (sane && !(P.qual_absent && P.qual_absent[r])) ? l_seq : 0;
   }
   // validity bitmaps: one 32-bit word per warp (rows are warp aligned)
   uint32_t m;
@@ -286,7 +291,7 @@ decode_fixed_warp_kernel(const DecodeParams P) {
       for (int s2 = 16; s2; s2 >>= 1) { span += __shfl_xor_sync(0xffffffffu, span, s2); cig_txt += __shfl_xor_sync(0xffffffffu, cig_txt, s2); }
       if (__any_sync(0xffffffffu, bad_op) && lane == 0) set_err(P.err, DEC_ERR_CIGAR_OP, r);
     }
-    const bool has_start = sane && pos >= 0, has_end = has_start && span > 0, has_mstart = sane && npos >= 0;
+    const bool has_start = sane && pos >= 0, has_end = has_start && (span > 0 || (P.end_zero_span && pos > 0)), has_mstart = sane && npos >= 0;
     if (lane == 0) {
       if (P.start) P.start[r] = has_start ? (uint32_t)pos + (P.zero_based ? 0u : 1u) : 0u;
       if (P.end) P.end[r] = has_end ? (uint32_t)pos + span : 0u;
@@ -299,7 +304,7 @@ decode_fixed_warp_kernel(const DecodeParams P) {
       if (P.l_mchrom) P.l_mchrom[r] = (sane && nref >= 0) ? (int32_t)(P.ref_name_off[nref + 1] - P.ref_name_off[nref]) : 0;
       if (P.l_cigar) P.l_cigar[r] = sane ? (int32_t)(P.binary_cigar ? 4u * n_cig : cig_txt) : 0;
       if (P.l_seq) P.l_seq[r] = sane ? l_seq : 0;
-      if (P.l_qual) P.l_qual[r] = sane ? l_seq : 0;
+      if (P.l_qual) P.l_qual[r] = (sane && !(P.qual_absent && P.qual_absent[r])) ? l_seq : 0;
     }
     const uint32_t bit = 1u << (r & 31u), word = r >> 5;
     if (lane == 0) {
@@ -614,7 +619,7 @@ decode_var_kernel(const DecodeParams P) {
     const uint32_t c0 = head + (nw << 2);
     if (c0 + (uint32_t)gl < l_seq) { const uint32_t c = c0 + gl; uint16_t two = seq_lut[ps[c >> 1]]; dst[c] = (uint8_t)((c & 1u) ? (two >> 8) : two); }
   }
-  if (P.d_qual && on) {
+  if (P.d_qual && on && !(P.qual_absent && P.qual_absent[r])) {
     uint8_t* dst = P.d_qual + DV_OFF(qual, l_qual);
     if (grp_map4<G>(dst, U + o_qual, l_seq, gl, 0x21212121u)) set_err(P.err, DEC_ERR_QUAL, r);
   }

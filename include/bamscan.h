@@ -104,7 +104,9 @@ typedef struct BamScanStats {
   uint64_t compressed_bytes, inflated_bytes, arrow_bytes;   /* B_comp, B_inflated, B_arrow (SURVEY 8d) */
   uint64_t h2d_bytes, d2h_bytes;
   uint64_t blocks, kernel_launches, boundary_repairs;
-  double ms_total, ms_inflate, ms_boundary, ms_decode;      /* CUDA-event device times */
+  double ms_total, ms_inflate, ms_boundary, ms_decode;      /* CUDA-event device times.  Plain SAM (no inflate): compressed_bytes ==
+                                                             * inflated_bytes == text bytes, ms_inflate is the ingest copy of the
+                                                             * text, ms_boundary the line framing plus the SAM -> BAM transcode */
   uint64_t boundary_seam_mismatches;                        /* seams the parallel check rejected (each triggers the repair walk) */
   /* Block-range partitions: inflated offset of the first record this partition owned (UINT64_MAX: none) and the offset at
    * which its record chain landed at or after its stop offset.  Partition p > 0 SPECULATES its first record; the scan of the
@@ -121,6 +123,9 @@ typedef struct BamScanStats {
 int bamscan_check_partition_seams(const BamScanStats* stats, int32_t n_partitions);
 
 /* == BamTableProvider::new (table_provider.rs:381-529): header read, tag-type inference, schema, index discovery.
+ * A path ending in ".sam" (any case) is read as plain SAM text, as the reference's `is_sam` does: header = the leading '@'
+ * lines (references from @SQ SN / LN), each line transcoded to a BAM record on the device, the same columns; no index is
+ * discovered or read.  A ".sam" file that starts with the gzip magic is refused with BAMSCAN_ERR_UNSUPPORTED.
  * index_path_or_null: NULL => discover `<path>.bai`, `<stem>.bai`, then `<path>.csi` (index_utils.rs:43-76); a BAI or a CSI
  *   (CSIv1, BGZF or plain, any min_shift / depth up to 9 levels) is read -- the reference discovers a CSI but parses it as a BAI;
  * "" => behave as if no index existed (sequential single-partition scans). */

@@ -5,7 +5,10 @@
 // produces), zlib raw deflate at --level (default 6), 28-byte EOF marker; optional .bai.
 //
 //   bamgen --mode short|long --reads N --seed S --out file.bam [--threads T] [--level 6] [--bai]
-//          [--unmapped K] [--flush-header]
+//          [--unmapped K] [--flush-header] [--sam]
+//
+// --sam: the same records (same header text, same reads for the same arguments) as plain SAM text instead of BGZF BAM, in
+// `samtools view -h` layout; `f` values would be printed with 9 significant digits, which reads back as the same f32.
 //
 // short: 150 bp paired-end, coordinate-sorted, 25 GRCh38 contigs, tags NM:C MD:Z AS:C XS:C RG:Z MC:Z MQ:C
 // long : ~10 kb lognormal single-end reads, ~1 CIGAR op / 8 bases, tags NM:i MD:Z MM:Z ML:B:C
@@ -215,6 +218,63 @@ static void gen_long_chunk(uint64_t seed, int64_t c, int64_t i0, int64_t i1, int
   }
 }
 
+// One BAM record (block_size first) -> one SAM line, '\n' included.
+static void render_sam(const uint8_t* p, std::string& o) {
+  auto r32 = [](const uint8_t* q) { uint32_t v; memcpy(&v, q, 4); return v; };
+  auto r16 = [](const uint8_t* q) { uint16_t v; memcpy(&v, q, 2); return v; };
+  const uint32_t bs = r32(p); const uint8_t* b = p + 4;
+  const int32_t ref = (int32_t)r32(b), pos = (int32_t)r32(b + 4), nref = (int32_t)r32(b + 20), npos = (int32_t)r32(b + 24), tlen = (int32_t)r32(b + 28);
+  const uint32_t l_name = b[8], mapq = b[9], n_cig = r16(b + 12), flag = r16(b + 14), l_seq = r32(b + 16);
+  size_t k = 32;
+  char t[64];
+  o.append((const char*)b + k, l_name - 1); k += l_name;
+  o += '\t'; o += std::to_string(flag); o += '\t'; o += ref >= 0 ? kNames[ref] : "*";
+  o += '\t'; o += std::to_string(pos + 1); o += '\t'; o += std::to_string(mapq); o += '\t';
+  if (!n_cig) o += '*';
+  for (uint32_t c = 0; c < n_cig; c++, k += 4) { const uint32_t w = r32(b + k); o += std::to_string(w >> 4); o += "MIDNSHP=X"[w & 15]; }
+  o += '\t'; o += nref < 0 ? "*" : nref == ref ? "=" : kNames[nref];
+  o += '\t'; o += std::to_string(npos + 1); o += '\t'; o += std::to_string(tlen); o += '\t';
+  if (!l_seq) o += '*';
+  for (uint32_t i = 0; i < l_seq; i++) o += "=ACMGRSVTWYHKDBN"[(b[k + i / 2] >> ((i & 1) ? 0 : 4)) & 15];
+  k += (l_seq + 1) / 2;
+  o += '\t';
+  bool missing = true;
+  for (uint32_t i = 0; i < l_seq; i++) missing &= b[k + i] == 0xff;
+  if (!l_seq || missing) o += '*'; else for (uint32_t i = 0; i < l_seq; i++) o += (char)(b[k + i] + 33);
+  k += l_seq;
+  while (k + 3 <= bs) {
+    o += '\t'; o.append((const char*)b + k, 2); const char ty = (char)b[k + 2]; k += 3;
+    switch (ty) {
+      case 'A': o += ":A:"; o += (char)b[k]; k += 1; break;
+      case 'c': o += ":i:"; o += std::to_string((int8_t)b[k]); k += 1; break;
+      case 'C': o += ":i:"; o += std::to_string(b[k]); k += 1; break;
+      case 's': o += ":i:"; o += std::to_string((int16_t)r16(b + k)); k += 2; break;
+      case 'S': o += ":i:"; o += std::to_string(r16(b + k)); k += 2; break;
+      case 'i': o += ":i:"; o += std::to_string((int32_t)r32(b + k)); k += 4; break;
+      case 'I': o += ":i:"; o += std::to_string(r32(b + k)); k += 4; break;
+      case 'f': { float f; memcpy(&f, b + k, 4); snprintf(t, sizeof t, ":f:%.9g", f); o += t; k += 4; break; }
+      case 'Z': case 'H': { o += ':'; o += ty; o += ':'; const size_t n = strlen((const char*)b + k); o.append((const char*)b + k, n); k += n + 1; break; }
+      default: {   // 'B'
+        const char st = (char)b[k]; const uint32_t cnt = r32(b + k + 1); k += 5;
+        o += ":B:"; o += st;
+        for (uint32_t e = 0; e < cnt; e++) {
+          o += ',';
+          switch (st) {
+            case 'c': o += std::to_string((int8_t)b[k]); k += 1; break;
+            case 'C': o += std::to_string(b[k]); k += 1; break;
+            case 's': o += std::to_string((int16_t)r16(b + k)); k += 2; break;
+            case 'S': o += std::to_string(r16(b + k)); k += 2; break;
+            case 'i': o += std::to_string((int32_t)r32(b + k)); k += 4; break;
+            case 'I': o += std::to_string(r32(b + k)); k += 4; break;
+            default: { float f; memcpy(&f, b + k, 4); snprintf(t, sizeof t, "%.9g", f); o += t; k += 4; }
+          }
+        }
+      }
+    }
+  }
+  o += '\n';
+}
+
 // ------------------------------------------------------------------------------------------
 struct BaiRef { std::map<uint32_t, std::vector<std::pair<uint64_t, uint64_t>>> bins; std::vector<uint64_t> lin; uint64_t beg = ~0ull, end = 0, n_mapped = 0, n_unmapped = 0; };
 
@@ -233,16 +293,17 @@ static size_t deflate_block(const uint8_t* src, size_t n, int level, uint8_t* ds
 }
 
 int main(int argc, char** argv) {
-  std::string mode = "short", out; int64_t N = 1000000; uint64_t seed = 1; int threads = (int)std::thread::hardware_concurrency(); int level = 6; bool bai = false; int64_t n_unmapped = 0;
+  std::string mode = "short", out; int64_t N = 1000000; uint64_t seed = 1; int threads = (int)std::thread::hardware_concurrency(); int level = 6; bool bai = false; int64_t n_unmapped = 0; bool sam = false;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
     auto nxt = [&]() { if (i + 1 >= argc) { fprintf(stderr, "missing value for %s\n", a.c_str()); exit(1); } return std::string(argv[++i]); };
     if (a == "--mode") mode = nxt(); else if (a == "--reads") N = atoll(nxt().c_str()); else if (a == "--seed") seed = strtoull(nxt().c_str(), 0, 10);
     else if (a == "--out") out = nxt(); else if (a == "--threads") threads = atoi(nxt().c_str()); else if (a == "--level") level = atoi(nxt().c_str());
-    else if (a == "--bai") bai = true; else if (a == "--unmapped") n_unmapped = atoll(nxt().c_str());
+    else if (a == "--bai") bai = true; else if (a == "--unmapped") n_unmapped = atoll(nxt().c_str()); else if (a == "--sam") sam = true;
     else { fprintf(stderr, "unknown arg %s\n", a.c_str()); return 1; }
   }
-  if (out.empty() || N <= 0) { fprintf(stderr, "usage: bamgen --mode short|long --reads N --seed S --out f.bam [--threads T] [--level L] [--bai] [--unmapped K]\n"); return 1; }
+  if (out.empty() || N <= 0) { fprintf(stderr, "usage: bamgen --mode short|long --reads N --seed S --out f.bam [--threads T] [--level L] [--bai] [--unmapped K] [--sam]\n"); return 1; }
+  if (sam && bai) { fprintf(stderr, "--bai needs BAM output\n"); return 1; }
   if (threads < 1) threads = 1;
   bool is_long = mode == "long";
   if (!is_long && (N & 1)) N++;
@@ -253,6 +314,30 @@ int main(int argc, char** argv) {
   for (int i = 0; i < 25; i++) text += std::string("@SQ\tSN:") + kNames[i] + "\tLN:" + std::to_string(kLens[i]) + "\n";
   text += "@RG\tID:rg1\tSM:sample1\tPL:ILLUMINA\tLB:lib1\tPU:unit1\n";
   text += "@PG\tID:bamgen\tPN:bamgen\tVN:1.0\tCL:bamgen --mode " + mode + " --reads " + std::to_string(N) + " --seed " + std::to_string(seed) + "\n";
+  if (sam) {
+    // the same records as text, rendered in parallel per chunk, written in order
+    if (fwrite(text.data(), 1, text.size(), fp) != text.size()) { perror("write"); return 2; }
+    const int64_t units = is_long ? N : N / 2, per_chunk = is_long ? 512 : 16384, n_chunks = (units + per_chunk - 1) / per_chunk, group = (int64_t)threads * 2;
+    for (int64_t c0 = 0; c0 < n_chunks; c0 += group) {
+      const int64_t c1 = std::min(n_chunks, c0 + group);
+      std::vector<std::string> txt((size_t)(c1 - c0));
+      std::vector<std::thread> th;
+      for (int t = 0; t < threads; t++) th.emplace_back([&, t]() {
+        for (int64_t c = c0 + t; c < c1; c += threads) {
+          Chunk ch;
+          const int64_t u0 = c * per_chunk, u1 = std::min(units, u0 + per_chunk);
+          if (is_long) gen_long_chunk(seed, c, u0, u1, units, G, ch); else gen_short_chunk(seed, c, u0, u1, units, G, ch);
+          std::string& o = txt[(size_t)(c - c0)];
+          o.reserve(ch.bytes.size() * 2);
+          for (auto& r : ch.recs) render_sam(ch.bytes.data() + r.off, o);
+        } });
+      for (auto& t : th) t.join();
+      for (auto& o : txt) if (fwrite(o.data(), 1, o.size(), fp) != o.size()) { perror("write"); return 2; }
+    }
+    if (n_unmapped > 0) { fprintf(stderr, "--unmapped needs BAM output\n"); return 1; }
+    fclose(fp);
+    return 0;
+  }
   std::vector<uint8_t> pend;     // inflated stream bytes not yet written; pend[0] is at absolute offset pend_abs
   uint64_t pend_abs = 0;
   pend.insert(pend.end(), {'B', 'A', 'M', 1}); put32(pend, (uint32_t)text.size()); pend.insert(pend.end(), text.begin(), text.end());
