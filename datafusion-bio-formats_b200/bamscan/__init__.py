@@ -33,6 +33,7 @@ EXPORTED_SYMBOLS = [
     "bamscan_stream_free", "bamscan_run_device_resident", "bamscan_stream_stats", "bamscan_bench_inflate",
     "bamscan_probe_pcie", "bamscan_check_partition_seams", "bamscan_last_error", "bamscan_version",
     "bamscan_writer_open", "bamscan_writer_write", "bamscan_writer_write_device", "bamscan_writer_finish", "bamscan_writer_stats", "bamscan_writer_free",
+    "bamscan_fastq_writer_open",
 ]
 
 
@@ -150,6 +151,7 @@ def load_library():
     L.bamscan_writer_finish.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
     L.bamscan_writer_stats.argtypes = [C.c_void_p, C.POINTER(WriteStats)]
     L.bamscan_writer_free.argtypes = [C.c_void_p]
+    L.bamscan_fastq_writer_open.argtypes = [C.c_char_p, C.c_void_p, C.POINTER(_WriteOptions), C.POINTER(C.c_void_p)]
     _lib = L
     return L
 
@@ -644,31 +646,78 @@ class BamWriteExec:
         finally:
             if cs.release:
                 C.CFUNCTYPE(None, C.c_void_p)(cs.release)(C.addressof(cs))
+        n, self.stats = _drive_writer(h, batches, self.schema)
+        return n
+
+
+def _drive_writer(h, batches, schema: pa.Schema):
+    """Feeds `batches` (pyarrow.RecordBatch or DeviceBatch with `schema`'s columns) to an open writer handle, finishes it and
+    frees it.  -> (rows written, stats dict)."""
+    L = load_library()
+    try:
+        for b in batches:
+            if b.schema.names != schema.names:
+                raise BamScanError(-7, "batch columns differ from the writer's input schema")
+            if isinstance(b, DeviceBatch):                   # stays in HBM: bamscan_writer_write_device
+                _check(L.bamscan_writer_write_device(h, C.byref(b._dev)))
+                continue
+            ca = _ArrowArrayStruct()
+            sa = b.to_struct_array()
+            sa._export_to_c(C.addressof(ca))
+            try:
+                _check(L.bamscan_writer_write(h, C.addressof(ca)))
+            finally:
+                if ca.release:
+                    C.CFUNCTYPE(None, C.c_void_p)(ca.release)(C.addressof(ca))
+        n = C.c_uint64()
+        _check(L.bamscan_writer_finish(h, C.byref(n)))
+        st = WriteStats()
+        _check(L.bamscan_writer_stats(h, C.byref(st)))
+        return int(n.value), st.as_dict()
+    finally:
+        L.bamscan_writer_free(h)
+
+
+FASTQ_SCHEMA = pa.schema([pa.field("name", pa.string(), False), pa.field("description", pa.string(), True),
+                          pa.field("sequence", pa.string(), False), pa.field("quality_scores", pa.string(), False)])
+
+
+def fastq_compression_for(output_path) -> int:
+    """Compression a FASTQ path asks for by its extension: `.bgz`, `.bgzf` and `.gz` -> BGZF (0), anything else -> plain text
+    (2).  BGZF is valid multi-member gzip, so a `.gz` file is written as BGZF too."""
+    return 0 if str(output_path).lower().endswith((".bgz", ".bgzf", ".gz")) else 2
+
+
+class FastqWriteExec:
+    """The FASTQ write path (bamscan_fastq_writer_open): rows of `input_schema`'s name / description / sequence / quality_scores
+    columns (looked up by name; description optional; other columns ignored) encoded as FASTQ text on the device, into BGZF
+    members (compression 0, or 1 = stored blocks) or plain text (2).  compression None: by the path's extension
+    (fastq_compression_for).  `execute` takes pyarrow.RecordBatch or DeviceBatch and returns the row count; `.stats` after it.
+    Bases and qualities are written as stored: reads of a BAM scan are not reverse-complemented."""
+
+    def __init__(self, output_path, input_schema: pa.Schema, compression=None, *, device_id=0):
+        self.output_path = str(output_path)
+        self.schema = input_schema
+        self.compression = fastq_compression_for(output_path) if compression is None else int(compression)
+        self.device_id = device_id
+        self.stats = None
+
+    def execute(self, batches) -> int:
+        L = load_library()
+        o = _WriteOptions()
+        o.struct_size = C.sizeof(_WriteOptions)
+        o.device_id = self.device_id
+        o.compression = self.compression
+        cs = _ArrowSchemaStruct()
+        pa.struct(list(self.schema))._export_to_c(C.addressof(cs))
+        h = C.c_void_p()
         try:
-            for b in batches:
-                if isinstance(b, DeviceBatch):               # stays in HBM: bamscan_writer_write_device
-                    if b.schema.names != self.schema.names:
-                        raise BamScanError(-7, "batch columns differ from the writer's input schema")
-                    _check(L.bamscan_writer_write_device(h, C.byref(b._dev)))
-                    continue
-                if b.schema.names != self.schema.names:
-                    raise BamScanError(-7, "batch columns differ from the writer's input schema")
-                ca = _ArrowArrayStruct()
-                sa = b.to_struct_array()
-                sa._export_to_c(C.addressof(ca))
-                try:
-                    _check(L.bamscan_writer_write(h, C.addressof(ca)))
-                finally:
-                    if ca.release:
-                        C.CFUNCTYPE(None, C.c_void_p)(ca.release)(C.addressof(ca))
-            n = C.c_uint64()
-            _check(L.bamscan_writer_finish(h, C.byref(n)))
-            st = WriteStats()
-            _check(L.bamscan_writer_stats(h, C.byref(st)))
-            self.stats = st.as_dict()
-            return int(n.value)
+            _check(L.bamscan_fastq_writer_open(self.output_path.encode(), C.addressof(cs), C.byref(o), C.byref(h)))
         finally:
-            L.bamscan_writer_free(h)
+            if cs.release:
+                C.CFUNCTYPE(None, C.c_void_p)(cs.release)(C.addressof(cs))
+        n, self.stats = _drive_writer(h, batches, self.schema)
+        return n
 
 
 class FastqTableProvider(BamTableProvider):
@@ -693,12 +742,34 @@ class FastqTableProvider(BamTableProvider):
         self._h = C.c_void_p()
         _check(L.bamscan_open_fastq(str(file_path).encode(), C.byref(o), C.byref(self._h)))
         self.file_path = str(file_path)
+        self.device_id = device_id
         self._schema = None
 
     def scan(self, projection=None, filters=None, limit=None, *, target_partitions=1, partition_mode=None) -> BamExec:
         if partition_mode is None:
             partition_mode = "block_range" if target_partitions > 1 else "reference"
         return super().scan(projection, None, limit, target_partitions=target_partitions, partition_mode=partition_mode)
+
+    @classmethod
+    def new_for_write(cls, output_path, schema: pa.Schema = None, *, device_id=0):
+        """A provider for a FASTQ file that does not exist yet (default schema: the FASTQ scan's); only schema() and
+        insert_into() are meaningful on it."""
+        self = cls.__new__(cls)
+        self._h = None
+        self.file_path = str(output_path)
+        self.device_id = device_id
+        self._schema = FASTQ_SCHEMA if schema is None else schema
+        return self
+
+    def insert_into(self, batches, insert_op="overwrite", *, compression=None):
+        """`INSERT OVERWRITE` of `batches` (pyarrow.RecordBatch or DeviceBatch with this provider's schema) into this provider's
+        file through FastqWriteExec; compression None picks BGZF or plain text by the file's extension.  Returns the row count."""
+        if insert_op != "overwrite":
+            raise NotImplementedError("FASTQ insert_into only supports OVERWRITE mode")
+        ex = FastqWriteExec(self.file_path, self.schema(), compression, device_id=getattr(self, "device_id", 0))
+        n = ex.execute(batches)
+        self.last_write_stats = ex.stats
+        return n
 
 
 def check_partition_seams(stats_list):

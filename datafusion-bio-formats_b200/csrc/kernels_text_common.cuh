@@ -75,8 +75,10 @@ __device__ __forceinline__ void st_u16(uint8_t* p, uint32_t v) { p[0] = (uint8_t
 // dst[i] = op(src[i]) for i < n by a group of G lanes, with destination-aligned 32-bit stores (head / tail bytes singly); `op`
 // maps four bytes at a time.  Records are byte packed, so a plain byte loop costs one store instruction and one 32-byte
 // sector write per byte (ncu: 9.5 x store-sector amplification in the first version of this kernel).
+// grp_xform4_ref takes the op by reference, so an op can also accumulate state over the words it sees (a byte check fused
+// into the copy); the single head / tail bytes reach it as words whose upper three bytes are zero.
 template <int G, class OP>
-__device__ __forceinline__ void grp_xform4(uint8_t* dst, const uint8_t* src, uint32_t n, int gl, OP op) {
+__device__ __forceinline__ void grp_xform4_ref(uint8_t* dst, const uint8_t* src, uint32_t n, int gl, OP& op) {
   const uint32_t head = min(n, (uint32_t)((4u - (reinterpret_cast<uintptr_t>(dst) & 3u)) & 3u));
   if ((uint32_t)gl < head) dst[gl] = (uint8_t)op((uint32_t)src[gl]);
   const uint32_t nw = (n - head) >> 2;
@@ -86,6 +88,8 @@ __device__ __forceinline__ void grp_xform4(uint8_t* dst, const uint8_t* src, uin
   const uint32_t t0 = head + (nw << 2);
   if (t0 + (uint32_t)gl < n) dst[t0 + gl] = (uint8_t)op((uint32_t)src[t0 + gl]);
 }
+template <int G, class OP>
+__device__ __forceinline__ void grp_xform4(uint8_t* dst, const uint8_t* src, uint32_t n, int gl, OP op) { grp_xform4_ref<G>(dst, src, n, gl, op); }
 struct OpCopy { __device__ __forceinline__ uint32_t operator()(uint32_t v) const { return v; } };
 struct OpQual { __device__ __forceinline__ uint32_t operator()(uint32_t v) const { return __vsubus4(v, 0x21212121u); } };   // byte-wise saturating - 33
 

@@ -5,6 +5,10 @@
 // Here: Arrow buffers of a batch -> H2D -> enc_size_kernel -> scan -> enc_records_kernel into the uncompressed stream in HBM
 // -> bgzf_deflate_kernel over every full 0xff00-byte member -> gather -> D2H -> write(2).  The tail that does not fill a
 // member stays in HBM for the next batch; bamscan_writer_finish flushes it and appends the EOF marker.
+//
+// FASTQ writers (bamscan_fastq_writer_open) share everything but the encoder: no header, fq_enc_size_kernel -> scan ->
+// fq_enc_records_kernel write the text into the same stream buffer, which is deflated into the same members -- or, in plain
+// mode (compression 2), copied to the file as it is.
 #include <fcntl.h>
 #include <unistd.h>
 
@@ -27,6 +31,7 @@
 #include "bamscan_internal.h"
 #include "kernels_deflate.cuh"
 #include "kernels_encode.cuh"
+#include "kernels_fastq_encode.cuh"
 
 namespace bamscan {
 
@@ -71,6 +76,7 @@ struct DevBuf {
 };
 
 struct WTag { int col; int32_t kind; uint8_t tag[2], sam_type, subtype; };
+enum : int { FMT_BAM = 0, FMT_FASTQ = 1 };
 
 // Device buffers, pinned staging, stream and events of a writer.  One set per device is kept between writers (cudaMalloc /
 // cudaHostAlloc / cudaFree of a few GB cost more than writing a few million records).
@@ -107,7 +113,10 @@ struct BamWriter : bamscan::WriterRes {
   int device = 0;
   bool zero_based = true, cigar_binary = false, finished = false;
   int compression = 0;
-  int col[11] = {};                      // name chrom start flags cigar mapq mate_chrom mate_start seq qual tlen
+  int format = FMT_BAM;
+  bool plain = false;                    // FASTQ compression 2: the text goes to the file as it is (no BGZF, no EOF marker)
+  int col[11] = {};                      // BAM: name chrom start flags cigar mapq mate_chrom mate_start seq qual tlen;
+                                         // FASTQ: name description (-1: absent) sequence quality_scores
   std::vector<WTag> tags;
   int n_cols = 0;
   int n_ref = 0;
@@ -190,6 +199,8 @@ static int32_t kind_of_format(const ArrowSchema* c) {
 }
 
 static int writer_flush_members(BamWriter* w, uint64_t total, bool final_flush);
+static int writer_open_device(BamWriter* w, int device_id);
+static int writer_open_file(BamWriter* w, const char* output_path);
 
 static int writer_open_impl(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
                             const int32_t* ref_lengths, const ArrowSchema* schema, const BamWriteOptions* options, BamWriter** out) {
@@ -249,17 +260,48 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
     if ((int)w->tags.size() >= enc::MAX_WTAGS) { set_error("more than %d tag columns are not supported by the writer", enc::MAX_WTAGS); return BAMSCAN_ERR_UNSUPPORTED; }
     w->tags.push_back(g);
   }
-  // device
+  int rc;
+  if ((rc = writer_open_device(w.get(), opt.device_id))) return rc;
+  // reference dictionary, sorted bytewise; a later duplicate wins like the reference's HashMap collect
+  {
+    std::map<std::string, int32_t> m;
+    for (int32_t i = 0; i < n_ref; i++) m[ref_names[i]] = i;
+    std::string blob; std::vector<int32_t> off{0}, ids;
+    for (auto& kv : m) { blob += kv.first; off.push_back((int32_t)blob.size()); ids.push_back(kv.second); }
+    w->n_ref = (int)ids.size();
+    if ((rc = w->ref_blob.reserve(blob.size() + 16)) || (rc = w->ref_off.reserve(off.size() * 4)) || (rc = w->ref_ids.reserve(ids.size() * 4 + 4))) return rc;
+    if (!blob.empty()) WCU_TRY(cudaMemcpy(w->ref_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice));
+    WCU_TRY(cudaMemcpy(w->ref_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice));
+    if (!ids.empty()) WCU_TRY(cudaMemcpy(w->ref_ids.p, ids.data(), ids.size() * 4, cudaMemcpyHostToDevice));
+  }
+  // BAM header bytes open the uncompressed stream (bam::io::Writer::write_header)
+  std::string hdr("BAM\1", 4);
+  {
+    const std::string text = sam_header_text ? sam_header_text : "";
+    auto put32 = [&](int32_t v) { hdr.append(reinterpret_cast<const char*>(&v), 4); };
+    put32((int32_t)text.size()); hdr += text; put32(n_ref);
+    for (int32_t i = 0; i < n_ref; i++) { const std::string n = ref_names[i]; put32((int32_t)n.size() + 1); hdr += n; hdr.push_back('\0'); put32(ref_lengths[i]); }
+  }
+  if ((rc = w->stream_buf.reserve(hdr.size() + SLICE_BYTES + 65536))) return rc;
+  WCU_TRY(cudaMemcpy(w->stream_buf.p, hdr.data(), hdr.size(), cudaMemcpyHostToDevice));
+  w->pending = hdr.size();
+  if ((rc = writer_open_file(w.get(), output_path))) return rc;
+  *out = w.release();
+  return BAMSCAN_OK;
+}
+
+// Device, pooled resources and the CRC table of the deflate kernel: the part of opening a writer that needs the GPU.
+static int writer_open_device(BamWriter* w, int device_id) {
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); set_error("bamscan_writer_open: no CUDA device (this library has no CPU path)"); return BAMSCAN_ERR_CUDA; }
-  if (opt.device_id < 0 || opt.device_id >= ndev) { set_error("device_id %d out of range (%d devices)", opt.device_id, ndev); return BAMSCAN_ERR_INVALID; }
-  WCU_TRY(cudaSetDevice(opt.device_id));
+  if (device_id < 0 || device_id >= ndev) { set_error("device_id %d out of range (%d devices)", device_id, ndev); return BAMSCAN_ERR_INVALID; }
+  WCU_TRY(cudaSetDevice(device_id));
   cudaDeviceProp prop;
-  WCU_TRY(cudaGetDeviceProperties(&prop, opt.device_id));
+  WCU_TRY(cudaGetDeviceProperties(&prop, device_id));
   w->n_sms = prop.multiProcessorCount;
   {
     std::lock_guard<std::mutex> lk(g_res_mu);
-    WriterRes& pooled = g_res_pool[opt.device_id & 63];
+    WriterRes& pooled = g_res_pool[device_id & 63];
     if (pooled.ready) { static_cast<WriterRes&>(*w) = pooled; pooled = WriterRes(); }
   }
   if (!w->ready) {
@@ -280,35 +322,15 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
     WCU_TRY(cudaMemcpyToSymbol(dfl::c_xpow8, tab, sizeof tab));
     WCU_TRY(cudaFuncSetAttribute(dfl::bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(dfl::Smem)));
   }
-  // reference dictionary, sorted bytewise; a later duplicate wins like the reference's HashMap collect
-  {
-    std::map<std::string, int32_t> m;
-    for (int32_t i = 0; i < n_ref; i++) m[ref_names[i]] = i;
-    std::string blob; std::vector<int32_t> off{0}, ids;
-    for (auto& kv : m) { blob += kv.first; off.push_back((int32_t)blob.size()); ids.push_back(kv.second); }
-    w->n_ref = (int)ids.size();
-    int rc;
-    if ((rc = w->ref_blob.reserve(blob.size() + 16)) || (rc = w->ref_off.reserve(off.size() * 4)) || (rc = w->ref_ids.reserve(ids.size() * 4 + 4))) return rc;
-    if (!blob.empty()) WCU_TRY(cudaMemcpy(w->ref_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-    WCU_TRY(cudaMemcpy(w->ref_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice));
-    if (!ids.empty()) WCU_TRY(cudaMemcpy(w->ref_ids.p, ids.data(), ids.size() * 4, cudaMemcpyHostToDevice));
-  }
-  // BAM header bytes open the uncompressed stream (bam::io::Writer::write_header)
-  std::string hdr("BAM\1", 4);
-  {
-    const std::string text = sam_header_text ? sam_header_text : "";
-    auto put32 = [&](int32_t v) { hdr.append(reinterpret_cast<const char*>(&v), 4); };
-    put32((int32_t)text.size()); hdr += text; put32(n_ref);
-    for (int32_t i = 0; i < n_ref; i++) { const std::string n = ref_names[i]; put32((int32_t)n.size() + 1); hdr += n; hdr.push_back('\0'); put32(ref_lengths[i]); }
-  }
-  int rc = w->stream_buf.reserve(hdr.size() + SLICE_BYTES + 65536);
-  if (rc) return rc;
-  WCU_TRY(cudaMemcpy(w->stream_buf.p, hdr.data(), hdr.size(), cudaMemcpyHostToDevice));
-  w->pending = hdr.size();
+  return BAMSCAN_OK;
+}
+
+// Creates the output file and starts the file threads.
+static int writer_open_file(BamWriter* w, const char* output_path) {
   w->fd = ::open(output_path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
   if (w->fd < 0) { set_error("Failed to create output file: %s", output_path); return BAMSCAN_ERR_IO; }
   {
-    BamWriter* wp = w.get();
+    BamWriter* wp = w;
     for (auto& th : wp->file_thread) th = std::thread([wp] {
       for (;;) {
         BamWriter::FileJob job;
@@ -329,6 +351,36 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
       }
     });
   }
+  return BAMSCAN_OK;
+}
+
+// FASTQ writer: columns by name (name, sequence, quality_scores required, description optional, all Utf8; any other column is
+// ignored), no header bytes, compression 0 / 1 (BGZF) or 2 (plain text).
+static int fastq_writer_open_impl(const char* output_path, const ArrowSchema* schema, const BamWriteOptions* options, BamWriter** out) {
+  if (!output_path || !schema || !out) { set_error("bamscan_fastq_writer_open: null argument"); return BAMSCAN_ERR_INVALID; }
+  BamWriteOptions opt;
+  memset(&opt, 0, sizeof opt);
+  if (options) memcpy(&opt, options, std::min<size_t>(sizeof opt, options->struct_size ? options->struct_size : sizeof opt));
+  if (!schema->format || strcmp(schema->format, "+s") != 0) { set_error("bamscan_fastq_writer_open: input_schema must be a struct"); return BAMSCAN_ERR_INVALID; }
+  if (opt.compression < 0 || opt.compression > 2) { set_error("bamscan_fastq_writer_open: compression %d (0: BGZF, 1: BGZF stored blocks, 2: plain text)", opt.compression); return BAMSCAN_ERR_INVALID; }
+  std::unique_ptr<BamWriter, void (*)(BamWriter*)> w(new BamWriter(), [](BamWriter* p) { bamscan_writer_free(p); });
+  w->path = output_path; w->device = opt.device_id; w->compression = opt.compression;
+  w->format = FMT_FASTQ; w->plain = opt.compression == 2;
+  w->n_cols = (int)schema->n_children;
+  static const char* const names[4] = {"name", "description", "sequence", "quality_scores"};
+  for (int k = 0; k < 4; k++) {
+    int idx = -1;
+    for (int64_t c = 0; c < schema->n_children; c++) if (schema->children[c]->name && strcmp(schema->children[c]->name, names[k]) == 0) { idx = (int)c; break; }
+    if (idx < 0 && k == 1) { w->col[k] = -1; continue; }
+    if (idx < 0) { set_error("Required column '%s' not found in batch", names[k]); return BAMSCAN_ERR_SCHEMA; }
+    if (kind_of_format(schema->children[idx]) != HK_Utf8) { set_error("Column '%s' must be Utf8", names[k]); return BAMSCAN_ERR_SCHEMA; }
+    w->col[k] = idx;
+  }
+  int rc;
+  if ((rc = writer_open_device(w.get(), opt.device_id))) return rc;
+  if ((rc = w->stream_buf.reserve(SLICE_BYTES + 65536))) return rc;
+  w->pending = 0;
+  if ((rc = writer_open_file(w.get(), output_path))) return rc;
   *out = w.release();
   return BAMSCAN_OK;
 }
@@ -422,6 +474,125 @@ static int stage_prim(BamWriter* w, size_t* cur, const HostCol& c, int64_t n, en
   return stage_validity(w, cur, c, n, &out->valid);
 }
 
+// Byte count of a slice from the record lengths in rec_len: tile sums on the device, exclusive tile offsets into h_small[0 ..
+// n_tiles) on the host.  The slice's error words come back beside them (h_small + 4096), read by the caller.
+static int sum_lengths(BamWriter* w, uint32_t rows, const uint32_t* d_err, uint64_t* total) {
+  const uint32_t n_tiles = (rows + 4095) / 4096;
+  unsigned long long* d_tiles = static_cast<unsigned long long*>(w->tile_sums.p);
+  dfl::len_tile_sums_kernel<<<n_tiles, 256, 0, w->stream>>>(static_cast<uint32_t*>(w->rec_len.p), rows, d_tiles);
+  w->st.kernel_launches += 1;
+  WCU_TRY(cudaMemcpyAsync(w->h_small, d_tiles, (size_t)n_tiles * 8, cudaMemcpyDeviceToHost, w->stream));
+  WCU_TRY(cudaMemcpyAsync(w->h_small + 4096, d_err, 16, cudaMemcpyDeviceToHost, w->stream));
+  WCU_TRY(cudaStreamSynchronize(w->stream));
+  uint64_t t = 0;
+  for (uint32_t k = 0; k < n_tiles; k++) { const uint64_t s = w->h_small[k]; w->h_small[k] = t; t += s; }
+  *total = t;
+  return BAMSCAN_OK;
+}
+
+// 64-bit record offsets rec_off[0 .. rows] in the stream buffer, behind its pending bytes (grown when one slice does not fit).
+static int place_records(BamWriter* w, uint32_t rows, uint64_t total) {
+  const uint32_t n_tiles = (rows + 4095) / 4096;
+  unsigned long long* d_tiles = static_cast<unsigned long long*>(w->tile_sums.p);
+  if (w->pending + total + 65536 > w->stream_buf.cap) {    // one record larger than a slice: grow, keeping the pending bytes
+    DevBuf bigger;
+    int rc;
+    if ((rc = bigger.reserve(w->pending + total + 65536))) return rc;
+    WCU_TRY(cudaMemcpyAsync(bigger.p, w->stream_buf.p, w->pending, cudaMemcpyDeviceToDevice, w->stream));
+    WCU_TRY(cudaStreamSynchronize(w->stream));
+    w->stream_buf.release(); w->stream_buf = bigger;
+  }
+  WCU_TRY(cudaMemcpyAsync(d_tiles + n_tiles + 1, w->h_small, (size_t)n_tiles * 8, cudaMemcpyHostToDevice, w->stream));
+  dfl::len_offsets_kernel<<<n_tiles, 256, 0, w->stream>>>(static_cast<uint32_t*>(w->rec_len.p), rows, d_tiles + n_tiles + 1, w->pending,
+                                                         static_cast<unsigned long long*>(w->rec_off.p));
+  w->st.kernel_launches += 1;
+  w->h_small[6000] = w->pending + total;                    // (rows % 4096 == 0: no tile of the kernel above owns element `rows`)
+  WCU_TRY(cudaMemcpyAsync(static_cast<unsigned long long*>(w->rec_off.p) + rows, w->h_small + 6000, 8, cudaMemcpyHostToDevice, w->stream));
+  return BAMSCAN_OK;
+}
+
+static const char* fq_err_text(uint32_t code) {
+  switch (code) {
+    case fqenc::FQ_ERR_NULL_NAME: return "name is NULL";
+    case fqenc::FQ_ERR_NULL_SEQ: return "sequence is NULL";
+    case fqenc::FQ_ERR_NULL_QUAL: return "quality_scores is NULL";
+    case fqenc::FQ_ERR_EOL_NAME: return "line break in name";
+    case fqenc::FQ_ERR_WS_NAME: return "space or tab in name";
+    case fqenc::FQ_ERR_EOL_DESC: return "line break in description";
+    case fqenc::FQ_ERR_EOL_SEQ: return "line break in sequence";
+    case fqenc::FQ_ERR_EOL_QUAL: return "line break in quality_scores";
+    case fqenc::FQ_ERR_REC_LEN: return "record larger than 2 GiB";
+    default: return "encode error";
+  }
+}
+
+// The FASTQ branch of bamscan_writer_write(_device): stage the four Utf8 columns, then per slice of rows sizes -> offsets ->
+// text -> members (or, plain, the file).
+static int fastq_write_impl(BamWriter* w, const ArrowArray* batch, int64_t n) {
+  auto hc = [&](int idx) { return HostCol{batch->children[idx], batch->offset + batch->children[idx]->offset}; };
+  for (int k = 0; k < 4; k++) {
+    if (w->col[k] < 0) continue;
+    const ArrowArray* a = batch->children[w->col[k]];
+    if (!a || !a->buffers || a->n_buffers < 3 || !a->buffers[1] || a->length + a->offset < n + batch->offset) {
+      set_error("bamscan_writer_write: column %d of the batch does not have the layout of the writer's input schema", w->col[k]);
+      return BAMSCAN_ERR_INVALID;
+    }
+  }
+  size_t need = 4096;
+  if (!w->src_on_device) for (int k = 0; k < 4; k++) if (w->col[k] >= 0) need += utf8_bytes(w, hc(w->col[k]), n);
+  int rc;
+  const double t_w0 = now_ms();
+  if ((rc = w->in.reserve(need))) return rc;
+  fqenc::FqArgs A;
+  memset(&A, 0, sizeof A);
+  size_t cur = 0;
+  A.has_desc = w->col[1] >= 0;
+  if ((rc = stage_utf8(w, &cur, hc(w->col[0]), n, &A.name)) || (A.has_desc && (rc = stage_utf8(w, &cur, hc(w->col[1]), n, &A.desc))) ||
+      (rc = stage_utf8(w, &cur, hc(w->col[2]), n, &A.seq)) || (rc = stage_utf8(w, &cur, hc(w->col[3]), n, &A.qual)))
+    return rc;
+  WTRACE("[writer] FASTQ batch of %lld rows: staged %.1f MB in %.1f ms\n", (long long)n, cur / 1e6, now_ms() - t_w0);
+  if ((rc = w->small.reserve(4096))) return rc;
+  uint32_t* d_err = static_cast<uint32_t*>(w->small.p);
+  const uint32_t* h_err = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
+  int64_t r0 = 0;
+  uint32_t want_rows = w->slice_rows;
+  while (r0 < n) {
+    const uint32_t rows = (uint32_t)std::min<int64_t>(want_rows, n - r0);
+    if ((rc = w->rec_len.reserve((size_t)rows * 4)) || (rc = w->rec_off.reserve(((size_t)rows + 1) * 8)) || (rc = w->tile_sums.reserve(((size_t)rows / 4096 + 2) * 16)))
+      return rc;
+    A.row0 = (uint32_t)r0; A.n_rows = rows;
+    WCU_TRY(cudaEventRecord(w->ev[0], w->stream));
+    WCU_TRY(cudaMemsetAsync(d_err, 0, 16, w->stream));
+    fqenc::fq_enc_size_kernel<<<(rows + 255) / 256, 256, 0, w->stream>>>(A, static_cast<uint32_t*>(w->rec_len.p), d_err);
+    w->st.kernel_launches += 1;
+    uint64_t total = 0;
+    if ((rc = sum_lengths(w, rows, d_err, &total))) return rc;
+    if (h_err[0]) { set_error("FASTQ write error: row %u: %s", h_err[1], fq_err_text(h_err[0])); return BAMSCAN_ERR_FORMAT; }
+    if (total > SLICE_BYTES && rows > 1) {                   // long reads: fewer rows per pass
+      want_rows = std::max<uint32_t>(1, (uint32_t)((double)rows * (double)SLICE_BYTES / (double)total * 0.9));
+      w->slice_rows = want_rows;
+      continue;
+    }
+    if ((rc = place_records(w, rows, total))) return rc;
+    const unsigned long long* d_off = static_cast<const unsigned long long*>(w->rec_off.p);
+    uint8_t* d_out = static_cast<uint8_t*>(w->stream_buf.p);
+    if (total / rows > 2048) fqenc::fq_enc_records_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_off, d_out, d_err);   // long reads: a warp per row
+    else fqenc::fq_enc_records_kernel<8><<<(((rows + 3) / 4) * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_off, d_out, d_err);
+    w->st.kernel_launches += 1;
+    WCU_TRY(cudaEventRecord(w->ev[1], w->stream));
+    WCU_TRY(cudaMemcpyAsync(w->h_small + 4096, d_err, 16, cudaMemcpyDeviceToHost, w->stream));
+    WCU_TRY(cudaStreamSynchronize(w->stream));
+    if (h_err[0]) { set_error("FASTQ write error: row %u: %s", h_err[1], fq_err_text(h_err[0])); return BAMSCAN_ERR_FORMAT; }
+    { float ms = 0; cudaEventElapsedTime(&ms, w->ev[0], w->ev[1]); w->st.ms_encode += ms; w->st.ms_total += ms; }
+    w->st.rows += rows; w->st.bam_bytes += total;
+    const double t_f0 = now_ms();
+    if ((rc = writer_flush_members(w, w->pending + total, false))) return rc;
+    WTRACE("[writer] FASTQ slice of %u rows: encode done at +%.1f ms, flushed in %.1f ms\n", rows, t_f0 - t_w0, now_ms() - t_f0);
+    r0 += rows;
+  }
+  return BAMSCAN_OK;
+}
+
 static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
   if (!w || !batch) { set_error("bamscan_writer_write: null argument"); return BAMSCAN_ERR_INVALID; }
   if (w->finished) { set_error("bamscan_writer_write: the writer is finished"); return BAMSCAN_ERR_INVALID; }
@@ -430,6 +601,7 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
   w->st.batches++;
   if (n == 0) return BAMSCAN_OK;
   WCU_TRY(cudaSetDevice(w->device));
+  if (w->format == FMT_FASTQ) return fastq_write_impl(w, batch, n);
   auto hc = [&](int idx) { return HostCol{batch->children[idx], batch->offset + batch->children[idx]->offset}; };
   // shape checks before any buffer is touched (the arrays carry no type: the schema given at open decides how they are read)
   auto shape_ok = [&](int idx, int64_t want_buffers, bool list) {
@@ -525,14 +697,9 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
     enc::enc_cigar_kernel<8><<<(((rows + 3) / 4) * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, d_cig_span, d_err);
     enc::enc_size_kernel<<<(rows + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, d_cig_span, static_cast<uint32_t*>(w->rec_len.p), static_cast<int32_t*>(w->ref_pairs.p),
                                                                    static_cast<uint32_t*>(w->cig_bin.p), d_err);
-    w->st.kernel_launches += 1;
-    const uint32_t n_tiles = (rows + 4095) / 4096;
-    unsigned long long* d_tiles = static_cast<unsigned long long*>(w->tile_sums.p);
-    dfl::len_tile_sums_kernel<<<n_tiles, 256, 0, w->stream>>>(static_cast<uint32_t*>(w->rec_len.p), rows, d_tiles);
     w->st.kernel_launches += 2;
-    WCU_TRY(cudaMemcpyAsync(w->h_small, d_tiles, (size_t)n_tiles * 8, cudaMemcpyDeviceToHost, w->stream));
-    WCU_TRY(cudaMemcpyAsync(w->h_small + 4096, d_err, 16, cudaMemcpyDeviceToHost, w->stream));
-    WCU_TRY(cudaStreamSynchronize(w->stream));
+    uint64_t total = 0;
+    if ((rc = sum_lengths(w, rows, d_err, &total))) return rc;
     {
       const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
       if (e[0]) {
@@ -541,26 +708,13 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
                : e[0] == enc::ENC_ERR_CIGAR_OPS ? BAMSCAN_ERR_UNSUPPORTED : BAMSCAN_ERR_FORMAT;
       }
     }
-    uint64_t total = 0;
-    for (uint32_t t = 0; t < n_tiles; t++) { const uint64_t s = w->h_small[t]; w->h_small[t] = total; total += s; }
     if (total > SLICE_BYTES && rows > 1) {                   // long reads: fewer rows per pass
       want_rows = std::max<uint32_t>(1, (uint32_t)((double)rows * (double)SLICE_BYTES / (double)total * 0.9));
       w->slice_rows = want_rows;                               // (the next batch starts from this estimate)
       continue;
     }
-    if (w->pending + total + 65536 > w->stream_buf.cap) {    // one record larger than a slice: grow, keeping the pending bytes
-      DevBuf bigger;
-      if ((rc = bigger.reserve(w->pending + total + 65536))) return rc;
-      WCU_TRY(cudaMemcpyAsync(bigger.p, w->stream_buf.p, w->pending, cudaMemcpyDeviceToDevice, w->stream));
-      WCU_TRY(cudaStreamSynchronize(w->stream));
-      w->stream_buf.release(); w->stream_buf = bigger;
-    }
-    WCU_TRY(cudaMemcpyAsync(d_tiles + n_tiles + 1, w->h_small, (size_t)n_tiles * 8, cudaMemcpyHostToDevice, w->stream));
-    dfl::len_offsets_kernel<<<n_tiles, 256, 0, w->stream>>>(static_cast<uint32_t*>(w->rec_len.p), rows, d_tiles + n_tiles + 1, w->pending,
-                                                           static_cast<unsigned long long*>(w->rec_off.p));
-    w->h_small[6000] = w->pending + total;                    // (rows % 4096 == 0: no tile of the kernel above owns element `rows`)
-    WCU_TRY(cudaMemcpyAsync(static_cast<unsigned long long*>(w->rec_off.p) + rows, w->h_small + 6000, 8, cudaMemcpyHostToDevice, w->stream));
-    if (total / rows > 2048) {                                 // long reads: a warp per row
+    if ((rc = place_records(w, rows, total))) return rc;
+    if (total / rows > 2048) {                                // long reads: a warp per row
       enc::enc_records_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, static_cast<unsigned long long*>(w->rec_off.p), static_cast<int32_t*>(w->ref_pairs.p),
                                                                                    static_cast<uint32_t*>(w->cig_bin.p), static_cast<uint8_t*>(w->stream_buf.p), d_err);
     } else {
@@ -568,7 +722,7 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
       enc::enc_records_kernel<8><<<(warps * 32 + 255) / 256, 256, 0, w->stream>>>(A, static_cast<unsigned long long*>(w->rec_off.p), static_cast<int32_t*>(w->ref_pairs.p),
                                                                                    static_cast<uint32_t*>(w->cig_bin.p), static_cast<uint8_t*>(w->stream_buf.p), d_err);
     }
-    w->st.kernel_launches += 2;
+    w->st.kernel_launches += 1;
     WCU_TRY(cudaEventRecord(w->ev[1], w->stream));
     WCU_TRY(cudaMemcpyAsync(w->h_small + 4096, d_err, 16, cudaMemcpyDeviceToHost, w->stream));
     WCU_TRY(cudaStreamSynchronize(w->stream));
@@ -586,9 +740,46 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
   return BAMSCAN_OK;
 }
 
+// Appends `bytes` device bytes to the file: D2H into a free pinned staging buffer, then its pieces go to the file threads.
+// Returns once every D2H has landed (the device bytes may be overwritten then).
+static int writer_emit(BamWriter* w, const uint8_t* dev, uint64_t bytes) {
+  for (uint64_t at = 0; at < bytes; at += OUT_CHUNK) {
+    const size_t nb = (size_t)std::min<uint64_t>(OUT_CHUNK, bytes - at);
+    int slot = -1;
+    {
+      std::unique_lock<std::mutex> lk(w->mu);
+      w->cv.wait(lk, [&] { for (int b = 0; b < OUT_BUFS; b++) if (!w->out_busy[b]) { slot = b; return true; } return w->file_failed; });
+      if (w->file_failed || slot < 0) { set_error("Failed to write %s record: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      w->out_busy[slot] = FILE_THREADS;
+    }
+    WCU_TRY(cudaMemcpyAsync(w->h_out[slot], dev + at, nb, cudaMemcpyDeviceToHost, w->stream));
+    WCU_TRY(cudaStreamSynchronize(w->stream));
+    {
+      std::lock_guard<std::mutex> lk(w->mu);
+      const size_t per = (nb + FILE_THREADS - 1) / FILE_THREADS;
+      for (int t = 0; t < FILE_THREADS; t++) {
+        const size_t b = std::min(nb, per * t), e = std::min(nb, b + per);
+        w->file_q.push_back(BamWriter::FileJob{slot, b, e - b, w->file_off + b});
+      }
+      w->file_off += nb;
+    }
+    w->cv.notify_all();
+  }
+  WCU_TRY(cudaStreamSynchronize(w->stream));
+  return BAMSCAN_OK;
+}
+
 // Compresses the full members of the first `total` bytes of the stream buffer (all of them when final_flush) and appends them
-// to the file; the remaining tail moves to the front of the buffer.
+// to the file; the remaining tail moves to the front of the buffer.  Plain (FASTQ compression 2): the bytes go to the file as
+// they are, nothing stays behind.
 static int writer_flush_members(BamWriter* w, uint64_t total, bool final_flush) {
+  if (w->plain) {
+    int rc;
+    if (total && (rc = writer_emit(w, static_cast<const uint8_t*>(w->stream_buf.p), total))) return rc;
+    w->st.compressed_bytes += total;
+    w->pending = 0;
+    return BAMSCAN_OK;
+  }
   const uint64_t n_members = final_flush ? (total + dfl::BLOCK - 1) / dfl::BLOCK : total / dfl::BLOCK;
   if (n_members == 0) { w->pending = total; return BAMSCAN_OK; }
   const uint64_t consumed = std::min<uint64_t>(total, n_members * dfl::BLOCK);
@@ -620,29 +811,7 @@ static int writer_flush_members(BamWriter* w, uint64_t total, bool final_flush) 
   // the tail moves to the front (source and destination cannot overlap: the tail is shorter than one member)
   const uint64_t tail = total - consumed;
   if (tail) WCU_TRY(cudaMemcpyAsync(w->stream_buf.p, static_cast<uint8_t*>(w->stream_buf.p) + consumed, tail, cudaMemcpyDeviceToDevice, w->stream));
-  for (uint64_t at = 0; at < packed_bytes; at += OUT_CHUNK) {
-    const size_t nb = (size_t)std::min<uint64_t>(OUT_CHUNK, packed_bytes - at);
-    int slot = -1;
-    {
-      std::unique_lock<std::mutex> lk(w->mu);
-      w->cv.wait(lk, [&] { for (int b = 0; b < OUT_BUFS; b++) if (!w->out_busy[b]) { slot = b; return true; } return w->file_failed; });
-      if (w->file_failed || slot < 0) { set_error("Failed to write BAM record: write(%s) failed", w->path.c_str()); return BAMSCAN_ERR_IO; }
-      w->out_busy[slot] = FILE_THREADS;
-    }
-    WCU_TRY(cudaMemcpyAsync(w->h_out[slot], static_cast<uint8_t*>(w->packed.p) + at, nb, cudaMemcpyDeviceToHost, w->stream));
-    WCU_TRY(cudaStreamSynchronize(w->stream));
-    {
-      std::lock_guard<std::mutex> lk(w->mu);
-      const size_t per = (nb + FILE_THREADS - 1) / FILE_THREADS;
-      for (int t = 0; t < FILE_THREADS; t++) {
-        const size_t b = std::min(nb, per * t), e = std::min(nb, b + per);
-        w->file_q.push_back(BamWriter::FileJob{slot, b, e - b, w->file_off + b});
-      }
-      w->file_off += nb;
-    }
-    w->cv.notify_all();
-  }
-  WCU_TRY(cudaStreamSynchronize(w->stream));
+  if ((rc = writer_emit(w, static_cast<const uint8_t*>(w->packed.p), packed_bytes))) return rc;
   WTRACE("[writer] %llu members, %.1f MB packed: gather + D2H + queueing %.1f ms\n", (unsigned long long)n_members, packed_bytes / 1e6, now_ms() - t_d);
   { float ms = 0, ms2 = 0; cudaEventElapsedTime(&ms, w->ev[2], w->ev[3]); cudaEventElapsedTime(&ms2, w->ev2[0], w->ev2[1]); w->st.ms_deflate += ms + ms2; w->st.ms_total += ms + ms2; }
   w->st.members += n_members; w->st.compressed_bytes += packed_bytes;
@@ -661,11 +830,13 @@ static int writer_finish_impl(BamWriter* w, uint64_t* rows_written) {
     {
       std::unique_lock<std::mutex> lk(w->mu);
       w->cv.wait(lk, [&] { if (!w->file_q.empty()) return false; for (int b = 0; b < OUT_BUFS; b++) if (w->out_busy[b]) return false; return true; });
-      if (w->file_failed) { set_error("Failed to finish BAM stream: write(%s) failed", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (w->file_failed) { set_error("Failed to finish %s stream: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
     }
-    static const uint8_t eof_marker[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-    if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish BAM stream: write(%s) failed", w->path.c_str()); return BAMSCAN_ERR_IO; }
-    w->st.compressed_bytes += 28;
+    if (!w->plain) {
+      static const uint8_t eof_marker[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+      if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish %s stream: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      w->st.compressed_bytes += 28;
+    }
     ::close(w->fd); w->fd = -1;
     w->finished = true;
     WTRACE("[writer] finish: %.1f ms\n", now_ms() - t_fin);
@@ -687,6 +858,9 @@ extern "C" {
 int bamscan_writer_open(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
                         const int32_t* ref_lengths, const struct ArrowSchema* input_schema, const BamWriteOptions* options, BamWriter** out) {
   WRITER_GUARD(writer_open_impl(output_path, sam_header_text, n_ref, ref_names, ref_lengths, input_schema, options, out))
+}
+int bamscan_fastq_writer_open(const char* output_path, const struct ArrowSchema* input_schema, const BamWriteOptions* options, BamWriter** out) {
+  WRITER_GUARD(fastq_writer_open_impl(output_path, input_schema, options, out))
 }
 int bamscan_writer_write(BamWriter* w, const struct ArrowArray* batch) { WRITER_GUARD(writer_write_impl(w, batch)) }
 static int writer_write_device_impl(BamWriter* w, const struct ArrowDeviceArray* batch) {

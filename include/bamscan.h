@@ -285,6 +285,23 @@ int bamscan_writer_finish(BamWriter* w, uint64_t* rows_written);
 int bamscan_writer_stats(const BamWriter* w, BamWriteStats* out);
 void bamscan_writer_free(BamWriter* w);
 
+/* ---- the FASTQ write path: Arrow batches -> FASTQ text encoded on the device -> BGZF members (or plain text) -> file ----
+ * Opens a writer whose handle works with bamscan_writer_write, _write_device, _finish, _stats and _free exactly as above.
+ * `input_schema` columns are looked up BY NAME: name, sequence and quality_scores are required, description is optional, all
+ * Utf8; other columns are ignored, so a BAM scan's batch can be written as FASTQ too (its bases and qualities are written as
+ * stored: reverse-strand reads are NOT reverse-complemented).  Schema errors (BAMSCAN_ERR_SCHEMA) come before the device is
+ * touched; without a device the call fails with BAMSCAN_ERR_CUDA and creates no file.
+ * Options read: struct_size, device_id, compression -- 0 (default) BGZF with LZ77 + dynamic Huffman, 1 BGZF with stored
+ * blocks, 2 plain text (no BGZF, no EOF marker; accepted by FASTQ writers only).  BGZF members hold 0xff00 bytes of text, the
+ * file ends with the BGZF EOF marker.
+ * Each row is written as '@' name [' ' description] '\n' sequence '\n' '+' '\n' quality '\n'; the description and its separator
+ * are left out when it is NULL or empty.  Bytes are written as given (no case folding, sequence and quality lengths are not
+ * compared).  A NULL name / sequence / quality, a '\n' or '\r' in any field, or a space or tab in the name (the file would not
+ * read back as the same rows) is BAMSCAN_ERR_FORMAT with the row in the message.
+ * BamWriteStats of a FASTQ writer: bam_bytes = uncompressed FASTQ text bytes; members and ms_deflate are 0 in plain mode. */
+int bamscan_fastq_writer_open(const char* output_path, const struct ArrowSchema* input_schema, const BamWriteOptions* options,
+                              BamWriter** out);
+
 const char* bamscan_last_error(void);   /* thread-local message of the last failing call on this thread */
 const char* bamscan_version(void);
 

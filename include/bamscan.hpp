@@ -224,4 +224,23 @@ class BamWriteExec {
   BamWriter* w_ = nullptr;
 };
 
+// The FASTQ write path (bamscan_fastq_writer_open): name / description / sequence / quality_scores of input_schema, looked up
+// by name (description optional, other columns ignored).  compression: 0 BGZF, 1 BGZF with stored blocks, 2 plain text.
+class FastqWriteExec {
+ public:
+  FastqWriteExec(const std::string& output_path, const ArrowSchema* input_schema, int32_t compression = 0, int32_t device_id = 0) {
+    BamWriteOptions o; std::memset(&o, 0, sizeof o);
+    o.struct_size = sizeof o; o.device_id = device_id; o.compression = compression;
+    check(bamscan_fastq_writer_open(output_path.c_str(), input_schema, &o, &w_));
+  }
+  FastqWriteExec(FastqWriteExec&& o) noexcept : w_(o.w_) { o.w_ = nullptr; }
+  FastqWriteExec(const FastqWriteExec&) = delete;
+  ~FastqWriteExec() { if (w_) bamscan_writer_free(w_); }
+  void write(const ArrowArray* batch) { check(bamscan_writer_write(w_, batch)); }          // one RecordBatch (struct array), not released here
+  uint64_t finish() { uint64_t n = 0; check(bamscan_writer_finish(w_, &n)); return n; }    // rows written
+  BamWriteStats stats() const { BamWriteStats st; std::memset(&st, 0, sizeof st); check(bamscan_writer_stats(w_, &st)); return st; }
+ private:
+  BamWriter* w_ = nullptr;
+};
+
 }  // namespace bamscan_cpp

@@ -103,6 +103,13 @@ unsafe extern "C" {
     pub fn bamscan_writer_write(w: *mut BamWriter, batch: *const FFI_ArrowArray) -> c_int;
     pub fn bamscan_writer_finish(w: *mut BamWriter, rows_written: *mut u64) -> c_int;
     pub fn bamscan_writer_free(w: *mut BamWriter);
+    // FASTQ write path: the same BamWriter handle and calls; options read: struct_size, device_id, compression (0/1 BGZF, 2 plain)
+    pub fn bamscan_fastq_writer_open(
+        output_path: *const c_char,
+        input_schema: *const FFI_ArrowSchema,
+        options: *const BamWriteOptions,
+        out: *mut *mut BamWriter,
+    ) -> c_int;
 }
 
 #[repr(C)]

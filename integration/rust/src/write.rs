@@ -81,3 +81,56 @@ impl Drop for GpuBamWriter {
         unsafe { ffi::bamscan_writer_free(self.0) }
     }
 }
+
+/// FASTQ output for `FastqTableProvider::insert_into`: `bamscan_fastq_writer_open` + the same `bamscan_writer_*` calls.  The
+/// name / description / sequence / quality_scores columns are looked up by name (description optional, other columns ignored);
+/// `compression`: 0 BGZF, 1 BGZF with stored blocks, 2 plain text.  Bases are written as stored (no reverse-complementing).
+pub struct GpuFastqWriter(*mut ffi::BamWriter);
+unsafe impl Send for GpuFastqWriter {}
+
+impl GpuFastqWriter {
+    /// `compression` None: BGZF for `.bgz` / `.bgzf` / `.gz` paths, plain text otherwise.
+    pub fn open(output_path: &str, input_schema: &SchemaRef, compression: Option<i32>, device_id: i32) -> Result<Self> {
+        let c_path = CString::new(output_path).map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let lower = output_path.to_ascii_lowercase();
+        let bgzf = [".bgz", ".bgzf", ".gz"].iter().any(|s| lower.ends_with(s));
+        let c_schema = FFI_ArrowSchema::try_from(&DataType::Struct(input_schema.fields().clone()))?;
+        let opts = ffi::BamWriteOptions {
+            struct_size: std::mem::size_of::<ffi::BamWriteOptions>() as u32,
+            coordinate_system_zero_based: 1,
+            n_tag_fields: 0,
+            tag_fields: std::ptr::null(),
+            device_id,
+            compression: compression.unwrap_or(if bgzf { 0 } else { 2 }),
+        };
+        let mut raw: *mut ffi::BamWriter = std::ptr::null_mut();
+        if unsafe { ffi::bamscan_fastq_writer_open(c_path.as_ptr(), &c_schema, &opts, &mut raw) } != 0 {
+            return Err(last_error());
+        }
+        Ok(Self(raw))
+    }
+
+    /// One batch (host memory), not consumed.
+    pub fn write(&mut self, batch: &RecordBatch) -> Result<()> {
+        let (array, _schema) = to_ffi(&StructArray::from(batch.clone()).into_data())?;
+        if unsafe { ffi::bamscan_writer_write(self.0, &array) } != 0 {
+            return Err(last_error());
+        }
+        Ok(())
+    }
+
+    /// Flushes the last member and the EOF marker (BGZF) and closes the file; returns the row count.
+    pub fn finish(self) -> Result<u64> {
+        let mut rows = 0u64;
+        if unsafe { ffi::bamscan_writer_finish(self.0, &mut rows) } != 0 {
+            return Err(last_error());
+        }
+        Ok(rows)
+    }
+}
+
+impl Drop for GpuFastqWriter {
+    fn drop(&mut self) {
+        unsafe { ffi::bamscan_writer_free(self.0) }
+    }
+}
