@@ -33,7 +33,7 @@ EXPORTED_SYMBOLS = [
     "bamscan_stream_free", "bamscan_run_device_resident", "bamscan_stream_stats", "bamscan_bench_inflate",
     "bamscan_probe_pcie", "bamscan_check_partition_seams", "bamscan_last_error", "bamscan_version",
     "bamscan_writer_open", "bamscan_writer_write", "bamscan_writer_write_device", "bamscan_writer_finish", "bamscan_writer_stats", "bamscan_writer_free",
-    "bamscan_fastq_writer_open",
+    "bamscan_fastq_writer_open", "bamscan_sam_writer_open",
 ]
 
 
@@ -152,6 +152,7 @@ def load_library():
     L.bamscan_writer_stats.argtypes = [C.c_void_p, C.POINTER(WriteStats)]
     L.bamscan_writer_free.argtypes = [C.c_void_p]
     L.bamscan_fastq_writer_open.argtypes = [C.c_char_p, C.c_void_p, C.POINTER(_WriteOptions), C.POINTER(C.c_void_p)]
+    L.bamscan_sam_writer_open.argtypes = L.bamscan_writer_open.argtypes
     _lib = L
     return L
 
@@ -545,7 +546,8 @@ class BamTableProvider:
         """== TableProvider::insert_into (table_provider.rs:1117-1177) + BamWriteExec::execute: `INSERT OVERWRITE` of `batches`
         (an iterable of pyarrow.RecordBatch with this provider's schema) into this provider's file.  Returns the row count (the
         reference's one-row `count` batch).  sort_on_write is DataFusion's SortExec in front of the writer, not part of it: the
-        rows are written in arrival order and only the header's SO field follows the flag, as in the reference."""
+        rows are written in arrival order and only the header's SO field follows the flag, as in the reference.  A `.sam` path
+        (is_sam_path) is written as plain SAM text through SamWriteExec; `compression` applies to BAM only."""
         if insert_op != "overwrite":
             raise NotImplementedError("BAM insert_into only supports OVERWRITE mode")
         schema = self.schema()
@@ -558,8 +560,13 @@ class BamTableProvider:
         if sort_on_write is None:
             sort_on_write = getattr(self, "_sort_on_write", False)
         overrides = {"bio.bam.sort_order": "coordinate" if sort_on_write else "unsorted"}
-        ex = BamWriteExec(self.file_path, schema, tags, zero_based, overrides, device_id=getattr(self, "device_id", 0), compression=compression)
-        return ex.execute(batches)
+        if is_sam_path(self.file_path):                                                          # plain SAM text (compression is not read)
+            ex = SamWriteExec(self.file_path, schema, tags, zero_based, overrides, device_id=getattr(self, "device_id", 0))
+        else:
+            ex = BamWriteExec(self.file_path, schema, tags, zero_based, overrides, device_id=getattr(self, "device_id", 0), compression=compression)
+        n = ex.execute(batches)
+        self.last_write_stats = ex.stats
+        return n
 
 
 # ---- SURVEY 8 f4: the write path -------------------------------------------------------------------------------------
@@ -609,12 +616,12 @@ def build_bam_header(schema: pa.Schema, tag_fields=None, overrides=None):
 class BamWriteExec:
     """== BamWriteExec (bio-format-bam/src/write_exec.rs:43-110): new(input, output_path, compression, tag_fields,
     coordinate_system_zero_based, schema_metadata_overrides, sort_on_write); `execute` consumes the batches and returns the
-    count.  Only BGZF BAM output (a `.sam` path is the reference's plain-text writer: out of scope)."""
+    count.  Only BGZF BAM output: a `.sam` path is refused here, SamWriteExec writes plain SAM."""
 
     def __init__(self, output_path, input_schema: pa.Schema, tag_fields=None, coordinate_system_zero_based=True,
                  schema_metadata_overrides=None, *, device_id=0, compression=0):
-        if str(output_path).lower().endswith(".sam"):
-            raise BamScanError(-5, "plain SAM output is out of scope for this build (BGZF BAM only)")
+        if is_sam_path(output_path):
+            raise BamScanError(-5, "plain SAM output is out of scope for BamWriteExec (BGZF BAM only): use SamWriteExec")
         self.output_path = str(output_path)
         self.schema = input_schema
         self.tag_fields = list(tag_fields or [])
@@ -625,29 +632,60 @@ class BamWriteExec:
         self.stats = None
 
     def execute(self, batches) -> int:
-        L = load_library()
-        text, names, lens = build_bam_header(self.schema, self.tag_fields, self.overrides)
-        o = _WriteOptions()
-        o.struct_size = C.sizeof(_WriteOptions)
-        o.coordinate_system_zero_based = int(self.zero_based)
-        tag_arr, _keep = _strs(self.tag_fields)
-        o.n_tag_fields = len(self.tag_fields)
-        if tag_arr is not None:
-            o.tag_fields = tag_arr
-        o.device_id = self.device_id
-        o.compression = self.compression
-        name_arr, _keep2 = _strs(names)
-        len_arr = (C.c_int32 * max(1, len(lens)))(*lens)
-        cs = _ArrowSchemaStruct()
-        pa.struct(list(self.schema))._export_to_c(C.addressof(cs))
-        h = C.c_void_p()
-        try:
-            _check(L.bamscan_writer_open(self.output_path.encode(), text.encode(), len(names), name_arr, len_arr, C.addressof(cs), C.byref(o), C.byref(h)))
-        finally:
-            if cs.release:
-                C.CFUNCTYPE(None, C.c_void_p)(cs.release)(C.addressof(cs))
-        n, self.stats = _drive_writer(h, batches, self.schema)
+        n, self.stats = _open_and_drive(load_library().bamscan_writer_open, self, batches)
         return n
+
+
+def is_sam_path(path) -> bool:
+    """The reference's `is_sam`: a path ending in `.sam`, in any case, is plain SAM text (scan and write)."""
+    return str(path).lower().endswith(".sam")
+
+
+class SamWriteExec:
+    """The SAM write path (bamscan_sam_writer_open): the rows BamWriteExec accepts, written as plain SAM text -- the header of
+    build_bam_header(input_schema, tag_fields, overrides), then one line per row in arrival order (no BGZF).  Rows the BAM writer
+    refuses are refused with the same error; so are rows whose line would not read back as the same row (DESIGN 3.9).
+    `execute` takes pyarrow.RecordBatch or DeviceBatch and returns the row count; `.stats` after it."""
+
+    def __init__(self, output_path, input_schema: pa.Schema, tag_fields=None, coordinate_system_zero_based=True,
+                 schema_metadata_overrides=None, *, device_id=0):
+        self.output_path = str(output_path)
+        self.schema = input_schema
+        self.tag_fields = list(tag_fields or [])
+        self.zero_based = bool(coordinate_system_zero_based)
+        self.overrides = dict(schema_metadata_overrides or {})
+        self.device_id = device_id
+        self.compression = 0
+        self.stats = None
+
+    def execute(self, batches) -> int:
+        n, self.stats = _open_and_drive(load_library().bamscan_sam_writer_open, self, batches)
+        return n
+
+
+def _open_and_drive(open_fn, ex, batches):
+    """bamscan_writer_open / bamscan_sam_writer_open with ex's header, references, tags and options, then _drive_writer."""
+    text, names, lens = build_bam_header(ex.schema, ex.tag_fields, ex.overrides)
+    o = _WriteOptions()
+    o.struct_size = C.sizeof(_WriteOptions)
+    o.coordinate_system_zero_based = int(ex.zero_based)
+    tag_arr, _keep = _strs(ex.tag_fields)
+    o.n_tag_fields = len(ex.tag_fields)
+    if tag_arr is not None:
+        o.tag_fields = tag_arr
+    o.device_id = ex.device_id
+    o.compression = ex.compression
+    name_arr, _keep2 = _strs(names)
+    len_arr = (C.c_int32 * max(1, len(lens)))(*lens)
+    cs = _ArrowSchemaStruct()
+    pa.struct(list(ex.schema))._export_to_c(C.addressof(cs))
+    h = C.c_void_p()
+    try:
+        _check(open_fn(ex.output_path.encode(), text.encode(), len(names), name_arr, len_arr, C.addressof(cs), C.byref(o), C.byref(h)))
+    finally:
+        if cs.release:
+            C.CFUNCTYPE(None, C.c_void_p)(cs.release)(C.addressof(cs))
+    return _drive_writer(h, batches, ex.schema)
 
 
 def _drive_writer(h, batches, schema: pa.Schema):

@@ -9,6 +9,9 @@
 // FASTQ writers (bamscan_fastq_writer_open) share everything but the encoder: no header, fq_enc_size_kernel -> scan ->
 // fq_enc_records_kernel write the text into the same stream buffer, which is deflated into the same members -- or, in plain
 // mode (compression 2), copied to the file as it is.
+// SAM writers (bamscan_sam_writer_open) are BAM writers up to enc_size_kernel -- the same staging, row rules and reference
+// lookup -- then sam_size_kernel -> scan -> sam_records_kernel write SAM lines behind the header text, and the plain path
+// copies them to the file.
 #include <fcntl.h>
 #include <unistd.h>
 
@@ -32,6 +35,7 @@
 #include "kernels_deflate.cuh"
 #include "kernels_encode.cuh"
 #include "kernels_fastq_encode.cuh"
+#include "kernels_sam_encode.cuh"
 
 namespace bamscan {
 
@@ -76,7 +80,7 @@ struct DevBuf {
 };
 
 struct WTag { int col; int32_t kind; uint8_t tag[2], sam_type, subtype; };
-enum : int { FMT_BAM = 0, FMT_FASTQ = 1 };
+enum : int { FMT_BAM = 0, FMT_FASTQ = 1, FMT_SAM = 2 };
 
 // Device buffers, pinned staging, stream and events of a writer.  One set per device is kept between writers (cudaMalloc /
 // cudaHostAlloc / cudaFree of a few GB cost more than writing a few million records).
@@ -114,8 +118,8 @@ struct BamWriter : bamscan::WriterRes {
   bool zero_based = true, cigar_binary = false, finished = false;
   int compression = 0;
   int format = FMT_BAM;
-  bool plain = false;                    // FASTQ compression 2: the text goes to the file as it is (no BGZF, no EOF marker)
-  int col[11] = {};                      // BAM: name chrom start flags cigar mapq mate_chrom mate_start seq qual tlen;
+  bool plain = false;                    // FASTQ compression 2, SAM: the text goes to the file as it is (no BGZF, no EOF marker)
+  int col[11] = {};                      // BAM, SAM: name chrom start flags cigar mapq mate_chrom mate_start seq qual tlen;
                                          // FASTQ: name description (-1: absent) sequence quality_scores
   std::vector<WTag> tags;
   int n_cols = 0;
@@ -153,9 +157,23 @@ static const char* enc_err_text(uint32_t code) {
     case enc::ENC_ERR_CIGAR_BIN: return "Failed to decode binary CIGAR";
     case enc::ENC_ERR_REC_LEN: return "record larger than 2 GiB";
     case enc::ENC_ERR_POS: return "position does not fit the 32-bit BAM field";
+    case samenc::SAM_ERR_QNAME: return "invalid QNAME (SAM allows 1 to 254 characters of [!-?A-~])";
+    case samenc::SAM_ERR_SEQ: return "invalid SEQ (SAM allows [A-Za-z=.])";
+    case samenc::SAM_ERR_QUAL: return "invalid QUAL (a quality character above '~')";
+    case samenc::SAM_ERR_TAG_Z: return "invalid Z tag value (SAM allows [ !-~])";
+    case samenc::SAM_ERR_TAG_A: return "invalid A tag value (SAM allows one character of [!-~])";
+    case samenc::SAM_ERR_LINE_LEN: return "SAM line larger than 2 GiB";
+    case samenc::SAM_ERR_INTERNAL: return "internal error: a SAM line does not have its sized length";
     default: return "encode error";
   }
 }
+
+// error class of an encoder code: tag value checks are schema errors, CG-tag overflow is unsupported, the rest format errors
+static int enc_err_class(uint32_t code) {
+  return (code == enc::ENC_ERR_TAG_RANGE || code == enc::ENC_ERR_TAG_HEX || code == enc::ENC_ERR_TAG_CHAR) ? BAMSCAN_ERR_SCHEMA
+         : code == enc::ENC_ERR_CIGAR_OPS ? BAMSCAN_ERR_UNSUPPORTED : BAMSCAN_ERR_FORMAT;
+}
+static const char* fmt_name(const BamWriter* w) { return w->format == FMT_FASTQ ? "FASTQ" : w->format == FMT_SAM ? "SAM" : "BAM"; }
 
 static std::map<std::string, std::string> parse_metadata(const char* md) {
   std::map<std::string, std::string> out;
@@ -203,7 +221,8 @@ static int writer_open_device(BamWriter* w, int device_id);
 static int writer_open_file(BamWriter* w, const char* output_path);
 
 static int writer_open_impl(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
-                            const int32_t* ref_lengths, const ArrowSchema* schema, const BamWriteOptions* options, BamWriter** out) {
+                            const int32_t* ref_lengths, const ArrowSchema* schema, const BamWriteOptions* options, BamWriter** out,
+                            int format = FMT_BAM) {
   if (!output_path || !schema || !out || (n_ref > 0 && (!ref_names || !ref_lengths))) { set_error("bamscan_writer_open: null argument"); return BAMSCAN_ERR_INVALID; }
   BamWriteOptions opt;
   memset(&opt, 0, sizeof opt);
@@ -212,6 +231,7 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
   if (!schema->format || strcmp(schema->format, "+s") != 0) { set_error("bamscan_writer_open: input_schema must be a struct"); return BAMSCAN_ERR_INVALID; }
   std::unique_ptr<BamWriter, void (*)(BamWriter*)> w(new BamWriter(), [](BamWriter* p) { bamscan_writer_free(p); });   // (error paths give the pooled resources back)
   w->path = output_path; w->device = opt.device_id; w->zero_based = opt.coordinate_system_zero_based != 0; w->compression = opt.compression;
+  w->format = format; w->plain = format == FMT_SAM;        // (SAM: plain text, `compression` is not read)
   w->n_cols = (int)schema->n_children;
   // columns by name (sam_record_serializer.rs:27-37: every core column is required; `end` is not read)
   static const char* const names[11] = {"name", "chrom", "start", "flags", "cigar", "mapping_quality", "mate_chrom", "mate_start", "sequence", "quality_scores", "template_length"};
@@ -233,6 +253,10 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
     if (idx < 0) continue;
     const auto md = parse_metadata(schema->children[idx]->metadata);
     if (!md.count("bio.bam.tag.tag") || strlen(tn) != 2) continue;
+    auto alpha = [](char c) { return (c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z'); };
+    if (format == FMT_SAM && !(alpha(tn[0]) && (alpha(tn[1]) || (tn[1] >= '0' && tn[1] <= '9')))) {   // the SAM reader refuses other names
+      set_error("tag column '%s': a SAM tag name must match [A-Za-z][A-Za-z0-9]", tn); return BAMSCAN_ERR_SCHEMA;
+    }
     std::string spec = md.count("bio.bam.tag.type") ? md.at("bio.bam.tag.type") : "Z";
     WTag g; g.col = idx; g.kind = kind_of_format(schema->children[idx]); g.tag[0] = (uint8_t)tn[0]; g.tag[1] = (uint8_t)tn[1]; g.subtype = 0;
     if (spec.size() == 1) g.sam_type = (uint8_t)spec[0];
@@ -274,16 +298,17 @@ static int writer_open_impl(const char* output_path, const char* sam_header_text
     WCU_TRY(cudaMemcpy(w->ref_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice));
     if (!ids.empty()) WCU_TRY(cudaMemcpy(w->ref_ids.p, ids.data(), ids.size() * 4, cudaMemcpyHostToDevice));
   }
-  // BAM header bytes open the uncompressed stream (bam::io::Writer::write_header)
+  // BAM header bytes open the uncompressed stream (bam::io::Writer::write_header); a SAM file starts with the header text as given
   std::string hdr("BAM\1", 4);
-  {
+  if (format == FMT_SAM) { hdr = sam_header_text ? sam_header_text : ""; w->st.bam_bytes = hdr.size(); }
+  else {
     const std::string text = sam_header_text ? sam_header_text : "";
     auto put32 = [&](int32_t v) { hdr.append(reinterpret_cast<const char*>(&v), 4); };
     put32((int32_t)text.size()); hdr += text; put32(n_ref);
     for (int32_t i = 0; i < n_ref; i++) { const std::string n = ref_names[i]; put32((int32_t)n.size() + 1); hdr += n; hdr.push_back('\0'); put32(ref_lengths[i]); }
   }
   if ((rc = w->stream_buf.reserve(hdr.size() + SLICE_BYTES + 65536))) return rc;
-  WCU_TRY(cudaMemcpy(w->stream_buf.p, hdr.data(), hdr.size(), cudaMemcpyHostToDevice));
+  if (!hdr.empty()) WCU_TRY(cudaMemcpy(w->stream_buf.p, hdr.data(), hdr.size(), cudaMemcpyHostToDevice));
   w->pending = hdr.size();
   if ((rc = writer_open_file(w.get(), output_path))) return rc;
   *out = w.release();
@@ -699,14 +724,15 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
                                                                    static_cast<uint32_t*>(w->cig_bin.p), d_err);
     w->st.kernel_launches += 2;
     uint64_t total = 0;
+    const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
     if ((rc = sum_lengths(w, rows, d_err, &total))) return rc;
-    {
-      const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
-      if (e[0]) {
-        set_error("BAM write error: row %u: %s", e[1], enc_err_text(e[0]));
-        return (e[0] == enc::ENC_ERR_TAG_RANGE || e[0] == enc::ENC_ERR_TAG_HEX || e[0] == enc::ENC_ERR_TAG_CHAR) ? BAMSCAN_ERR_SCHEMA
-               : e[0] == enc::ENC_ERR_CIGAR_OPS ? BAMSCAN_ERR_UNSUPPORTED : BAMSCAN_ERR_FORMAT;
-      }
+    if (e[0]) { set_error("%s write error: row %u: %s", fmt_name(w), e[1], enc_err_text(e[0])); return enc_err_class(e[0]); }
+    if (w->format == FMT_SAM) {                                // the rows passed the BAM rules: SAM line lengths + the SAM-only checks
+      if (total / rows > 2048) samenc::sam_size_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint32_t*>(w->rec_len.p), d_err);
+      else samenc::sam_size_kernel<8><<<(((rows + 3) / 4) * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint32_t*>(w->rec_len.p), d_err);
+      w->st.kernel_launches += 1;
+      if ((rc = sum_lengths(w, rows, d_err, &total))) return rc;
+      if (e[0]) { set_error("SAM write error: row %u: %s", e[1], enc_err_text(e[0])); return enc_err_class(e[0]); }
     }
     if (total > SLICE_BYTES && rows > 1) {                   // long reads: fewer rows per pass
       want_rows = std::max<uint32_t>(1, (uint32_t)((double)rows * (double)SLICE_BYTES / (double)total * 0.9));
@@ -714,7 +740,11 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
       continue;
     }
     if ((rc = place_records(w, rows, total))) return rc;
-    if (total / rows > 2048) {                                // long reads: a warp per row
+    if (w->format == FMT_SAM) {
+      const unsigned long long* d_off = static_cast<const unsigned long long*>(w->rec_off.p);
+      if (total / rows > 2048) samenc::sam_records_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_off, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint8_t*>(w->stream_buf.p), d_err);
+      else samenc::sam_records_kernel<8><<<(((rows + 3) / 4) * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_off, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint8_t*>(w->stream_buf.p), d_err);
+    } else if (total / rows > 2048) {                         // long reads: a warp per row
       enc::enc_records_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, static_cast<unsigned long long*>(w->rec_off.p), static_cast<int32_t*>(w->ref_pairs.p),
                                                                                    static_cast<uint32_t*>(w->cig_bin.p), static_cast<uint8_t*>(w->stream_buf.p), d_err);
     } else {
@@ -728,7 +758,7 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
     WCU_TRY(cudaStreamSynchronize(w->stream));
     {
       const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
-      if (e[0]) { set_error("BAM write error: row %u: %s", e[1], enc_err_text(e[0])); return BAMSCAN_ERR_SCHEMA; }
+      if (e[0]) { set_error("%s write error: row %u: %s", fmt_name(w), e[1], enc_err_text(e[0])); return w->format == FMT_SAM ? BAMSCAN_ERR_INVALID : BAMSCAN_ERR_SCHEMA; }
       float ms = 0; cudaEventElapsedTime(&ms, w->ev[0], w->ev[1]); w->st.ms_encode += ms; w->st.ms_total += ms;
     }
     w->st.rows += rows; w->st.bam_bytes += total;
@@ -749,7 +779,7 @@ static int writer_emit(BamWriter* w, const uint8_t* dev, uint64_t bytes) {
     {
       std::unique_lock<std::mutex> lk(w->mu);
       w->cv.wait(lk, [&] { for (int b = 0; b < OUT_BUFS; b++) if (!w->out_busy[b]) { slot = b; return true; } return w->file_failed; });
-      if (w->file_failed || slot < 0) { set_error("Failed to write %s record: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (w->file_failed || slot < 0) { set_error("Failed to write %s record: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
       w->out_busy[slot] = FILE_THREADS;
     }
     WCU_TRY(cudaMemcpyAsync(w->h_out[slot], dev + at, nb, cudaMemcpyDeviceToHost, w->stream));
@@ -830,11 +860,11 @@ static int writer_finish_impl(BamWriter* w, uint64_t* rows_written) {
     {
       std::unique_lock<std::mutex> lk(w->mu);
       w->cv.wait(lk, [&] { if (!w->file_q.empty()) return false; for (int b = 0; b < OUT_BUFS; b++) if (w->out_busy[b]) return false; return true; });
-      if (w->file_failed) { set_error("Failed to finish %s stream: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (w->file_failed) { set_error("Failed to finish %s stream: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
     }
     if (!w->plain) {
       static const uint8_t eof_marker[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-      if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish %s stream: write(%s) failed", w->format == FMT_FASTQ ? "FASTQ" : "BAM", w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish %s stream: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
       w->st.compressed_bytes += 28;
     }
     ::close(w->fd); w->fd = -1;
@@ -861,6 +891,10 @@ int bamscan_writer_open(const char* output_path, const char* sam_header_text, in
 }
 int bamscan_fastq_writer_open(const char* output_path, const struct ArrowSchema* input_schema, const BamWriteOptions* options, BamWriter** out) {
   WRITER_GUARD(fastq_writer_open_impl(output_path, input_schema, options, out))
+}
+int bamscan_sam_writer_open(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
+                            const int32_t* ref_lengths, const struct ArrowSchema* input_schema, const BamWriteOptions* options, BamWriter** out) {
+  WRITER_GUARD(writer_open_impl(output_path, sam_header_text, n_ref, ref_names, ref_lengths, input_schema, options, out, FMT_SAM))
 }
 int bamscan_writer_write(BamWriter* w, const struct ArrowArray* batch) { WRITER_GUARD(writer_write_impl(w, batch)) }
 static int writer_write_device_impl(BamWriter* w, const struct ArrowDeviceArray* batch) {

@@ -302,6 +302,25 @@ void bamscan_writer_free(BamWriter* w);
 int bamscan_fastq_writer_open(const char* output_path, const struct ArrowSchema* input_schema, const BamWriteOptions* options,
                               BamWriter** out);
 
+/* ---- the SAM write path: Arrow batches -> SAM text lines encoded on the device -> plain text file ----
+ * Arguments, schema checks and tag handling are bamscan_writer_open's, and the handle works with bamscan_writer_write,
+ * _write_device, _finish, _stats and _free exactly as above.  The file starts with sam_header_text as given (the text passed to
+ * bamscan_writer_open); each row becomes one line, in arrival order; there is no BGZF and no EOF marker; zero rows leave the
+ * header alone.  Options read: struct_size, coordinate_system_zero_based, n_tag_fields, tag_fields, device_id (`compression` is
+ * not read: BGZF-compressed SAM is not built).
+ * A row is accepted or refused exactly as bamscan_writer_open's writer would, with the same error class and reason; on top of
+ * that a row whose line would not read back as the same row is BAMSCAN_ERR_FORMAT with the row in the message: a name outside
+ * SAMv1 [!-?A-~]{1,254} (NULL or "*" write '*'), a sequence outside [A-Za-z=.] (written as given, no case folding), a quality
+ * character above '~' (characters below '!' are written as '!'), a Z value outside [ !-~], an A value outside [!-~].
+ * A tag column named outside [A-Za-z][A-Za-z0-9] is BAMSCAN_ERR_SCHEMA before the device is touched.
+ * Fields: RNAME / RNEXT are the resolved reference's name, '*' for none, RNEXT '=' for the record's own reference; POS / PNEXT
+ * are 1-based, 0 when missing; CIGAR is rendered from its parsed operations ('*' for none); integer tags are written as
+ * TG:i:<decimal>, f values as Rust's f32 Display prints them (NaN, inf, -inf), H values upper-cased (DESIGN 3.9).
+ * BamWriteStats of a SAM writer: bam_bytes = SAM text bytes (header included) = compressed_bytes; members and ms_deflate are 0. */
+int bamscan_sam_writer_open(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
+                            const int32_t* ref_lengths, const struct ArrowSchema* input_schema, const BamWriteOptions* options,
+                            BamWriter** out);
+
 const char* bamscan_last_error(void);   /* thread-local message of the last failing call on this thread */
 const char* bamscan_version(void);
 

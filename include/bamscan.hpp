@@ -243,4 +243,31 @@ class FastqWriteExec {
   BamWriter* w_ = nullptr;
 };
 
+// The SAM write path (bamscan_sam_writer_open): BamWriteExec's arguments and row rules, written as plain SAM text -- the header
+// text as given, then one line per row (no BGZF).  Rows whose line would not read back as the same row are refused (DESIGN 3.9).
+class SamWriteExec {
+ public:
+  SamWriteExec(const std::string& output_path, const std::string& sam_header_text, const std::vector<std::string>& ref_names,
+               const std::vector<int32_t>& ref_lengths, const ArrowSchema* input_schema, const std::vector<std::string>& tag_fields = {},
+               bool coordinate_system_zero_based = true, int32_t device_id = 0) {
+    if (ref_names.size() != ref_lengths.size()) throw Error(BAMSCAN_ERR_INVALID, "ref_names and ref_lengths differ in length");
+    std::vector<const char*> names, tags;
+    for (auto& n : ref_names) names.push_back(n.c_str());
+    for (auto& t : tag_fields) tags.push_back(t.c_str());
+    BamWriteOptions o; std::memset(&o, 0, sizeof o);
+    o.struct_size = sizeof o; o.coordinate_system_zero_based = coordinate_system_zero_based; o.device_id = device_id;
+    o.n_tag_fields = (int32_t)tags.size(); o.tag_fields = tags.empty() ? nullptr : tags.data();
+    check(bamscan_sam_writer_open(output_path.c_str(), sam_header_text.c_str(), (int32_t)names.size(), names.empty() ? nullptr : names.data(),
+                                  ref_lengths.empty() ? nullptr : ref_lengths.data(), input_schema, &o, &w_));
+  }
+  SamWriteExec(SamWriteExec&& o) noexcept : w_(o.w_) { o.w_ = nullptr; }
+  SamWriteExec(const SamWriteExec&) = delete;
+  ~SamWriteExec() { if (w_) bamscan_writer_free(w_); }
+  void write(const ArrowArray* batch) { check(bamscan_writer_write(w_, batch)); }          // one RecordBatch (struct array), not released here
+  uint64_t finish() { uint64_t n = 0; check(bamscan_writer_finish(w_, &n)); return n; }    // rows written
+  BamWriteStats stats() const { BamWriteStats st; std::memset(&st, 0, sizeof st); check(bamscan_writer_stats(w_, &st)); return st; }
+ private:
+  BamWriter* w_ = nullptr;
+};
+
 }  // namespace bamscan_cpp

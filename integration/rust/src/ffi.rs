@@ -110,6 +110,17 @@ unsafe extern "C" {
         options: *const BamWriteOptions,
         out: *mut *mut BamWriter,
     ) -> c_int;
+    // SAM write path: bamscan_writer_open's arguments, plain SAM text (header text as given, one line per row); compression not read
+    pub fn bamscan_sam_writer_open(
+        output_path: *const c_char,
+        sam_header_text: *const c_char,
+        n_ref: i32,
+        ref_names: *const *const c_char,
+        ref_lengths: *const i32,
+        input_schema: *const FFI_ArrowSchema,
+        options: *const BamWriteOptions,
+        out: *mut *mut BamWriter,
+    ) -> c_int;
 }
 
 #[repr(C)]

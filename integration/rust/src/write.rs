@@ -134,3 +134,70 @@ impl Drop for GpuFastqWriter {
         unsafe { ffi::bamscan_writer_free(self.0) }
     }
 }
+
+/// SAM output for `.sam` targets (the reference's `is_sam` rule): `bamscan_sam_writer_open` with `GpuBamWriter::open`'s
+/// arguments, then the same `bamscan_writer_*` calls.  The file is the header text as given and one SAM line per row (no BGZF).
+/// Rows are accepted and refused as by the BAM writer, plus the SAM-only refusals of DESIGN 3.9.  SOURCE-ONLY: never compiled here.
+pub struct GpuSamWriter(*mut ffi::BamWriter);
+unsafe impl Send for GpuSamWriter {}
+
+impl GpuSamWriter {
+    pub fn open(
+        output_path: &str,
+        sam_header_text: &str,
+        references: &[(String, i32)],
+        input_schema: &SchemaRef,
+        tag_fields: &[String],
+        coordinate_system_zero_based: bool,
+        device_id: i32,
+    ) -> Result<Self> {
+        let c_path = CString::new(output_path).map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let c_text = CString::new(sam_header_text).map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let names: Vec<CString> = references.iter().map(|(n, _)| CString::new(n.as_str()).unwrap()).collect();
+        let name_ptrs: Vec<*const c_char> = names.iter().map(|n| n.as_ptr()).collect();
+        let lens: Vec<i32> = references.iter().map(|(_, l)| *l).collect();
+        let tags: Vec<CString> = tag_fields.iter().map(|t| CString::new(t.as_str()).unwrap()).collect();
+        let tag_ptrs: Vec<*const c_char> = tags.iter().map(|t| t.as_ptr()).collect();
+        let c_schema = FFI_ArrowSchema::try_from(&DataType::Struct(input_schema.fields().clone()))?;
+        let opts = ffi::BamWriteOptions {
+            struct_size: std::mem::size_of::<ffi::BamWriteOptions>() as u32,
+            coordinate_system_zero_based: coordinate_system_zero_based as i32,
+            n_tag_fields: tag_ptrs.len() as i32,
+            tag_fields: tag_ptrs.as_ptr(),
+            device_id,
+            compression: 0,
+        };
+        let mut raw: *mut ffi::BamWriter = std::ptr::null_mut();
+        let rc = unsafe {
+            ffi::bamscan_sam_writer_open(c_path.as_ptr(), c_text.as_ptr(), names.len() as i32, name_ptrs.as_ptr(), lens.as_ptr(), &c_schema, &opts, &mut raw)
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(Self(raw))
+    }
+
+    /// One batch (host memory), not consumed.
+    pub fn write(&mut self, batch: &RecordBatch) -> Result<()> {
+        let (array, _schema) = to_ffi(&StructArray::from(batch.clone()).into_data())?;
+        if unsafe { ffi::bamscan_writer_write(self.0, &array) } != 0 {
+            return Err(last_error());
+        }
+        Ok(())
+    }
+
+    /// Writes the remaining lines and closes the file; returns the row count.
+    pub fn finish(self) -> Result<u64> {
+        let mut rows = 0u64;
+        if unsafe { ffi::bamscan_writer_finish(self.0, &mut rows) } != 0 {
+            return Err(last_error());
+        }
+        Ok(rows)
+    }
+}
+
+impl Drop for GpuSamWriter {
+    fn drop(&mut self) {
+        unsafe { ffi::bamscan_writer_free(self.0) }
+    }
+}
