@@ -1,9 +1,13 @@
 // f32_text.h -- a float tag rendered into a Utf8 column: Rust's `f32::to_string()` (sam_tag_io.rs:670-676).
 //
-// Rust prints the SHORTEST decimal that parses back to the same f32, without an exponent ("0.0000001", "100000000000000000000").
-// The spec used here is the oracle's restatement (oracle/bam_oracle.c::rust_f32_to_string): the smallest number N <= 9 of
-// significant digits for which the value, correctly rounded to N digits (round-half-even on the EXACT binary value), reads
-// back as the same float; then those digits in plain positional notation.
+// Rust prints the SHORTEST decimal that parses back to the same f32, without an exponent ("0.0000001", "100000000000000000000"):
+// the fewest significant digits of any decimal inside the float's rounding interval, and of two such decimals the closer
+// (the even last digit on a tie).  Computed here as: the smallest number N <= 9 of significant digits for which the value,
+// correctly rounded to N digits (round-half-even on the EXACT binary value), reads back as the same float -- or, when that
+// rounded down at a power of two (m = 2^23, where the float below is half as far away as the one above), the N-digit value
+// one unit above, which can lie inside the wider upper half when the rounded one misses the narrow lower half (2^87:
+// 1.5474250e26 does not read back, 1.5474251e26 does).  Then those digits in plain positional notation.  The exact
+// reference is oracle/f32_exact.py::display (tests/test_f32_exact.py).
 //
 // No floating point and no library: the exact decimal expansion of m * 2^e is built with a small big-integer (m * 5^-e for
 // e < 0, at most 370 bits), rounded on its digit string, and the round-trip test |R - v| < half an ulp (ties: even mantissa)
@@ -90,20 +94,28 @@ F32T_HD F32T_NOINLINE inline uint32_t f32_to_text(uint32_t bits, uint8_t* out) {
       if (dv[N] > 5) up = true;
       else if (dv[N] == 5) { bool rest = false; for (int i = N + 1; i < n; i++) if (dv[i]) rest = true; up = rest || (dv[N - 1] & 1); }
     }
-    if (up) { int i = N; while (i >= 0) { if (rv[i] == 9) { rv[i] = 0; i--; } else { rv[i]++; break; } } }
     if (N >= n) break;                               // all digits: exact
-    // diff = |rv - dv| as n + 1 digits, then two more zeros (units of 10^-(F+2))
-    uint8_t df[136];
-    int borrow = 0;
-    for (int i = n; i >= 0; i--) {
-      const int a = up ? rv[i] : (i ? dv[i - 1] : 0), b = up ? (i ? dv[i - 1] : 0) : rv[i];
-      int d = a - b - borrow;
-      if (d < 0) { d += 10; borrow = 1; } else borrow = 0;
-      df[i] = (uint8_t)d;
+    bool inside = false;
+    for (;;) {
+      if (up) { int i = N; while (i >= 0) { if (rv[i] == 9) { rv[i] = 0; i--; } else { rv[i]++; break; } } }
+      // diff = |rv - dv| as n + 1 digits, then two more zeros (units of 10^-(F+2))
+      uint8_t df[136];
+      int borrow = 0;
+      for (int i = n; i >= 0; i--) {
+        const int a = up ? rv[i] : (i ? dv[i - 1] : 0), b = up ? (i ? dv[i - 1] : 0) : rv[i];
+        int d = a - b - borrow;
+        if (d < 0) { d += 10; borrow = 1; } else borrow = 0;
+        df[i] = (uint8_t)d;
+      }
+      df[n + 1] = 0; df[n + 2] = 0;
+      const int c = up ? f32t_cmp(df, n + 3, hu, nhu) : f32t_cmp(df, n + 3, hd, nhd);
+      inside = c < 0 || (c == 0 && (m & 1u) == 0u);
+      // rounded down at a power of two and outside the narrow lower half: the N-digit value one unit above v may still be
+      // inside the upper half, which is twice as wide
+      if (inside || up || !boundary) break;
+      up = true;
     }
-    df[n + 1] = 0; df[n + 2] = 0;
-    const int c = up ? f32t_cmp(df, n + 3, hu, nhu) : f32t_cmp(df, n + 3, hd, nhd);
-    if (c < 0 || (c == 0 && (m & 1u) == 0u)) break;
+    if (inside) break;
   }
   if (N > 9) N = 9;
   // significant digits of the candidate and its decimal exponent

@@ -422,13 +422,36 @@ static int append_array(Col *c, uint8_t st, const uint8_t *p, int32_t count, cha
   return 0;
 }
 
-/* Rust `f32::to_string()` (shortest round-trip digits, never exponent form). */
+/* "%.*e" text `s` (no sign) -> the decimal one unit above it in the last digit, with as many digits ("9.9e5" -> "1.0e6"). */
+static void f32_next_up(const char *s, char *out, size_t cap) {
+  char d[16]; int nd = 0; const char *p = s;
+  for (; *p != 'e'; p++) if (*p != '.') d[nd++] = *p;
+  int x = atoi(p + 1), i = nd - 1;
+  while (i >= 0 && d[i] == '9') d[i--] = '0';
+  if (i >= 0) d[i]++; else { d[0] = '1'; x++; }
+  snprintf(out, cap, "%c.%.*se%d", d[0], nd - 1, d + 1, x);
+}
+
+/* Rust `f32::to_string()` (shortest digits inside the rounding interval, the closer of two; never exponent form): the
+ * smallest precision whose correctly rounded "%.*e" reads back -- or, when that rounded down, the value one unit above it,
+ * which can read back where the rounded one does not only at a power of two (the float below is half as far away as the
+ * one above).  oracle/f32_exact.py is the exact reference. */
 static size_t rust_f32_to_string(float v, char *out, size_t cap) {
   if (v != v) return (size_t)snprintf(out, cap, "NaN");
   if (v == 1.0f / 0.0f) return (size_t)snprintf(out, cap, "inf");
   if (v == -1.0f / 0.0f) return (size_t)snprintf(out, cap, "-inf");
-  char tmp[64]; int prec;
-  for (prec = 1; prec <= 9; prec++) { snprintf(tmp, sizeof tmp, "%.*e", prec - 1, (double)v); if (strtof(tmp, NULL) == v) break; }
+  char tmp[64], alt[64]; int prec;
+  const int minus = v < 0 || (v == 0 && 1.0f / v < 0);
+  const float a = minus ? -v : v;
+  for (prec = 1; prec <= 9; prec++) {
+    snprintf(tmp, sizeof tmp, "%.*e", prec - 1, (double)a);
+    if (strtof(tmp, NULL) == a) break;
+    if (strtod(tmp, NULL) < (double)a) {
+      f32_next_up(tmp, alt, sizeof alt);
+      if (strtof(alt, NULL) == a) { memcpy(tmp, alt, sizeof tmp); break; }
+    }
+  }
+  if (minus) { memmove(tmp + 1, tmp, strlen(tmp) + 1); tmp[0] = '-'; }
   /* tmp = d.ddddde[+-]XX -> expand to plain decimal */
   char digits[16]; int nd = 0; int neg = 0; const char *s = tmp;
   if (*s == '-') { neg = 1; s++; }

@@ -41,7 +41,9 @@ class WriteError(Exception):
 
 # ---------------------------------------------------------------------------------------------------------------------
 # f32 text: oracle/bam_oracle.c::rust_f32_to_string -- the smallest precision N <= 9 whose correctly rounded "%.{N-1}e" reads
-# back as the same f32, written in plain positional notation
+# back as the same f32, or, when that rounded down, whose value one unit above reads back (possible only at a power of two,
+# where the float below is half as far away as the one above), written in plain positional notation.  The exact reference
+# is oracle/f32_exact.py.
 
 def _f32_value(bits: int) -> Fraction:
     e, m = (bits >> 23) & 0xff, bits & 0x7fffff
@@ -59,6 +61,16 @@ def _reads_back(text: str, bits: int) -> bool:
     return abs(r - v) < gap or (abs(r - v) == gap and bits % 2 == 0)
 
 
+def _next_up(t: str) -> str:
+    """The "d.ddde+x" decimal one unit above `t` in its last digit, with as many digits ("9.9e+05" -> "1.0e+06")."""
+    mant, exp10 = t.split("e")
+    digits = mant.replace(".", "")
+    up, x = str(int(digits) + 1), int(exp10)
+    if len(up) > len(digits):
+        up, x = up[:-1], x + 1
+    return f"{up[0]}.{up[1:]}e{x}" if len(up) > 1 else f"{up}e{x}"
+
+
 def f32_text(bits: int) -> str:
     bits &= 0xffffffff
     sign, mag = bits >> 31, bits & 0x7fffffff
@@ -73,6 +85,10 @@ def f32_text(bits: int) -> str:
         t = f"{x:.{prec - 1}e}"
         if _reads_back(t, mag):
             break
+        if Fraction(t) < x:
+            t = _next_up(t)
+            if _reads_back(t, mag):
+                break
     mant, exp10 = t.split("e")
     digits, exp10 = mant.replace(".", "").rstrip("0") or "0", int(exp10)
     if exp10 < 0:

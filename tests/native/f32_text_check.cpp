@@ -1,5 +1,6 @@
 // Checks csrc/f32_text.h (integer-only shortest round-trip text of an f32, what the GPU runs) against the oracle's rule
-// (oracle/bam_oracle.c::rust_f32_to_string: smallest precision whose correctly rounded "%.*e" reads back with strtof).
+// (oracle/bam_oracle.c::rust_f32_to_string: smallest precision whose correctly rounded "%.*e" reads back with strtof, or
+// when that rounded down, the value one unit above it -- the power-of-two case).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -7,12 +8,31 @@
 #include <random>
 #include "../../datafusion-bio-formats_b200/csrc/f32_text.h"
 
+static void next_up(const char* s, char* out, size_t cap) {
+  char d[16]; int nd = 0; const char* p = s;
+  for (; *p != 'e'; p++) if (*p != '.') d[nd++] = *p;
+  int x = atoi(p + 1), i = nd - 1;
+  while (i >= 0 && d[i] == '9') d[i--] = '0';
+  if (i >= 0) d[i]++; else { d[0] = '1'; x++; }
+  snprintf(out, cap, "%c.%.*se%d", d[0], nd - 1, d + 1, x);
+}
+
 static size_t oracle_rule(float v, char* out) {
   if (v != v) return (size_t)sprintf(out, "NaN");
   if (v == 1.0f / 0.0f) return (size_t)sprintf(out, "inf");
   if (v == -1.0f / 0.0f) return (size_t)sprintf(out, "-inf");
-  char tmp[64]; int prec;
-  for (prec = 1; prec <= 9; prec++) { snprintf(tmp, sizeof tmp, "%.*e", prec - 1, (double)v); if (strtof(tmp, NULL) == v) break; }
+  char tmp[64], alt[64]; int prec;
+  const bool minus = v < 0 || (v == 0 && 1.0f / v < 0);
+  const float a = minus ? -v : v;
+  for (prec = 1; prec <= 9; prec++) {
+    snprintf(tmp, sizeof tmp, "%.*e", prec - 1, (double)a);
+    if (strtof(tmp, NULL) == a) break;
+    if (strtod(tmp, NULL) < (double)a) {
+      next_up(tmp, alt, sizeof alt);
+      if (strtof(alt, NULL) == a) { memcpy(tmp, alt, sizeof tmp); break; }
+    }
+  }
+  if (minus) { memmove(tmp + 1, tmp, strlen(tmp) + 1); tmp[0] = '-'; }
   char digits[16]; int nd = 0, neg = 0; const char* s = tmp;
   if (*s == '-') { neg = 1; s++; }
   for (; *s && *s != 'e'; s++) if (*s != '.') digits[nd++] = *s;

@@ -134,7 +134,7 @@ def test_insert_into_overwrites_the_providers_file(tmp_path):
     """== `INSERT OVERWRITE`: TableProvider::insert_into (table_provider.rs:1117-1177)."""
     import shutil, bamscan
     dst = tmp_path / "t.bam"
-    shutil.copy(GOLDEN / "multi_chrom.bam", dst)
+    shutil.copyfile(GOLDEN / "multi_chrom.bam", dst)      # contents only: a read-only checkout's mode would make dst read-only
     p = bamscan.BamTableProvider(str(dst), None, True, ["NM"], index_path="")
     batches = list(p.scan(None, [], None).execute(0))
     keep = [b.slice(0, b.num_rows // 2) for b in batches]
