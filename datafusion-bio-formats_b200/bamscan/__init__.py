@@ -26,7 +26,7 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE.parent / "libbamscan.so"
 
 EXPORTED_SYMBOLS = [
-    "bamscan_open", "bamscan_open_fastq", "bamscan_close", "bamscan_schema", "bamscan_describe_tags", "bamscan_classify_filters", "bamscan_plan",
+    "bamscan_open", "bamscan_open_fastq", "bamscan_open_fasta", "bamscan_close", "bamscan_schema", "bamscan_describe_tags", "bamscan_classify_filters", "bamscan_plan",
     "bamscan_plan_num_partitions", "bamscan_plan_schema", "bamscan_plan_free", "bamscan_plan_num_ranges",
     "bamscan_plan_range_info", "bamscan_plan_partition_regions", "bamscan_extract_regions", "bamscan_balance_partitions",
     "bamscan_execute", "bamscan_next", "bamscan_execute_device", "bamscan_next_device",
@@ -121,6 +121,7 @@ def load_library():
     L.bamscan_version.restype = C.c_char_p
     L.bamscan_open.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
     L.bamscan_open_fastq.argtypes = [C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
+    L.bamscan_open_fasta.argtypes = [C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
     L.bamscan_close.argtypes = [C.c_void_p]
     L.bamscan_schema.argtypes = [C.c_void_p, C.c_void_p]
     L.bamscan_describe_tags.argtypes = [C.c_void_p, C.c_int32, C.c_char_p, C.c_uint64, C.POINTER(C.c_uint64)]
@@ -808,6 +809,35 @@ class FastqTableProvider(BamTableProvider):
         n = ex.execute(batches)
         self.last_write_stats = ex.stats
         return n
+
+
+class FastaTableProvider(BamTableProvider):
+    """A provider for BGZF-compressed FASTA (bamscan_open_fasta): `FastaTableProvider(file_path, object_storage_options)`;
+    schema name / description / sequence (Utf8, description nullable).  `scan` with target_partitions > 1 uses BGZF block ranges
+    balanced by compressed bytes (a record belongs to the range that holds its '>'); no filter is pushed down and `limit` is not
+    applied, as for FastqTableProvider; everything else is BamTableProvider's."""
+
+    def __init__(self, file_path, object_storage_options=None, *, device_id=0, batch_rows=0, chunk_inflated_bytes=0,
+                 skip_crc=False, debug_flags=0):
+        if object_storage_options is not None:
+            raise BamScanError(-5, "remote object storage is out of scope for this build (local files only)")
+        L = load_library()
+        o = _Options()
+        o.struct_size = C.sizeof(_Options)
+        o.device_id = device_id
+        o.batch_rows = batch_rows
+        o.chunk_inflated_bytes = chunk_inflated_bytes
+        o.skip_crc = int(skip_crc)
+        o.debug_flags = debug_flags
+        self._h = C.c_void_p()
+        _check(L.bamscan_open_fasta(str(file_path).encode(), C.byref(o), C.byref(self._h)))
+        self.file_path = str(file_path)
+        self.device_id = device_id
+        self._schema = None
+
+    def scan(self, projection=None, filters=None, limit=None, *, target_partitions=1) -> BamExec:
+        mode = "block_range" if target_partitions > 1 else "reference"
+        return super().scan(projection, None, limit, target_partitions=target_partitions, partition_mode=mode)
 
 
 def check_partition_seams(stats_list):

@@ -62,7 +62,8 @@ struct BaiIndex {
 // == BamTableProvider (table_provider.rs:314-335)
 struct BamFile {
   int format = 0;            // 0: BAM; 1: BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index;
-                             // 2: plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index
+                             // 2: plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index;
+                             // 3: BGZF-compressed FASTA (kernels_fasta.cuh): three Utf8 columns, records of up to 1 GiB, no index
   std::string path, index_path;
   uint8_t* data = nullptr;   // whole file: read-only mapping (O_RDONLY / PROT_READ, not page-locked); small files: a plain copy
   uint64_t size = 0;

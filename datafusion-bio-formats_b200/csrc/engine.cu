@@ -35,6 +35,7 @@
 #include "kernels_inflate.cuh"
 #include "kernels_inflate_cta.cuh"
 #include "kernels_fastq.cuh"
+#include "kernels_fasta.cuh"
 #include "kernels_sam.cuh"
 
 namespace bamscan {
@@ -54,6 +55,7 @@ bool filter_is_record_pushable(const BamFile& f, const BamScanFilter& flt);
 constexpr uint32_t HEADROOM = 16u << 20;      // room in front of a chunk for the carried-over tail record
 constexpr uint32_t INFL_PAD = 1u << 20;   // slack behind a chunk: literal runs of a corrupt member may overshoot before the check
 constexpr uint32_t MAX_BLOCK_SIZE = 256u << 20;
+constexpr int FA_HFLAGS = 620;            // FASTA flag words [16, 64) of a chunk on the mapped flags page (nothing else uses [620, 668))
 
 static bool g_have_device = false;
 // Page-locked host memory.  Without a device (planning-only use: open / schema / classify / plan) plain memory is
@@ -197,6 +199,7 @@ struct PendingBatch {
   uint64_t rows = 0;
   size_t arena_bytes = 0;
   size_t err_off = 0;
+  uint64_t row0 = 0;               // rows of the partition in front of this batch (FASTA error messages)
   cudaEvent_t done = nullptr;
   bool valid = false;
 };
@@ -227,6 +230,11 @@ struct BamScanStream {
   size_t range_idx = 0;
   std::vector<ChunkPlan> chunks; size_t chunk_idx = 0; bool range_open = false; bool finished = false;
   uint32_t carry_len = 0; bool have_h2d_ahead = false; uint32_t ext_blocks = 8; bool need_spec = false;
+  // room in front of a chunk for the carried tail record: HEADROOM for BAM, SAM and FASTQ; a FASTA record may be far longer, so
+  // for FASTA it grows to the carried record.  desc_base: the room a slot's member descriptors were built for (issue_h2d)
+  uint32_t headroom = HEADROOM, desc_base[2] = {HEADROOM, HEADROOM};
+  bool fa_lead_nl = true;     // FASTA: the byte in front of the next chunk is a '\n' (its first byte starts a line)
+  bool fa_leading = false;    // FASTA: the range owns the file's first byte and no '>' was found yet
   // unique decoded columns
   std::vector<int32_t> dec_cols;          // schema indices, unique
   std::vector<int32_t> out_to_dec;        // projection position -> index into dec_cols
@@ -235,6 +243,8 @@ struct BamScanStream {
   // SAM (format 2): per slot the parsed lines, record sizes -> offsets, "QUAL is *" flags, scan tiles and the transcoded BAM records;
   // the reference names sorted bytewise for RNAME / RNEXT lookups
   DeviceBuf d_samline[2], d_samsize[2], d_qabs[2], d_samtiles[2], d_bam[2], d_samrefs;
+  // FASTA (format 3): per slot the line index of every record start and every line's destination in the sequence text
+  DeviceBuf d_fastarts[2], d_faseq[2];
   cudaEvent_t ev_text_free[2] = {nullptr, nullptr}, ev_ing[2][2] = {};   // the write pass has read a slot's text; ingest copy timing
   bool tail_seen = false, range_stop = false;   // per-reference unmapped tail state (physical_exec.rs:1203-1215)
   const uint8_t* d_comp_all = nullptr; DeviceBuf d_comp_all_buf; uint64_t comp_all_c0 = 0;
@@ -246,7 +256,10 @@ struct BamScanStream {
   // rows of the current chunk that are not decoded yet: a chunk is one inflate wave, a batch is one slice of its rows
   bool slice_pending = false;    // a decode slice whose time / error word has not been collected (flush_slice)
   int64_t launched_chunk = -1;   // index in `chunks` of a chunk whose inflate + boundary kernels are already queued (run_chunk phase 1)
-  struct { const uint8_t* U = nullptr; const uint32_t* recoff = nullptr; const uint8_t* qabs = nullptr; uint32_t n = 0, pos = 0, rows_per_slice = 0; bool long_records = false; uint64_t ubytes = 0; cudaStream_t cs = nullptr; } cur;
+  struct { const uint8_t* U = nullptr; const uint32_t* recoff = nullptr; const uint8_t* qabs = nullptr; uint32_t n = 0, pos = 0, rows_per_slice = 0; bool long_records = false; uint64_t ubytes = 0; cudaStream_t cs = nullptr;
+           // FASTA: the chunk's lines, their destinations, the newline scan's tile bases and the decode slices (first record, first byte)
+           const uint32_t* fa_lines = nullptr; const uint32_t* fa_seqpos = nullptr; const uint32_t* fa_tile_base = nullptr; uint32_t fa_lo = 0, fa_hi = 0;
+           uint32_t fa_slice_rec[FA_MAX_SLICES + 1] = {}, fa_slice_byte[FA_MAX_SLICES + 1] = {}, fa_slice = 0; } cur;
   PendingBatch pending;
   std::vector<ReadyBatch> ready; size_t ready_pos = 0;
   BamScanStats st{};
@@ -341,6 +354,7 @@ static int stream_init(BamScanStream* s) {
   // per-scan state
   s->range_idx = 0; s->chunks.clear(); s->chunk_idx = 0; s->range_open = false; s->finished = false;
   s->carry_len = 0; s->have_h2d_ahead = false; s->ext_blocks = 8; s->need_spec = false; s->tail_seen = false; s->range_stop = false;
+  s->headroom = HEADROOM; s->desc_base[0] = s->desc_base[1] = HEADROOM;
   s->dec_cols.clear(); s->out_to_dec.clear(); s->arena_flip = 0; s->cur.n = s->cur.pos = 0; s->launched_chunk = -1; s->slice_pending = false; s->pending = PendingBatch(); s->ready.clear(); s->ready_pos = 0;
   s->st = BamScanStats{}; s->st.first_record_uoff = ~0ull; s->error = 0; s->d_comp_all = nullptr; s->comp_all_c0 = 0;
   if (!s->resources_ready) {
@@ -433,7 +447,8 @@ static void stream_destroy(BamScanStream* s, bool recycle = true) {
   }
   for (auto* b : {&s->d_comp[0], &s->d_comp[1], &s->d_blk[0], &s->d_blk[1], &s->d_infl[0], &s->d_infl[1], &s->d_carry, &s->d_status[0], &s->d_status[1], &s->d_flags[0], &s->d_flags[1], &s->d_seg[0], &s->d_seg[1],
                   &s->d_recoff[0], &s->d_recoff[1], &s->d_recoff2[0], &s->d_recoff2[1], &s->d_keep[0], &s->d_keep[1], &s->d_tiles, &s->d_totals, &s->d_scratch, &s->d_arena[0], &s->d_arena[1], &s->d_refs, &s->d_comp_all_buf, &s->d_sorted,
-                  &s->d_samline[0], &s->d_samline[1], &s->d_samsize[0], &s->d_samsize[1], &s->d_qabs[0], &s->d_qabs[1], &s->d_samtiles[0], &s->d_samtiles[1], &s->d_bam[0], &s->d_bam[1], &s->d_samrefs}) b->release();
+                  &s->d_samline[0], &s->d_samline[1], &s->d_samsize[0], &s->d_samsize[1], &s->d_qabs[0], &s->d_qabs[1], &s->d_samtiles[0], &s->d_samtiles[1], &s->d_bam[0], &s->d_bam[1], &s->d_samrefs,
+                  &s->d_fastarts[0], &s->d_fastarts[1], &s->d_faseq[0], &s->d_faseq[1]}) b->release();
   if (s->h_flags) cudaFreeHost(s->h_flags);
   for (auto& hd : s->h_descs) if (hd) cudaFreeHost(hd);
   for (auto& hs : s->h_stage) if (hs) cudaFreeHost(hs);
@@ -463,7 +478,8 @@ static const uint64_t SLICE_BYTES = 768ull << 20;
 static uint64_t chunk_cap_bytes(const BamFile& f) {
   if (f.chunk_bytes) return f.chunk_bytes;
   if (f.format == 2) return 512ull << 20;          // SAM: text bytes per chunk (no inflate wave to fill)
-  return std::min<uint64_t>((uint64_t)inflate_wave_members(f.device) * 65280ull + 65536ull, 3ull << 30);
+  // FASTA: the carried record (up to 1 GiB) sits in front of the chunk, and chunk offsets are u32
+  return std::min<uint64_t>((uint64_t)inflate_wave_members(f.device) * 65280ull + 65536ull, f.format == 3 ? 2ull << 30 : 3ull << 30);
 }
 static void plan_chunks(const BamFile& f, uint32_t b0, uint32_t b1, bool extension, std::vector<ChunkPlan>* out) {
   const uint32_t wave = inflate_wave_members(f.device);
@@ -552,7 +568,8 @@ static int issue_h2d(BamScanStream* s, const ChunkPlan& c, int slot) {
     s->h_descs_cap[slot] = cap;
   }
   BlockDesc* descs = s->h_descs[slot];
-  uint32_t uoff = HEADROOM, nb = 0;
+  uint32_t uoff = s->headroom, nb = 0;
+  s->desc_base[slot] = s->headroom;
   for (uint32_t b = c.b0; b < c.b1; b++) {
     const BgzfBlock& B = f->blocks[b];
     if (B.isize) { BlockDesc d; d.cdata_off = (uint32_t)(B.coff - c.c0) + B.cdata_off; d.cdata_len = B.csize - B.cdata_off - 8; d.isize = B.isize; d.crc = B.crc; d.uoff = uoff; descs[nb++] = d; }
@@ -600,7 +617,12 @@ static int decode_slice(BamScanStream* s, bool* produced) {
   int rc;
   if ((rc = flush_slice(s))) return rc;
   const uint8_t* U = s->cur.U;
-  const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
+  const bool fasta = f->format == 3;
+  // FASTA: the slices fa_frame cut (each holds whole records, about SLICE_BYTES of text); otherwise rows_per_slice rows
+  const uint32_t n = fasta ? s->cur.fa_slice_rec[s->cur.fa_slice + 1] - s->cur.pos : std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
+  const uint32_t fa_b0 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice] : 0, fa_b1 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice + 1] : 0;
+  if (fasta) s->cur.fa_slice++;
+  const uint64_t row0 = s->st.rows;
   const uint32_t* d_recoff = s->cur.recoff + (size_t)s->cur.pos * (f->format == 1 ? 4 : 1);
   const uint8_t* d_qabs = s->cur.qabs ? s->cur.qabs + s->cur.pos : nullptr;
   s->cur.pos += n;
@@ -618,7 +640,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       ColLayout& L = cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = f->fields[L.schema_idx].kind;
       const int c_id = L.schema_idx;
       bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-      L.has_validity = f->format == 1 ? c_id == 1 : (c_id >= 12 || c_id == 1 || c_id == 2 || c_id == 3 || c_id == 7 || c_id == 8);
+      L.has_validity = (f->format == 1 || fasta) ? c_id == 1 : (c_id >= 12 || c_id == 1 || c_id == 2 || c_id == 3 || c_id == 7 || c_id == 8);
       if (L.has_validity) L.validity_off = AB.take(bm_bytes);
       if (is_var) L.offsets_off = AB.take(off_bytes); else L.values_off = AB.take(val_bytes);
       if (c_id >= 12 && is_var) { src_off[i] = scratch; scratch += align_up(val_bytes, 256); }
@@ -647,8 +669,8 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       uint32_t* v = L.has_validity ? reinterpret_cast<uint32_t*>(A + L.validity_off) : nullptr;
       int32_t* offs = reinterpret_cast<int32_t*>(A + L.offsets_off);
       uint32_t* vals = reinterpret_cast<uint32_t*>(A + L.values_off);
-      static const int fq_slot[4] = {0, 1, 9, 10};      // FASTQ: name, description (nullable Utf8 like chrom), sequence, quality_scores
-      switch (f->format == 1 ? fq_slot[L.schema_idx] : L.schema_idx) {
+      static const int fq_slot[4] = {0, 1, 9, 10};      // FASTQ: name, description (nullable Utf8 like chrom), sequence, quality_scores; FASTA: the first three
+      switch ((f->format == 1 || fasta) ? fq_slot[L.schema_idx] : L.schema_idx) {
         case 0: DP.l_name = offs; break;
         case 1: DP.l_chrom = offs; DP.v_chrom = v; break;
         case 2: DP.start = vals; DP.v_start = v; break;
@@ -678,9 +700,14 @@ static int decode_slice(BamScanStream* s, bool* produced) {
     DP.n_tags = n_tags;
     CU_TRY(cudaMemsetAsync(A + err_off, 0, 64, cs));
     FastqCols FC;
+    FastaCols AC;
     if (f->format == 1) {
       FC = FastqCols{U, d_recoff, n, DP.l_name, DP.l_chrom, DP.l_seq, DP.l_qual, DP.v_chrom, nullptr, nullptr, nullptr, nullptr, DP.err};
       fq_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(FC);
+    }
+    else if (fasta) {
+      AC = FastaCols{U, s->cur.fa_lines, d_recoff, s->cur.fa_seqpos, n, DP.l_name, DP.l_chrom, DP.l_seq, DP.v_chrom, nullptr, nullptr, DP.err};
+      fa_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(AC);
     }
     else if (s->cur.long_records) {
       CU_TRY(cudaMemsetAsync(A, 0, regionA, cs));                                        // validity words are OR-ed in
@@ -735,7 +762,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
         uint8_t* d = A + L.data_off;
         switch (L.schema_idx) {
           case 0: DP.d_name = d; break; case 1: DP.d_chrom = d; break; case 5: DP.d_cigar = d; break; case 7: DP.d_mchrom = d; break;
-          case 2: if (f->format == 1) DP.d_seq = d; break; case 3: if (f->format == 1) DP.d_qual = d; break;
+          case 2: if (f->format == 1 || fasta) DP.d_seq = d; break; case 3: if (f->format == 1) DP.d_qual = d; break;
           case 9: DP.d_seq = d; break; case 10: DP.d_qual = d; break;
           default: DP.tags[tag_slot[i]].data = d;
         }
@@ -745,12 +772,23 @@ static int decode_slice(BamScanStream* s, bool* produced) {
         FC.d_name = DP.d_name; FC.d_desc = DP.d_chrom; FC.d_seq = DP.d_seq; FC.d_qual = DP.d_qual;
         fq_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(FC);
       }
+      else if (fasta) {
+        AC.l_name = DP.l_name; AC.l_desc = DP.l_chrom; AC.l_seq = DP.l_seq; AC.v_desc = DP.v_chrom; AC.err = DP.err;      // (rebased with the arena)
+        AC.d_name = DP.d_name; AC.d_desc = DP.d_chrom;
+        if (AC.d_name || AC.d_desc) { fa_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(AC); s->st.kernel_launches++; }
+        if (DP.d_seq && fa_b1 > fa_b0) {
+          const uint32_t t0 = (fa_b0 - s->cur.fa_lo) / FQ_TILE, t1 = (fa_b1 - s->cur.fa_lo + FQ_TILE - 1) / FQ_TILE;
+          FastaSeq SQ{U, s->cur.fa_lines, s->cur.fa_seqpos, s->cur.fa_tile_base, d_recoff, n, s->cur.fa_lo, s->cur.fa_hi, t0, DP.d_seq, DP.err};
+          fa_seq_kernel<<<t1 - t0, 256, 0, cs>>>(SQ);
+          s->st.kernel_launches++;
+        }
+      }
       // short reads: 8 lanes per record (4 records per warp); long reads (and debug_flags bit 1): a warp per record
       else if (s->cur.long_records)
         decode_var_kernel<32><<<std::min<uint32_t>((n + VAR_WARPS - 1) / VAR_WARPS, 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
       else
         decode_var_kernel<8><<<std::min<uint32_t>((n + VAR_WARPS * 4 - 1) / (VAR_WARPS * 4), 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
-      s->st.kernel_launches++;
+      if (!fasta) s->st.kernel_launches++;
     }
     const size_t arena_bytes = AB.pos;
     s->st.rows += n; s->st.batches++;
@@ -769,7 +807,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       P.owner = new BatchOwner();
       P.owner->device = f->device; P.owner->refs = 1;
       if (cudaMalloc(&P.owner->dev, arena_bytes) != cudaSuccess) { delete P.owner; P.owner = nullptr; set_error("cudaMalloc(%zu) for a device batch failed", arena_bytes); return BAMSCAN_ERR_CUDA; }
-      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.valid = true;
+      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
       if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
       CU_TRY(cudaEventCreateWithFlags(&P.owner->dev_ready, cudaEventDisableTiming));
       CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
@@ -786,7 +824,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       P.owner->arena = arena_acquire(arena_bytes);
       if (!P.owner->arena.p) { delete P.owner; P.owner = nullptr; return BAMSCAN_ERR_CUDA; }
       P.owner->refs = 1;
-      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.valid = true;
+      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
       if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
       CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
       CU_TRY(cudaMemcpyAsync(P.owner->arena.p, A, arena_bytes, cudaMemcpyDeviceToHost, s->s_d2h));
@@ -872,13 +910,16 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   const double tw0 = wall_ms();
   const uint32_t nb_all = c.b1 - c.b0;
   (void)nb_all;
-  const uint32_t data_hi = s->chunk_data_hi[slot], seg0 = HEADROOM;
+  // H: room in front of the chunk (HEADROOM except for FASTA, where it grows to the carried record); the slot's member descriptors
+  // were built for desc_base, so the inflate output moves up by the difference
+  const uint32_t H = s->headroom, shift = H - s->desc_base[slot];
+  const uint32_t data_hi = s->chunk_data_hi[slot] + shift, seg0 = H;
   const uint32_t nb = s->n_descs[slot];
   int rc;
-  if ((rc = s->d_infl[slot].ensure((size_t)HEADROOM + c.ubytes + INFL_PAD))) return rc;
+  if ((rc = s->d_infl[slot].ensure((size_t)H + c.ubytes + INFL_PAD))) return rc;
   if ((rc = s->d_status[slot].ensure(4 * std::max<uint32_t>(nb, 1)))) return rc;
-  if ((rc = s->d_flags[slot].ensure(256))) return rc;
-  if ((rc = s->d_carry.ensure(HEADROOM))) return rc;
+  if ((rc = s->d_flags[slot].ensure(f->format == 3 ? 1024 : 256))) return rc;
+  if ((rc = s->d_carry.ensure(H))) return rc;
   // Long records (the previous chunk's mean above 2 KiB): 64 KiB segments.  seg_candidates tests every byte offset of a segment up
   // to its first record start, i.e. about half a record per segment (and all of it when a 10 kb record covers the segment): with
   // 16 KiB segments that scan was 9.5 % of the long-read scan.
@@ -904,16 +945,16 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   const uint32_t carry = s->carry_len;
   // ---- boundaries
   BoundaryParams BP;
-  BP.U = U; BP.data_lo = HEADROOM - carry; BP.data_hi = data_hi; BP.seg0 = seg0; BP.seg_bytes = seg_bytes; BP.n_seg = n_seg;
+  BP.U = U; BP.data_lo = H - carry; BP.data_hi = data_hi; BP.seg0 = seg0; BP.seg_bytes = seg_bytes; BP.n_seg = n_seg;
   BP.n_ref = (int32_t)f->ref_names.size(); BP.ref_len = s->d_refs.as<int32_t>(); BP.max_block_size = MAX_BLOCK_SIZE;
-  if (carry) BP.first_start = HEADROOM - carry;
+  if (carry) BP.first_start = H - carry;
   else if (s->need_spec) BP.first_start = SEG_NONE;                 // shard without a known start: speculate
-  else if (!first_of_range) BP.first_start = HEADROOM;
-  else BP.first_start = HEADROOM + (uint32_t)(range.first_uoff - c.u0);
+  else if (!first_of_range) BP.first_start = H;
+  else BP.first_start = H + (uint32_t)(range.first_uoff - c.u0);
   // ownership bound inside this chunk
   uint64_t own = data_hi;
   if (c.extension) own = seg0;
-  if (range.stop_uoff != ~0ull && range.stop_uoff < c.u0 + c.ubytes) own = std::min<uint64_t>(own, range.stop_uoff >= c.u0 ? HEADROOM + (range.stop_uoff - c.u0) : seg0);
+  if (range.stop_uoff != ~0ull && range.stop_uoff < c.u0 + c.ubytes) own = std::min<uint64_t>(own, range.stop_uoff >= c.u0 ? H + (range.stop_uoff - c.u0) : seg0);
   BP.own_hi = (uint32_t)own;
   if (phase != 2) {
   CU_TRY(cudaStreamWaitEvent(cs, s->ev_h2d[slot], 0));   // descriptors (+ compressed bytes) of this chunk have landed
@@ -925,14 +966,14 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   CU_TRY(cudaEventRecord(s->ev_t[slot][0], cs));
   if (nb) {
     int nl = 0;
-    if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, d_flags + 15, &s->d_sorted, &nl))) return rc;
+    if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U + shift, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, d_flags + 15, &s->d_sorted, &nl))) return rc;
     s->st.kernel_launches += nl;
   }
   CU_TRY(cudaEventRecord(s->ev_t[slot][1], cs));
   // ---- carry-in
   if (carry) {
     CU_TRY(cudaStreamWaitEvent(cs, s->ev_carry, 0));                  // the previous chunk's tail was copied out on the other stream
-    CU_TRY(cudaMemcpyAsync(U + HEADROOM - carry, s->d_carry.p, carry, cudaMemcpyDeviceToDevice, cs));
+    CU_TRY(cudaMemcpyAsync(U + H - carry, s->d_carry.p, carry, cudaMemcpyDeviceToDevice, cs));
   }
   if (f->format == 1) {
     // FASTQ: line starts of the chunk -> d_recoff (kernels_fastq.cuh); the flags come out as the seg_* kernels report them
@@ -950,6 +991,35 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     fq_frame_kernel<<<1, 32, 0, cs>>>(FF, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
     s->st.kernel_launches += 2;
     publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+    CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+    if (phase == 1) return BAMSCAN_OK;
+  } else if (f->format == 3) {
+    // FASTA: line starts (the FASTQ newline scan) and the lines that start with '>' (kernels_fasta.cuh)
+    const uint32_t lo = BP.data_lo, span = data_hi - lo;
+    const uint32_t n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
+    if ((rc = s->d_seg[slot].ensure(16ull * n_tiles + 64))) return rc;
+    uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>(); uint32_t* d_tile_base = d_tile_count + n_tiles;
+    uint32_t* d_st_count = d_tile_base + n_tiles; uint32_t* d_st_base = d_st_count + n_tiles;
+    const uint32_t line_cap = span / 4 + 4096;                                          // lines[] capacity: beyond that the scan fails loudly
+    if ((rc = s->d_recoff[slot].ensure(4ull * line_cap)) || (rc = s->d_fastarts[slot].ensure(4ull * line_cap))) return rc;
+    // ownership starts at the range's first byte (the member in front of it is inflated too, and owned by the range before) or at
+    // the carried record; the chunk's first byte starts a line at the file start, for a carried record, or behind a '\n'
+    const uint32_t own_lo = first_of_range && !carry ? H + (uint32_t)std::min<uint64_t>(range.first_uoff - c.u0, data_hi - H) : lo;
+    const uint32_t lead_ok = carry || (first_of_range ? c.u0 == 0 : s->fa_lead_nl);
+    FastaFrame FF{U, lo, data_hi, own_lo, BP.own_hi, lead_ok, (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap, (uint32_t)SLICE_BYTES};
+    CU_TRY(cudaMemsetAsync(d_flags + 16, 0, 4 * 48, cs));
+    fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
+    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + FA_F_NEWLINES);
+    fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
+    fa_count_kernel<<<n_tiles, 256, 0, cs>>>(FF, d_st_count);
+    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_st_count, d_st_base, n_tiles, d_flags + FA_F_STARTS);
+    fa_starts_kernel<<<n_tiles, 256, 0, cs>>>(FF, d_tile_base, d_st_base, s->d_fastarts[slot].as<uint32_t>());
+    fa_frame_kernel<<<1, 32, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags);
+    s->st.kernel_launches += 7;
+    if (s->fa_leading) { fa_leading_kernel<<<n_tiles, 256, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags); s->st.kernel_launches++; }
+    publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+    publish_kernel<<<1, 64, 0, cs>>>(d_flags + 16, s->d_hflags + FA_HFLAGS, 48);
+    s->st.kernel_launches += 2;
     CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
     if (phase == 1) return BAMSCAN_OK;
   } else if (f->format == 2) {
@@ -1007,7 +1077,14 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   }
   if (hf[1] && f->format == 1) { set_error("FASTQ read error: more lines in one chunk than supported (lines shorter than 8 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
   if (hf[1] && f->format == 2) { set_error("SAM read error: lines shorter than 8 bytes on average (a SAM record has 11 fields)"); return BAMSCAN_ERR_FORMAT; }
-  if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - HEADROOM))); return BAMSCAN_ERR_FORMAT; }
+  if (hf[1] && f->format == 3) { set_error("FASTA read error: more lines in one chunk than supported (lines shorter than 4 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
+  if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - H))); return BAMSCAN_ERR_FORMAT; }
+  const uint32_t* fa_hf = s->h_flags + FA_HFLAGS - 16;     // FASTA words, indexed as in d_flags
+  if (f->format == 3) {
+    if (fa_hf[FA_F_LEADING]) { set_error("FASTA read error: record %llu of the partition (0-based): bytes other than whitespace in front of the first '>'", (unsigned long long)s->st.rows); return BAMSCAN_ERR_FORMAT; }
+    if (fa_hf[FA_F_STARTS]) s->fa_leading = false;
+    if (data_hi > BP.data_lo) s->fa_lead_nl = fa_hf[FA_F_LAST_NL] != 0;
+  }
   s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10]; s->st.inflate_retries += hf[15];
   const uint32_t n_rec = hf[3];
   if (f->format == 1) { if (n_rec > 0) s->need_spec = false; }
@@ -1016,7 +1093,12 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   if (tail_off > data_hi) tail_off = data_hi;
   *owned_done = tail_off >= BP.own_hi;
   *new_carry = *owned_done ? 0 : data_hi - tail_off;
-  if (*new_carry > HEADROOM) { set_error("%s larger than %u bytes is not supported", f->format == 2 ? "SAM line" : "BAM record", HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; }
+  if (f->format == 3) {
+    if (*new_carry > FA_MAX_RECORD) { set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", (unsigned long long)(s->st.rows + n_rec), (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED; }
+    if (*new_carry > s->headroom) s->headroom = (uint32_t)align_up(*new_carry, 1u << 20);     // the next chunk's room (this chunk's U is unchanged)
+    if ((rc = s->d_carry.ensure(*new_carry))) return rc;
+  }
+  else if (*new_carry > HEADROOM) { set_error("%s larger than %u bytes is not supported", f->format == 2 ? "SAM line" : "BAM record", HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; }
   if (*new_carry) { CU_TRY(cudaMemcpyAsync(s->d_carry.p, U + tail_off, *new_carry, cudaMemcpyDeviceToDevice, cs)); CU_TRY(cudaEventRecord(s->ev_carry, cs)); }
   const uint8_t* U_rows = U;               // the bytes the decode stage reads: the inflated chunk, or the SAM chunk's BAM records
   const uint32_t* sam_recoff = nullptr;
@@ -1026,8 +1108,10 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   } else s->cur.qabs = nullptr;
   s->st.chunks++; s->st.blocks += nb; s->st.inflated_bytes += c.ubytes; s->st.compressed_bytes += c.c1 - c.c0;
   // seam evidence of block-range partitions (BamScanStats): where the first owned record starts, where the chain lands
-  if (n_rec > 0 && s->st.first_record_uoff == ~0ull && hf[13] != 0xffffffffu && hf[13] >= HEADROOM) s->st.first_record_uoff = c.u0 + (hf[13] - HEADROOM);
-  if (*owned_done) s->st.end_chain_uoff = c.u0 + (uint64_t)tail_off - HEADROOM;
+  // (FASTA: the first record may have been carried in, in front of H)
+  if (n_rec > 0 && s->st.first_record_uoff == ~0ull && hf[13] != 0xffffffffu && (hf[13] >= H || f->format == 3)) s->st.first_record_uoff = c.u0 + (uint64_t)hf[13] - H;
+  // (FASTA: the chain ends at the next record start; a chunk without one says nothing about where that is)
+  if (*owned_done && (f->format != 3 || hf[2] != 0xffffffffu)) s->st.end_chain_uoff = c.u0 + (uint64_t)tail_off - H;
   CU_TRY(cudaEventRecord(s->ev_t[slot][2], cs));
   if (n_rec == 0) { CU_TRY(cudaEventRecord(s->ev_t[slot][3], cs)); goto timing; }
   {
@@ -1035,6 +1119,27 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     uint32_t* d_recoff;
     if (f->format == 1) d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14];       // lines[] from the first record's line on: 4 per row
     else if (f->format == 2) d_recoff = const_cast<uint32_t*>(sam_recoff);
+    else if (f->format == 3) {
+      // every line's destination in the chunk's sequence text: content bytes per line, scanned (the decode slices read it)
+      const uint32_t n_lines = fa_hf[FA_F_LINES];
+      if ((rc = s->d_faseq[slot].ensure(4ull * (n_lines + 1) + 64))) return rc;
+      uint32_t* d_seqpos = s->d_faseq[slot].as<uint32_t>();
+      fa_lines_kernel<<<(n_lines + 255) / 256, 256, 0, cs>>>(U, s->d_recoff[slot].as<uint32_t>(), n_lines, d_seqpos);
+      ScanCols LC; memset(&LC, 0, sizeof LC);
+      LC.col[0] = reinterpret_cast<int32_t*>(d_seqpos); LC.n_cols = 1; LC.n = n_lines + 1;
+      const uint32_t n_st = (LC.n + SCAN_TILE - 1) / SCAN_TILE;
+      if ((rc = s->d_tiles.ensure(8ull * n_st)) || (rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS))) return rc;
+      multi_scan_reduce_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
+      multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_tiles.as<uint64_t>(), n_st, s->d_totals.as<uint64_t>());
+      multi_scan_apply_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
+      s->st.kernel_launches += 4;
+      d_recoff = s->d_fastarts[slot].as<uint32_t>();
+      s->cur.fa_lines = s->d_recoff[slot].as<uint32_t>(); s->cur.fa_seqpos = d_seqpos;
+      s->cur.fa_tile_base = s->d_seg[slot].as<uint32_t>() + std::max<uint32_t>(1, (data_hi - BP.data_lo + FQ_TILE - 1) / FQ_TILE);
+      s->cur.fa_lo = BP.data_lo; s->cur.fa_hi = data_hi; s->cur.fa_slice = 0;
+      const uint32_t n_sl = fa_hf[FA_F_SLICES];
+      for (uint32_t k = 0; k <= n_sl; k++) { s->cur.fa_slice_rec[k] = fa_hf[FA_F_SLICE_REC + k]; s->cur.fa_slice_byte[k] = fa_hf[FA_F_SLICE_BYTE + k]; }
+    }
     else {
       if ((rc = s->d_recoff[slot].ensure(4ull * (n_rec + 1)))) return rc;
       d_recoff = s->d_recoff[slot].as<uint32_t>();
@@ -1077,9 +1182,9 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     const uint32_t n_slices = (uint32_t)std::max<uint64_t>(1, (c.ubytes + SLICE_BYTES - 1) / SLICE_BYTES);
     s->cur.U = U_rows; s->cur.recoff = d_recoff; s->cur.n = n; s->cur.pos = 0; s->cur.cs = cs;
     s->cur.rows_per_slice = (n + n_slices - 1) / n_slices;
-    s->mean_record_bytes = (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)(data_hi - HEADROOM) / std::max<uint32_t>(n_rec, 1));
+    s->mean_record_bytes = (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)(data_hi - H) / std::max<uint32_t>(n_rec, 1));
     s->cur.long_records = (f->debug_flags & 2) || s->mean_record_bytes > 2048;
-    s->cur.ubytes = c.ubytes / n_slices + (HEADROOM / 4);
+    s->cur.ubytes = c.ubytes / n_slices + (H / 4);
     CU_TRY(cudaEventRecord(s->ev_t[slot][3], cs));
   }
 timing:
@@ -1144,6 +1249,7 @@ static int advance(BamScanStream* s, bool* produced) {
       if (r.region_mode < 0) { set_error("BAM region query failed: a region names a reference sequence that is not in the BAM header"); return BAMSCAN_ERR_INVALID; }
       s->tail_seen = false; s->range_stop = false;
       s->chunks.clear(); s->chunk_idx = 0; s->carry_len = 0; s->have_h2d_ahead = false; s->ext_blocks = 8; s->need_spec = !r.exact_start;
+      s->fa_leading = f->format == 3 && r.first_uoff == 0;
       plan_chunks(*f, r.block_begin, r.block_end, false, &s->chunks);
       s->range_open = true;
       if (s->chunks.empty()) { s->range_open = false; s->range_idx++; continue; }
@@ -1154,7 +1260,7 @@ static int advance(BamScanStream* s, bool* produced) {
       uint32_t last = s->chunks.back().b1;
       if (s->carry_len == 0 || last >= f->blocks.size()) {
         if (s->carry_len) {
-          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", f->format == 1 ? "FASTQ" : f->format == 2 ? "SAM" : "BAM", s->carry_len);
+          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", f->format == 1 ? "FASTQ" : f->format == 2 ? "SAM" : f->format == 3 ? "FASTA" : "BAM", s->carry_len);
           return BAMSCAN_ERR_FORMAT;
         }
         s->range_open = false; s->range_idx++;
@@ -1247,7 +1353,9 @@ static void export_batch(const BamScanStream* s, const ReadyBatch& rb, ArrowArra
   }
 }
 
-static int decode_error_to_rc(uint32_t code, uint32_t row) {
+// row: in the batch; row0: rows of the partition in front of the batch
+static int decode_error_to_rc(uint32_t code, uint32_t row, uint64_t row0) {
+  const unsigned long long prow = row0 + row;
   switch (code) {
     case DEC_ERR_FIELDS: set_error("BAM read error: record %u: fields exceed block_size", row); return BAMSCAN_ERR_FORMAT;
     case DEC_ERR_REF: set_error("BAM read error: record %u: reference sequence id out of range", row); return BAMSCAN_ERR_FORMAT;
@@ -1260,6 +1368,9 @@ static int decode_error_to_rc(uint32_t code, uint32_t row) {
     case FQ_ERR_NAME_PREFIX: set_error("FASTQ read error: record %u of the batch does not start with '@'", row); return BAMSCAN_ERR_FORMAT;
     case FQ_ERR_PLUS: set_error("FASTQ read error: record %u of the batch: third line does not start with '+'", row); return BAMSCAN_ERR_FORMAT;
     case FQ_ERR_UTF8: set_error("FASTQ record %u of the batch: non-ASCII byte (not supported by this build)", row); return BAMSCAN_ERR_UNSUPPORTED;
+    case FA_ERR_NAME: set_error("FASTA read error: record %llu of the partition (0-based): empty name", prow); return BAMSCAN_ERR_FORMAT;
+    case FA_ERR_UTF8: set_error("FASTA read error: record %llu of the partition (0-based): byte 0x80 or above", prow); return BAMSCAN_ERR_FORMAT;
+    case FA_ERR_TOO_LONG: set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", prow, (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED;
   }
   set_error("decode error %u at record %u", code, row);
   return BAMSCAN_ERR_FORMAT;
@@ -1273,7 +1384,7 @@ static int finalize_pending(BamScanStream* s) {
   CU_TRY(cudaEventSynchronize(P.done));
   P.valid = false;
   const uint32_t* err = s->device_export ? s->h_flags + 514 : reinterpret_cast<const uint32_t*>(P.owner->arena.p + P.err_off);
-  if (err[0]) { int rc = decode_error_to_rc(err[0], err[1]); owner_unref(P.owner); P.owner = nullptr; return rc; }
+  if (err[0]) { int rc = decode_error_to_rc(err[0], err[1], P.row0); owner_unref(P.owner); P.owner = nullptr; return rc; }
   s->ready.clear(); s->ready_pos = 0;
   uint64_t step = s->f->batch_rows > 0 ? (uint64_t)s->f->batch_rows : P.rows;
   for (uint64_t r0 = 0; r0 < P.rows; r0 += step) {
@@ -1342,6 +1453,13 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
     *out = h.release();
     return BAMSCAN_OK;
   }
+  if (format == 3) {
+    // FASTA: name, description (NULL when empty), sequence; no metadata, as for FASTQ
+    if (rc) { release_file(&f); return rc; }
+    f.fields = {FieldDef{"name", HK_Utf8, false, {}}, FieldDef{"description", HK_Utf8, true, {}}, FieldDef{"sequence", HK_Utf8, false, {}}};
+    *out = h.release();
+    return BAMSCAN_OK;
+  }
   if ((rc = build_schema(&f, &opt))) { release_file(&f); return rc; }
   if (format == 2) { *out = h.release(); return BAMSCAN_OK; }     // SAM: no index (the reference discovers none for SAM paths)
   if (index_path_or_null) f.index_path = index_path_or_null; else f.index_path = discover_index(f.path);   // "" = no index
@@ -1355,6 +1473,10 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
 
 int bamscan_open_fastq(const char* path, const BamScanOptions* options, BamScanHandle** out) {
   BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, 1))
+}
+
+int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanHandle** out) {
+  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, 3))
 }
 
 void bamscan_close(BamScanHandle* h) {
@@ -1372,7 +1494,7 @@ int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out) {
 
 static int bamscan_describe_tags_impl(BamScanHandle* h, int32_t sample_size, char* buf, uint64_t cap, uint64_t* needed) {
   if (!h || !needed || (cap && !buf)) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == 1) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
+  if (h->file.format == 1 || h->file.format == 3) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
   if (!h->file.header_ok) { set_error("BAM header could not be read: %s", h->file.path.c_str()); return BAMSCAN_ERR_FORMAT; }
   std::map<std::string, std::pair<char, int32_t>> found;
   infer_tag_types(h->file, {}, sample_size > 0 ? sample_size : 100, &found, true);
@@ -1401,7 +1523,7 @@ int bamscan_describe_tags(BamScanHandle* h, int32_t sample_size, char* buf, uint
 
 int bamscan_classify_filters(BamScanHandle* h, const BamScanFilter* filters, int32_t n_filters, uint8_t* out_pushdown) {
   if (!h || (n_filters && (!filters || !out_pushdown))) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == 1) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // FastqTableProvider pushes no filter down
+  if (h->file.format == 1 || h->file.format == 3) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // FastqTableProvider and FastaTableProvider push no filter down
   return classify_filters(h->file, filters, n_filters, out_pushdown);
 }
 

@@ -292,7 +292,7 @@ int load_file(BamFile* f) {
   if (f->format == 2) return load_sam(f);
   int rc = walk_blocks(f);
   if (rc) return rc;
-  if (f->format == 1) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ: records start at inflated offset 0
+  if (f->format == 1 || f->format == 3) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ, FASTA: no header
 
   // BAM header (noodles-bam read_header): magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
   HostStream hs(*f);

@@ -112,6 +112,13 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
         owns = r.first_uoff < std::min<uint64_t>(r.stop_uoff, f->size);
         if (owns) r.block_begin = block_of_uoff(*f, r.first_uoff);
       }
+      if (f->format == 3 && owns) {
+        // FASTA: a record belongs to the range that holds its '>'.  Whether the range's first byte starts a line depends on the byte in
+        // front of it, so the last non-empty member in front of the range is inflated too, and nothing in it is owned (first_uoff)
+        r.exact_start = true;
+        r.first_uoff = f->blocks[b].uoff;
+        for (uint32_t q = b; q > 0; q--) if (f->blocks[q - 1].isize) { r.block_begin = q - 1; break; }
+      }
       if (owns) part.ranges.push_back(r);
       part.estimated_bytes = (e > b && b < n_blocks) ? ((e < n_blocks ? f->blocks[e].coff : f->size) - f->blocks[b].coff) : 0;
       plan->partitions.push_back(part);

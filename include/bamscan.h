@@ -149,6 +149,18 @@ void bamscan_close(BamScanHandle* h);
  * refused (BAMSCAN_ERR_FORMAT): this build reads BGZF. */
 int bamscan_open_fastq(const char* path, const BamScanOptions* options, BamScanHandle** out);
 
+/* A BGZF-compressed FASTA file (a provider like bio-format-fasta's).  The handle is used with the same calls as a FASTQ handle:
+ * bamscan_schema gives name (Utf8), description (Utf8, nullable) and sequence (Utf8).  A record is a line that starts with '>'
+ * (its text up to the line end, without one trailing '\r', split at the first space or tab into name and description; an empty
+ * description is NULL) followed by every line up to the next '>' line or the end of the file, joined without their line breaks
+ * (and one trailing '\r' each); bytes are kept as given.  bamscan_plan with BAMSCAN_PARTITION_BLOCK_RANGE balances BGZF block
+ * ranges by compressed bytes (a record belongs to the range that holds its '>'); otherwise one partition.  BAMSCAN_ERR_FORMAT,
+ * naming the record of the partition: an empty name, a byte of 0x80 or above in a projected column, bytes other than whitespace in
+ * front of the first '>'.  A record of more than 1 GiB of text is BAMSCAN_ERR_UNSUPPORTED.  No filter is pushed down, there is
+ * no index, describe is refused, the options that concern BAM columns are ignored.  Plain gzip and uncompressed FASTA are
+ * refused (BAMSCAN_ERR_FORMAT): this build reads BGZF. */
+int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanHandle** out);
+
 /* == TableProvider::schema (table_provider.rs:933-935): the full, unprojected schema with all metadata. */
 int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out);
 

@@ -197,6 +197,33 @@ class FastqTableProvider {
   BamScanHandle* h_ = nullptr;
 };
 
+// A provider for BGZF-compressed FASTA (bamscan_open_fasta): name, description (nullable), sequence.  scan() with
+// target_partitions > 1 cuts BGZF block ranges balanced by compressed bytes; no filter is pushed down.
+class FastaTableProvider {
+ public:
+  explicit FastaTableProvider(const std::string& file_path, const std::optional<std::string>& object_storage_options = std::nullopt,
+                              int32_t device_id = 0, int32_t batch_rows = 0) {
+    if (object_storage_options) throw Error(BAMSCAN_ERR_UNSUPPORTED, "remote object storage is out of scope for this build (local files only)");
+    BamScanOptions o; std::memset(&o, 0, sizeof o);
+    o.struct_size = sizeof o; o.device_id = device_id; o.batch_rows = batch_rows;
+    check(bamscan_open_fasta(file_path.c_str(), &o, &h_));
+  }
+  FastaTableProvider(FastaTableProvider&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+  FastaTableProvider(const FastaTableProvider&) = delete;
+  ~FastaTableProvider() { if (h_) bamscan_close(h_); }
+  void schema(ArrowSchema* out) const { check(bamscan_schema(h_, out)); }
+  const char* table_type() const { return "Base"; }
+  BamExec scan(const std::optional<std::vector<int32_t>>& projection, std::optional<int64_t> limit, int32_t target_partitions = 1) const {
+    BamScanPlan* p = nullptr;
+    check(bamscan_plan(h_, projection && !projection->empty() ? projection->data() : nullptr, projection ? (int32_t)projection->size() : -1,
+                       nullptr, 0, limit.value_or(-1), target_partitions,
+                       target_partitions > 1 ? BAMSCAN_PARTITION_BLOCK_RANGE : BAMSCAN_PARTITION_REFERENCE, &p));
+    return BamExec(p);
+  }
+ private:
+  BamScanHandle* h_ = nullptr;
+};
+
 // == BamWriteExec (bio-format-bam/src/write_exec.rs:43-110, 195-350): INSERT OVERWRITE into a BGZF BAM.  The SAM header text and
 // the reference dictionary are the caller's (the Rust host keeps build_bam_header, header_builder.rs:43-186; INTEGRATION.md 3c).
 class BamWriteExec {

@@ -65,6 +65,8 @@ pub const PARTITION_BLOCK_RANGE: i32 = 1;
 
 unsafe extern "C" {
     pub fn bamscan_open(path: *const c_char, index_path_or_null: *const c_char, options: *const BamScanOptions, out: *mut *mut BamScanHandle) -> c_int;
+    /// BGZF-compressed FASTA: the same handle and calls; schema name / description (nullable) / sequence, all Utf8.
+    pub fn bamscan_open_fasta(path: *const c_char, options: *const BamScanOptions, out: *mut *mut BamScanHandle) -> c_int;
     pub fn bamscan_close(h: *mut BamScanHandle);
     pub fn bamscan_schema(h: *mut BamScanHandle, out: *mut FFI_ArrowSchema) -> c_int;
     /// describe(): "TAG\tsam_type\tarrow_type\tdescription\n" per aux tag of the first `sample_size` records.

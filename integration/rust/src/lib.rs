@@ -398,3 +398,110 @@ impl ExecutionPlan for GpuBamExec {
         Ok(Box::pin(RecordBatchStreamAdapter::new(self.schema.clone(), futures::stream::iter(it))))
     }
 }
+
+/// A provider for BGZF-compressed FASTA (`bamscan_open_fasta`), shaped like the BAM one: name, description (nullable) and
+/// sequence; no filter is pushed down (DataFusion applies them), `limit` is passed on and not applied, and with
+/// `target_partitions` > 1 the file is cut into BGZF block ranges balanced by compressed bytes (a record belongs to the range
+/// that holds its '>').  Scans return `GpuBamExec`, which streams the batches exactly as for BAM.
+pub struct GpuFastaTableProvider {
+    handle: Arc<Handle>,
+    schema: SchemaRef,
+    device_id: i32,
+}
+
+impl GpuFastaTableProvider {
+    /// `object_storage_options` must be `None` (local files only).  `device_id` selects the GPU.
+    pub fn new(file_path: String, object_storage_options: Option<String>, device_id: i32) -> Result<Self> {
+        if object_storage_options.is_some() {
+            return Err(DataFusionError::NotImplemented("remote object storage is out of scope for this build (local files only)".into()));
+        }
+        let c_path = CString::new(file_path).map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let opts = ffi::BamScanOptions {
+            struct_size: std::mem::size_of::<ffi::BamScanOptions>() as u32,
+            coordinate_system_zero_based: 1,
+            binary_cigar: 0,
+            has_tag_fields: 0,
+            n_tag_fields: 0,
+            tag_fields: std::ptr::null(),
+            infer_tag_types: 0,
+            infer_tag_sample_size: 0,
+            n_tag_type_hints: 0,
+            tag_type_hints: std::ptr::null(),
+            device_id,
+            batch_rows: 0,
+            chunk_inflated_bytes: 0,
+            segment_bytes: 0,
+            skip_crc: 0,
+            debug_flags: 0,
+        };
+        let mut raw = std::ptr::null_mut();
+        if unsafe { ffi::bamscan_open_fasta(c_path.as_ptr(), &opts, &mut raw) } != 0 {
+            return Err(last_error());
+        }
+        let handle = Arc::new(Handle(raw));
+        let mut c_schema = FFI_ArrowSchema::empty();
+        if unsafe { ffi::bamscan_schema(handle.0, &mut c_schema) } != 0 {
+            return Err(last_error());
+        }
+        let schema = Arc::new(Schema::try_from(&c_schema)?);
+        Ok(Self { handle, schema, device_id })
+    }
+
+    pub fn device_id(&self) -> i32 {
+        self.device_id
+    }
+}
+
+impl Debug for GpuFastaTableProvider {
+    fn fmt(&self, f: &mut Formatter<'_>) -> std::fmt::Result {
+        f.debug_struct("GpuFastaTableProvider").field("device_id", &self.device_id).finish()
+    }
+}
+
+#[async_trait]
+impl TableProvider for GpuFastaTableProvider {
+    fn as_any(&self) -> &dyn Any {
+        self
+    }
+    fn schema(&self) -> SchemaRef {
+        self.schema.clone()
+    }
+    fn table_type(&self) -> TableType {
+        TableType::Base
+    }
+
+    fn supports_filters_pushdown(&self, filters: &[&Expr]) -> Result<Vec<TableProviderFilterPushDown>> {
+        Ok(vec![TableProviderFilterPushDown::Unsupported; filters.len()])
+    }
+
+    async fn scan(&self, state: &dyn Session, projection: Option<&Vec<usize>>, _filters: &[Expr], limit: Option<usize>) -> Result<Arc<dyn ExecutionPlan>> {
+        let proj: Option<Vec<i32>> = projection.map(|p| p.iter().map(|&i| i as i32).collect());
+        let (proj_ptr, n_proj) = match &proj {
+            Some(p) => (p.as_ptr(), p.len() as i32),
+            None => (std::ptr::null(), -1),
+        };
+        let target = state.config().target_partitions() as i32;
+        let mode = if target > 1 { ffi::PARTITION_BLOCK_RANGE } else { ffi::PARTITION_REFERENCE };
+        let mut raw_plan = std::ptr::null_mut();
+        let rc = unsafe {
+            ffi::bamscan_plan(self.handle.0, proj_ptr, n_proj, std::ptr::null(), 0, limit.map(|l| l as i64).unwrap_or(-1), target, mode, &mut raw_plan)
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        let plan = Arc::new(Plan { raw: raw_plan, _handle: self.handle.clone() });
+        let mut c_schema = FFI_ArrowSchema::empty();
+        if unsafe { ffi::bamscan_plan_schema(plan.raw, &mut c_schema) } != 0 {
+            return Err(last_error());
+        }
+        let schema: SchemaRef = Arc::new(Schema::try_from(&c_schema)?);
+        let n = unsafe { ffi::bamscan_plan_num_partitions(plan.raw) };
+        let cache = PlanProperties::new(
+            EquivalenceProperties::new(schema.clone()),
+            Partitioning::UnknownPartitioning(n as usize),
+            EmissionType::Final,
+            Boundedness::Bounded,
+        );
+        Ok(Arc::new(GpuBamExec { plan, schema, cache: Arc::new(cache) }))
+    }
+}

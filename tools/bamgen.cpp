@@ -5,6 +5,7 @@
 // produces), zlib raw deflate at --level (default 6), 28-byte EOF marker; optional .bai.
 //
 //   bamgen --mode short|long --reads N --seed S --out file.bam [--threads T] [--level 6] [--bai]
+//   bamgen --fasta genome|short --reads N --seed S --out file.fa.bgz [--threads T] [--level 6]   (BGZF FASTA, see write_fasta)
 //          [--unmapped K] [--flush-header] [--sam]
 //
 // --sam: the same records (same header text, same reads for the same arguments) as plain SAM text instead of BGZF BAM, in
@@ -292,19 +293,79 @@ static size_t deflate_block(const uint8_t* src, size_t n, int level, uint8_t* ds
   return total;
 }
 
+// BGZF FASTA of one of two shapes, members of exactly 0xff00 inflated bytes + the EOF marker.
+//   genome: the 25 records of kNames / kLens (about 3.1 Gb), 60-column lines, runs of lower case (soft-masked) and of N;
+//   short:  N records of 300 residues, even records on one line, odd ones wrapped at 60 columns.
+static int write_fasta(const std::string& shape, const std::string& out, int64_t N, uint64_t seed, int threads, int level) {
+  const bool genome = shape == "genome";
+  if (!genome && shape != "short") { fprintf(stderr, "--fasta genome|short\n"); return 1; }
+  const int64_t units = genome ? 25 : N, per = genome ? 1 : 65536, n_pieces = (units + per - 1) / per;
+  std::vector<std::string> piece((size_t)n_pieces);
+  std::vector<std::thread> th;
+  for (int t = 0; t < threads; t++) th.emplace_back([&, t]() {
+    for (int64_t c = t; c < n_pieces; c += threads) {
+      Rng r(seed * 1000003ull + (uint64_t)c);
+      std::string& o = piece[(size_t)c];
+      for (int64_t u = c * per; u < std::min(units, (c + 1) * per); u++) {
+        const int64_t len = genome ? kLens[u] : 300;
+        o += genome ? std::string(">") + kNames[u] + " synthetic chromosome " + std::to_string(u + 1) + " len=" + std::to_string(len) + "\n"
+                    : ">seq" + std::to_string(u) + ((u % 3) ? " sample=" + std::to_string(r.below(1000)) : std::string()) + "\n";
+        const int64_t width = (genome || (u & 1)) ? 60 : len;
+        o.reserve(o.size() + (size_t)(len + len / 60 + 2));
+        int64_t run = 0; char kind = 'U';                // U upper, l lower, N
+        for (int64_t i = 0; i < len; i += width) {
+          const int64_t w = std::min(width, len - i);
+          for (int64_t k = 0; k < w; k++) {
+            if (run == 0) { const uint32_t x = r.below(100); kind = x < 70 ? 'U' : x < 95 ? 'l' : 'N'; run = 1 + r.below(kind == 'N' ? 2000 : 400); }
+            run--;
+            static const char up[4] = {'A', 'C', 'G', 'T'}, lo[4] = {'a', 'c', 'g', 't'};
+            o += kind == 'N' ? 'N' : kind == 'U' ? up[r.next() >> 62] : lo[r.next() >> 62];
+          }
+          o += '\n';
+        }
+      }
+    } });
+  for (auto& x : th) x.join();
+  FILE* fp = fopen(out.c_str(), "wb"); if (!fp) { perror("open"); return 1; }
+  const size_t P = 0xff00;
+  std::string pend;
+  uint64_t inflated = 0, compressed = 0, blocks = 0;
+  auto flush = [&](bool final) {
+    const size_t nb = pend.size() / P, tail = pend.size() - nb * P, total = nb + ((final && tail) ? 1 : 0);
+    std::vector<std::vector<uint8_t>> comp(total);
+    std::vector<std::thread> ft;
+    for (int t = 0; t < threads; t++) ft.emplace_back([&, t]() {
+      std::vector<uint8_t> tmp(65536 + 64);
+      for (size_t b = (size_t)t; b < total; b += (size_t)threads) { const size_t c = deflate_block((const uint8_t*)pend.data() + b * P, b < nb ? P : tail, level, tmp.data()); comp[b].assign(tmp.begin(), tmp.begin() + (long)c); } });
+    for (auto& x : ft) x.join();
+    for (auto& cb : comp) { if (fwrite(cb.data(), 1, cb.size(), fp) != cb.size()) { perror("write"); exit(2); } compressed += cb.size(); blocks++; }
+    const size_t used = std::min(pend.size(), total * P);
+    inflated += used; pend.erase(0, used);
+  };
+  for (auto& x : piece) { pend += x; std::string().swap(x); if (pend.size() >= (256u << 20)) flush(false); }
+  flush(true);
+  static const uint8_t eof_marker[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  fwrite(eof_marker, 1, 28, fp); fclose(fp);
+  printf("{\"fasta\": \"%s\", \"records\": %lld, \"seed\": %llu, \"compressed_bytes\": %llu, \"inflated_bytes\": %llu, \"blocks\": %llu, \"level\": %d}\n",
+         shape.c_str(), (long long)units, (unsigned long long)seed, (unsigned long long)(compressed + 28), (unsigned long long)inflated, (unsigned long long)blocks + 1, level);
+  return 0;
+}
+
 int main(int argc, char** argv) {
-  std::string mode = "short", out; int64_t N = 1000000; uint64_t seed = 1; int threads = (int)std::thread::hardware_concurrency(); int level = 6; bool bai = false; int64_t n_unmapped = 0; bool sam = false;
+  std::string mode = "short", out; int64_t N = 1000000; uint64_t seed = 1; int threads = (int)std::thread::hardware_concurrency(); int level = 6; bool bai = false; int64_t n_unmapped = 0; bool sam = false; std::string fasta;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
     auto nxt = [&]() { if (i + 1 >= argc) { fprintf(stderr, "missing value for %s\n", a.c_str()); exit(1); } return std::string(argv[++i]); };
     if (a == "--mode") mode = nxt(); else if (a == "--reads") N = atoll(nxt().c_str()); else if (a == "--seed") seed = strtoull(nxt().c_str(), 0, 10);
     else if (a == "--out") out = nxt(); else if (a == "--threads") threads = atoi(nxt().c_str()); else if (a == "--level") level = atoi(nxt().c_str());
     else if (a == "--bai") bai = true; else if (a == "--unmapped") n_unmapped = atoll(nxt().c_str()); else if (a == "--sam") sam = true;
+    else if (a == "--fasta") fasta = nxt();
     else { fprintf(stderr, "unknown arg %s\n", a.c_str()); return 1; }
   }
   if (out.empty() || N <= 0) { fprintf(stderr, "usage: bamgen --mode short|long --reads N --seed S --out f.bam [--threads T] [--level L] [--bai] [--unmapped K] [--sam]\n"); return 1; }
   if (sam && bai) { fprintf(stderr, "--bai needs BAM output\n"); return 1; }
   if (threads < 1) threads = 1;
+  if (!fasta.empty()) return write_fasta(fasta, out, N, seed, threads, level);
   bool is_long = mode == "long";
   if (!is_long && (N & 1)) N++;
   Genome G;
