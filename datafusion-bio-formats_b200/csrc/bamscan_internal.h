@@ -59,11 +59,25 @@ struct BaiIndex {
   uint64_t max_pos() const { return 1ull << (min_shift + 3 * depth); }
 };
 
+// The file formats a scan reads (BamFile::format); the writer writes the first three
+enum ScanFormat : int {
+  FMT_BAM = 0,
+  FMT_FASTQ = 1,   // BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index
+  FMT_SAM = 2,     // plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index
+  FMT_FASTA = 3,   // BGZF-compressed FASTA (kernels_fasta.cuh): three Utf8 columns, records of up to 1 GiB, no index
+};
+inline const char* format_name(int format) {
+  switch (format) {
+    case FMT_FASTQ: return "FASTQ";
+    case FMT_SAM: return "SAM";
+    case FMT_FASTA: return "FASTA";
+  }
+  return "BAM";
+}
+
 // == BamTableProvider (table_provider.rs:314-335)
 struct BamFile {
-  int format = 0;            // 0: BAM; 1: BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index;
-                             // 2: plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index;
-                             // 3: BGZF-compressed FASTA (kernels_fasta.cuh): three Utf8 columns, records of up to 1 GiB, no index
+  int format = FMT_BAM;      // a ScanFormat; stored as int because code built against this header (the host test drivers) assigns plain integers
   std::string path, index_path;
   uint8_t* data = nullptr;   // whole file: read-only mapping (O_RDONLY / PROT_READ, not page-locked); small files: a plain copy
   uint64_t size = 0;
@@ -131,7 +145,7 @@ struct Plan {
 // host_file.cpp
 int load_file(BamFile* f);                       // reads the file into pinned memory, walks BGZF, parses header
 bool is_sam_path(const std::string& path);      // BamTableProvider's `is_sam`: the path ends in ".sam", any case
-int load_sam(BamFile* f);                        // format 2: header lines, @SQ references, pseudo-blocks over the text body
+int load_sam(BamFile* f);                        // FMT_SAM: header lines, @SQ references, pseudo-blocks over the text body
 uint64_t sam_record_start_at(const BamFile& f, uint64_t off);   // first line start at or after off (a record belongs to the range holding its first byte)
 int infer_tag_types(const BamFile& f, const std::vector<std::string>& tags, int sample_size,
                     std::map<std::string, std::pair<char, int32_t>>* out, bool all = false);   // table_provider.rs:145-202

@@ -240,10 +240,10 @@ struct BamScanStream {
   std::vector<int32_t> out_to_dec;        // projection position -> index into dec_cols
   // device memory
   DeviceBuf d_comp[2], d_blk[2], d_infl[2], d_carry, d_status[2], d_flags[2], d_seg[2], d_recoff[2], d_recoff2[2], d_keep[2], d_tiles, d_totals, d_scratch, d_arena[2], d_refs, d_sorted;
-  // SAM (format 2): per slot the parsed lines, record sizes -> offsets, "QUAL is *" flags, scan tiles and the transcoded BAM records;
+  // SAM: per slot the parsed lines, record sizes -> offsets, "QUAL is *" flags, scan tiles and the transcoded BAM records;
   // the reference names sorted bytewise for RNAME / RNEXT lookups
   DeviceBuf d_samline[2], d_samsize[2], d_qabs[2], d_samtiles[2], d_bam[2], d_samrefs;
-  // FASTA (format 3): per slot the line index of every record start and every line's destination in the sequence text
+  // FASTA: per slot the line index of every record start and every line's destination in the sequence text
   DeviceBuf d_fastarts[2], d_faseq[2];
   cudaEvent_t ev_text_free[2] = {nullptr, nullptr}, ev_ing[2][2] = {};   // the write pass has read a slot's text; ingest copy timing
   bool tail_seen = false, range_stop = false;   // per-reference unmapped tail state (physical_exec.rs:1203-1215)
@@ -392,7 +392,7 @@ static int stream_init(BamScanStream* s) {
   if (n_ref) CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_len, f->ref_lens.data(), 4 * n_ref, cudaMemcpyHostToDevice));
   CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_off, offs.data(), 4 * (n_ref + 1), cudaMemcpyHostToDevice));
   if (!blob.empty()) CU_TRY(cudaMemcpy(s->d_refs.as<uint8_t>() + o_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-  if (f->format == 2) {
+  if (f->format == FMT_SAM) {
     // SAM: names sorted bytewise + their ids (enc::lookup_ref), laid out as [offsets n_ref + 1][ids n_ref][names]
     std::vector<int32_t> ids(n_ref);
     std::iota(ids.begin(), ids.end(), 0);
@@ -477,9 +477,9 @@ static uint32_t inflate_wave_members(int device) { return (uint32_t)device_sms(d
 static const uint64_t SLICE_BYTES = 768ull << 20;
 static uint64_t chunk_cap_bytes(const BamFile& f) {
   if (f.chunk_bytes) return f.chunk_bytes;
-  if (f.format == 2) return 512ull << 20;          // SAM: text bytes per chunk (no inflate wave to fill)
+  if (f.format == FMT_SAM) return 512ull << 20;    // SAM: text bytes per chunk (no inflate wave to fill)
   // FASTA: the carried record (up to 1 GiB) sits in front of the chunk, and chunk offsets are u32
-  return std::min<uint64_t>((uint64_t)inflate_wave_members(f.device) * 65280ull + 65536ull, f.format == 3 ? 2ull << 30 : 3ull << 30);
+  return std::min<uint64_t>((uint64_t)inflate_wave_members(f.device) * 65280ull + 65536ull, f.format == FMT_FASTA ? 2ull << 30 : 3ull << 30);
 }
 static void plan_chunks(const BamFile& f, uint32_t b0, uint32_t b1, bool extension, std::vector<ChunkPlan>* out) {
   const uint32_t wave = inflate_wave_members(f.device);
@@ -558,7 +558,7 @@ static int issue_h2d_text(BamScanStream* s, const ChunkPlan& c, int slot) {
 static int issue_h2d(BamScanStream* s, const ChunkPlan& c, int slot) {
   NvtxRange nv("bamscan: stage + H2D of a chunk's compressed members");
   const BamFile* f = s->f;
-  if (f->format == 2) return issue_h2d_text(s, c, slot);
+  if (f->format == FMT_SAM) return issue_h2d_text(s, c, slot);
   const uint32_t nb_all = c.b1 - c.b0;
   if (s->h_descs_cap[slot] < nb_all) {
     if (s->h_descs[slot]) cudaFreeHost(s->h_descs[slot]);
@@ -617,13 +617,14 @@ static int decode_slice(BamScanStream* s, bool* produced) {
   int rc;
   if ((rc = flush_slice(s))) return rc;
   const uint8_t* U = s->cur.U;
-  const bool fasta = f->format == 3;
+  const bool fasta = f->format == FMT_FASTA;
+  const bool fastx = f->format == FMT_FASTQ || fasta;     // the columns map onto the BAM decode slots through fq_slot
   // FASTA: the slices fa_frame cut (each holds whole records, about SLICE_BYTES of text); otherwise rows_per_slice rows
   const uint32_t n = fasta ? s->cur.fa_slice_rec[s->cur.fa_slice + 1] - s->cur.pos : std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
   const uint32_t fa_b0 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice] : 0, fa_b1 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice + 1] : 0;
   if (fasta) s->cur.fa_slice++;
   const uint64_t row0 = s->st.rows;
-  const uint32_t* d_recoff = s->cur.recoff + (size_t)s->cur.pos * (f->format == 1 ? 4 : 1);
+  const uint32_t* d_recoff = s->cur.recoff + (size_t)s->cur.pos * (f->format == FMT_FASTQ ? 4 : 1);
   const uint8_t* d_qabs = s->cur.qabs ? s->cur.qabs + s->cur.pos : nullptr;
   s->cur.pos += n;
   CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
@@ -640,7 +641,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       ColLayout& L = cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = f->fields[L.schema_idx].kind;
       const int c_id = L.schema_idx;
       bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-      L.has_validity = (f->format == 1 || fasta) ? c_id == 1 : (c_id >= 12 || c_id == 1 || c_id == 2 || c_id == 3 || c_id == 7 || c_id == 8);
+      L.has_validity = fastx ? c_id == 1 : (c_id >= 12 || c_id == 1 || c_id == 2 || c_id == 3 || c_id == 7 || c_id == 8);
       if (L.has_validity) L.validity_off = AB.take(bm_bytes);
       if (is_var) L.offsets_off = AB.take(off_bytes); else L.values_off = AB.take(val_bytes);
       if (c_id >= 12 && is_var) { src_off[i] = scratch; scratch += align_up(val_bytes, 256); }
@@ -655,7 +656,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
     memset(&DP, 0, sizeof DP);
     DP.U = U; DP.rec_off = d_recoff; DP.n = n; DP.zero_based = f->zero_based; DP.binary_cigar = f->binary_cigar;
     DP.n_ref = (int32_t)f->ref_names.size();
-    DP.end_zero_span = f->format == 2; DP.qual_absent = d_qabs;
+    DP.end_zero_span = f->format == FMT_SAM; DP.qual_absent = d_qabs;
     size_t n_ref = f->ref_names.size();
     DP.ref_name_off = reinterpret_cast<const uint32_t*>(s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16));
     DP.ref_names = s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16) + align_up(4 * (n_ref + 1), 16);
@@ -670,7 +671,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       int32_t* offs = reinterpret_cast<int32_t*>(A + L.offsets_off);
       uint32_t* vals = reinterpret_cast<uint32_t*>(A + L.values_off);
       static const int fq_slot[4] = {0, 1, 9, 10};      // FASTQ: name, description (nullable Utf8 like chrom), sequence, quality_scores; FASTA: the first three
-      switch ((f->format == 1 || fasta) ? fq_slot[L.schema_idx] : L.schema_idx) {
+      switch (fastx ? fq_slot[L.schema_idx] : L.schema_idx) {
         case 0: DP.l_name = offs; break;
         case 1: DP.l_chrom = offs; DP.v_chrom = v; break;
         case 2: DP.start = vals; DP.v_start = v; break;
@@ -701,7 +702,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
     CU_TRY(cudaMemsetAsync(A + err_off, 0, 64, cs));
     FastqCols FC;
     FastaCols AC;
-    if (f->format == 1) {
+    if (f->format == FMT_FASTQ) {
       FC = FastqCols{U, d_recoff, n, DP.l_name, DP.l_chrom, DP.l_seq, DP.l_qual, DP.v_chrom, nullptr, nullptr, nullptr, nullptr, DP.err};
       fq_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(FC);
     }
@@ -762,12 +763,12 @@ static int decode_slice(BamScanStream* s, bool* produced) {
         uint8_t* d = A + L.data_off;
         switch (L.schema_idx) {
           case 0: DP.d_name = d; break; case 1: DP.d_chrom = d; break; case 5: DP.d_cigar = d; break; case 7: DP.d_mchrom = d; break;
-          case 2: if (f->format == 1 || fasta) DP.d_seq = d; break; case 3: if (f->format == 1) DP.d_qual = d; break;
+          case 2: if (fastx) DP.d_seq = d; break; case 3: if (f->format == FMT_FASTQ) DP.d_qual = d; break;
           case 9: DP.d_seq = d; break; case 10: DP.d_qual = d; break;
           default: DP.tags[tag_slot[i]].data = d;
         }
       }
-      if (f->format == 1) {
+      if (f->format == FMT_FASTQ) {
         FC.l_name = DP.l_name; FC.l_desc = DP.l_chrom; FC.l_seq = DP.l_seq; FC.l_qual = DP.l_qual; FC.err = DP.err;      // (rebased with the arena)
         FC.d_name = DP.d_name; FC.d_desc = DP.d_chrom; FC.d_seq = DP.d_seq; FC.d_qual = DP.d_qual;
         fq_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(FC);
@@ -899,6 +900,152 @@ static int transcode_sam(BamScanStream* s, int slot, cudaStream_t cs, const uint
   return BAMSCAN_OK;
 }
 
+// ---- chunk framing: one function per format queues the kernels that find the chunk's records behind its inflate, publishes the
+// flag words (kernels_boundary.cuh's convention in [0, 16)) to the mapped page and records ev_flags[slot].
+
+struct LineScan { uint32_t n_tiles, line_cap; uint32_t* tile_base; };
+
+// The newline scan of FASTQ, SAM and FASTA (kernels_fastq.cuh): the line starts of U[lo, hi) -> d_recoff[slot], which holds
+// (hi - lo) / line_divisor + 4096 of them (beyond that the framing kernel fails loudly); the line count -> d_flags[16].  d_seg[slot]
+// holds tile_words words per tile: the newline counts, their scan (L->tile_base), then whatever the caller keeps there.
+static int launch_line_scan(BamScanStream* s, int slot, cudaStream_t cs, const uint8_t* U, uint32_t lo, uint32_t hi, uint32_t tile_words,
+                            uint32_t line_divisor, LineScan* L) {
+  const uint32_t span = hi - lo;
+  L->n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
+  L->line_cap = span / line_divisor + 4096;
+  int rc;
+  if ((rc = s->d_seg[slot].ensure(4ull * tile_words * L->n_tiles + 64)) || (rc = s->d_recoff[slot].ensure(4ull * L->line_cap))) return rc;
+  uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>();
+  L->tile_base = d_tile_count + L->n_tiles;
+  fq_count_kernel<<<L->n_tiles, 256, 0, cs>>>(U, lo, hi, d_tile_count);
+  fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, L->tile_base, L->n_tiles, s->d_flags[slot].as<uint32_t>() + 16);
+  fq_lines_kernel<<<L->n_tiles, 256, 0, cs>>>(U, lo, hi, L->tile_base, s->d_recoff[slot].as<uint32_t>(), L->line_cap);
+  s->st.kernel_launches += 3;
+  return BAMSCAN_OK;
+}
+
+// BAM: record chains walked from candidate starts per segment, the seams between segments checked and repaired (kernels_boundary.cuh)
+static int frame_bam(BamScanStream* s, int slot, const BoundaryParams& BP, const WalkOut& W, uint32_t* d_seg_base) {
+  const BamFile* f = s->f;
+  cudaStream_t cs = s->s_chunk[slot];
+  const uint32_t n_seg = BP.n_seg;
+  seg_candidates_kernel<<<(n_seg * 32 + 255) / 256, 256, 0, cs>>>(BP, W.seg_start, (f->debug_flags & 1) ? 1 : 0);
+  seg_walk_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
+  seg_check_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
+  if (!(f->debug_flags & 64)) {
+    // parallel repair rounds (no-ops when every seam agreed); debug_flags bit 6 leaves everything to the sequential repair
+    for (int round = 0; round < 3; round++) {
+      seg_fix_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W, round);
+      seg_reset_kernel<<<1, 1, 0, cs>>>(W);
+      seg_check_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
+    }
+    s->st.kernel_launches += 9;
+  }
+  seg_repair_kernel<<<1, 1, 0, cs>>>(BP, W);
+  seg_scan_kernel<<<1, 1024, 0, cs>>>(W.seg_count, W.seg_start, W.seg_exit, W.seg_tail, d_seg_base, n_seg, W.flags);
+  s->st.kernel_launches += 5;
+  publish_kernel<<<1, 32, 0, cs>>>(W.flags, s->d_hflags, 16);
+  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+  return BAMSCAN_OK;
+}
+
+// FASTQ: line starts of the chunk -> d_recoff (kernels_fastq.cuh); the flags come out as the seg_* kernels report them
+static int frame_fastq(BamScanStream* s, const ChunkPlan& c, int slot, const BoundaryParams& BP) {
+  cudaStream_t cs = s->s_chunk[slot];
+  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
+  LineScan L;
+  // lines[] capacity: FASTQ lines average far more than 8 bytes
+  if (int rc = launch_line_scan(s, slot, cs, BP.U, BP.data_lo, BP.data_hi, 2, 8, &L)) return rc;
+  FastqFrame FF{BP.U, BP.data_lo, BP.data_hi, BP.own_hi, (uint32_t)(s->need_spec ? 1 : 0), (uint32_t)(c.b1 == s->f->blocks.size() ? 1 : 0), L.line_cap};
+  fq_frame_kernel<<<1, 32, 0, cs>>>(FF, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
+  s->st.kernel_launches++;
+  publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+  return BAMSCAN_OK;
+}
+
+// SAM: line starts of the chunk (the newline scan), one record per line (kernels_sam.cuh)
+static int frame_sam(BamScanStream* s, const ChunkPlan& c, int slot, const BoundaryParams& BP) {
+  cudaStream_t cs = s->s_chunk[slot];
+  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
+  LineScan L;
+  // a SAM record has 11 fields: lines average far more than 8 bytes
+  if (int rc = launch_line_scan(s, slot, cs, BP.U, BP.data_lo, BP.data_hi, 2, 8, &L)) return rc;
+  FastqFrame FF{BP.U, BP.data_lo, BP.data_hi, BP.own_hi, 0u, (uint32_t)(c.b1 == s->f->blocks.size() ? 1 : 0), L.line_cap};
+  sam::sam_frame_kernel<<<1, 32, 0, cs>>>(FF, BP.first_start, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
+  s->st.kernel_launches++;
+  publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+  return BAMSCAN_OK;
+}
+
+// FASTA: line starts (the newline scan) and the lines that start with '>' (kernels_fasta.cuh).  Its own flag words [16, 64) go to
+// [FA_HFLAGS, FA_HFLAGS + 48) of the mapped page.
+static int frame_fasta(BamScanStream* s, const ChunkPlan& c, const ScanRange& range, int slot, const BoundaryParams& BP, bool first_of_range) {
+  cudaStream_t cs = s->s_chunk[slot];
+  uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
+  const uint32_t lo = BP.data_lo, data_hi = BP.data_hi, H = BP.seg0, carry = s->carry_len;
+  int rc;
+  CU_TRY(cudaMemsetAsync(d_flags + 16, 0, 4 * 48, cs));
+  LineScan L;
+  // lines[] capacity; d_seg also holds the '>' line counts and their scan
+  if ((rc = launch_line_scan(s, slot, cs, BP.U, lo, data_hi, 4, 4, &L)) || (rc = s->d_fastarts[slot].ensure(4ull * L.line_cap))) return rc;
+  uint32_t* d_st_count = L.tile_base + L.n_tiles; uint32_t* d_st_base = d_st_count + L.n_tiles;
+  // ownership starts at the range's first byte (the member in front of it is inflated too, and owned by the range before) or at
+  // the carried record; the chunk's first byte starts a line at the file start, for a carried record, or behind a '\n'
+  const uint32_t own_lo = first_of_range && !carry ? H + (uint32_t)std::min<uint64_t>(range.first_uoff - c.u0, data_hi - H) : lo;
+  const uint32_t lead_ok = carry || (first_of_range ? c.u0 == 0 : s->fa_lead_nl);
+  FastaFrame FF{BP.U, lo, data_hi, own_lo, BP.own_hi, lead_ok, (uint32_t)(c.b1 == s->f->blocks.size() ? 1 : 0), L.line_cap, (uint32_t)SLICE_BYTES};
+  fa_count_kernel<<<L.n_tiles, 256, 0, cs>>>(FF, d_st_count);
+  fq_scan_kernel<<<1, 1024, 0, cs>>>(d_st_count, d_st_base, L.n_tiles, d_flags + FA_F_STARTS);
+  fa_starts_kernel<<<L.n_tiles, 256, 0, cs>>>(FF, L.tile_base, d_st_base, s->d_fastarts[slot].as<uint32_t>());
+  fa_frame_kernel<<<1, 32, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags);
+  s->st.kernel_launches += 4;
+  if (s->fa_leading) { fa_leading_kernel<<<L.n_tiles, 256, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags); s->st.kernel_launches++; }
+  publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
+  publish_kernel<<<1, 64, 0, cs>>>(d_flags + 16, s->d_hflags + FA_HFLAGS, 48);
+  s->st.kernel_launches += 2;
+  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+  return BAMSCAN_OK;
+}
+
+// The host's reading of a framed chunk's flags, per format: the framing error in hf[1], FASTA's own flag words, whether the next
+// chunk still has to speculate where a record starts (need_spec), and the longest record the next chunk can take in (new_carry).
+static int read_frame_flags(BamScanStream* s, const ChunkPlan& c, uint32_t H, uint32_t data_lo, uint32_t data_hi, uint32_t n_rec, uint32_t new_carry) {
+  const uint32_t* hf = s->h_flags;
+  const bool start_known = n_rec > 0 || hf[2] != 0xffffffffu;
+  auto over_headroom = [](const char* what) { set_error("%s larger than %u bytes is not supported", what, HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; };
+  switch (s->f->format) {
+    case FMT_BAM:
+      if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - H))); return BAMSCAN_ERR_FORMAT; }
+      if (start_known) s->need_spec = false;
+      if (new_carry > HEADROOM) return over_headroom("BAM record");
+      break;
+    case FMT_FASTQ:
+      if (hf[1]) { set_error("FASTQ read error: more lines in one chunk than supported (lines shorter than 8 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
+      if (n_rec > 0) s->need_spec = false;
+      if (new_carry > HEADROOM) return over_headroom("BAM record");
+      break;
+    case FMT_SAM:
+      if (hf[1]) { set_error("SAM read error: lines shorter than 8 bytes on average (a SAM record has 11 fields)"); return BAMSCAN_ERR_FORMAT; }
+      if (start_known) s->need_spec = false;
+      if (new_carry > HEADROOM) return over_headroom("SAM line");
+      break;
+    case FMT_FASTA: {
+      if (hf[1]) { set_error("FASTA read error: more lines in one chunk than supported (lines shorter than 4 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
+      const uint32_t* fa_hf = s->h_flags + FA_HFLAGS - 16;     // FASTA words, indexed as in d_flags
+      if (fa_hf[FA_F_LEADING]) { set_error("FASTA read error: record %llu of the partition (0-based): bytes other than whitespace in front of the first '>'", (unsigned long long)s->st.rows); return BAMSCAN_ERR_FORMAT; }
+      if (fa_hf[FA_F_STARTS]) s->fa_leading = false;
+      if (data_hi > data_lo) s->fa_lead_nl = fa_hf[FA_F_LAST_NL] != 0;
+      if (start_known) s->need_spec = false;
+      if (new_carry > FA_MAX_RECORD) { set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", (unsigned long long)(s->st.rows + n_rec), (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED; }
+      if (new_carry > s->headroom) s->headroom = (uint32_t)align_up(new_carry, 1u << 20);     // the next chunk's room (this chunk's U is unchanged)
+      return s->d_carry.ensure(new_carry);
+    }
+  }
+  return BAMSCAN_OK;
+}
+
 // Runs one chunk.  On success *produced tells whether a batch went into s->pending (previous pending must have been consumed).
 // phase 1 queues H2D wait + inflate + record boundaries and returns without waiting (the host can then wait for an older
 // batch's D2H while the GPU works); phase 2 picks the chunk up from there; phase 0 does both.
@@ -908,8 +1055,6 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   NvtxRange nv(phase == 1 ? "bamscan: queue inflate + record boundaries (ahead)" : phase == 2 ? "bamscan: chunk boundaries -> rows" : "bamscan: inflate + record boundaries");
   static const bool trace2 = getenv("BAMSCAN_TRACE") && atoi(getenv("BAMSCAN_TRACE")) >= 2;
   const double tw0 = wall_ms();
-  const uint32_t nb_all = c.b1 - c.b0;
-  (void)nb_all;
   // H: room in front of the chunk (HEADROOM except for FASTA, where it grows to the carried record); the slot's member descriptors
   // were built for desc_base, so the inflate output moves up by the difference
   const uint32_t H = s->headroom, shift = H - s->desc_base[slot];
@@ -918,7 +1063,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   int rc;
   if ((rc = s->d_infl[slot].ensure((size_t)H + c.ubytes + INFL_PAD))) return rc;
   if ((rc = s->d_status[slot].ensure(4 * std::max<uint32_t>(nb, 1)))) return rc;
-  if ((rc = s->d_flags[slot].ensure(f->format == 3 ? 1024 : 256))) return rc;
+  if ((rc = s->d_flags[slot].ensure(f->format == FMT_FASTA ? 1024 : 256))) return rc;
   if ((rc = s->d_carry.ensure(H))) return rc;
   // Long records (the previous chunk's mean above 2 KiB): 64 KiB segments.  seg_candidates tests every byte offset of a segment up
   // to its first record start, i.e. about half a record per segment (and all of it when a 10 kb record covers the segment): with
@@ -934,8 +1079,9 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   uint8_t* d_seg_tail = reinterpret_cast<uint8_t*>(d_seg_base + n_seg);
   // [0..7] boundary / filter flags, [8] inflate ticket, [9] inflate error, [10] seams rejected, [11] first disagreeing seam,
   // [12] retry ticket, [13] first owned record, [14] FASTQ first record line, [15] members the CTA inflate kernel refused:
-  // these 16 words are published to the host.  [16] FASTQ newline count (device only).
+  // these 16 words are published to the host.  [16] line count of the newline scan (device only; FASTA publishes [16, 64)).
   uint32_t* d_flags = s->d_flags[slot].as<uint32_t>();
+  const WalkOut W{d_seg_start, d_seg_exit, d_seg_count, d_seg_tail, d_flags};
 
   cudaStream_t cs = s->s_chunk[slot];
   const uint8_t* d_comp;
@@ -957,109 +1103,32 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
   if (range.stop_uoff != ~0ull && range.stop_uoff < c.u0 + c.ubytes) own = std::min<uint64_t>(own, range.stop_uoff >= c.u0 ? H + (range.stop_uoff - c.u0) : seg0);
   BP.own_hi = (uint32_t)own;
   if (phase != 2) {
-  CU_TRY(cudaStreamWaitEvent(cs, s->ev_h2d[slot], 0));   // descriptors (+ compressed bytes) of this chunk have landed
-  CU_TRY(cudaMemsetAsync(d_flags, 0, 64, cs));
-  CU_TRY(cudaMemsetAsync(d_flags + 2, 0xff, 4, cs));     // [2] tail offset
-  CU_TRY(cudaMemsetAsync(d_flags + 5, 0xff, 8, cs));     // [5] first row of the target reference, [6] stop row
-  CU_TRY(cudaMemsetAsync(d_flags + 11, 0xff, 4, cs));    // [11] first disagreeing seam
-  CU_TRY(cudaMemsetAsync(d_flags + 13, 0xff, 4, cs));    // [13] first owned record of the chunk
-  CU_TRY(cudaEventRecord(s->ev_t[slot][0], cs));
-  if (nb) {
-    int nl = 0;
-    if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U + shift, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, d_flags + 15, &s->d_sorted, &nl))) return rc;
-    s->st.kernel_launches += nl;
-  }
-  CU_TRY(cudaEventRecord(s->ev_t[slot][1], cs));
-  // ---- carry-in
-  if (carry) {
-    CU_TRY(cudaStreamWaitEvent(cs, s->ev_carry, 0));                  // the previous chunk's tail was copied out on the other stream
-    CU_TRY(cudaMemcpyAsync(U + H - carry, s->d_carry.p, carry, cudaMemcpyDeviceToDevice, cs));
-  }
-  if (f->format == 1) {
-    // FASTQ: line starts of the chunk -> d_recoff (kernels_fastq.cuh); the flags come out as the seg_* kernels report them
-    const uint32_t lo = BP.data_lo, span = data_hi - lo;
-    const uint32_t n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
-    if ((rc = s->d_seg[slot].ensure(8ull * n_tiles + 64))) return rc;
-    uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>(); uint32_t* d_tile_base = d_tile_count + n_tiles;
-    const uint32_t line_cap = span / 8 + 4096;                                          // lines[] capacity: FASTQ lines average far more than 8 bytes; beyond that the scan fails loudly
-    if ((rc = s->d_recoff[slot].ensure(4ull * line_cap))) return rc;
-    fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
-    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + 16);
-    s->st.kernel_launches += 2;
-    fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
-    FastqFrame FF{U, lo, data_hi, BP.own_hi, (uint32_t)(s->need_spec ? 1 : 0), (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap};
-    fq_frame_kernel<<<1, 32, 0, cs>>>(FF, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
-    s->st.kernel_launches += 2;
-    publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
-    CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
-    if (phase == 1) return BAMSCAN_OK;
-  } else if (f->format == 3) {
-    // FASTA: line starts (the FASTQ newline scan) and the lines that start with '>' (kernels_fasta.cuh)
-    const uint32_t lo = BP.data_lo, span = data_hi - lo;
-    const uint32_t n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
-    if ((rc = s->d_seg[slot].ensure(16ull * n_tiles + 64))) return rc;
-    uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>(); uint32_t* d_tile_base = d_tile_count + n_tiles;
-    uint32_t* d_st_count = d_tile_base + n_tiles; uint32_t* d_st_base = d_st_count + n_tiles;
-    const uint32_t line_cap = span / 4 + 4096;                                          // lines[] capacity: beyond that the scan fails loudly
-    if ((rc = s->d_recoff[slot].ensure(4ull * line_cap)) || (rc = s->d_fastarts[slot].ensure(4ull * line_cap))) return rc;
-    // ownership starts at the range's first byte (the member in front of it is inflated too, and owned by the range before) or at
-    // the carried record; the chunk's first byte starts a line at the file start, for a carried record, or behind a '\n'
-    const uint32_t own_lo = first_of_range && !carry ? H + (uint32_t)std::min<uint64_t>(range.first_uoff - c.u0, data_hi - H) : lo;
-    const uint32_t lead_ok = carry || (first_of_range ? c.u0 == 0 : s->fa_lead_nl);
-    FastaFrame FF{U, lo, data_hi, own_lo, BP.own_hi, lead_ok, (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap, (uint32_t)SLICE_BYTES};
-    CU_TRY(cudaMemsetAsync(d_flags + 16, 0, 4 * 48, cs));
-    fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
-    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + FA_F_NEWLINES);
-    fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
-    fa_count_kernel<<<n_tiles, 256, 0, cs>>>(FF, d_st_count);
-    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_st_count, d_st_base, n_tiles, d_flags + FA_F_STARTS);
-    fa_starts_kernel<<<n_tiles, 256, 0, cs>>>(FF, d_tile_base, d_st_base, s->d_fastarts[slot].as<uint32_t>());
-    fa_frame_kernel<<<1, 32, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags);
-    s->st.kernel_launches += 7;
-    if (s->fa_leading) { fa_leading_kernel<<<n_tiles, 256, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags); s->st.kernel_launches++; }
-    publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
-    publish_kernel<<<1, 64, 0, cs>>>(d_flags + 16, s->d_hflags + FA_HFLAGS, 48);
-    s->st.kernel_launches += 2;
-    CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
-    if (phase == 1) return BAMSCAN_OK;
-  } else if (f->format == 2) {
-    // SAM: line starts of the chunk (the FASTQ newline scan), one record per line (kernels_sam.cuh)
-    const uint32_t lo = BP.data_lo, span = data_hi - lo;
-    const uint32_t n_tiles = std::max<uint32_t>(1, (span + FQ_TILE - 1) / FQ_TILE);
-    if ((rc = s->d_seg[slot].ensure(8ull * n_tiles + 64))) return rc;
-    uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>(); uint32_t* d_tile_base = d_tile_count + n_tiles;
-    const uint32_t line_cap = span / 8 + 4096;                                          // a SAM record has 11 fields: lines average far more than 8 bytes
-    if ((rc = s->d_recoff[slot].ensure(4ull * line_cap))) return rc;
-    fq_count_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_count);
-    fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, d_tile_base, n_tiles, d_flags + 16);
-    fq_lines_kernel<<<n_tiles, 256, 0, cs>>>(U, lo, data_hi, d_tile_base, s->d_recoff[slot].as<uint32_t>(), line_cap);
-    FastqFrame FF{U, lo, data_hi, BP.own_hi, 0u, (uint32_t)(c.b1 == f->blocks.size() ? 1 : 0), line_cap};
-    sam::sam_frame_kernel<<<1, 32, 0, cs>>>(FF, BP.first_start, d_flags + 16, s->d_recoff[slot].as<uint32_t>(), d_flags);
-    s->st.kernel_launches += 4;
-    publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
-    CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
-    if (phase == 1) return BAMSCAN_OK;
-  } else {
-  WalkOut W{d_seg_start, d_seg_exit, d_seg_count, d_seg_tail, d_flags};
-  seg_candidates_kernel<<<(n_seg * 32 + 255) / 256, 256, 0, cs>>>(BP, d_seg_start, (f->debug_flags & 1) ? 1 : 0);
-  seg_walk_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
-  seg_check_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
-  if (!(f->debug_flags & 64)) {
-    // parallel repair rounds (no-ops when every seam agreed); debug_flags bit 6 leaves everything to the sequential repair
-    for (int round = 0; round < 3; round++) {
-      seg_fix_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W, round);
-      seg_reset_kernel<<<1, 1, 0, cs>>>(W);
-      seg_check_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, W);
+    CU_TRY(cudaStreamWaitEvent(cs, s->ev_h2d[slot], 0));   // descriptors (+ compressed bytes) of this chunk have landed
+    CU_TRY(cudaMemsetAsync(d_flags, 0, 64, cs));
+    CU_TRY(cudaMemsetAsync(d_flags + 2, 0xff, 4, cs));     // [2] tail offset
+    CU_TRY(cudaMemsetAsync(d_flags + 5, 0xff, 8, cs));     // [5] first row of the target reference, [6] stop row
+    CU_TRY(cudaMemsetAsync(d_flags + 11, 0xff, 4, cs));    // [11] first disagreeing seam
+    CU_TRY(cudaMemsetAsync(d_flags + 13, 0xff, 4, cs));    // [13] first owned record of the chunk
+    CU_TRY(cudaEventRecord(s->ev_t[slot][0], cs));
+    if (nb) {
+      int nl = 0;
+      if ((rc = launch_inflate(f, cs, d_comp, s->d_blk[slot].as<BlockDesc>(), nb, U + shift, s->d_status[slot].as<uint32_t>(), d_flags + 8, d_flags + 9, d_flags + 12, d_flags + 15, &s->d_sorted, &nl))) return rc;
+      s->st.kernel_launches += nl;
     }
-    s->st.kernel_launches += 9;
-  }
-  seg_repair_kernel<<<1, 1, 0, cs>>>(BP, W);
-  seg_scan_kernel<<<1, 1024, 0, cs>>>(d_seg_count, d_seg_start, d_seg_exit, d_seg_tail, d_seg_base, n_seg, d_flags);
-  s->st.kernel_launches += 5;
-  publish_kernel<<<1, 32, 0, cs>>>(d_flags, s->d_hflags, 16);
-  CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
+    CU_TRY(cudaEventRecord(s->ev_t[slot][1], cs));
+    // ---- carry-in
+    if (carry) {
+      CU_TRY(cudaStreamWaitEvent(cs, s->ev_carry, 0));                  // the previous chunk's tail was copied out on the other stream
+      CU_TRY(cudaMemcpyAsync(U + H - carry, s->d_carry.p, carry, cudaMemcpyDeviceToDevice, cs));
+    }
+    switch (f->format) {
+      case FMT_BAM: rc = frame_bam(s, slot, BP, W, d_seg_base); break;
+      case FMT_FASTQ: rc = frame_fastq(s, c, slot, BP); break;
+      case FMT_SAM: rc = frame_sam(s, c, slot, BP); break;
+      case FMT_FASTA: rc = frame_fasta(s, c, range, slot, BP, first_of_range); break;
+    }
+    if (rc) return rc;
     if (phase == 1) return BAMSCAN_OK;
-  }
   }
   CU_TRY(cudaEventSynchronize(s->ev_flags[slot]));
   CU_TRY(cudaGetLastError());
@@ -1075,76 +1144,63 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     set_error("BAM read error: BGZF member %u (file offset %llu): inflate failed: %s", blk, (unsigned long long)f->blocks[blk].coff, code < 10 ? names[code] : "?");
     return BAMSCAN_ERR_CRC;
   }
-  if (hf[1] && f->format == 1) { set_error("FASTQ read error: more lines in one chunk than supported (lines shorter than 8 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
-  if (hf[1] && f->format == 2) { set_error("SAM read error: lines shorter than 8 bytes on average (a SAM record has 11 fields)"); return BAMSCAN_ERR_FORMAT; }
-  if (hf[1] && f->format == 3) { set_error("FASTA read error: more lines in one chunk than supported (lines shorter than 4 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
-  if (hf[1]) { set_error("BAM read error: invalid record block_size at inflated offset %llu", (unsigned long long)(c.u0 + ((hf[1] & ~1u) - H))); return BAMSCAN_ERR_FORMAT; }
-  const uint32_t* fa_hf = s->h_flags + FA_HFLAGS - 16;     // FASTA words, indexed as in d_flags
-  if (f->format == 3) {
-    if (fa_hf[FA_F_LEADING]) { set_error("FASTA read error: record %llu of the partition (0-based): bytes other than whitespace in front of the first '>'", (unsigned long long)s->st.rows); return BAMSCAN_ERR_FORMAT; }
-    if (fa_hf[FA_F_STARTS]) s->fa_leading = false;
-    if (data_hi > BP.data_lo) s->fa_lead_nl = fa_hf[FA_F_LAST_NL] != 0;
-  }
-  s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10]; s->st.inflate_retries += hf[15];
   const uint32_t n_rec = hf[3];
-  if (f->format == 1) { if (n_rec > 0) s->need_spec = false; }
-  else if (n_rec > 0 || hf[2] != 0xffffffffu) s->need_spec = false;
   uint32_t tail_off = hf[2] == 0xffffffffu ? data_hi : hf[2];
   if (tail_off > data_hi) tail_off = data_hi;
   *owned_done = tail_off >= BP.own_hi;
   *new_carry = *owned_done ? 0 : data_hi - tail_off;
-  if (f->format == 3) {
-    if (*new_carry > FA_MAX_RECORD) { set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", (unsigned long long)(s->st.rows + n_rec), (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED; }
-    if (*new_carry > s->headroom) s->headroom = (uint32_t)align_up(*new_carry, 1u << 20);     // the next chunk's room (this chunk's U is unchanged)
-    if ((rc = s->d_carry.ensure(*new_carry))) return rc;
-  }
-  else if (*new_carry > HEADROOM) { set_error("%s larger than %u bytes is not supported", f->format == 2 ? "SAM line" : "BAM record", HEADROOM); return BAMSCAN_ERR_UNSUPPORTED; }
+  if ((rc = read_frame_flags(s, c, H, BP.data_lo, data_hi, n_rec, *new_carry))) return rc;
+  s->st.boundary_repairs += hf[4]; s->st.boundary_seam_mismatches += hf[10]; s->st.inflate_retries += hf[15];
   if (*new_carry) { CU_TRY(cudaMemcpyAsync(s->d_carry.p, U + tail_off, *new_carry, cudaMemcpyDeviceToDevice, cs)); CU_TRY(cudaEventRecord(s->ev_carry, cs)); }
   const uint8_t* U_rows = U;               // the bytes the decode stage reads: the inflated chunk, or the SAM chunk's BAM records
   const uint32_t* sam_recoff = nullptr;
-  if (f->format == 2 && n_rec > 0) {
+  if (f->format == FMT_SAM && n_rec > 0) {
     if ((rc = transcode_sam(s, slot, cs, U, s->d_recoff[slot].as<uint32_t>() + hf[14], n_rec, &U_rows, &sam_recoff))) return rc;
     s->cur.qabs = s->d_qabs[slot].as<uint8_t>();
   } else s->cur.qabs = nullptr;
   s->st.chunks++; s->st.blocks += nb; s->st.inflated_bytes += c.ubytes; s->st.compressed_bytes += c.c1 - c.c0;
   // seam evidence of block-range partitions (BamScanStats): where the first owned record starts, where the chain lands
   // (FASTA: the first record may have been carried in, in front of H)
-  if (n_rec > 0 && s->st.first_record_uoff == ~0ull && hf[13] != 0xffffffffu && (hf[13] >= H || f->format == 3)) s->st.first_record_uoff = c.u0 + (uint64_t)hf[13] - H;
+  if (n_rec > 0 && s->st.first_record_uoff == ~0ull && hf[13] != 0xffffffffu && (hf[13] >= H || f->format == FMT_FASTA)) s->st.first_record_uoff = c.u0 + (uint64_t)hf[13] - H;
   // (FASTA: the chain ends at the next record start; a chunk without one says nothing about where that is)
-  if (*owned_done && (f->format != 3 || hf[2] != 0xffffffffu)) s->st.end_chain_uoff = c.u0 + (uint64_t)tail_off - H;
+  if (*owned_done && (f->format != FMT_FASTA || hf[2] != 0xffffffffu)) s->st.end_chain_uoff = c.u0 + (uint64_t)tail_off - H;
   CU_TRY(cudaEventRecord(s->ev_t[slot][2], cs));
   if (n_rec == 0) { CU_TRY(cudaEventRecord(s->ev_t[slot][3], cs)); goto timing; }
   {
     // ---- record offsets
-    uint32_t* d_recoff;
-    if (f->format == 1) d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14];       // lines[] from the first record's line on: 4 per row
-    else if (f->format == 2) d_recoff = const_cast<uint32_t*>(sam_recoff);
-    else if (f->format == 3) {
-      // every line's destination in the chunk's sequence text: content bytes per line, scanned (the decode slices read it)
-      const uint32_t n_lines = fa_hf[FA_F_LINES];
-      if ((rc = s->d_faseq[slot].ensure(4ull * (n_lines + 1) + 64))) return rc;
-      uint32_t* d_seqpos = s->d_faseq[slot].as<uint32_t>();
-      fa_lines_kernel<<<(n_lines + 255) / 256, 256, 0, cs>>>(U, s->d_recoff[slot].as<uint32_t>(), n_lines, d_seqpos);
-      ScanCols LC; memset(&LC, 0, sizeof LC);
-      LC.col[0] = reinterpret_cast<int32_t*>(d_seqpos); LC.n_cols = 1; LC.n = n_lines + 1;
-      const uint32_t n_st = (LC.n + SCAN_TILE - 1) / SCAN_TILE;
-      if ((rc = s->d_tiles.ensure(8ull * n_st)) || (rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS))) return rc;
-      multi_scan_reduce_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
-      multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_tiles.as<uint64_t>(), n_st, s->d_totals.as<uint64_t>());
-      multi_scan_apply_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
-      s->st.kernel_launches += 4;
-      d_recoff = s->d_fastarts[slot].as<uint32_t>();
-      s->cur.fa_lines = s->d_recoff[slot].as<uint32_t>(); s->cur.fa_seqpos = d_seqpos;
-      s->cur.fa_tile_base = s->d_seg[slot].as<uint32_t>() + std::max<uint32_t>(1, (data_hi - BP.data_lo + FQ_TILE - 1) / FQ_TILE);
-      s->cur.fa_lo = BP.data_lo; s->cur.fa_hi = data_hi; s->cur.fa_slice = 0;
-      const uint32_t n_sl = fa_hf[FA_F_SLICES];
-      for (uint32_t k = 0; k <= n_sl; k++) { s->cur.fa_slice_rec[k] = fa_hf[FA_F_SLICE_REC + k]; s->cur.fa_slice_byte[k] = fa_hf[FA_F_SLICE_BYTE + k]; }
-    }
-    else {
-      if ((rc = s->d_recoff[slot].ensure(4ull * (n_rec + 1)))) return rc;
-      d_recoff = s->d_recoff[slot].as<uint32_t>();
-      seg_emit_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, d_seg_start, d_seg_count, d_seg_base, d_recoff, n_rec, tail_off);
-      s->st.kernel_launches++;
+    uint32_t* d_recoff = nullptr;
+    switch (f->format) {
+      case FMT_BAM:
+        if ((rc = s->d_recoff[slot].ensure(4ull * (n_rec + 1)))) return rc;
+        d_recoff = s->d_recoff[slot].as<uint32_t>();
+        seg_emit_kernel<<<(n_seg + 127) / 128, 128, 0, cs>>>(BP, d_seg_start, d_seg_count, d_seg_base, d_recoff, n_rec, tail_off);
+        s->st.kernel_launches++;
+        break;
+      case FMT_FASTQ: d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14]; break;       // lines[] from the first record's line on: 4 per row
+      case FMT_SAM: d_recoff = const_cast<uint32_t*>(sam_recoff); break;
+      case FMT_FASTA: {
+        // every line's destination in the chunk's sequence text: content bytes per line, scanned (the decode slices read it)
+        const uint32_t* fa_hf = s->h_flags + FA_HFLAGS - 16;     // FASTA words, indexed as in d_flags
+        const uint32_t n_lines = fa_hf[FA_F_LINES];
+        if ((rc = s->d_faseq[slot].ensure(4ull * (n_lines + 1) + 64))) return rc;
+        uint32_t* d_seqpos = s->d_faseq[slot].as<uint32_t>();
+        fa_lines_kernel<<<(n_lines + 255) / 256, 256, 0, cs>>>(U, s->d_recoff[slot].as<uint32_t>(), n_lines, d_seqpos);
+        ScanCols LC; memset(&LC, 0, sizeof LC);
+        LC.col[0] = reinterpret_cast<int32_t*>(d_seqpos); LC.n_cols = 1; LC.n = n_lines + 1;
+        const uint32_t n_st = (LC.n + SCAN_TILE - 1) / SCAN_TILE;
+        if ((rc = s->d_tiles.ensure(8ull * n_st)) || (rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS))) return rc;
+        multi_scan_reduce_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
+        multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_tiles.as<uint64_t>(), n_st, s->d_totals.as<uint64_t>());
+        multi_scan_apply_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
+        s->st.kernel_launches += 4;
+        d_recoff = s->d_fastarts[slot].as<uint32_t>();
+        s->cur.fa_lines = s->d_recoff[slot].as<uint32_t>(); s->cur.fa_seqpos = d_seqpos;
+        s->cur.fa_tile_base = s->d_seg[slot].as<uint32_t>() + std::max<uint32_t>(1, (data_hi - BP.data_lo + FQ_TILE - 1) / FQ_TILE);
+        s->cur.fa_lo = BP.data_lo; s->cur.fa_hi = data_hi; s->cur.fa_slice = 0;
+        const uint32_t n_sl = fa_hf[FA_F_SLICES];
+        for (uint32_t k = 0; k <= n_sl; k++) { s->cur.fa_slice_rec[k] = fa_hf[FA_F_SLICE_REC + k]; s->cur.fa_slice_byte[k] = fa_hf[FA_F_SLICE_BYTE + k]; }
+        break;
+      }
     }
     uint32_t n = n_rec;
     if (range.region_mode > 0) {
@@ -1193,7 +1249,7 @@ timing:
   {
     float a = 0, b = 0, d = 0;
     cudaEventElapsedTime(&a, s->ev_t[slot][0], s->ev_t[slot][1]);
-    if (f->format == 2) cudaEventElapsedTime(&a, s->ev_ing[slot][0], s->ev_ing[slot][1]);     // SAM: the ingest copy
+    if (f->format == FMT_SAM) cudaEventElapsedTime(&a, s->ev_ing[slot][0], s->ev_ing[slot][1]);     // SAM: the ingest copy
     cudaEventElapsedTime(&b, s->ev_t[slot][1], s->ev_t[slot][2]);
     cudaEventElapsedTime(&d, s->ev_t[slot][2], s->ev_t[slot][3]);
     s->st.ms_inflate += a; s->st.ms_boundary += b; s->st.ms_decode += d;
@@ -1249,7 +1305,7 @@ static int advance(BamScanStream* s, bool* produced) {
       if (r.region_mode < 0) { set_error("BAM region query failed: a region names a reference sequence that is not in the BAM header"); return BAMSCAN_ERR_INVALID; }
       s->tail_seen = false; s->range_stop = false;
       s->chunks.clear(); s->chunk_idx = 0; s->carry_len = 0; s->have_h2d_ahead = false; s->ext_blocks = 8; s->need_spec = !r.exact_start;
-      s->fa_leading = f->format == 3 && r.first_uoff == 0;
+      s->fa_leading = f->format == FMT_FASTA && r.first_uoff == 0;
       plan_chunks(*f, r.block_begin, r.block_end, false, &s->chunks);
       s->range_open = true;
       if (s->chunks.empty()) { s->range_open = false; s->range_idx++; continue; }
@@ -1260,7 +1316,7 @@ static int advance(BamScanStream* s, bool* produced) {
       uint32_t last = s->chunks.back().b1;
       if (s->carry_len == 0 || last >= f->blocks.size()) {
         if (s->carry_len) {
-          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", f->format == 1 ? "FASTQ" : f->format == 2 ? "SAM" : f->format == 3 ? "FASTA" : "BAM", s->carry_len);
+          set_error("%s read error: unexpected EOF inside a record (%u trailing bytes)", format_name(f->format), s->carry_len);
           return BAMSCAN_ERR_FORMAT;
         }
         s->range_open = false; s->range_idx++;
@@ -1405,7 +1461,7 @@ extern "C" {
 const char* bamscan_last_error(void) { return last_error_cstr(); }
 const char* bamscan_version(void) { return "bamscan-b200 0.1 (sm_100a)"; }
 
-static int bamscan_open_impl(const char* path, const char* index_path_or_null, const BamScanOptions* options, BamScanHandle** out, int format = 0);
+static int bamscan_open_impl(const char* path, const char* index_path_or_null, const BamScanOptions* options, BamScanHandle** out, ScanFormat format = FMT_BAM);
 
 // No C++ exception may cross the C ABI (a corrupt file can ask for absurd allocations): they become BAMSCAN_ERR_FORMAT.
 #define BAMSCAN_GUARD(call)                                                                                          \
@@ -1418,9 +1474,9 @@ int bamscan_open(const char* path, const char* index_path_or_null, const BamScan
   BAMSCAN_GUARD(bamscan_open_impl(path, index_path_or_null, options, out))
 }
 
-static int bamscan_open_impl(const char* path, const char* index_path_or_null, const BamScanOptions* options, BamScanHandle** out, int format) {
+static int bamscan_open_impl(const char* path, const char* index_path_or_null, const BamScanOptions* options, BamScanHandle** out, ScanFormat format) {
   if (!path || !out) { set_error("bamscan_open: null argument"); return BAMSCAN_ERR_INVALID; }
-  if (format == 0 && is_sam_path(path)) format = 2;
+  if (format == FMT_BAM && is_sam_path(path)) format = FMT_SAM;
   BamScanOptions opt;
   memset(&opt, 0, sizeof opt);
   opt.coordinate_system_zero_based = 1; opt.infer_tag_types = 1; opt.infer_tag_sample_size = 100;
@@ -1443,17 +1499,17 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
   if (opt.segment_bytes) { f.seg_bytes = std::max<uint32_t>(256, opt.segment_bytes); f.seg_bytes_set = true; }
   f.skip_crc = opt.skip_crc != 0; f.debug_flags = opt.debug_flags; f.decode_all_tags = opt.decode_all_tag_fields != 0;
   int rc = load_file(&f);
-  if (rc == BAMSCAN_ERR_IO || rc == BAMSCAN_ERR_CUDA || (format == 2 && rc)) { release_file(&f); return rc; }
+  if (rc == BAMSCAN_ERR_IO || rc == BAMSCAN_ERR_CUDA || (format == FMT_SAM && rc)) { release_file(&f); return rc; }
   // a file whose header cannot be read still yields a provider with empty metadata (table_provider.rs:423-426);
   // scans on it fail later
-  if (format == 1) {
+  if (format == FMT_FASTQ) {
     // == determine_schema of bio-format-fastq/src/table_provider.rs:22-32
     if (rc) { release_file(&f); return rc; }
     f.fields = {FieldDef{"name", HK_Utf8, false, {}}, FieldDef{"description", HK_Utf8, true, {}}, FieldDef{"sequence", HK_Utf8, false, {}}, FieldDef{"quality_scores", HK_Utf8, false, {}}};
     *out = h.release();
     return BAMSCAN_OK;
   }
-  if (format == 3) {
+  if (format == FMT_FASTA) {
     // FASTA: name, description (NULL when empty), sequence; no metadata, as for FASTQ
     if (rc) { release_file(&f); return rc; }
     f.fields = {FieldDef{"name", HK_Utf8, false, {}}, FieldDef{"description", HK_Utf8, true, {}}, FieldDef{"sequence", HK_Utf8, false, {}}};
@@ -1461,7 +1517,7 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
     return BAMSCAN_OK;
   }
   if ((rc = build_schema(&f, &opt))) { release_file(&f); return rc; }
-  if (format == 2) { *out = h.release(); return BAMSCAN_OK; }     // SAM: no index (the reference discovers none for SAM paths)
+  if (format == FMT_SAM) { *out = h.release(); return BAMSCAN_OK; }     // SAM: no index (the reference discovers none for SAM paths)
   if (index_path_or_null) f.index_path = index_path_or_null; else f.index_path = discover_index(f.path);   // "" = no index
   if (!f.index_path.empty()) {
     f.bai.reset(new BaiIndex());
@@ -1472,11 +1528,11 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
 }
 
 int bamscan_open_fastq(const char* path, const BamScanOptions* options, BamScanHandle** out) {
-  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, 1))
+  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, FMT_FASTQ))
 }
 
 int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanHandle** out) {
-  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, 3))
+  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, FMT_FASTA))
 }
 
 void bamscan_close(BamScanHandle* h) {
@@ -1494,7 +1550,7 @@ int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out) {
 
 static int bamscan_describe_tags_impl(BamScanHandle* h, int32_t sample_size, char* buf, uint64_t cap, uint64_t* needed) {
   if (!h || !needed || (cap && !buf)) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == 1 || h->file.format == 3) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
+  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
   if (!h->file.header_ok) { set_error("BAM header could not be read: %s", h->file.path.c_str()); return BAMSCAN_ERR_FORMAT; }
   std::map<std::string, std::pair<char, int32_t>> found;
   infer_tag_types(h->file, {}, sample_size > 0 ? sample_size : 100, &found, true);
@@ -1523,7 +1579,7 @@ int bamscan_describe_tags(BamScanHandle* h, int32_t sample_size, char* buf, uint
 
 int bamscan_classify_filters(BamScanHandle* h, const BamScanFilter* filters, int32_t n_filters, uint8_t* out_pushdown) {
   if (!h || (n_filters && (!filters || !out_pushdown))) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == 1 || h->file.format == 3) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // FastqTableProvider and FastaTableProvider push no filter down
+  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // FastqTableProvider and FastaTableProvider push no filter down
   return classify_filters(h->file, filters, n_filters, out_pushdown);
 }
 
@@ -1776,7 +1832,7 @@ int bamscan_bench_inflate(BamScanPlan* plan, int32_t partition, int32_t repeats,
   int rc = make_stream(plan, partition, true, &s);
   if (rc) return rc;
   BamFile* f = s->f;
-  if (f->format == 2) { stream_destroy(s); set_error("a SAM scan has no inflate to benchmark"); return BAMSCAN_ERR_INVALID; }
+  if (f->format == FMT_SAM) { stream_destroy(s); set_error("a SAM scan has no inflate to benchmark"); return BAMSCAN_ERR_INVALID; }
   if (s->part->ranges.empty()) { stream_destroy(s); set_error("empty partition"); return BAMSCAN_ERR_INVALID; }
   const ScanRange& r = s->part->ranges[0];
   std::vector<ChunkPlan> chunks;

@@ -89,7 +89,7 @@ static int walk_blocks(BamFile* f) {
   return BAMSCAN_OK;
 }
 
-// ---- plain SAM (format 2) ----
+// ---- plain SAM ----
 // The text body is described as pseudo-blocks with csize == isize and coff == uoff == the file offset, so that planning, chunking
 // and the seam evidence of block-range partitions work on it unchanged.
 constexpr uint32_t SAM_BLOCK = 65536;
@@ -289,10 +289,10 @@ int load_file(BamFile* f) {
     memset(f->data + f->size, 0, 4096);
   }
   fclose(fp);
-  if (f->format == 2) return load_sam(f);
+  if (f->format == FMT_SAM) return load_sam(f);
   int rc = walk_blocks(f);
   if (rc) return rc;
-  if (f->format == 1 || f->format == 3) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ, FASTA: no header
+  if (f->format == FMT_FASTQ || f->format == FMT_FASTA) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ, FASTA: no header
 
   // BAM header (noodles-bam read_header): magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
   HostStream hs(*f);
@@ -322,7 +322,7 @@ int load_file(BamFile* f) {
 // `all` (BamTableProvider::describe, table_provider.rs:715-745): every tag met in the sample, first occurrence wins.
 int infer_tag_types(const BamFile& f, const std::vector<std::string>& tags, int sample_size,
                     std::map<std::string, std::pair<char, int32_t>>* out, bool all) {
-  if (f.format == 2) return infer_tag_types_sam(f, tags, sample_size, out, all);
+  if (f.format == FMT_SAM) return infer_tag_types_sam(f, tags, sample_size, out, all);
   HostStream hs(f);
   // position on the first record
   while (hs.base_uoff + hs.buf.size() <= f.first_record_uoff) if (!hs.fill()) return BAMSCAN_OK;

@@ -104,7 +104,7 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
       r.first_uoff = (p == 0) ? f->first_record_uoff : (b < n_blocks ? f->blocks[b].uoff : f->total_inflated);
       r.stop_uoff = e < n_blocks ? f->blocks[e].uoff : ~0ull;
       bool owns = b < e;
-      if (f->format == 2 && owns) {
+      if (f->format == FMT_SAM && owns) {
         // SAM: a record is a line; the host sees whether the byte in front of the range is '\n', so every range starts exactly
         // on its first owned line (one that begins in front of the range's end), in the block that holds it
         r.exact_start = true;
@@ -112,7 +112,7 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
         owns = r.first_uoff < std::min<uint64_t>(r.stop_uoff, f->size);
         if (owns) r.block_begin = block_of_uoff(*f, r.first_uoff);
       }
-      if (f->format == 3 && owns) {
+      if (f->format == FMT_FASTA && owns) {
         // FASTA: a record belongs to the range that holds its '>'.  Whether the range's first byte starts a line depends on the byte in
         // front of it, so the last non-empty member in front of the range is inflated too, and nothing in it is owned (first_uoff)
         r.exact_start = true;
@@ -131,7 +131,7 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
   // FASTQ, reference rule (bio-format-fastq/src/physical_exec.rs:94-116, 140-175): a BGZF file with a companion `<path>.gzi`
   // is cut into min(target, blocks) runs of whole blocks by block COUNT (num_blocks / n, the first num_blocks % n runs one
   // longer), where blocks = the GZI entries plus the implicit first member; without a GZI the scan is sequential.
-  if (f->format == 1 && target_partitions > 1) {
+  if (f->format == FMT_FASTQ && target_partitions > 1) {
     std::vector<std::pair<uint64_t, uint64_t>> gzi;
     int rc = load_gzi(f->path + ".gzi", &gzi);
     if (rc == BAMSCAN_OK) {

@@ -80,7 +80,6 @@ struct DevBuf {
 };
 
 struct WTag { int col; int32_t kind; uint8_t tag[2], sam_type, subtype; };
-enum : int { FMT_BAM = 0, FMT_FASTQ = 1, FMT_SAM = 2 };
 
 // Device buffers, pinned staging, stream and events of a writer.  One set per device is kept between writers (cudaMalloc /
 // cudaHostAlloc / cudaFree of a few GB cost more than writing a few million records).
@@ -117,7 +116,7 @@ struct BamWriter : bamscan::WriterRes {
   int device = 0;
   bool zero_based = true, cigar_binary = false, finished = false;
   int compression = 0;
-  int format = FMT_BAM;
+  ScanFormat format = FMT_BAM;
   bool plain = false;                    // FASTQ compression 2, SAM: the text goes to the file as it is (no BGZF, no EOF marker)
   int col[11] = {};                      // BAM, SAM: name chrom start flags cigar mapq mate_chrom mate_start seq qual tlen;
                                          // FASTQ: name description (-1: absent) sequence quality_scores
@@ -173,7 +172,6 @@ static int enc_err_class(uint32_t code) {
   return (code == enc::ENC_ERR_TAG_RANGE || code == enc::ENC_ERR_TAG_HEX || code == enc::ENC_ERR_TAG_CHAR) ? BAMSCAN_ERR_SCHEMA
          : code == enc::ENC_ERR_CIGAR_OPS ? BAMSCAN_ERR_UNSUPPORTED : BAMSCAN_ERR_FORMAT;
 }
-static const char* fmt_name(const BamWriter* w) { return w->format == FMT_FASTQ ? "FASTQ" : w->format == FMT_SAM ? "SAM" : "BAM"; }
 
 static std::map<std::string, std::string> parse_metadata(const char* md) {
   std::map<std::string, std::string> out;
@@ -222,7 +220,7 @@ static int writer_open_file(BamWriter* w, const char* output_path);
 
 static int writer_open_impl(const char* output_path, const char* sam_header_text, int32_t n_ref, const char* const* ref_names,
                             const int32_t* ref_lengths, const ArrowSchema* schema, const BamWriteOptions* options, BamWriter** out,
-                            int format = FMT_BAM) {
+                            ScanFormat format = FMT_BAM) {
   if (!output_path || !schema || !out || (n_ref > 0 && (!ref_names || !ref_lengths))) { set_error("bamscan_writer_open: null argument"); return BAMSCAN_ERR_INVALID; }
   BamWriteOptions opt;
   memset(&opt, 0, sizeof opt);
@@ -726,7 +724,7 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
     uint64_t total = 0;
     const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
     if ((rc = sum_lengths(w, rows, d_err, &total))) return rc;
-    if (e[0]) { set_error("%s write error: row %u: %s", fmt_name(w), e[1], enc_err_text(e[0])); return enc_err_class(e[0]); }
+    if (e[0]) { set_error("%s write error: row %u: %s", format_name(w->format), e[1], enc_err_text(e[0])); return enc_err_class(e[0]); }
     if (w->format == FMT_SAM) {                                // the rows passed the BAM rules: SAM line lengths + the SAM-only checks
       if (total / rows > 2048) samenc::sam_size_kernel<32><<<(rows * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint32_t*>(w->rec_len.p), d_err);
       else samenc::sam_size_kernel<8><<<(((rows + 3) / 4) * 32 + 255) / 256, 256, 0, w->stream>>>(A, d_cig_ops, static_cast<int32_t*>(w->ref_pairs.p), static_cast<uint32_t*>(w->rec_len.p), d_err);
@@ -758,7 +756,7 @@ static int writer_write_impl(BamWriter* w, const ArrowArray* batch) {
     WCU_TRY(cudaStreamSynchronize(w->stream));
     {
       const uint32_t* e = reinterpret_cast<const uint32_t*>(w->h_small + 4096);
-      if (e[0]) { set_error("%s write error: row %u: %s", fmt_name(w), e[1], enc_err_text(e[0])); return w->format == FMT_SAM ? BAMSCAN_ERR_INVALID : BAMSCAN_ERR_SCHEMA; }
+      if (e[0]) { set_error("%s write error: row %u: %s", format_name(w->format), e[1], enc_err_text(e[0])); return w->format == FMT_SAM ? BAMSCAN_ERR_INVALID : BAMSCAN_ERR_SCHEMA; }
       float ms = 0; cudaEventElapsedTime(&ms, w->ev[0], w->ev[1]); w->st.ms_encode += ms; w->st.ms_total += ms;
     }
     w->st.rows += rows; w->st.bam_bytes += total;
@@ -779,7 +777,7 @@ static int writer_emit(BamWriter* w, const uint8_t* dev, uint64_t bytes) {
     {
       std::unique_lock<std::mutex> lk(w->mu);
       w->cv.wait(lk, [&] { for (int b = 0; b < OUT_BUFS; b++) if (!w->out_busy[b]) { slot = b; return true; } return w->file_failed; });
-      if (w->file_failed || slot < 0) { set_error("Failed to write %s record: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (w->file_failed || slot < 0) { set_error("Failed to write %s record: write(%s) failed", format_name(w->format), w->path.c_str()); return BAMSCAN_ERR_IO; }
       w->out_busy[slot] = FILE_THREADS;
     }
     WCU_TRY(cudaMemcpyAsync(w->h_out[slot], dev + at, nb, cudaMemcpyDeviceToHost, w->stream));
@@ -860,11 +858,11 @@ static int writer_finish_impl(BamWriter* w, uint64_t* rows_written) {
     {
       std::unique_lock<std::mutex> lk(w->mu);
       w->cv.wait(lk, [&] { if (!w->file_q.empty()) return false; for (int b = 0; b < OUT_BUFS; b++) if (w->out_busy[b]) return false; return true; });
-      if (w->file_failed) { set_error("Failed to finish %s stream: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (w->file_failed) { set_error("Failed to finish %s stream: write(%s) failed", format_name(w->format), w->path.c_str()); return BAMSCAN_ERR_IO; }
     }
     if (!w->plain) {
       static const uint8_t eof_marker[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-      if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish %s stream: write(%s) failed", fmt_name(w), w->path.c_str()); return BAMSCAN_ERR_IO; }
+      if (::pwrite(w->fd, eof_marker, 28, (off_t)w->file_off) != 28) { set_error("Failed to finish %s stream: write(%s) failed", format_name(w->format), w->path.c_str()); return BAMSCAN_ERR_IO; }
       w->st.compressed_bytes += 28;
     }
     ::close(w->fd); w->fd = -1;
