@@ -610,6 +610,19 @@ static int flush_slice(BamScanStream* s) {
   return BAMSCAN_OK;
 }
 
+// Arrow offsets from per-row lengths (kernels_decode.cuh phase 2): every column of SC is exclusive-scanned in place, column k's
+// total -> totals[k].  tiles holds the tile sums and is sized here.
+static int launch_offsets_scan(BamScanStream* s, cudaStream_t cs, const ScanCols& SC, DeviceBuf& tiles, uint64_t* totals) {
+  const uint32_t n_tiles = (SC.n + SCAN_TILE - 1) / SCAN_TILE;
+  if (int rc = tiles.ensure(8ull * n_tiles * SC.n_cols)) return rc;
+  uint64_t* d_tiles = tiles.as<uint64_t>();
+  multi_scan_reduce_kernel<<<dim3(n_tiles, SC.n_cols), SCAN_TPB, 0, cs>>>(SC, d_tiles, n_tiles);
+  cta_scan_kernel<<<SC.n_cols, CTA_SCAN_THREADS, 0, cs>>>(d_tiles, d_tiles, n_tiles, totals);
+  multi_scan_apply_kernel<<<dim3(n_tiles, SC.n_cols), SCAN_TPB, 0, cs>>>(SC, d_tiles, n_tiles);
+  s->st.kernel_launches += 3;
+  return BAMSCAN_OK;
+}
+
 static int decode_slice(BamScanStream* s, bool* produced) {
   NvtxRange nv("bamscan: decode slice (fixed, scan, var) + D2H issue");
   BamFile* f = s->f;
@@ -719,13 +732,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
     s->st.kernel_launches++;
     uint64_t* h_totals = reinterpret_cast<uint64_t*>(s->h_flags + 16);
     if (SC.n_cols) {
-      uint32_t n_tiles = (SC.n + SCAN_TILE - 1) / SCAN_TILE;
-      if ((rc = s->d_tiles.ensure(8ull * n_tiles * SC.n_cols))) return rc;
-      if ((rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS))) return rc;
-      multi_scan_reduce_kernel<<<dim3(n_tiles, SC.n_cols), SCAN_TPB, 0, cs>>>(SC, s->d_tiles.as<uint64_t>(), n_tiles);
-      multi_scan_tiles_kernel<<<SC.n_cols, 1024, 0, cs>>>(s->d_tiles.as<uint64_t>(), n_tiles, s->d_totals.as<uint64_t>());
-      multi_scan_apply_kernel<<<dim3(n_tiles, SC.n_cols), SCAN_TPB, 0, cs>>>(SC, s->d_tiles.as<uint64_t>(), n_tiles);
-      s->st.kernel_launches += 3;
+      if ((rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS)) || (rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>()))) return rc;
       publish_kernel<<<1, 128, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, 2 * SC.n_cols);      // [16, 16 + 2 * MAX_SCAN_COLS) of the mapped flags page; the decode error words live at [512, 516)
       CU_TRY(cudaEventRecord(s->ev_dflags, cs));
       CU_TRY(cudaEventSynchronize(s->ev_dflags));
@@ -875,13 +882,9 @@ static int transcode_sam(BamScanStream* s, int slot, cudaStream_t cs, const uint
   sam::sam_size_kernel<<<(n + 255) / 256, 256, 0, cs>>>(A);
   ScanCols SC; memset(&SC, 0, sizeof SC);
   SC.col[0] = reinterpret_cast<int32_t*>(A.sizes); SC.n_cols = 1; SC.n = n + 1;
-  const uint32_t n_tiles = (SC.n + SCAN_TILE - 1) / SCAN_TILE;
-  if ((rc = s->d_samtiles[slot].ensure(8ull * n_tiles))) return rc;
-  multi_scan_reduce_kernel<<<dim3(n_tiles, 1), SCAN_TPB, 0, cs>>>(SC, s->d_samtiles[slot].as<uint64_t>(), n_tiles);
-  multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_samtiles[slot].as<uint64_t>(), n_tiles, reinterpret_cast<uint64_t*>(d_flags + 26));
-  multi_scan_apply_kernel<<<dim3(n_tiles, 1), SCAN_TPB, 0, cs>>>(SC, s->d_samtiles[slot].as<uint64_t>(), n_tiles);
+  if ((rc = launch_offsets_scan(s, cs, SC, s->d_samtiles[slot], reinterpret_cast<uint64_t*>(d_flags + 26)))) return rc;
   publish_kernel<<<1, 32, 0, cs>>>(d_err, s->d_hflags + 600, 4);     // [600, 604) of the mapped page: nothing else uses it
-  s->st.kernel_launches += 5;
+  s->st.kernel_launches += 2;
   CU_TRY(cudaEventRecord(s->ev_flags[slot], cs));
   CU_TRY(cudaEventSynchronize(s->ev_flags[slot]));
   CU_TRY(cudaGetLastError());
@@ -918,7 +921,7 @@ static int launch_line_scan(BamScanStream* s, int slot, cudaStream_t cs, const u
   uint32_t* d_tile_count = s->d_seg[slot].as<uint32_t>();
   L->tile_base = d_tile_count + L->n_tiles;
   fq_count_kernel<<<L->n_tiles, 256, 0, cs>>>(U, lo, hi, d_tile_count);
-  fq_scan_kernel<<<1, 1024, 0, cs>>>(d_tile_count, L->tile_base, L->n_tiles, s->d_flags[slot].as<uint32_t>() + 16);
+  cta_scan_kernel<<<1, CTA_SCAN_THREADS, 0, cs>>>(d_tile_count, L->tile_base, L->n_tiles, s->d_flags[slot].as<uint32_t>() + 16);
   fq_lines_kernel<<<L->n_tiles, 256, 0, cs>>>(U, lo, hi, L->tile_base, s->d_recoff[slot].as<uint32_t>(), L->line_cap);
   s->st.kernel_launches += 3;
   return BAMSCAN_OK;
@@ -997,7 +1000,7 @@ static int frame_fasta(BamScanStream* s, const ChunkPlan& c, const ScanRange& ra
   const uint32_t lead_ok = carry || (first_of_range ? c.u0 == 0 : s->fa_lead_nl);
   FastaFrame FF{BP.U, lo, data_hi, own_lo, BP.own_hi, lead_ok, (uint32_t)(c.b1 == s->f->blocks.size() ? 1 : 0), L.line_cap, (uint32_t)SLICE_BYTES};
   fa_count_kernel<<<L.n_tiles, 256, 0, cs>>>(FF, d_st_count);
-  fq_scan_kernel<<<1, 1024, 0, cs>>>(d_st_count, d_st_base, L.n_tiles, d_flags + FA_F_STARTS);
+  cta_scan_kernel<<<1, CTA_SCAN_THREADS, 0, cs>>>(d_st_count, d_st_base, L.n_tiles, d_flags + FA_F_STARTS);
   fa_starts_kernel<<<L.n_tiles, 256, 0, cs>>>(FF, L.tile_base, d_st_base, s->d_fastarts[slot].as<uint32_t>());
   fa_frame_kernel<<<1, 32, 0, cs>>>(FF, s->d_recoff[slot].as<uint32_t>(), s->d_fastarts[slot].as<uint32_t>(), d_flags);
   s->st.kernel_launches += 4;
@@ -1185,14 +1188,10 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
         if ((rc = s->d_faseq[slot].ensure(4ull * (n_lines + 1) + 64))) return rc;
         uint32_t* d_seqpos = s->d_faseq[slot].as<uint32_t>();
         fa_lines_kernel<<<(n_lines + 255) / 256, 256, 0, cs>>>(U, s->d_recoff[slot].as<uint32_t>(), n_lines, d_seqpos);
+        s->st.kernel_launches++;
         ScanCols LC; memset(&LC, 0, sizeof LC);
         LC.col[0] = reinterpret_cast<int32_t*>(d_seqpos); LC.n_cols = 1; LC.n = n_lines + 1;
-        const uint32_t n_st = (LC.n + SCAN_TILE - 1) / SCAN_TILE;
-        if ((rc = s->d_tiles.ensure(8ull * n_st)) || (rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS))) return rc;
-        multi_scan_reduce_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
-        multi_scan_tiles_kernel<<<1, 1024, 0, cs>>>(s->d_tiles.as<uint64_t>(), n_st, s->d_totals.as<uint64_t>());
-        multi_scan_apply_kernel<<<dim3(n_st, 1), SCAN_TPB, 0, cs>>>(LC, s->d_tiles.as<uint64_t>(), n_st);
-        s->st.kernel_launches += 4;
+        if ((rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS)) || (rc = launch_offsets_scan(s, cs, LC, s->d_tiles, s->d_totals.as<uint64_t>()))) return rc;
         d_recoff = s->d_fastarts[slot].as<uint32_t>();
         s->cur.fa_lines = s->d_recoff[slot].as<uint32_t>(); s->cur.fa_seqpos = d_seqpos;
         s->cur.fa_tile_base = s->d_seg[slot].as<uint32_t>() + std::max<uint32_t>(1, (data_hi - BP.data_lo + FQ_TILE - 1) / FQ_TILE);

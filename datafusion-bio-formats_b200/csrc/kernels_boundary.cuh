@@ -21,6 +21,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "kernels_scan.cuh"
+
 namespace bamscan {
 
 constexpr uint32_t SEG_NONE = 0xffffffffu;
@@ -246,41 +248,19 @@ __global__ void seg_repair_kernel(BoundaryParams P, WalkOut W) {
 __global__ void __launch_bounds__(1024)
 seg_scan_kernel(const uint32_t* __restrict__ seg_count, const uint32_t* __restrict__ seg_start, const uint32_t* __restrict__ seg_exit,
                 const uint8_t* __restrict__ seg_tail, uint32_t* __restrict__ seg_base, uint32_t n_seg, uint32_t* __restrict__ flags) {
-  __shared__ uint32_t warp_sums[32];
-  __shared__ uint32_t carry;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n_seg; base += 1024) {
-    uint32_t i = base + tid;
-    uint32_t v = i < n_seg ? seg_count[i] : 0u;
+  const uint32_t total = cta_exclusive_scan<uint32_t>(n_seg, [&](uint32_t i) {
+    const uint32_t v = i < n_seg ? seg_count[i] : 0u;
     {
       // offset of the first owned record of the chunk: one atomic per warp that holds one (a 1.5 GB chunk has 90 k segments with
       // records; one same-address atomic each made this kernel the slowest of the stage)
       const uint32_t mine = v ? seg_start[i] : 0xffffffffu;
       const uint32_t wmin = __reduce_min_sync(0xffffffffu, mine);
-      if (lane == 0 && wmin != 0xffffffffu && wmin < flags[13]) atomicMin(&flags[13], wmin);
+      if ((threadIdx.x & 31) == 0 && wmin != 0xffffffffu && wmin < flags[13]) atomicMin(&flags[13], wmin);
     }
     if (i < n_seg && seg_start[i] != SEG_NONE && seg_tail[i] == 2) atomicExch(&flags[1], seg_exit[i] | 1u);   // corrupt block_size on the live chain
-    uint32_t x = v;
-    #pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-    if (lane == 31) warp_sums[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = warp_sums[lane];
-      #pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += y; }
-      warp_sums[lane] = w;
-    }
-    __syncthreads();
-    uint32_t excl = carry + (warp ? warp_sums[warp - 1] : 0u) + x - v;
-    if (i < n_seg) seg_base[i] = excl;
-    __syncthreads();
-    if (tid == 1023) carry = excl + v;
-    __syncthreads();
-  }
-  if (tid == 0) flags[3] = carry;
+    return v;
+  }, [&](uint32_t i, uint32_t excl, uint32_t) { seg_base[i] = excl; });
+  if (threadIdx.x == 0) flags[3] = total;
 }
 
 // one thread per segment: emit record offsets

@@ -9,8 +9,8 @@
 //   decode_fixed_kernel  : one THREAD per record.  Fixed-width columns, validity bitmaps (warp ballots),
 //                          per-row byte lengths of every projected var-len column, one aux walk that
 //                          locates / converts every requested tag.
-//   multi_scan_*         : exclusive prefix sums turning the length arrays into Arrow i32 offsets
-//                          (all var-len columns in one launch, grid.y = column).
+//   multi_scan_reduce -> cta_scan_kernel -> multi_scan_apply : exclusive prefix sums turning the length arrays into Arrow
+//                          i32 offsets (all var-len columns in each launch: grid.y = column, one scan CTA per column).
 //   decode_var_kernel    : a group of 8 lanes (short reads) or a whole warp (long reads) per record.  Copies / transcodes the var-len payloads to their final
 //                          offsets: name, chrom / mate_chrom (dictionary expand), CIGAR text (or raw words),
 //                          sequence (4-bit -> ASCII via shared LUT), qualities (+33), Z/H/A/int-as-text tags,
@@ -22,6 +22,7 @@
 #include "f32_text.h"
 
 #include "kernels_boundary.cuh"
+#include "kernels_scan.cuh"
 
 namespace bamscan {
 
@@ -377,78 +378,29 @@ constexpr int MAX_SCAN_COLS = 6 + MAX_TAGS;
 
 struct ScanCols { int32_t* col[MAX_SCAN_COLS]; int n_cols; uint32_t n; /* elements per column = rows + 1 */ };
 
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* total, uint32_t* ws) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t x = v;
-  #pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-  if (lane == 31) ws[warp] = x;
-  __syncthreads();
-  if (warp == 0) {
-    uint32_t w = lane < (SCAN_TPB / 32) ? ws[lane] : 0u;
-    #pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += y; }
-    ws[lane] = w;
-  }
-  __syncthreads();
-  uint32_t excl = (warp ? ws[warp - 1] : 0u) + x - v;
-  *total = ws[SCAN_TPB / 32 - 1];
-  __syncthreads();
-  return excl;
-}
-
+// per column: tile sums (multi_scan_reduce), their scan (cta_scan_kernel<uint64_t, uint64_t>, in place, one CTA per column), the
+// tile's rows (multi_scan_apply)
 __global__ void __launch_bounds__(SCAN_TPB)
 multi_scan_reduce_kernel(ScanCols C, uint64_t* __restrict__ tile_sums, uint32_t n_tiles) {
-  __shared__ uint32_t ws[32];
+  __shared__ uint32_t ws[SCAN_TPB / 32];
   const int32_t* col = C.col[blockIdx.y];
   uint32_t base = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_ITEMS;
   uint32_t s = 0;
   #pragma unroll
   for (int k = 0; k < SCAN_ITEMS; k++) if (base + k < C.n - 1u) s += (uint32_t)col[base + k];   // element n-1 is the sentinel slot
-  uint32_t total;
-  block_exclusive_scan(s, &total, ws);
+  const uint32_t total = block_sum<SCAN_TPB>(s, ws);
   if (threadIdx.x == 0) tile_sums[(size_t)blockIdx.y * n_tiles + blockIdx.x] = total;
-}
-
-// one CTA per column: exclusive scan of the tile sums (64-bit), total -> totals[col]
-__global__ void __launch_bounds__(1024)
-multi_scan_tiles_kernel(uint64_t* __restrict__ tile_sums, uint32_t n_tiles, uint64_t* __restrict__ totals) {
-  __shared__ uint64_t sh[1024];
-  __shared__ uint64_t carry;
-  uint64_t* ts = tile_sums + (size_t)blockIdx.x * n_tiles;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n_tiles; base += 1024) {
-    uint32_t i = base + threadIdx.x;
-    uint64_t v = i < n_tiles ? ts[i] : 0ull;
-    sh[threadIdx.x] = v;
-    __syncthreads();
-    for (int o = 1; o < 1024; o <<= 1) {
-      uint64_t y = threadIdx.x >= (uint32_t)o ? sh[threadIdx.x - o] : 0ull;
-      __syncthreads();
-      sh[threadIdx.x] += y;
-      __syncthreads();
-    }
-    uint64_t incl = sh[threadIdx.x];
-    if (i < n_tiles) ts[i] = carry + incl - v;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry += incl;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) totals[blockIdx.x] = carry;
 }
 
 __global__ void __launch_bounds__(SCAN_TPB)
 multi_scan_apply_kernel(ScanCols C, const uint64_t* __restrict__ tile_sums, uint32_t n_tiles) {
-  __shared__ uint32_t ws[32];
+  __shared__ uint32_t ws[SCAN_TPB / 32];
   int32_t* col = C.col[blockIdx.y];
   uint32_t base = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_ITEMS;
   uint32_t v[SCAN_ITEMS], s = 0;
   #pragma unroll
   for (int k = 0; k < SCAN_ITEMS; k++) { v[k] = (base + k < C.n - 1u) ? (uint32_t)col[base + k] : 0u; s += v[k]; }
-  uint32_t total;
-  uint32_t excl = block_exclusive_scan(s, &total, ws);
-  uint32_t run = (uint32_t)tile_sums[(size_t)blockIdx.y * n_tiles + blockIdx.x] + excl;
+  uint32_t run = (uint32_t)tile_sums[(size_t)blockIdx.y * n_tiles + blockIdx.x] + block_exclusive_scan<SCAN_TPB>(s, ws);
   #pragma unroll
   for (int k = 0; k < SCAN_ITEMS; k++) { if (base + k < C.n) col[base + k] = (int32_t)run; run += v[k]; }
 }

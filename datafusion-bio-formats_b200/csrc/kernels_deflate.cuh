@@ -25,10 +25,12 @@
 //      shared-memory atomicOr into the member image, which reuses the input buffer), end-of-block, CRC-32 + ISIZE trailer,
 //      and the finished member (gzip header with the BC extra field included) leaves with 16-byte stores.
 //   A member that would not shrink is written as a stored block.
-// bgzf_offsets_kernel / bgzf_gather_kernel: exclusive scan of the member sizes, then the members are packed back to back.
+// cta_scan_kernel (kernels_scan.cuh) / bgzf_gather_kernel: exclusive scan of the member sizes, then the members are packed back to back.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
+
+#include "kernels_scan.cuh"
 
 namespace bamscan {
 namespace dfl {
@@ -536,32 +538,6 @@ bgzf_deflate_kernel(const uint8_t* __restrict__ stream, unsigned long long strea
   }
 }
 
-// member sizes -> byte offsets of the packed file image (one CTA)
-__global__ void __launch_bounds__(1024)
-bgzf_offsets_kernel(const uint32_t* __restrict__ sizes, uint32_t n, unsigned long long* __restrict__ offsets, unsigned long long* __restrict__ total) {
-  __shared__ unsigned long long sh[1024];
-  __shared__ unsigned long long carry;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t b = 0; b < n; b += 1024) {
-    const uint32_t i = b + threadIdx.x;
-    const unsigned long long v = i < n ? sizes[i] : 0ull;
-    sh[threadIdx.x] = v;
-    __syncthreads();
-    for (int o = 1; o < 1024; o <<= 1) {
-      const unsigned long long y = threadIdx.x >= (uint32_t)o ? sh[threadIdx.x - o] : 0ull;
-      __syncthreads();
-      sh[threadIdx.x] += y;
-      __syncthreads();
-    }
-    if (i < n) offsets[i] = carry + sh[threadIdx.x] - v;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry += sh[1023];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *total = carry;
-}
-
 __global__ void __launch_bounds__(256)
 bgzf_gather_kernel(const uint8_t* __restrict__ slots, const uint32_t* __restrict__ sizes, const unsigned long long* __restrict__ offsets, uint8_t* __restrict__ out) {
   const uint32_t m = blockIdx.x, n = sizes[m];
@@ -587,11 +563,8 @@ len_tile_sums_kernel(const uint32_t* __restrict__ len, uint32_t n, unsigned long
   unsigned long long s = 0;
   #pragma unroll
   for (int k = 0; k < 16; k++) if (base + k < n) s += len[base + k];
-  #pragma unroll
-  for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(FULL, s, o);
-  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = s;
-  __syncthreads();
-  if (threadIdx.x == 0) { unsigned long long t = 0; for (int w = 0; w < 8; w++) t += ws[w]; tile_sums[blockIdx.x] = t; }
+  const unsigned long long t = block_sum<256>(s, ws);
+  if (threadIdx.x == 0) tile_sums[blockIdx.x] = t;
 }
 __global__ void __launch_bounds__(256)
 len_offsets_kernel(const uint32_t* __restrict__ len, uint32_t n, const unsigned long long* __restrict__ tile_offsets, unsigned long long first,
@@ -601,13 +574,7 @@ len_offsets_kernel(const uint32_t* __restrict__ len, uint32_t n, const unsigned 
   uint32_t v[16]; unsigned long long s = 0;
   #pragma unroll
   for (int k = 0; k < 16; k++) { v[k] = base + k < n ? len[base + k] : 0u; s += v[k]; }
-  unsigned long long incl = s;
-  #pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { const unsigned long long y = __shfl_up_sync(FULL, incl, o); if ((threadIdx.x & 31) >= (uint32_t)o) incl += y; }
-  if ((threadIdx.x & 31) == 31) ws[threadIdx.x >> 5] = incl;
-  __syncthreads();
-  unsigned long long run = first + tile_offsets[blockIdx.x] + incl - s;
-  for (uint32_t w = 0; w < (threadIdx.x >> 5); w++) run += ws[w];
+  unsigned long long run = first + tile_offsets[blockIdx.x] + block_exclusive_scan<256>(s, ws);
   #pragma unroll
   for (int k = 0; k < 16; k++) { if (base + k <= n) offsets[base + k] = run; run += v[k]; }
 }

@@ -3,12 +3,13 @@
 // Inflate, chunking, carry of the incomplete tail record, Arrow layout and export are the engine's (engine.cu), as for FASTQ.
 // A FASTA record is a '>' definition line followed by any number of sequence lines, joined with their line breaks removed:
 //
-//   framing   fq_count -> fq_scan -> fq_lines (kernels_fastq.cuh): the offset of every line start of the chunk.
-//             fa_count -> fq_scan -> fa_starts: the line index of every line that starts with '>' (a record start), in order.
+//   framing   fq_count -> cta_scan_kernel -> fq_lines (kernels_fastq.cuh): the offset of every line start of the chunk.
+//             fa_count -> cta_scan_kernel -> fa_starts: the line index of every line starting with '>' (a record start), in order.
 //             fa_frame (one thread) turns them into rows / tail offset / first record as fq_frame reports them, owns the records
 //             whose '>' lies in [own_lo, own_hi), and cuts the owned records into decode slices of about SLICE bytes of text.
 //   lengths   fa_lines_kernel: per line its content bytes (without '\n' and one trailing '\r'; 0 for a definition line), which
-//             one scan (multi_scan_*) turns into each line's destination in the chunk's compacted sequence text.
+//             one offsets scan (multi_scan_reduce -> cta_scan_kernel -> multi_scan_apply) turns into each line's destination in
+//             the chunk's compacted sequence text.
 //             fa_lengths_kernel (thread per record): name / description split of the definition line (fq_definition's rule),
 //             sequence length = the difference of that scan at the record's two boundary lines.
 //   copy      fa_copy_kernel (8 lanes per record): name and description, as fq_copy does.
@@ -21,6 +22,7 @@
 #include <cuda_runtime.h>
 
 #include "kernels_fastq.cuh"
+#include "kernels_scan.cuh"
 
 namespace bamscan {
 
@@ -65,24 +67,8 @@ fa_count_kernel(const FastaFrame P, uint32_t* __restrict__ tile_count) {
   const uint32_t o = P.data_lo + blockIdx.x * FQ_TILE + threadIdx.x * 16;
   uint32_t c = __popc(fa_start_mask16(P.U, o, P.data_lo, P.data_hi, P.own_lo));
   if (blockIdx.x == 0 && threadIdx.x == 0) c += fa_lead_start(P);
-  #pragma unroll
-  for (int s = 16; s; s >>= 1) c += __shfl_xor_sync(0xffffffffu, c, s);
-  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) { uint32_t t = 0; for (int i = 0; i < 8; i++) t += ws[i]; tile_count[blockIdx.x] = t; }
-}
-
-// exclusive scan of v over the 256 threads of the CTA
-__device__ __forceinline__ uint32_t fa_block_excl(uint32_t v, uint32_t* ws) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t x = v;
-  #pragma unroll
-  for (int s = 1; s < 32; s <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, x, s); if (lane >= s) x += y; }
-  if (lane == 31) ws[warp] = x;
-  __syncthreads();
-  uint32_t wb = 0;
-  for (int w = 0; w < warp; w++) wb += ws[w];
-  return wb + x - v;
+  const uint32_t t = block_sum<256>(c, ws);
+  if (threadIdx.x == 0) tile_count[blockIdx.x] = t;
 }
 
 // starts[j] = line index of the j-th record start
@@ -93,8 +79,8 @@ fa_starts_kernel(const FastaFrame P, const uint32_t* __restrict__ nl_base, const
   const uint32_t nm = fq_newline_mask16(P.U, o, P.data_lo, P.data_hi);
   uint32_t sm = fa_start_mask16(P.U, o, P.data_lo, P.data_hi, P.own_lo);
   const uint32_t lead = (blockIdx.x == 0 && threadIdx.x == 0) ? fa_lead_start(P) : 0u;
-  const uint32_t nl_ex = fa_block_excl(__popc(nm), ws[0]);
-  uint32_t k = st_base[blockIdx.x] + fa_block_excl(__popc(sm) + lead, ws[1]);
+  const uint32_t nl_ex = block_exclusive_scan<256>((uint32_t)__popc(nm), ws[0]);
+  uint32_t k = st_base[blockIdx.x] + block_exclusive_scan<256>(__popc(sm) + lead, ws[1]);
   if (lead && k < P.cap) starts[k++] = 0;
   const uint32_t line0 = nl_base[blockIdx.x] + nl_ex;
   while (sm) {
@@ -228,7 +214,7 @@ struct FastaSeq {
   const uint8_t* U;
   const uint32_t* lines;
   const uint32_t* seqpos;
-  const uint32_t* tile_base;  // newlines in front of each FQ_TILE of [data_lo, data_hi) (fq_scan)
+  const uint32_t* tile_base;  // newlines in front of each FQ_TILE of [data_lo, data_hi) (the newline scan)
   const uint32_t* rec;        // the slice's records: rec[0 .. n]
   uint32_t n, data_lo, data_hi, t0;
   uint8_t* dst;               // the slice's sequence column data
@@ -263,7 +249,7 @@ fa_seq_kernel(const FastaSeq P) {
   uint32_t nm = 0;
   #pragma unroll
   for (int k = 0; k < 16; k++) if (o + k < P.data_hi && in[k] == '\n') nm |= 1u << k;
-  uint32_t li = P.tile_base[t] + fa_block_excl(__popc(nm), ws);
+  uint32_t li = P.tile_base[t] + block_exclusive_scan<256>((uint32_t)__popc(nm), ws);
   const uint32_t dlo = s_dlo;
   uint32_t cur = 0xffffffffu, ls = 0, len = 0, d = 0, kept = 0, bad = 0;
   #pragma unroll

@@ -6,7 +6,7 @@
 // Inflate, chunking, carry of the incomplete tail record, slicing into batches, arena layout and Arrow export are the BAM
 // engine's (engine.cu); only the two places that look INSIDE the inflated bytes differ:
 //
-//   framing   fq_count -> fq_scan -> fq_lines: the offset of every line start of the chunk, in order (lines[0] = first record
+//   framing   fq_count -> cta_scan_kernel -> fq_lines: the offset of every line start of the chunk, in order (lines[0] = first record
 //             start).  A FASTQ record is four lines (noodles-fastq reads exactly four: name, sequence, '+' line, qualities), so
 //             record r is lines[4r .. 4r + 4) and the "record offsets" the decode stage is given are that array itself.
 //             fq_frame (one warp) turns the line count into rows / tail offset / first record exactly as kernels_boundary.cuh
@@ -22,6 +22,7 @@
 #include <cuda_runtime.h>
 
 #include "kernels_decode.cuh"
+#include "kernels_scan.cuh"
 
 namespace bamscan {
 
@@ -41,62 +42,17 @@ __global__ void __launch_bounds__(256)
 fq_count_kernel(const uint8_t* __restrict__ U, uint32_t data_lo, uint32_t data_hi, uint32_t* __restrict__ tile_count) {
   __shared__ uint32_t ws[8];
   const uint32_t o = data_lo + blockIdx.x * FQ_TILE + threadIdx.x * 16;
-  uint32_t c = __popc(fq_newline_mask16(U, o, data_lo, data_hi));
-  #pragma unroll
-  for (int s = 16; s; s >>= 1) c += __shfl_xor_sync(0xffffffffu, c, s);
-  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) { uint32_t t = 0; for (int i = 0; i < 8; i++) t += ws[i]; tile_count[blockIdx.x] = t; }
-}
-
-// single CTA: exclusive scan of tile_count -> tile_base, total -> *total
-__global__ void __launch_bounds__(1024)
-fq_scan_kernel(const uint32_t* __restrict__ tile_count, uint32_t* __restrict__ tile_base, uint32_t n_tiles, uint32_t* __restrict__ total) {
-  __shared__ uint32_t ws[32];
-  __shared__ uint32_t carry;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n_tiles; base += 1024) {
-    const uint32_t i = base + tid;
-    const uint32_t v = i < n_tiles ? tile_count[i] : 0u;
-    uint32_t x = v;
-    #pragma unroll
-    for (int s = 1; s < 32; s <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, x, s); if (lane >= s) x += y; }
-    if (lane == 31) ws[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = ws[lane];
-      #pragma unroll
-      for (int s = 1; s < 32; s <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, w, s); if (lane >= s) w += y; }
-      ws[lane] = w;
-    }
-    __syncthreads();
-    const uint32_t excl = carry + (warp ? ws[warp - 1] : 0u) + x - v;
-    if (i < n_tiles) tile_base[i] = excl;
-    __syncthreads();
-    if (tid == 1023) carry = excl + v;
-    __syncthreads();
-  }
-  if (tid == 0) *total = carry;
+  const uint32_t t = block_sum<256>((uint32_t)__popc(fq_newline_mask16(U, o, data_lo, data_hi)), ws);
+  if (threadIdx.x == 0) tile_count[blockIdx.x] = t;
 }
 
 // lines[0] = data_lo; lines[k + 1] = offset behind the k-th newline
 __global__ void __launch_bounds__(256)
 fq_lines_kernel(const uint8_t* __restrict__ U, uint32_t data_lo, uint32_t data_hi, const uint32_t* __restrict__ tile_base, uint32_t* __restrict__ lines, uint32_t cap) {
   __shared__ uint32_t ws[8];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t o = data_lo + blockIdx.x * FQ_TILE + threadIdx.x * 16;
   uint32_t m = fq_newline_mask16(U, o, data_lo, data_hi);
-  const uint32_t c = __popc(m);
-  uint32_t x = c;
-  #pragma unroll
-  for (int s = 1; s < 32; s <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, x, s); if (lane >= s) x += y; }
-  if (lane == 31) ws[warp] = x;
-  __syncthreads();
-  uint32_t wb = 0;
-  for (int w = 0; w < warp; w++) wb += ws[w];
-  uint32_t k = tile_base[blockIdx.x] + wb + x - c;
+  uint32_t k = tile_base[blockIdx.x] + block_exclusive_scan<256>((uint32_t)__popc(m), ws);
   if (blockIdx.x == 0 && threadIdx.x == 0) lines[0] = data_lo;
   while (m) { const uint32_t b = (uint32_t)__ffs((int)m) - 1u; m &= m - 1u; if (++k < cap) lines[k] = o + b + 1u; }     // (fq_frame reports the overflow)
 }

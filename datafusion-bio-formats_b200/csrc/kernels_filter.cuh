@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 
 #include "kernels_boundary.cuh"
+#include "kernels_scan.cuh"
 
 namespace bamscan {
 
@@ -104,34 +105,10 @@ rule_keep_kernel(const uint8_t* __restrict__ U, const uint32_t* __restrict__ rec
 // single CTA: exclusive scan of keep[i] (cut at the stop index) -> pos[i]; total -> flags[7]
 __global__ void __launch_bounds__(1024)
 rule_scan_kernel(const uint32_t* __restrict__ keep, uint32_t* __restrict__ pos, uint32_t n, uint32_t* __restrict__ flags) {
-  __shared__ uint32_t ws[32];
-  __shared__ uint32_t carry;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t stop = flags[6];
-  if (tid == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n; base += 1024) {
-    uint32_t i = base + tid;
-    uint32_t v = (i < n && i < stop) ? keep[i] : 0u;
-    uint32_t x = v;
-    #pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-    if (lane == 31) ws[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = ws[lane];
-      #pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += y; }
-      ws[lane] = w;
-    }
-    __syncthreads();
-    uint32_t excl = carry + (warp ? ws[warp - 1] : 0u) + x - v;
-    if (i < n) pos[i] = v ? excl : 0xffffffffu;
-    __syncthreads();
-    if (tid == 1023) carry = excl + v;
-    __syncthreads();
-  }
-  if (tid == 0) flags[7] = carry;
+  const uint32_t total = cta_exclusive_scan<uint32_t>(n, [&](uint32_t i) { return (i < n && i < stop) ? keep[i] : 0u; },
+                                                      [&](uint32_t i, uint32_t excl, uint32_t v) { pos[i] = v ? excl : 0xffffffffu; });
+  if (threadIdx.x == 0) flags[7] = total;
 }
 
 __global__ void __launch_bounds__(256)

@@ -5,13 +5,13 @@
 // RecordBuf per line).  Column rules, tag coercions, binary CIGAR, the f32 -> text rendering, arenas and the Arrow export are
 // the BAM path's; only the text parsing is here:
 //
-//   framing    fq_count -> fq_scan -> fq_lines (kernels_fastq.cuh: every line start of the chunk), then sam_frame_kernel: one
+//   framing    fq_count -> cta_scan_kernel -> fq_lines (kernels_fastq.cuh: every line start of the chunk), then sam_frame_kernel: one
 //              record per line, rows / tail offset / first record / ownership bound reported as the seg_* kernels report them.
 //   size       sam_size_kernel: a thread per line.  Splits the 11 mandatory fields, parses and range-checks every one of them,
 //              resolves RNAME / RNEXT against the header's reference names, counts and validates the CIGAR, checks SEQ / QUAL,
 //              sizes every aux field.  Out: the BAM record size, a SamLine with the parsed values, the "QUAL is *" flag.  The
 //              first error (code + row) goes to err[0..1] (enc::report).
-//   offsets    multi_scan_* over the sizes (kernels_decode.cuh): the record offsets in the chunk's BAM buffer.
+//   offsets    the offsets scan over the sizes (launch_offsets_scan, engine.cu): the record offsets in the chunk's BAM buffer.
 //   write      sam_records_kernel<G>: a group of G lanes per line writes the record: block_size, the fixed 32 bytes, name + NUL,
 //              CIGAR ops (group-parallel text parse, as the write path's enc_records_kernel), packed bases, qualities - 33 (0xFF
 //              when QUAL is *), aux fields.  Nothing is validated here: the size pass has.

@@ -823,7 +823,7 @@ static int writer_flush_members(BamWriter* w, uint64_t total, bool final_flush) 
   dfl::bgzf_deflate_kernel<<<grid, dfl::NT, sizeof(dfl::Smem), w->stream>>>(static_cast<const uint8_t*>(w->stream_buf.p), consumed, (uint32_t)n_members,
                                                                            static_cast<uint8_t*>(w->slots.p), static_cast<uint32_t*>(w->sizes.p),
                                                                            static_cast<uint32_t*>(w->tok.p), d_ticket, w->compression == 1);
-  dfl::bgzf_offsets_kernel<<<1, 1024, 0, w->stream>>>(static_cast<uint32_t*>(w->sizes.p), (uint32_t)n_members, static_cast<unsigned long long*>(w->offsets.p), d_total);
+  cta_scan_kernel<<<1, CTA_SCAN_THREADS, 0, w->stream>>>(static_cast<const uint32_t*>(w->sizes.p), static_cast<unsigned long long*>(w->offsets.p), (uint32_t)n_members, d_total);
   WCU_TRY(cudaEventRecord(w->ev[3], w->stream));
   WCU_TRY(cudaMemcpyAsync(w->h_small + 5000, d_total, 8, cudaMemcpyDeviceToHost, w->stream));
   WCU_TRY(cudaStreamSynchronize(w->stream));
