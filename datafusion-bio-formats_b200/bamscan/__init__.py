@@ -26,7 +26,7 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE.parent / "libbamscan.so"
 
 EXPORTED_SYMBOLS = [
-    "bamscan_open", "bamscan_open_fastq", "bamscan_open_fasta", "bamscan_close", "bamscan_schema", "bamscan_describe_tags", "bamscan_classify_filters", "bamscan_plan",
+    "bamscan_open", "bamscan_open_fastq", "bamscan_open_fasta", "bamscan_open_vcf", "bamscan_close", "bamscan_schema", "bamscan_describe_tags", "bamscan_classify_filters", "bamscan_plan",
     "bamscan_plan_num_partitions", "bamscan_plan_schema", "bamscan_plan_free", "bamscan_plan_num_ranges",
     "bamscan_plan_range_info", "bamscan_plan_partition_regions", "bamscan_extract_regions", "bamscan_balance_partitions",
     "bamscan_execute", "bamscan_next", "bamscan_execute_device", "bamscan_next_device",
@@ -122,6 +122,7 @@ def load_library():
     L.bamscan_open.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
     L.bamscan_open_fastq.argtypes = [C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
     L.bamscan_open_fasta.argtypes = [C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
+    L.bamscan_open_vcf.argtypes = [C.c_char_p, C.POINTER(_Options), C.POINTER(C.c_void_p)]
     L.bamscan_close.argtypes = [C.c_void_p]
     L.bamscan_schema.argtypes = [C.c_void_p, C.c_void_p]
     L.bamscan_describe_tags.argtypes = [C.c_void_p, C.c_int32, C.c_char_p, C.c_uint64, C.POINTER(C.c_uint64)]
@@ -396,7 +397,8 @@ class DeviceBatch:
                 return pa.Array.from_buffers(typ, n, [validity, offs], null_count=-1, offset=off, children=[child])
             data = self._host(bufs[2], int(o[-1]) if len(o) else 0)
             return pa.Array.from_buffers(typ, n, [validity, offs, data], null_count=-1, offset=off)
-        return pa.Array.from_buffers(typ, n, [validity, self._host(bufs[1], (off + n) * (typ.bit_width // 8))], null_count=-1, offset=off)
+        nbytes = (off + n + 7) // 8 if pa.types.is_boolean(typ) else (off + n) * (typ.bit_width // 8)
+        return pa.Array.from_buffers(typ, n, [validity, self._host(bufs[1], nbytes)], null_count=-1, offset=off)
 
     def to_host(self) -> pa.RecordBatch:
         if self._dev.sync_event:
@@ -831,6 +833,44 @@ class FastaTableProvider(BamTableProvider):
         o.debug_flags = debug_flags
         self._h = C.c_void_p()
         _check(L.bamscan_open_fasta(str(file_path).encode(), C.byref(o), C.byref(self._h)))
+        self.file_path = str(file_path)
+        self.device_id = device_id
+        self._schema = None
+
+    def scan(self, projection=None, filters=None, limit=None, *, target_partitions=1) -> BamExec:
+        mode = "block_range" if target_partitions > 1 else "reference"
+        return super().scan(projection, None, limit, target_partitions=target_partitions, partition_mode=mode)
+
+
+class VcfTableProvider(BamTableProvider):
+    """A provider for BGZF-compressed VCF (bamscan_open_vcf): `VcfTableProvider(file_path, info_fields, object_storage_options,
+    coordinate_system_zero_based)`; schema chrom / start / end / id / ref / alt / qual / filter, then one column per INFO field of the
+    header (info_fields None: all of them in header order; a list: those IDs in that order), typed as the header declares them.
+    `scan` with target_partitions > 1 uses BGZF block ranges balanced by compressed bytes (a line belongs to the range that holds its
+    first byte); no filter is pushed down and `limit` is not applied, as for FastqTableProvider; everything else is
+    BamTableProvider's.  At most 112 INFO columns can be projected in one scan: execute raises BamScanError -5 (unsupported)
+    above that, so a header with more ##INFO fields needs info_fields or a projection."""
+
+    def __init__(self, file_path, info_fields=None, object_storage_options=None, coordinate_system_zero_based=True, *, device_id=0,
+                 batch_rows=0, chunk_inflated_bytes=0, skip_crc=False, debug_flags=0):
+        if object_storage_options is not None:
+            raise BamScanError(-5, "remote object storage is out of scope for this build (local files only)")
+        L = load_library()
+        o = _Options()
+        o.struct_size = C.sizeof(_Options)
+        o.coordinate_system_zero_based = int(coordinate_system_zero_based)
+        o.has_tag_fields = int(info_fields is not None)
+        self._tag_arr, self._tag_enc = _strs(list(info_fields or []))
+        o.n_tag_fields = len(info_fields or [])
+        if self._tag_arr is not None:
+            o.tag_fields = self._tag_arr
+        o.device_id = device_id
+        o.batch_rows = batch_rows
+        o.chunk_inflated_bytes = chunk_inflated_bytes
+        o.skip_crc = int(skip_crc)
+        o.debug_flags = debug_flags
+        self._h = C.c_void_p()
+        _check(L.bamscan_open_vcf(str(file_path).encode(), C.byref(o), C.byref(self._h)))
         self.file_path = str(file_path)
         self.device_id = device_id
         self._schema = None

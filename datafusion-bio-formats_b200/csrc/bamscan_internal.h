@@ -16,7 +16,9 @@ void set_error(const char* fmt, ...);   // thread-local message for bamscan_last
 // column kinds (values shared with kernels_decode.cuh::ColKind)
 enum : int32_t {
   HK_Int32 = 1, HK_UInt32 = 2, HK_Float32 = 3, HK_Utf8 = 4, HK_Binary = 5,
-  HK_ListInt8 = 10, HK_ListUInt8 = 11, HK_ListInt16 = 12, HK_ListUInt16 = 13, HK_ListInt32 = 14, HK_ListUInt32 = 15, HK_ListFloat32 = 16
+  HK_Boolean = 6,                                             // VCF Flag columns only
+  HK_ListInt8 = 10, HK_ListUInt8 = 11, HK_ListInt16 = 12, HK_ListUInt16 = 13, HK_ListInt32 = 14, HK_ListUInt32 = 15, HK_ListFloat32 = 16,
+  HK_ListUtf8 = 17                                            // VCF String / Character lists only
 };
 
 struct TagDef { std::string tag; char sam_type; int32_t kind; std::string description; };
@@ -65,12 +67,14 @@ enum ScanFormat : int {
   FMT_FASTQ = 1,   // BGZF-compressed FASTQ (kernels_fastq.cuh): same engine, four Utf8 columns, no header / index
   FMT_SAM = 2,     // plain SAM (kernels_sam.cuh): the text is transcoded to BAM records on the device, no index
   FMT_FASTA = 3,   // BGZF-compressed FASTA (kernels_fasta.cuh): three Utf8 columns, records of up to 1 GiB, no index
+  FMT_VCF = 4,     // BGZF-compressed VCF (kernels_vcf.cuh): eight fixed columns and the typed INFO fields, no index
 };
 inline const char* format_name(int format) {
   switch (format) {
     case FMT_FASTQ: return "FASTQ";
     case FMT_SAM: return "SAM";
     case FMT_FASTA: return "FASTA";
+    case FMT_VCF: return "VCF";
   }
   return "BAM";
 }
@@ -106,6 +110,9 @@ struct BamFile {
   int32_t debug_flags = 0;
   bool decode_all_tags = false;           // BamScanOptions.decode_all_tag_fields
   std::unique_ptr<BaiIndex> bai;
+  // VCF: the header's ##INFO lines, in header order (Number, Type and Description as written)
+  struct VcfInfo { std::string id, number, type, description; };
+  std::vector<VcfInfo> vcf_info;
 };
 
 // genomic_filter.rs:16-32
@@ -155,6 +162,7 @@ int load_bai(const std::string& path, BaiIndex* out);     // BAI, or CSI when th
 
 // host_schema.cpp
 int build_schema(BamFile* f, const BamScanOptions* opt);   // determine_schema (table_provider.rs:42-140)
+int build_vcf_schema(BamFile* f, const BamScanOptions* opt);   // FMT_VCF: the eight fixed columns + the selected INFO fields
 int export_schema(const std::vector<FieldDef>& fields, const std::vector<std::pair<std::string, std::string>>& metadata,
                   struct ArrowSchema* out);
 

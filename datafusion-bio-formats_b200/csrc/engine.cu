@@ -37,6 +37,7 @@
 #include "kernels_fastq.cuh"
 #include "kernels_fasta.cuh"
 #include "kernels_sam.cuh"
+#include "kernels_vcf.cuh"
 
 namespace bamscan {
 
@@ -189,6 +190,8 @@ struct ColLayout {
   size_t validity_off = 0, offsets_off = 0, values_off = 0, data_off = 0;
   uint64_t data_bytes = 0;      // var-len data bytes / list child bytes
   uint64_t child_len = 0;       // list child element count
+  bool child_validity = false;  // VCF lists: the child has a validity bitmap (child_validity_off)
+  size_t child_validity_off = 0, child_offsets_off = 0;   // List<Utf8>: child_offsets_off holds the child's offsets
 };
 
 struct ChunkPlan { uint32_t b0 = 0, b1 = 0; uint64_t c0 = 0, c1 = 0, u0 = 0, ubytes = 0; bool extension = false; };
@@ -419,6 +422,12 @@ static int stream_init(BamScanStream* s) {
     if (it == s->dec_cols.end()) { s->out_to_dec.push_back((int32_t)s->dec_cols.size()); s->dec_cols.push_back(c); }
     else s->out_to_dec.push_back((int32_t)(it - s->dec_cols.begin()));
   }
+  if (f->format == FMT_VCF) {
+    int n_info = 0;
+    for (int32_t c : s->dec_cols) if (c >= 8) n_info++;          // INFO columns follow the eight fixed ones
+    if (n_info > vcf::MAX_INFO) { set_error("more than %d projected INFO columns are not supported by this build", vcf::MAX_INFO); return BAMSCAN_ERR_UNSUPPORTED; }
+    return BAMSCAN_OK;
+  }
   int n_tag_cols = 0;
   for (int32_t c : s->dec_cols) if (c >= 12) n_tag_cols++;
   if (f->decode_all_tags && n_tag_cols) {
@@ -623,6 +632,53 @@ static int launch_offsets_scan(BamScanStream* s, cudaStream_t cs, const ScanCols
   return BAMSCAN_OK;
 }
 
+// Hands a decoded slice's arena A (rows n, arena_bytes, error word at err_off) to the consumer: kept in HBM (device-resident runs),
+// copied into the batch's own device allocation (device export), or copied to a pinned host arena; queued as s->pending.
+static int hand_off_batch(BamScanStream* s, cudaStream_t cs, uint8_t* A, const std::vector<ColLayout>& cols, uint32_t n, size_t arena_bytes,
+                          size_t err_off, uint64_t row0, bool* produced) {
+  const BamFile* f = s->f;
+  if (s->device_resident) {
+    // keep everything in HBM: only the decode error word travels
+    publish_kernel<<<1, 32, 0, cs>>>(reinterpret_cast<const uint32_t*>(A + err_off), s->d_hflags + 512, 2);     // (checked by flush_slice)
+  } else if (s->device_export) {
+    // device hand-off: the batch gets its own exactly-sized device allocation (a device-to-device copy on the side
+    // stream, ~3 TB/s); only the decode error word travels to the host
+    CU_TRY(cudaEventRecord(s->ev_compute, cs));
+    PendingBatch& P = s->pending;
+    P.owner = new BatchOwner();
+    P.owner->device = f->device; P.owner->refs = 1;
+    if (cudaMalloc(&P.owner->dev, arena_bytes) != cudaSuccess) { delete P.owner; P.owner = nullptr; set_error("cudaMalloc(%zu) for a device batch failed", arena_bytes); return BAMSCAN_ERR_CUDA; }
+    P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
+    if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
+    CU_TRY(cudaEventCreateWithFlags(&P.owner->dev_ready, cudaEventDisableTiming));
+    CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
+    CU_TRY(cudaMemcpyAsync(P.owner->dev, A, arena_bytes, cudaMemcpyDeviceToDevice, s->s_d2h));
+    CU_TRY(cudaMemcpyAsync(s->h_flags + 514, A + err_off, 8, cudaMemcpyDeviceToHost, s->s_d2h));
+    CU_TRY(cudaEventRecord(P.owner->dev_ready, s->s_d2h));
+    CU_TRY(cudaEventRecord(P.done, s->s_d2h));
+    s->arena_flip ^= 1;
+    *produced = true;
+  } else {
+    CU_TRY(cudaEventRecord(s->ev_compute, cs));
+    PendingBatch& P = s->pending;
+    P.owner = new BatchOwner();
+    P.owner->arena = arena_acquire(arena_bytes);
+    if (!P.owner->arena.p) { delete P.owner; P.owner = nullptr; return BAMSCAN_ERR_CUDA; }
+    P.owner->refs = 1;
+    P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
+    if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
+    CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
+    CU_TRY(cudaMemcpyAsync(P.owner->arena.p, A, arena_bytes, cudaMemcpyDeviceToHost, s->s_d2h));
+    CU_TRY(cudaEventRecord(P.done, s->s_d2h));
+    s->st.d2h_bytes += arena_bytes;
+    s->arena_flip ^= 1;
+    // the next chunk must not overwrite this arena before the copy has read it: arenas are double buffered and the
+    // batch before this one has already been waited for (see bamscan_next)
+    *produced = true;
+  }
+  return BAMSCAN_OK;
+}
+
 static int decode_slice(BamScanStream* s, bool* produced) {
   NvtxRange nv("bamscan: decode slice (fixed, scan, var) + D2H issue");
   BamFile* f = s->f;
@@ -804,49 +860,176 @@ static int decode_slice(BamScanStream* s, bool* produced) {
       bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
       s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var ? off_bytes + L.data_bytes : val_bytes);
     }
-    if (s->device_resident) {
-      // keep everything in HBM: only the decode error word travels
-      publish_kernel<<<1, 32, 0, cs>>>(reinterpret_cast<const uint32_t*>(A + err_off), s->d_hflags + 512, 2);     // (checked by flush_slice)
-    } else if (s->device_export) {
-      // device hand-off: the batch gets its own exactly-sized device allocation (a device-to-device copy on the side
-      // stream, ~3 TB/s); only the decode error word travels to the host
-      CU_TRY(cudaEventRecord(s->ev_compute, cs));
-      PendingBatch& P = s->pending;
-      P.owner = new BatchOwner();
-      P.owner->device = f->device; P.owner->refs = 1;
-      if (cudaMalloc(&P.owner->dev, arena_bytes) != cudaSuccess) { delete P.owner; P.owner = nullptr; set_error("cudaMalloc(%zu) for a device batch failed", arena_bytes); return BAMSCAN_ERR_CUDA; }
-      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
-      if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
-      CU_TRY(cudaEventCreateWithFlags(&P.owner->dev_ready, cudaEventDisableTiming));
-      CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
-      CU_TRY(cudaMemcpyAsync(P.owner->dev, A, arena_bytes, cudaMemcpyDeviceToDevice, s->s_d2h));
-      CU_TRY(cudaMemcpyAsync(s->h_flags + 514, A + err_off, 8, cudaMemcpyDeviceToHost, s->s_d2h));
-      CU_TRY(cudaEventRecord(P.owner->dev_ready, s->s_d2h));
-      CU_TRY(cudaEventRecord(P.done, s->s_d2h));
-      s->arena_flip ^= 1;
-      *produced = true;
-    } else {
-      CU_TRY(cudaEventRecord(s->ev_compute, cs));
-      PendingBatch& P = s->pending;
-      P.owner = new BatchOwner();
-      P.owner->arena = arena_acquire(arena_bytes);
-      if (!P.owner->arena.p) { delete P.owner; P.owner = nullptr; return BAMSCAN_ERR_CUDA; }
-      P.owner->refs = 1;
-      P.cols = cols; P.rows = n; P.arena_bytes = arena_bytes; P.err_off = err_off; P.row0 = row0; P.valid = true;
-      if (!P.done) CU_TRY(cudaEventCreateWithFlags(&P.done, cudaEventDisableTiming));
-      CU_TRY(cudaStreamWaitEvent(s->s_d2h, s->ev_compute, 0));
-      CU_TRY(cudaMemcpyAsync(P.owner->arena.p, A, arena_bytes, cudaMemcpyDeviceToHost, s->s_d2h));
-      CU_TRY(cudaEventRecord(P.done, s->s_d2h));
-      s->st.d2h_bytes += arena_bytes;
-      s->arena_flip ^= 1;
-      // the next chunk must not overwrite this arena before the copy has read it: arenas are double buffered and the
-      // batch before this one has already been waited for (see bamscan_next)
-      *produced = true;
-    }
-    }
+    if ((rc = hand_off_batch(s, cs, A, cols, n, arena_bytes, err_off, row0, produced))) return rc;
+  }
   CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
   s->slice_pending = true;
   return BAMSCAN_OK;
+}
+
+// VCF: the next slice of the chunk's lines -> the projected columns (kernels_vcf.cuh), then the same hand-off as decode_slice.  One host
+// sync: the totals of the count columns (Utf8 bytes, list elements, List<Utf8> bytes) size the arena's second region.
+static int decode_slice_vcf(BamScanStream* s, bool* produced) {
+  NvtxRange nv("bamscan: VCF decode slice (fields, rows, scan, write) + D2H issue");
+  const BamFile* f = s->f;
+  cudaStream_t cs = s->cur.cs;
+  int rc;
+  if ((rc = flush_slice(s))) return rc;
+  const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
+  const uint64_t row0 = s->st.rows;
+  const uint32_t* lines = s->cur.recoff + s->cur.pos;
+  s->cur.pos += n;
+  CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
+  const size_t n_dec = s->dec_cols.size();
+  std::vector<ColLayout> cols(n_dec);
+  std::vector<int> info_col(n_dec, -1);           // dec column -> INFO column (key) index
+  ArenaBuilder AB;
+  const size_t bm_bytes = 4ull * ((n + 31) / 32), off_bytes = 4ull * (n + 1), val_bytes = 4ull * n;
+  const size_t err_off = AB.take(64);
+  int n_info = 0;
+  for (size_t i = 0; i < n_dec; i++) {
+    ColLayout& L = cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = f->fields[L.schema_idx].kind;
+    L.has_validity = f->fields[L.schema_idx].nullable;
+    if (L.has_validity) L.validity_off = AB.take(bm_bytes);
+    if (L.kind == HK_Utf8 || L.kind >= HK_ListInt8) L.offsets_off = AB.take(off_bytes);
+    else L.values_off = AB.take(L.kind == HK_Boolean ? bm_bytes : val_bytes);
+    if (L.schema_idx >= 8) info_col[i] = n_info++;
+  }
+  const size_t regionA = AB.pos;
+  // keys: the projected INFO IDs, then END unless it is one of them
+  std::vector<std::string> keys;
+  for (size_t i = 0; i < n_dec; i++) if (info_col[i] >= 0) keys.push_back(f->fields[cols[i].schema_idx].name);
+  int end_key = (int)(std::find(keys.begin(), keys.end(), std::string("END")) - keys.begin());
+  if (end_key == (int)keys.size()) keys.push_back("END");
+  // Keys::off and Params::cols hold MAX_INFO + 1 keys (stream_init refuses more projected INFO columns)
+  if (keys.size() > (size_t)vcf::MAX_INFO + 1) { set_error("more than %d projected INFO columns are not supported by this build", vcf::MAX_INFO); return BAMSCAN_ERR_UNSUPPORTED; }
+  std::unique_ptr<vcf::Params> P(new vcf::Params());
+  memset(P.get(), 0, sizeof(vcf::Params));
+  vcf::Keys& K = P->keys;
+  uint32_t blob = 0;
+  for (size_t k = 0; k < keys.size(); k++) {
+    if (blob + keys[k].size() > (size_t)vcf::KEY_BLOB) { set_error("the projected INFO IDs exceed %d bytes, which is not supported by this build", vcf::KEY_BLOB); return BAMSCAN_ERR_UNSUPPORTED; }
+    K.off[k] = (uint16_t)blob;
+    memcpy(K.blob + blob, keys[k].data(), keys[k].size()); blob += (uint32_t)keys[k].size();
+    uint32_t h = vcf::key_hash(reinterpret_cast<const uint8_t*>(keys[k].data()), (uint32_t)keys[k].size());
+    while (K.slot[h & (vcf::KEY_SLOTS - 1)]) h++;
+    K.slot[h & (vcf::KEY_SLOTS - 1)] = (uint16_t)(k + 1);
+  }
+  K.off[keys.size()] = (uint16_t)blob; K.n_keys = (int32_t)keys.size(); K.end_key = end_key;
+  // scratch: per row the field starts, per key the value tokens, per List<Utf8> column its byte counts
+  const size_t o_tok = align_up(sizeof(vcf::Row) * n, 256), o_blen = o_tok + align_up(8ull * n * keys.size(), 256);
+  size_t scratch = o_blen;
+  std::vector<size_t> blen_off(n_dec, 0);
+  for (size_t i = 0; i < n_dec; i++) if (cols[i].kind == HK_ListUtf8) { blen_off[i] = scratch; scratch += align_up(off_bytes, 256); }
+  if ((rc = s->d_scratch.ensure(scratch + 256))) return rc;
+  uint8_t* SCR = s->d_scratch.as<uint8_t>();
+  DeviceBuf& arena = s->d_arena[s->arena_flip];
+  if (arena.cap < regionA && (rc = arena.ensure(regionA + (size_t)s->cur.ubytes * 2))) return rc;
+  // the kernels' view of the arena (rebuilt when the arena grows)
+  auto bind = [&](uint8_t* A) {
+    P->U = s->cur.U; P->lines = lines; P->n = n; P->zero_based = f->zero_based; P->n_info = n_info;
+    P->rows = reinterpret_cast<vcf::Row*>(SCR); P->err = reinterpret_cast<uint32_t*>(A + err_off);
+    for (size_t k = 0; k < keys.size(); k++) P->cols[k].tok = reinterpret_cast<uint2*>(SCR + o_tok) + (size_t)k * n;
+    for (size_t i = 0; i < n_dec; i++) {
+      const ColLayout& L = cols[i];
+      uint32_t* v = L.has_validity ? reinterpret_cast<uint32_t*>(A + L.validity_off) : nullptr;
+      int32_t* offs = reinterpret_cast<int32_t*>(A + L.offsets_off);
+      uint32_t* vals = reinterpret_cast<uint32_t*>(A + L.values_off);
+      uint8_t* d = L.data_bytes || L.child_len ? A + L.data_off : nullptr;
+      switch (L.schema_idx) {
+        case 0: P->l_chrom = offs; P->d_chrom = d; break;
+        case 1: P->start = vals; break;
+        case 2: P->end = vals; break;
+        case 3: P->l_id = offs; P->v_id = v; P->d_id = d; break;
+        case 4: P->l_ref = offs; P->d_ref = d; break;
+        case 5: P->l_alt = offs; P->v_alt = v; P->d_alt = d; break;
+        case 6: P->qual = vals; P->v_qual = v; break;
+        case 7: P->l_filter = offs; P->v_filter = v; P->d_filter = d; break;
+        default: {
+          vcf::InfoCol& C = P->cols[info_col[i]];
+          C.kind = L.kind; C.valid = v;
+          if (L.kind == HK_Utf8 || L.kind >= HK_ListInt8) C.lens = offs; else C.values = vals;
+          if (L.kind == HK_ListUtf8) { C.blens = reinterpret_cast<int32_t*>(SCR + blen_off[i]); C.coffs = reinterpret_cast<int32_t*>(A + L.child_offsets_off); }
+          if (L.child_validity) C.cvalid = reinterpret_cast<uint32_t*>(A + L.child_validity_off);
+          C.data = A + L.data_off;
+        }
+      }
+    }
+  };
+  uint8_t* A = arena.as<uint8_t>();
+  bind(A);
+  CU_TRY(cudaMemsetAsync(A + err_off, 0, 64, cs));
+  CU_TRY(cudaMemsetAsync(SCR + o_tok, 0, 8ull * n * keys.size(), cs));
+  // 8 lanes per line; 32 when the previous chunk's lines averaged above 2 KiB (sam_records_kernel's rule)
+  const bool wide = (f->debug_flags & 2) || s->mean_record_bytes > 2048;
+  if (wide) vcf::vcf_fields_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
+  else vcf::vcf_fields_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
+  vcf::vcf_rows_kernel<<<(n + 255) / 256, 256, 0, cs>>>(*P);
+  s->st.kernel_launches += 2;
+  // count columns -> offsets, in launches of up to MAX_SCAN_COLS columns
+  std::vector<int32_t*> scan_cols;
+  std::vector<std::pair<size_t, bool>> scan_owner;     // (dec column, is the List<Utf8> byte column)
+  for (size_t i = 0; i < n_dec; i++) {
+    const ColLayout& L = cols[i];
+    if (!(L.kind == HK_Utf8 || L.kind >= HK_ListInt8)) continue;
+    scan_cols.push_back(reinterpret_cast<int32_t*>(A + L.offsets_off)); scan_owner.push_back({i, false});
+    if (L.kind == HK_ListUtf8) { scan_cols.push_back(reinterpret_cast<int32_t*>(SCR + blen_off[i])); scan_owner.push_back({i, true}); }
+  }
+  const size_t n_scan = scan_cols.size();
+  uint64_t* h_totals = reinterpret_cast<uint64_t*>(s->h_flags + 16);
+  if (n_scan) {
+    if ((rc = s->d_totals.ensure(8 * n_scan))) return rc;
+    for (size_t k0 = 0; k0 < n_scan; k0 += MAX_SCAN_COLS) {
+      ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = n + 1;
+      for (size_t k = k0; k < std::min(n_scan, k0 + MAX_SCAN_COLS); k++) SC.col[SC.n_cols++] = scan_cols[k];
+      if ((rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>() + k0))) return rc;
+    }
+    publish_kernel<<<1, 256, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, (int)(2 * n_scan));   // [16, 16 + 2 * 229) < 512
+    s->st.kernel_launches++;
+    CU_TRY(cudaEventRecord(s->ev_dflags, cs));
+    CU_TRY(cudaEventSynchronize(s->ev_dflags));
+    CU_TRY(cudaGetLastError());
+    for (size_t k = 0; k < n_scan; k++) {
+      ColLayout& L = cols[scan_owner[k].first];
+      const uint64_t tot = h_totals[k];
+      if (tot > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", f->fields[L.schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
+      if (scan_owner[k].second) { L.data_bytes = tot; L.data_off = AB.take((size_t)tot + 16); continue; }
+      if (L.kind == HK_Utf8) { L.data_bytes = tot; L.data_off = AB.take((size_t)tot + 16); continue; }
+      L.child_len = tot; L.child_validity = true;
+      L.child_validity_off = AB.take(4 * ((tot + 31) / 32));
+      if (L.kind == HK_ListUtf8) L.child_offsets_off = AB.take(4 * (tot + 1));
+      else { L.data_bytes = 4 * tot; L.data_off = AB.take(4 * (size_t)tot + 16); }
+    }
+  }
+  if (AB.pos > arena.cap) {
+    // grow, keeping region A
+    DeviceBuf bigger;
+    if ((rc = bigger.ensure(AB.pos))) return rc;
+    CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, regionA, cudaMemcpyDeviceToDevice, cs));
+    CU_TRY(cudaStreamSynchronize(cs));
+    arena.release(); arena = bigger; bigger.p = nullptr; bigger.cap = 0;
+    A = arena.as<uint8_t>();
+  }
+  bind(A);
+  for (const ColLayout& L : cols) if (L.child_validity) CU_TRY(cudaMemsetAsync(A + L.child_validity_off, 0, 4 * ((L.child_len + 31) / 32), cs));
+  if (wide) vcf::vcf_write_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
+  else vcf::vcf_write_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
+  s->st.kernel_launches++;
+  const size_t arena_bytes = AB.pos;
+  s->st.rows += n; s->st.batches++;
+  for (auto& L : cols) {
+    const bool is_var = L.kind == HK_Utf8 || L.kind >= HK_ListInt8;
+    s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var ? off_bytes + L.data_bytes : L.kind == HK_Boolean ? bm_bytes : val_bytes);
+  }
+  if ((rc = hand_off_batch(s, cs, A, cols, n, arena_bytes, err_off, row0, produced))) return rc;
+  CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
+  s->slice_pending = true;
+  return BAMSCAN_OK;
+}
+
+// the next slice of the current chunk's rows: VCF has its own decode path
+static int decode_next_slice(BamScanStream* s, bool* produced) {
+  return s->f->format == FMT_VCF ? decode_slice_vcf(s, produced) : decode_slice(s, produced);
 }
 
 static int sam_error_to_rc(uint32_t code, unsigned long long rec) {
@@ -982,6 +1165,13 @@ static int frame_sam(BamScanStream* s, const ChunkPlan& c, int slot, const Bound
   return BAMSCAN_OK;
 }
 
+// VCF: a record is a line, framed as a SAM line is.  A range owns the lines that start at or after its first owned byte
+// (BP.first_start): the member in front of a block range is inflated too, so that a line start there is seen behind its '\n'.  '#'
+// lines and empty lines are refused by vcf_rows_kernel, which knows the record number.
+static int frame_vcf(BamScanStream* s, const ChunkPlan& c, int slot, const BoundaryParams& BP) {
+  return frame_sam(s, c, slot, BP);
+}
+
 // FASTA: line starts (the newline scan) and the lines that start with '>' (kernels_fasta.cuh).  Its own flag words [16, 64) go to
 // [FA_HFLAGS, FA_HFLAGS + 48) of the mapped page.
 static int frame_fasta(BamScanStream* s, const ChunkPlan& c, const ScanRange& range, int slot, const BoundaryParams& BP, bool first_of_range) {
@@ -1033,6 +1223,11 @@ static int read_frame_flags(BamScanStream* s, const ChunkPlan& c, uint32_t H, ui
       if (hf[1]) { set_error("SAM read error: lines shorter than 8 bytes on average (a SAM record has 11 fields)"); return BAMSCAN_ERR_FORMAT; }
       if (start_known) s->need_spec = false;
       if (new_carry > HEADROOM) return over_headroom("SAM line");
+      break;
+    case FMT_VCF:
+      if (hf[1]) { set_error("VCF read error: lines shorter than 8 bytes on average (a VCF record has 8 fields)"); return BAMSCAN_ERR_FORMAT; }
+      if (start_known) s->need_spec = false;
+      if (new_carry > HEADROOM) return over_headroom("VCF line");
       break;
     case FMT_FASTA: {
       if (hf[1]) { set_error("FASTA read error: more lines in one chunk than supported (lines shorter than 4 bytes on average)"); return BAMSCAN_ERR_UNSUPPORTED; }
@@ -1128,6 +1323,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
       case FMT_BAM: rc = frame_bam(s, slot, BP, W, d_seg_base); break;
       case FMT_FASTQ: rc = frame_fastq(s, c, slot, BP); break;
       case FMT_SAM: rc = frame_sam(s, c, slot, BP); break;
+      case FMT_VCF: rc = frame_vcf(s, c, slot, BP); break;
       case FMT_FASTA: rc = frame_fasta(s, c, range, slot, BP, first_of_range); break;
     }
     if (rc) return rc;
@@ -1181,6 +1377,7 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
         break;
       case FMT_FASTQ: d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14]; break;       // lines[] from the first record's line on: 4 per row
       case FMT_SAM: d_recoff = const_cast<uint32_t*>(sam_recoff); break;
+      case FMT_VCF: d_recoff = s->d_recoff[slot].as<uint32_t>() + hf[14]; break;      // line starts: row r = [lines[r], lines[r + 1])
       case FMT_FASTA: {
         // every line's destination in the chunk's sequence text: content bytes per line, scanned (the decode slices read it)
         const uint32_t* fa_hf = s->h_flags + FA_HFLAGS - 16;     // FASTA words, indexed as in d_flags
@@ -1293,7 +1490,7 @@ static int advance(BamScanStream* s, bool* produced) {
   BamFile* f = s->f;
   for (;;) {
     if (s->cur.pos < s->cur.n) {   // rows of the current chunk still to decode
-      int rc = decode_slice(s, produced);
+      int rc = decode_next_slice(s, produced);
       if (!rc) rc = launch_next_chunk_early(s);
       return rc ? rc : 1;
     }
@@ -1342,7 +1539,7 @@ static int advance(BamScanStream* s, bool* produced) {
     else if (s->range_stop) { s->carry_len = 0; s->range_open = false; s->range_idx++; }                      // unmapped tail: another reference began
     // first slice now (its kernels get the whole GPU: decode_slice does not wait for them), then the next chunk's inflate on the
     // other stream -- a persistent kernel that fills the SMs as the decode CTAs drain and overlaps the remaining slices
-    if (s->cur.pos < s->cur.n && (rc = decode_slice(s, produced))) return rc;
+    if (s->cur.pos < s->cur.n && (rc = decode_next_slice(s, produced))) return rc;
     if ((rc = launch_next_chunk_early(s))) return rc;
     return 1;
   }
@@ -1396,8 +1593,13 @@ static void export_batch(const BamScanStream* s, const ReadyBatch& rb, ArrowArra
     if (is_list) {
       NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 2, 1);
       p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off;
-      NodePriv* cp = new_node(ch->children[0], rb.owner, (int64_t)L.child_len, 0, 0, 2, 0);
-      cp->buffers[0] = nullptr; cp->buffers[1] = H + L.data_off;
+      // VCF lists have nullable elements (child validity) and List<Utf8> a child with offsets; the BAM tag lists have neither
+      const bool utf8_items = L.kind == HK_ListUtf8;
+      const int64_t cnulls = L.child_validity ? (on_device ? -1 : count_nulls(H + L.child_validity_off, 0, L.child_len)) : 0;
+      NodePriv* cp = new_node(ch->children[0], rb.owner, (int64_t)L.child_len, cnulls, 0, utf8_items ? 3 : 2, 0);
+      cp->buffers[0] = cnulls ? H + L.child_validity_off : nullptr;
+      if (utf8_items) { cp->buffers[1] = H + L.child_offsets_off; cp->buffers[2] = H + L.data_off; }
+      else cp->buffers[1] = H + L.data_off;
     } else if (is_var) {
       NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 3, 0);
       p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off; p->buffers[2] = H + L.data_off;
@@ -1425,6 +1627,18 @@ static int decode_error_to_rc(uint32_t code, uint32_t row, uint64_t row0) {
     case FQ_ERR_UTF8: set_error("FASTQ record %u of the batch: non-ASCII byte (not supported by this build)", row); return BAMSCAN_ERR_UNSUPPORTED;
     case FA_ERR_NAME: set_error("FASTA read error: record %llu of the partition (0-based): empty name", prow); return BAMSCAN_ERR_FORMAT;
     case FA_ERR_UTF8: set_error("FASTA read error: record %llu of the partition (0-based): byte 0x80 or above", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_FIELDS: set_error("VCF read error: record %llu of the partition (0-based): fewer than 8 fields", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_HASH: set_error("VCF read error: record %llu of the partition (0-based): a '#' line or an empty line in the body", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_POS: set_error("VCF read error: record %llu of the partition (0-based): POS is not an integer in [1, 2^31 - 1]", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_CHROM: set_error("VCF read error: record %llu of the partition (0-based): empty CHROM", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_REF: set_error("VCF read error: record %llu of the partition (0-based): empty REF", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_END: set_error("VCF read error: record %llu of the partition (0-based): INFO END is below POS", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_DUP: set_error("VCF read error: record %llu of the partition (0-based): an INFO key is given twice", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_UTF8: set_error("VCF read error: record %llu of the partition (0-based): byte 0x80 or above in a text column", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_QUAL: set_error("VCF read error: record %llu of the partition (0-based): QUAL is not '.' or a number", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_VALUE: set_error("VCF read error: record %llu of the partition (0-based): an INFO value does not parse as its declared type", prow); return BAMSCAN_ERR_SCHEMA;
+    case vcf::VCF_ERR_POS0: set_error("VCF read error: record %llu of the partition (0-based): POS 0 (a telomere) is not supported by this build", prow); return BAMSCAN_ERR_UNSUPPORTED;
+    case vcf::VCF_ERR_LONG: set_error("VCF read error: record %llu of the partition (0-based): a line longer than %u bytes is not supported", prow, vcf::MAX_LINE); return BAMSCAN_ERR_UNSUPPORTED;
     case FA_ERR_TOO_LONG: set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", prow, (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED;
   }
   set_error("decode error %u at record %u", code, row);
@@ -1508,6 +1722,13 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
     *out = h.release();
     return BAMSCAN_OK;
   }
+  if (format == FMT_VCF) {
+    // VCF: the fixed columns and the INFO fields the header declares (info_fields travel as tag_fields); no metadata, no index
+    if (rc) { release_file(&f); return rc; }
+    if ((rc = build_vcf_schema(&f, &opt))) { release_file(&f); return rc; }
+    *out = h.release();
+    return BAMSCAN_OK;
+  }
   if (format == FMT_FASTA) {
     // FASTA: name, description (NULL when empty), sequence; no metadata, as for FASTQ
     if (rc) { release_file(&f); return rc; }
@@ -1534,6 +1755,10 @@ int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanH
   BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, FMT_FASTA))
 }
 
+int bamscan_open_vcf(const char* path, const BamScanOptions* options, BamScanHandle** out) {
+  BAMSCAN_GUARD(bamscan_open_impl(path, nullptr, options, out, FMT_VCF))
+}
+
 void bamscan_close(BamScanHandle* h) {
   if (!h) return;
   for (BamScanStream* s : h->idle_streams) stream_destroy(s, false);
@@ -1549,7 +1774,7 @@ int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out) {
 
 static int bamscan_describe_tags_impl(BamScanHandle* h, int32_t sample_size, char* buf, uint64_t cap, uint64_t* needed) {
   if (!h || !needed || (cap && !buf)) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
+  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA || h->file.format == FMT_VCF) { set_error("describe is a BamTableProvider call"); return BAMSCAN_ERR_INVALID; }
   if (!h->file.header_ok) { set_error("BAM header could not be read: %s", h->file.path.c_str()); return BAMSCAN_ERR_FORMAT; }
   std::map<std::string, std::pair<char, int32_t>> found;
   infer_tag_types(h->file, {}, sample_size > 0 ? sample_size : 100, &found, true);
@@ -1578,7 +1803,7 @@ int bamscan_describe_tags(BamScanHandle* h, int32_t sample_size, char* buf, uint
 
 int bamscan_classify_filters(BamScanHandle* h, const BamScanFilter* filters, int32_t n_filters, uint8_t* out_pushdown) {
   if (!h || (n_filters && (!filters || !out_pushdown))) { set_error("null argument"); return BAMSCAN_ERR_INVALID; }
-  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // FastqTableProvider and FastaTableProvider push no filter down
+  if (h->file.format == FMT_FASTQ || h->file.format == FMT_FASTA || h->file.format == FMT_VCF) { for (int i = 0; i < n_filters; i++) out_pushdown[i] = 0; return BAMSCAN_OK; }   // the FASTQ, FASTA and VCF providers push no filter down
   return classify_filters(h->file, filters, n_filters, out_pushdown);
 }
 

@@ -89,6 +89,8 @@ static int walk_blocks(BamFile* f) {
   return BAMSCAN_OK;
 }
 
+static int load_vcf_header(BamFile* f);
+
 // ---- plain SAM ----
 // The text body is described as pseudo-blocks with csize == isize and coff == uoff == the file offset, so that planning, chunking
 // and the seam evidence of block-range partitions work on it unchanged.
@@ -258,6 +260,75 @@ static int infer_tag_types_sam(const BamFile& f, const std::vector<std::string>&
   return BAMSCAN_OK;
 }
 
+// ---- VCF header ----
+// One ##INFO=<...> line -> *out.  Values may be quoted ("..." with \" and \\ escapes), so a quoted Description may hold ',' '=' '>'.
+// Keys other than ID, Number, Type and Description are skipped.  false: the line does not parse (or lacks ID, Number or Type).
+static bool vcf_info_line(const std::string& line, BamFile::VcfInfo* out) {
+  size_t k = 8;                                   // behind "##INFO=<"
+  bool has_id = false, has_num = false, has_type = false;
+  for (;;) {
+    const size_t eq = line.find('=', k);
+    if (eq == std::string::npos) return false;
+    const std::string key = line.substr(k, eq - k);
+    std::string val;
+    k = eq + 1;
+    if (k < line.size() && line[k] == '"') {
+      for (k++; k < line.size() && line[k] != '"'; k++) {
+        if (line[k] == '\\' && k + 1 < line.size()) k++;
+        val += line[k];
+      }
+      if (k >= line.size()) return false;
+      k++;
+    } else {
+      while (k < line.size() && line[k] != ',' && line[k] != '>') val += line[k++];
+    }
+    if (key == "ID") { out->id = val; has_id = true; }
+    else if (key == "Number") { out->number = val; has_num = true; }
+    else if (key == "Type") { out->type = val; has_type = true; }
+    else if (key == "Description") out->description = val;
+    if (k >= line.size()) return false;
+    if (line[k] == '>') return has_id && has_num && has_type && !out->id.empty() && k + 1 == line.size();
+    if (line[k] != ',') return false;
+    k++;
+  }
+}
+
+// The header of a BGZF VCF: the leading lines up to and including the #CHROM line (host zlib, as for a BAM header).  The first
+// line must start with "##fileformat=VCF"; ##INFO lines are kept in header order; the records start behind the #CHROM line.
+static int load_vcf_header(BamFile* f) {
+  HostStream hs(*f);
+  static const char kChrom[] = "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO";
+  for (uint64_t line_no = 0;; line_no++) {
+    size_t nl;
+    for (;;) {
+      const uint8_t* p = hs.buf.data() + hs.pos;
+      const void* q = memchr(p, '\n', hs.buf.size() - hs.pos);
+      if (q) { nl = (size_t)((const uint8_t*)q - p); break; }
+      if (!hs.fill()) { nl = hs.buf.size() - hs.pos; break; }
+    }
+    if (nl == 0 && hs.pos >= hs.buf.size()) { set_error("%s: VCF header without a #CHROM line", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
+    std::string line((const char*)hs.ptr(), nl);
+    hs.skip(std::min(nl + 1, hs.buf.size() - hs.pos));
+    if (!line.empty() && line.back() == '\r') line.pop_back();
+    if (line_no == 0 && line.compare(0, 16, "##fileformat=VCF") != 0) { set_error("%s: not a VCF file (the first line is not ##fileformat=VCF...)", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
+    f->text += line; f->text += '\n';
+    if (line.compare(0, 2, "##") == 0) {
+      if (line.compare(0, 8, "##INFO=<") != 0) continue;
+      BamFile::VcfInfo info;
+      if (!vcf_info_line(line, &info)) { set_error("%s: malformed ##INFO header line: %s", f->path.c_str(), line.c_str()); return BAMSCAN_ERR_FORMAT; }
+      for (const auto& o : f->vcf_info)
+        if (o.id == info.id) { set_error("%s: INFO field '%s' is declared twice in the header", f->path.c_str(), info.id.c_str()); return BAMSCAN_ERR_FORMAT; }
+      f->vcf_info.push_back(info);
+      continue;
+    }
+    const size_t n = sizeof kChrom - 1;
+    if (line.compare(0, n, kChrom) != 0 || (line.size() > n && line[n] != '\t')) { set_error("%s: VCF header without a #CHROM line", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
+    f->first_record_uoff = hs.uoff();
+    f->header_ok = true;
+    return BAMSCAN_OK;
+  }
+}
+
 void release_file(BamFile* f) {
   if (!f->data) return;
   if (f->mapped) unmap_file_pinned(f->data, f->size, f->registered); else pinned_free(f->data);
@@ -293,6 +364,7 @@ int load_file(BamFile* f) {
   int rc = walk_blocks(f);
   if (rc) return rc;
   if (f->format == FMT_FASTQ || f->format == FMT_FASTA) { f->first_record_uoff = 0; f->header_ok = true; return BAMSCAN_OK; }     // FASTQ, FASTA: no header
+  if (f->format == FMT_VCF) return load_vcf_header(f);
 
   // BAM header (noodles-bam read_header): magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
   HostStream hs(*f);

@@ -119,6 +119,14 @@ int make_plan(BamFile* f, const int32_t* projection, int32_t n_projection, const
         r.first_uoff = f->blocks[b].uoff;
         for (uint32_t q = b; q > 0; q--) if (f->blocks[q - 1].isize) { r.block_begin = q - 1; break; }
       }
+      if (f->format == FMT_VCF && owns && p > 0) {
+        // VCF: a line belongs to the range that holds its first byte, FASTA's rule: the member in front of the range is inflated
+        // too (it tells whether the range's first byte starts a line) and nothing in it is owned.  Range 0 starts at the first
+        // record, behind the #CHROM line.
+        r.exact_start = true;
+        r.first_uoff = std::max<uint64_t>(f->blocks[b].uoff, f->first_record_uoff);
+        for (uint32_t q = b; q > 0; q--) if (f->blocks[q - 1].isize) { r.block_begin = q - 1; break; }
+      }
       if (owns) part.ranges.push_back(r);
       part.estimated_bytes = (e > b && b < n_blocks) ? ((e < n_blocks ? f->blocks[e].coff : f->size) - f->blocks[b].coff) : 0;
       plan->partitions.push_back(part);

@@ -4,6 +4,7 @@
 //   bio-format-bam/src/table_provider.rs:42-140   determine_schema (inferred > hints > registry > Utf8)
 //   bio-format-core/src/tag_registry.rs:131-792   registry, hint grammar, type formatting
 //   bio-format-core/src/metadata.rs:321-485       extract_header_metadata (SAM header -> JSON strings)
+#include <algorithm>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -224,6 +225,46 @@ int build_schema(BamFile* f, const BamScanOptions* opt) {
   return BAMSCAN_OK;
 }
 
+// VCF: chrom, start, end, id, ref, alt, qual, filter, then one column per selected ##INFO field (DESIGN 3.11).  Type=Flag ->
+// Boolean (not null); Number=1 -> Int32 / Float32 / Utf8; any other Number -> a list of those.  The field metadata carries the
+// header's Number, Type and Description.  BAMSCAN_ERR_SCHEMA names the field: an ID the header does not declare, an ID equal to a
+// fixed column's name, an unknown Type, Number=0 on a type other than Flag.
+int build_vcf_schema(BamFile* f, const BamScanOptions* opt) {
+  static const char* fixed[] = {"chrom", "start", "end", "id", "ref", "alt", "qual", "filter"};
+  f->fields = {{"chrom", HK_Utf8, false, {}}, {"start", HK_UInt32, false, {}}, {"end", HK_UInt32, false, {}}, {"id", HK_Utf8, true, {}},
+               {"ref", HK_Utf8, false, {}}, {"alt", HK_Utf8, true, {}}, {"qual", HK_Float32, true, {}}, {"filter", HK_Utf8, true, {}}};
+  std::vector<const BamFile::VcfInfo*> sel;
+  if (opt->has_tag_fields) {
+    for (int i = 0; i < opt->n_tag_fields && opt->tag_fields; i++) {
+      const std::string id = opt->tag_fields[i] ? opt->tag_fields[i] : "";
+      const BamFile::VcfInfo* hit = nullptr;
+      for (const auto& d : f->vcf_info) if (d.id == id) { hit = &d; break; }
+      if (!hit) { set_error("INFO field '%s' is not declared in the VCF header", id.c_str()); return BAMSCAN_ERR_SCHEMA; }
+      if (std::find(sel.begin(), sel.end(), hit) != sel.end()) { set_error("INFO field '%s' is selected twice", id.c_str()); return BAMSCAN_ERR_SCHEMA; }
+      sel.push_back(hit);
+    }
+  } else {
+    for (const auto& d : f->vcf_info) sel.push_back(&d);
+  }
+  for (const BamFile::VcfInfo* d : sel) {
+    for (const char* c : fixed)
+      if (d->id == c) { set_error("INFO field '%s' has the name of a fixed VCF column", d->id.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    int32_t scalar;
+    if (d->type == "Flag") scalar = HK_Boolean;
+    else if (d->type == "Integer") scalar = HK_Int32;
+    else if (d->type == "Float") scalar = HK_Float32;
+    else if (d->type == "String" || d->type == "Character") scalar = HK_Utf8;
+    else { set_error("INFO field '%s' has the unknown Type '%s'", d->id.c_str(), d->type.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    if (scalar != HK_Boolean && d->number == "0") { set_error("INFO field '%s' has Number=0 but Type=%s (only a Flag may have Number=0)", d->id.c_str(), d->type.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    int32_t kind = scalar;
+    if (scalar != HK_Boolean && d->number != "1") kind = scalar == HK_Int32 ? HK_ListInt32 : scalar == HK_Float32 ? HK_ListFloat32 : HK_ListUtf8;
+    FieldDef fd{d->id, kind, scalar != HK_Boolean, {}};
+    fd.metadata = {{"bio.vcf.info.number", d->number}, {"bio.vcf.info.type", d->type}, {"bio.vcf.info.description", d->description}};
+    f->fields.push_back(fd);
+  }
+  return BAMSCAN_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // ArrowSchema export
 struct SchemaPriv {
@@ -251,13 +292,15 @@ static std::string encode_metadata(const std::vector<std::pair<std::string, std:
 static const char* kind_format(int32_t kind) {
   switch (kind) {
     case HK_Int32: return "i"; case HK_UInt32: return "I"; case HK_Float32: return "f"; case HK_Utf8: return "u"; case HK_Binary: return "z";
-    case HK_ListInt8: case HK_ListUInt8: case HK_ListInt16: case HK_ListUInt16: case HK_ListInt32: case HK_ListUInt32: case HK_ListFloat32: return "+l";
+    case HK_Boolean: return "b";
+    case HK_ListInt8: case HK_ListUInt8: case HK_ListInt16: case HK_ListUInt16: case HK_ListInt32: case HK_ListUInt32: case HK_ListFloat32:
+    case HK_ListUtf8: return "+l";
   }
   return "n";
 }
 static const char* list_item_format(int32_t kind) {
   switch (kind) { case HK_ListInt8: return "c"; case HK_ListUInt8: return "C"; case HK_ListInt16: return "s"; case HK_ListUInt16: return "S";
-                  case HK_ListInt32: return "i"; case HK_ListUInt32: return "I"; case HK_ListFloat32: return "f"; }
+                  case HK_ListInt32: return "i"; case HK_ListUInt32: return "I"; case HK_ListFloat32: return "f"; case HK_ListUtf8: return "u"; }
   return "n";
 }
 

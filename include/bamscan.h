@@ -161,6 +161,25 @@ int bamscan_open_fastq(const char* path, const BamScanOptions* options, BamScanH
  * refused (BAMSCAN_ERR_FORMAT): this build reads BGZF. */
 int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanHandle** out);
 
+/* A BGZF-compressed VCF file (a provider like bio-format-vcf's; the rules are this build's own, DESIGN 3.11 and oracle/vcf_oracle.py).
+ * The header (the leading lines up to the #CHROM line; the first line must start with "##fileformat=VCF") is read at open, and its
+ * ##INFO lines decide the schema: chrom (Utf8), start (UInt32, POS - 1 or POS), end (UInt32: INFO END if present, else
+ * POS + len(REF) - 1), id, ref, alt (Utf8), qual (Float32), filter (Utf8), then one column per selected INFO field: Type=Flag ->
+ * Boolean, Number=1 -> Int32 / Float32 / Utf8, any other Number -> List of those with nullable elements; '.' is NULL.  Options
+ * read: has_tag_fields / n_tag_fields / tag_fields carry info_fields (0 = every ##INFO field in header order, else those IDs in
+ * that order), coordinate_system_zero_based, batch_rows, chunk_inflated_bytes, skip_crc, device_id and the inflate bits of
+ * debug_flags; everything else is ignored.  Refused at open: a file that is not BGZF or not VCF, a duplicate INFO ID or a missing
+ * #CHROM line (BAMSCAN_ERR_FORMAT); an info_fields ID the header does not declare or that is given twice, an INFO ID equal to a
+ * fixed column's name, Number=0 on a type other than Flag (BAMSCAN_ERR_SCHEMA, naming the field).  Refused by the scan, naming
+ * the record of the partition: malformed lines (BAMSCAN_ERR_FORMAT), a projected INFO value that does not parse as its type
+ * (BAMSCAN_ERR_SCHEMA), POS 0 and lines over 16 MiB (BAMSCAN_ERR_UNSUPPORTED).  An INFO key given twice in one record is a
+ * format error only for the keys the scan looks up (the projected INFO fields and END): other keys are skipped unread, as
+ * their values are.  At most 112 INFO columns can be projected in one scan; bamscan_execute refuses more with
+ * BAMSCAN_ERR_UNSUPPORTED (a header with more ##INFO fields needs info_fields or a projection).  FORMAT and sample columns are skipped.  bamscan_plan with
+ * BAMSCAN_PARTITION_BLOCK_RANGE balances BGZF block ranges by compressed bytes (a line belongs to the range that holds its first
+ * byte); otherwise one partition.  No filter is pushed down, there is no index, describe is refused. */
+int bamscan_open_vcf(const char* path, const BamScanOptions* options, BamScanHandle** out);
+
 /* == TableProvider::schema (table_provider.rs:933-935): the full, unprojected schema with all metadata. */
 int bamscan_schema(BamScanHandle* h, struct ArrowSchema* out);
 

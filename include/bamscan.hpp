@@ -224,6 +224,40 @@ class FastaTableProvider {
   BamScanHandle* h_ = nullptr;
 };
 
+// A provider for BGZF-compressed VCF (bamscan_open_vcf): the eight fixed columns, then one column per selected ##INFO field
+// (info_fields nullopt: all of them, in header order).  scan() with target_partitions > 1 cuts BGZF block ranges balanced by
+// compressed bytes; no filter is pushed down.  At most 112 INFO columns can be projected in one scan (execute throws
+// BAMSCAN_ERR_UNSUPPORTED above that): pass info_fields or a projection for headers with more ##INFO fields.
+class VcfTableProvider {
+ public:
+  explicit VcfTableProvider(const std::string& file_path, const std::optional<std::vector<std::string>>& info_fields = std::nullopt,
+                            const std::optional<std::string>& object_storage_options = std::nullopt, bool coordinate_system_zero_based = true,
+                            int32_t device_id = 0, int32_t batch_rows = 0) {
+    if (object_storage_options) throw Error(BAMSCAN_ERR_UNSUPPORTED, "remote object storage is out of scope for this build (local files only)");
+    std::vector<const char*> ids;
+    if (info_fields) for (auto& i : *info_fields) ids.push_back(i.c_str());
+    BamScanOptions o; std::memset(&o, 0, sizeof o);
+    o.struct_size = sizeof o; o.device_id = device_id; o.batch_rows = batch_rows;
+    o.coordinate_system_zero_based = coordinate_system_zero_based;
+    o.has_tag_fields = info_fields.has_value(); o.n_tag_fields = (int32_t)ids.size(); o.tag_fields = ids.empty() ? nullptr : ids.data();
+    check(bamscan_open_vcf(file_path.c_str(), &o, &h_));
+  }
+  VcfTableProvider(VcfTableProvider&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+  VcfTableProvider(const VcfTableProvider&) = delete;
+  ~VcfTableProvider() { if (h_) bamscan_close(h_); }
+  void schema(ArrowSchema* out) const { check(bamscan_schema(h_, out)); }
+  const char* table_type() const { return "Base"; }
+  BamExec scan(const std::optional<std::vector<int32_t>>& projection, std::optional<int64_t> limit, int32_t target_partitions = 1) const {
+    BamScanPlan* p = nullptr;
+    check(bamscan_plan(h_, projection && !projection->empty() ? projection->data() : nullptr, projection ? (int32_t)projection->size() : -1,
+                       nullptr, 0, limit.value_or(-1), target_partitions,
+                       target_partitions > 1 ? BAMSCAN_PARTITION_BLOCK_RANGE : BAMSCAN_PARTITION_REFERENCE, &p));
+    return BamExec(p);
+  }
+ private:
+  BamScanHandle* h_ = nullptr;
+};
+
 // == BamWriteExec (bio-format-bam/src/write_exec.rs:43-110, 195-350): INSERT OVERWRITE into a BGZF BAM.  The SAM header text and
 // the reference dictionary are the caller's (the Rust host keeps build_bam_header, header_builder.rs:43-186; INTEGRATION.md 3c).
 class BamWriteExec {

@@ -505,3 +505,117 @@ impl TableProvider for GpuFastaTableProvider {
         Ok(Arc::new(GpuBamExec { plan, schema, cache: Arc::new(cache) }))
     }
 }
+
+/// A provider for BGZF-compressed VCF (`bamscan_open_vcf`), shaped like the BAM one: chrom, start, end, id, ref, alt, qual and
+/// filter, then one column per selected `##INFO` field (Flag -> Boolean, Number=1 -> Int32 / Float32 / Utf8, any other Number ->
+/// a list of those); FORMAT and sample columns are skipped.  `info_fields` `None` selects every `##INFO` field in header order;
+/// at most 112 INFO columns can be projected in one scan (more fail with BAMSCAN_ERR_UNSUPPORTED).  No filter is pushed down
+/// (DataFusion applies them), `limit` is passed on and not applied, and with `target_partitions` > 1 the file is cut into BGZF
+/// block ranges balanced by compressed bytes (a line belongs to the range that holds its first byte).  Scans return
+/// `GpuBamExec`, which streams the batches exactly as for BAM.
+pub struct GpuVcfTableProvider {
+    handle: Arc<Handle>,
+    schema: SchemaRef,
+    device_id: i32,
+}
+
+impl GpuVcfTableProvider {
+    /// `object_storage_options` must be `None` (local files only).  `device_id` selects the GPU.
+    pub fn new(file_path: String, info_fields: Option<Vec<String>>, object_storage_options: Option<String>, coordinate_system_zero_based: bool,
+               device_id: i32) -> Result<Self> {
+        if object_storage_options.is_some() {
+            return Err(DataFusionError::NotImplemented("remote object storage is out of scope for this build (local files only)".into()));
+        }
+        let c_path = CString::new(file_path).map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let c_ids: Vec<CString> = info_fields.iter().flatten().map(|s| CString::new(s.as_str())).collect::<std::result::Result<_, _>>()
+            .map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let id_ptrs: Vec<*const c_char> = c_ids.iter().map(|c| c.as_ptr()).collect();
+        let opts = ffi::BamScanOptions {
+            struct_size: std::mem::size_of::<ffi::BamScanOptions>() as u32,
+            coordinate_system_zero_based: coordinate_system_zero_based as i32,
+            binary_cigar: 0,
+            has_tag_fields: info_fields.is_some() as i32,
+            n_tag_fields: id_ptrs.len() as i32,
+            tag_fields: if id_ptrs.is_empty() { std::ptr::null() } else { id_ptrs.as_ptr() },
+            infer_tag_types: 0,
+            infer_tag_sample_size: 0,
+            n_tag_type_hints: 0,
+            tag_type_hints: std::ptr::null(),
+            device_id,
+            batch_rows: 0,
+            chunk_inflated_bytes: 0,
+            segment_bytes: 0,
+            skip_crc: 0,
+            debug_flags: 0,
+        };
+        let mut raw = std::ptr::null_mut();
+        if unsafe { ffi::bamscan_open_vcf(c_path.as_ptr(), &opts, &mut raw) } != 0 {
+            return Err(last_error());
+        }
+        let handle = Arc::new(Handle(raw));
+        let mut c_schema = FFI_ArrowSchema::empty();
+        if unsafe { ffi::bamscan_schema(handle.0, &mut c_schema) } != 0 {
+            return Err(last_error());
+        }
+        let schema = Arc::new(Schema::try_from(&c_schema)?);
+        Ok(Self { handle, schema, device_id })
+    }
+
+    pub fn device_id(&self) -> i32 {
+        self.device_id
+    }
+}
+
+impl Debug for GpuVcfTableProvider {
+    fn fmt(&self, f: &mut Formatter<'_>) -> std::fmt::Result {
+        f.debug_struct("GpuVcfTableProvider").field("device_id", &self.device_id).finish()
+    }
+}
+
+#[async_trait]
+impl TableProvider for GpuVcfTableProvider {
+    fn as_any(&self) -> &dyn Any {
+        self
+    }
+    fn schema(&self) -> SchemaRef {
+        self.schema.clone()
+    }
+    fn table_type(&self) -> TableType {
+        TableType::Base
+    }
+
+    fn supports_filters_pushdown(&self, filters: &[&Expr]) -> Result<Vec<TableProviderFilterPushDown>> {
+        Ok(vec![TableProviderFilterPushDown::Unsupported; filters.len()])
+    }
+
+    async fn scan(&self, state: &dyn Session, projection: Option<&Vec<usize>>, _filters: &[Expr], limit: Option<usize>) -> Result<Arc<dyn ExecutionPlan>> {
+        let proj: Option<Vec<i32>> = projection.map(|p| p.iter().map(|&i| i as i32).collect());
+        let (proj_ptr, n_proj) = match &proj {
+            Some(p) => (p.as_ptr(), p.len() as i32),
+            None => (std::ptr::null(), -1),
+        };
+        let target = state.config().target_partitions() as i32;
+        let mode = if target > 1 { ffi::PARTITION_BLOCK_RANGE } else { ffi::PARTITION_REFERENCE };
+        let mut raw_plan = std::ptr::null_mut();
+        let rc = unsafe {
+            ffi::bamscan_plan(self.handle.0, proj_ptr, n_proj, std::ptr::null(), 0, limit.map(|l| l as i64).unwrap_or(-1), target, mode, &mut raw_plan)
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        let plan = Arc::new(Plan { raw: raw_plan, _handle: self.handle.clone() });
+        let mut c_schema = FFI_ArrowSchema::empty();
+        if unsafe { ffi::bamscan_plan_schema(plan.raw, &mut c_schema) } != 0 {
+            return Err(last_error());
+        }
+        let schema: SchemaRef = Arc::new(Schema::try_from(&c_schema)?);
+        let n = unsafe { ffi::bamscan_plan_num_partitions(plan.raw) };
+        let cache = PlanProperties::new(
+            EquivalenceProperties::new(schema.clone()),
+            Partitioning::UnknownPartitioning(n as usize),
+            EmissionType::Final,
+            Boundedness::Bounded,
+        );
+        Ok(Arc::new(GpuBamExec { plan, schema, cache: Arc::new(cache) }))
+    }
+}
