@@ -607,9 +607,7 @@ struct ArenaBuilder {
   size_t take(size_t bytes) { size_t o = pos; pos = align_up(pos + bytes, 256); return o; }
 };
 
-// Decodes the next slice of the current chunk's rows into a fresh arena and queues its D2H (one batch).
-// A decode slice is queued without waiting for it; its time (and, for device-resident runs, its error word) is collected when
-// the next slice starts or the partition ends.
+// Collects the time and, for device-resident runs, the error word of the decode slice queued last (decode_slice).
 static int flush_slice(BamScanStream* s) {
   if (!s->slice_pending) return BAMSCAN_OK;
   s->slice_pending = false;
@@ -679,226 +677,254 @@ static int hand_off_batch(BamScanStream* s, cudaStream_t cs, uint8_t* A, const s
   return BAMSCAN_OK;
 }
 
-static int decode_slice(BamScanStream* s, bool* produced) {
-  NvtxRange nv("bamscan: decode slice (fixed, scan, var) + D2H issue");
-  BamFile* f = s->f;
-  cudaStream_t cs = s->cur.cs;
-  int rc;
-  if ((rc = flush_slice(s))) return rc;
-  const uint8_t* U = s->cur.U;
-  const bool fasta = f->format == FMT_FASTA;
-  const bool fastx = f->format == FMT_FASTQ || fasta;     // the columns map onto the BAM decode slots through fq_slot
-  // FASTA: the slices fa_frame cut (each holds whole records, about SLICE_BYTES of text); otherwise rows_per_slice rows
-  const uint32_t n = fasta ? s->cur.fa_slice_rec[s->cur.fa_slice + 1] - s->cur.pos : std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
-  const uint32_t fa_b0 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice] : 0, fa_b1 = fasta ? s->cur.fa_slice_byte[s->cur.fa_slice + 1] : 0;
-  if (fasta) s->cur.fa_slice++;
-  const uint64_t row0 = s->st.rows;
-  const uint32_t* d_recoff = s->cur.recoff + (size_t)s->cur.pos * (f->format == FMT_FASTQ ? 4 : 1);
-  const uint8_t* d_qabs = s->cur.qabs ? s->cur.qabs + s->cur.pos : nullptr;
-  s->cur.pos += n;
-  CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
-  {
-    // ---- arena region A
-    const size_t n_dec = s->dec_cols.size();
-    std::vector<ColLayout> cols(n_dec);
-    ArenaBuilder AB;
-    const size_t bm_bytes = 4ull * ((n + 31) / 32), off_bytes = 4ull * (n + 1), val_bytes = 4ull * n;
-    size_t err_off = AB.take(64);
-    std::vector<size_t> src_off(n_dec, 0);
-    size_t scratch = 0;
-    for (size_t i = 0; i < n_dec; i++) {
-      ColLayout& L = cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = f->fields[L.schema_idx].kind;
-      const int c_id = L.schema_idx;
-      bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-      L.has_validity = fastx ? c_id == 1 : (c_id >= 12 || c_id == 1 || c_id == 2 || c_id == 3 || c_id == 7 || c_id == 8);
-      if (L.has_validity) L.validity_off = AB.take(bm_bytes);
-      if (is_var) L.offsets_off = AB.take(off_bytes); else L.values_off = AB.take(val_bytes);
-      if (c_id >= 12 && is_var) { src_off[i] = scratch; scratch += align_up(val_bytes, 256); }
-    }
-    const size_t regionA = AB.pos;
-    if ((rc = s->d_scratch.ensure(scratch + 256))) return rc;
-    // a first arena sizing guess; grown after totals are known
-    DeviceBuf& arena = s->d_arena[s->arena_flip];
-    if (arena.cap < regionA) { if ((rc = arena.ensure(regionA + (size_t)s->cur.ubytes * 2))) return rc; }
-    uint8_t* A = arena.as<uint8_t>();
-    DecodeParams DP;
-    memset(&DP, 0, sizeof DP);
-    DP.U = U; DP.rec_off = d_recoff; DP.n = n; DP.zero_based = f->zero_based; DP.binary_cigar = f->binary_cigar;
-    DP.n_ref = (int32_t)f->ref_names.size();
-    DP.end_zero_span = f->format == FMT_SAM; DP.qual_absent = d_qabs;
-    size_t n_ref = f->ref_names.size();
-    DP.ref_name_off = reinterpret_cast<const uint32_t*>(s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16));
-    DP.ref_names = s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16) + align_up(4 * (n_ref + 1), 16);
-    DP.err = reinterpret_cast<uint32_t*>(A + err_off);
-    ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = n + 1;
-    std::vector<size_t> scan_owner;   // dec col index per scan column
-    int n_tags = 0;
-    std::vector<int> tag_slot(n_dec, -1);
-    for (size_t i = 0; i < n_dec; i++) {
-      ColLayout& L = cols[i];
-      uint32_t* v = L.has_validity ? reinterpret_cast<uint32_t*>(A + L.validity_off) : nullptr;
-      int32_t* offs = reinterpret_cast<int32_t*>(A + L.offsets_off);
-      uint32_t* vals = reinterpret_cast<uint32_t*>(A + L.values_off);
-      static const int fq_slot[4] = {0, 1, 9, 10};      // FASTQ: name, description (nullable Utf8 like chrom), sequence, quality_scores; FASTA: the first three
-      switch (fastx ? fq_slot[L.schema_idx] : L.schema_idx) {
-        case 0: DP.l_name = offs; break;
-        case 1: DP.l_chrom = offs; DP.v_chrom = v; break;
-        case 2: DP.start = vals; DP.v_start = v; break;
-        case 3: DP.end = vals; DP.v_end = v; break;
-        case 4: DP.flags = vals; break;
-        case 5: DP.l_cigar = offs; break;
-        case 6: DP.mapq = vals; break;
-        case 7: DP.l_mchrom = offs; DP.v_mchrom = v; break;
-        case 8: DP.mate_start = vals; DP.v_mstart = v; break;
-        case 9: DP.l_seq = offs; break;
-        case 10: DP.l_qual = offs; break;
-        case 11: DP.tlen = reinterpret_cast<int32_t*>(vals); break;
-        default: {
-          TagPlan& T = DP.tags[n_tags];
-          const std::string& tg = f->fields[L.schema_idx].name;
-          T.tag = tg.size() == 2 ? (uint16_t)((uint8_t)tg[0] | ((uint16_t)(uint8_t)tg[1] << 8)) : 0xffffu;   // names that are not 2 bytes never match (sam_tag_io.rs:58-68)
-          T.kind = L.kind; T.valid = v;
-          bool is_var = L.kind == HK_Utf8 || L.kind >= HK_ListInt8;
-          if (is_var) { T.lens = offs; T.src = reinterpret_cast<uint32_t*>(s->d_scratch.as<uint8_t>() + src_off[i]); }
-          else T.values = vals;
-          tag_slot[i] = n_tags++;
-        }
-      }
-      bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-      if (is_var) { SC.col[SC.n_cols++] = offs; scan_owner.push_back(i); }
-    }
-    DP.n_tags = n_tags;
-    CU_TRY(cudaMemsetAsync(A + err_off, 0, 64, cs));
-    FastqCols FC;
-    FastaCols AC;
-    if (f->format == FMT_FASTQ) {
-      FC = FastqCols{U, d_recoff, n, DP.l_name, DP.l_chrom, DP.l_seq, DP.l_qual, DP.v_chrom, nullptr, nullptr, nullptr, nullptr, DP.err};
-      fq_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(FC);
-    }
-    else if (fasta) {
-      AC = FastaCols{U, s->cur.fa_lines, d_recoff, s->cur.fa_seqpos, n, DP.l_name, DP.l_chrom, DP.l_seq, DP.v_chrom, nullptr, nullptr, DP.err};
-      fa_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(AC);
-    }
-    else if (s->cur.long_records) {
-      CU_TRY(cudaMemsetAsync(A, 0, regionA, cs));                                        // validity words are OR-ed in
-      decode_fixed_warp_kernel<<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(DP);     // long records: a warp per row, lanes co-operate inside the record
-    }
-    else
-      decode_fixed_kernel<<<(n + 255) / 256, 256, 0, cs>>>(DP);
-    s->st.kernel_launches++;
-    uint64_t* h_totals = reinterpret_cast<uint64_t*>(s->h_flags + 16);
-    if (SC.n_cols) {
-      if ((rc = s->d_totals.ensure(8ull * MAX_SCAN_COLS)) || (rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>()))) return rc;
-      publish_kernel<<<1, 128, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, 2 * SC.n_cols);      // [16, 16 + 2 * MAX_SCAN_COLS) of the mapped flags page; the decode error words live at [512, 516)
-      CU_TRY(cudaEventRecord(s->ev_dflags, cs));
-      CU_TRY(cudaEventSynchronize(s->ev_dflags));
-      CU_TRY(cudaGetLastError());
-      // ---- arena region B
-      for (int k = 0; k < SC.n_cols; k++) {
-        ColLayout& L = cols[scan_owner[k]];
-        uint64_t tot = h_totals[k];
-        if (tot > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", f->fields[L.schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
-        uint64_t bytes = tot;
-        if (L.kind >= HK_ListInt8) { L.child_len = tot; bytes = tot * ((L.kind == HK_ListInt8 || L.kind == HK_ListUInt8) ? 1 : (L.kind == HK_ListInt16 || L.kind == HK_ListUInt16) ? 2 : 4); }
-        L.data_bytes = bytes;
-        L.data_off = AB.take((size_t)bytes + 16);
-      }
-      if (AB.pos > arena.cap) {
-        // grow, preserving region A
-        DeviceBuf bigger;
-        if ((rc = bigger.ensure(AB.pos))) return rc;
-        CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, regionA, cudaMemcpyDeviceToDevice, cs));
-        CU_TRY(cudaStreamSynchronize(cs));
-        // rebase pointers
-        ptrdiff_t delta = (uint8_t*)bigger.p - A;
-        auto rb = [&](auto*& p) { if (p) p = reinterpret_cast<std::remove_reference_t<decltype(p)>>(reinterpret_cast<uint8_t*>(p) + delta); };
-        rb(DP.start); rb(DP.end); rb(DP.flags); rb(DP.mapq); rb(DP.mate_start); rb(DP.tlen);
-        rb(DP.v_chrom); rb(DP.v_start); rb(DP.v_end); rb(DP.v_mchrom); rb(DP.v_mstart);
-        rb(DP.l_name); rb(DP.l_chrom); rb(DP.l_cigar); rb(DP.l_mchrom); rb(DP.l_seq); rb(DP.l_qual); rb(DP.err);
-        for (int t = 0; t < n_tags; t++) { rb(DP.tags[t].valid); rb(DP.tags[t].values); rb(DP.tags[t].lens); }
-        arena.release(); arena = bigger; bigger.p = nullptr; bigger.cap = 0;
-        A = arena.as<uint8_t>();
-      }
-      for (size_t i = 0; i < n_dec; i++) {
-        ColLayout& L = cols[i];
-        bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-        if (!is_var) continue;
-        uint8_t* d = A + L.data_off;
-        switch (L.schema_idx) {
-          case 0: DP.d_name = d; break; case 1: DP.d_chrom = d; break; case 5: DP.d_cigar = d; break; case 7: DP.d_mchrom = d; break;
-          case 2: if (fastx) DP.d_seq = d; break; case 3: if (f->format == FMT_FASTQ) DP.d_qual = d; break;
-          case 9: DP.d_seq = d; break; case 10: DP.d_qual = d; break;
-          default: DP.tags[tag_slot[i]].data = d;
-        }
-      }
-      if (f->format == FMT_FASTQ) {
-        FC.l_name = DP.l_name; FC.l_desc = DP.l_chrom; FC.l_seq = DP.l_seq; FC.l_qual = DP.l_qual; FC.err = DP.err;      // (rebased with the arena)
-        FC.d_name = DP.d_name; FC.d_desc = DP.d_chrom; FC.d_seq = DP.d_seq; FC.d_qual = DP.d_qual;
-        fq_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(FC);
-      }
-      else if (fasta) {
-        AC.l_name = DP.l_name; AC.l_desc = DP.l_chrom; AC.l_seq = DP.l_seq; AC.v_desc = DP.v_chrom; AC.err = DP.err;      // (rebased with the arena)
-        AC.d_name = DP.d_name; AC.d_desc = DP.d_chrom;
-        if (AC.d_name || AC.d_desc) { fa_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(AC); s->st.kernel_launches++; }
-        if (DP.d_seq && fa_b1 > fa_b0) {
-          const uint32_t t0 = (fa_b0 - s->cur.fa_lo) / FQ_TILE, t1 = (fa_b1 - s->cur.fa_lo + FQ_TILE - 1) / FQ_TILE;
-          FastaSeq SQ{U, s->cur.fa_lines, s->cur.fa_seqpos, s->cur.fa_tile_base, d_recoff, n, s->cur.fa_lo, s->cur.fa_hi, t0, DP.d_seq, DP.err};
-          fa_seq_kernel<<<t1 - t0, 256, 0, cs>>>(SQ);
-          s->st.kernel_launches++;
-        }
-      }
-      // short reads: 8 lanes per record (4 records per warp); long reads (and debug_flags bit 1): a warp per record
-      else if (s->cur.long_records)
-        decode_var_kernel<32><<<std::min<uint32_t>((n + VAR_WARPS - 1) / VAR_WARPS, 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
-      else
-        decode_var_kernel<8><<<std::min<uint32_t>((n + VAR_WARPS * 4 - 1) / (VAR_WARPS * 4), 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
-      if (!fasta) s->st.kernel_launches++;
-    }
-    const size_t arena_bytes = AB.pos;
-    s->st.rows += n; s->st.batches++;
-    for (auto& L : cols) {
-      bool is_var = L.kind == HK_Utf8 || L.kind == HK_Binary || L.kind >= HK_ListInt8;
-      s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var ? off_bytes + L.data_bytes : val_bytes);
-    }
-    if ((rc = hand_off_batch(s, cs, A, cols, n, arena_bytes, err_off, row0, produced))) return rc;
+// ---- decode slices: one function per format picks the slice's rows, binds its kernels to the arena and launches them; the arena
+// steps are shared.  Region A (the error word, then per column its validity words and its offsets or fixed values) is laid out
+// before the count kernels run, region B (variable-length data, list children) once the scanned totals are known.
+
+static bool is_var(int32_t kind) { return kind == HK_Utf8 || kind == HK_Binary || kind >= HK_ListInt8; }     // Arrow offsets + data
+static size_t fixed_bytes(int32_t kind, uint32_t n) { return kind == HK_Boolean ? 4ull * ((n + 31) / 32) : 4ull * n; }   // Boolean: bitmap words
+// A column's buffers in the arena at A: valid is null without a validity bitmap, data until region B is laid out (region A starts
+// with the error word, so no data lies at offset 0)
+struct ColPtrs { uint32_t* valid; int32_t* offs; uint32_t* vals; uint8_t* data; };
+static ColPtrs col_ptrs(uint8_t* A, const ColLayout& L) {
+  return {L.has_validity ? reinterpret_cast<uint32_t*>(A + L.validity_off) : nullptr, reinterpret_cast<int32_t*>(A + L.offsets_off),
+          reinterpret_cast<uint32_t*>(A + L.values_off), L.data_off ? A + L.data_off : nullptr};
+}
+
+struct Slice {
+  uint32_t n = 0;                  // rows
+  std::vector<ColLayout> cols;     // one per s->dec_cols
+  ArenaBuilder AB;
+  size_t err_off = 0, region_a = 0;
+  uint8_t* A = nullptr;            // s->d_arena[s->arena_flip]
+};
+struct CountCol { int32_t* counts; size_t col; };   // a count column, scanned in place, and its index in Slice::cols
+
+// Region A of an n-row slice, in an arena that holds it (a first sizing guess, grown by layout_region_b), with the error word
+// cleared.  has_validity: the format's rule for which columns carry a validity bitmap.
+static int layout_region_a(BamScanStream* s, Slice& S, uint32_t n, bool (*has_validity)(const BamFile&, int32_t)) {
+  S.n = n;
+  S.err_off = S.AB.take(64);
+  S.cols.resize(s->dec_cols.size());
+  for (size_t i = 0; i < S.cols.size(); i++) {
+    ColLayout& L = S.cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = s->f->fields[L.schema_idx].kind;
+    L.has_validity = has_validity(*s->f, L.schema_idx);
+    if (L.has_validity) L.validity_off = S.AB.take(4ull * ((n + 31) / 32));
+    if (is_var(L.kind)) L.offsets_off = S.AB.take(4ull * (n + 1)); else L.values_off = S.AB.take(fixed_bytes(L.kind, n));
   }
-  CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
-  s->slice_pending = true;
+  S.region_a = S.AB.pos;
+  DeviceBuf& arena = s->d_arena[s->arena_flip];
+  if (arena.cap < S.region_a) { if (int rc = arena.ensure(S.region_a + (size_t)s->cur.ubytes * 2)) return rc; }
+  S.A = arena.as<uint8_t>();
+  CU_TRY(cudaMemsetAsync(S.A + S.err_off, 0, 64, s->cur.cs));
   return BAMSCAN_OK;
 }
 
-// VCF: the next slice of the chunk's lines -> the projected columns (kernels_vcf.cuh), then the same hand-off as decode_slice.  One host
-// sync: the totals of the count columns (Utf8 bytes, list elements, List<Utf8> bytes) size the arena's second region.
-static int decode_slice_vcf(BamScanStream* s, bool* produced) {
-  NvtxRange nv("bamscan: VCF decode slice (fields, rows, scan, write) + D2H issue");
+// The count columns of BAM, SAM, FASTQ and FASTA: the offsets of every variable-length column
+static std::vector<CountCol> offset_counts(const Slice& S) {
+  std::vector<CountCol> counts;
+  for (size_t i = 0; i < S.cols.size(); i++) if (is_var(S.cols[i].kind)) counts.push_back({reinterpret_cast<int32_t*>(S.A + S.cols[i].offsets_off), i});
+  return counts;
+}
+
+// Count columns -> Arrow offsets, in launches of up to MAX_SCAN_COLS columns.  The totals reach the host through the mapped flags
+// page at [16, 16 + 2 * counts) (VCF's 229 at most stay below the decode error words at [512, 516)) with one host sync, and each is
+// held to Arrow's 2^31-1 limit.  Region B then takes per column its data: the total's bytes (Utf8, Binary) or, for a list, the
+// child validity words when list_child_validity (VCF; BAM tag lists have none), then the child values, or for List<Utf8> the
+// child offsets and the bytes the next count column totals.  The arena grows when region B does not fit, keeping region A; the
+// format binds its kernels again afterwards.
+static int layout_region_b(BamScanStream* s, Slice& S, const std::vector<CountCol>& counts, bool list_child_validity) {
+  cudaStream_t cs = s->cur.cs;
+  const size_t n_scan = counts.size();
+  int rc;
+  if ((rc = s->d_totals.ensure(8 * n_scan))) return rc;
+  for (size_t k0 = 0; k0 < n_scan; k0 += MAX_SCAN_COLS) {
+    ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = S.n + 1;
+    for (size_t k = k0; k < std::min(n_scan, k0 + MAX_SCAN_COLS); k++) SC.col[SC.n_cols++] = counts[k].counts;
+    if ((rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>() + k0))) return rc;
+  }
+  publish_kernel<<<1, 256, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, (int)(2 * n_scan));
+  CU_TRY(cudaEventRecord(s->ev_dflags, cs));
+  CU_TRY(cudaEventSynchronize(s->ev_dflags));
+  CU_TRY(cudaGetLastError());
+  const uint64_t* T = reinterpret_cast<const uint64_t*>(s->h_flags + 16);
+  for (size_t k = 0; k < n_scan; k++)
+    if (T[k] > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", s->f->fields[S.cols[counts[k].col].schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
+  for (size_t k = 0; k < n_scan; k++) {
+    ColLayout& L = S.cols[counts[k].col];
+    uint64_t bytes = T[k];
+    if (L.kind >= HK_ListInt8) {
+      L.child_len = T[k];
+      if (list_child_validity) { L.child_validity = true; L.child_validity_off = S.AB.take(4 * ((T[k] + 31) / 32)); }
+      if (L.kind == HK_ListUtf8) { L.child_offsets_off = S.AB.take(4 * (T[k] + 1)); bytes = T[++k]; }
+      else bytes *= (L.kind == HK_ListInt8 || L.kind == HK_ListUInt8) ? 1 : (L.kind == HK_ListInt16 || L.kind == HK_ListUInt16) ? 2 : 4;
+    }
+    L.data_bytes = bytes;
+    L.data_off = S.AB.take((size_t)bytes + 16);
+  }
+  DeviceBuf& arena = s->d_arena[s->arena_flip];
+  if (S.AB.pos > arena.cap) {
+    DeviceBuf bigger;
+    if ((rc = bigger.ensure(S.AB.pos))) return rc;
+    CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, S.region_a, cudaMemcpyDeviceToDevice, cs));
+    CU_TRY(cudaStreamSynchronize(cs));
+    arena.release(); arena = bigger;
+    S.A = arena.as<uint8_t>();
+  }
+  return BAMSCAN_OK;
+}
+
+// FASTQ: fq_lengths -> scan -> fq_copy.  name, description, sequence and quality_scores (schema 0-3) are Utf8; description is the
+// nullable one.
+static int decode_fastq(BamScanStream* s, Slice& S) {
+  cudaStream_t cs = s->cur.cs;
+  const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
+  int rc;
+  if ((rc = layout_region_a(s, S, n, [](const BamFile&, int32_t c) { return c == 1; }))) return rc;
+  FastqCols FC{s->cur.U, s->cur.recoff + 4ull * s->cur.pos, n};        // (the column pointers: bind)
+  s->cur.pos += n;
+  auto bind = [&](uint8_t* A) {
+    FC.err = reinterpret_cast<uint32_t*>(A + S.err_off);
+    for (const ColLayout& L : S.cols) {
+      const ColPtrs c = col_ptrs(A, L);
+      switch (L.schema_idx) {
+        case 0: FC.l_name = c.offs; FC.d_name = c.data; break;
+        case 1: FC.l_desc = c.offs; FC.v_desc = c.valid; FC.d_desc = c.data; break;
+        case 2: FC.l_seq = c.offs; FC.d_seq = c.data; break;
+        case 3: FC.l_qual = c.offs; FC.d_qual = c.data; break;
+      }
+    }
+  };
+  bind(S.A);
+  fq_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(FC);
+  s->st.kernel_launches++;
+  const std::vector<CountCol> counts = offset_counts(S);
+  if (counts.empty() || (rc = layout_region_b(s, S, counts, false))) return rc;
+  bind(S.A);
+  fq_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(FC);
+  s->st.kernel_launches++;
+  return BAMSCAN_OK;
+}
+
+// FASTA: fa_lengths -> scan -> fa_copy (name, description) and fa_seq (the sequence lines joined).  The slices are the ones
+// frame_fasta cut: whole records, about SLICE_BYTES of text each.
+static int decode_fasta(BamScanStream* s, Slice& S) {
+  cudaStream_t cs = s->cur.cs;
+  const uint32_t k = s->cur.fa_slice++;
+  const uint32_t n = s->cur.fa_slice_rec[k + 1] - s->cur.pos, b0 = s->cur.fa_slice_byte[k], b1 = s->cur.fa_slice_byte[k + 1];
+  int rc;
+  if ((rc = layout_region_a(s, S, n, [](const BamFile&, int32_t c) { return c == 1; }))) return rc;
+  const uint32_t* rec = s->cur.recoff + s->cur.pos;
+  s->cur.pos += n;
+  FastaCols AC{s->cur.U, s->cur.fa_lines, rec, s->cur.fa_seqpos, n};
+  FastaSeq SQ{s->cur.U, s->cur.fa_lines, s->cur.fa_seqpos, s->cur.fa_tile_base, rec, n, s->cur.fa_lo, s->cur.fa_hi, (b0 - s->cur.fa_lo) / FQ_TILE, nullptr, nullptr};
+  auto bind = [&](uint8_t* A) {
+    AC.err = SQ.err = reinterpret_cast<uint32_t*>(A + S.err_off);
+    for (const ColLayout& L : S.cols) {
+      const ColPtrs c = col_ptrs(A, L);
+      switch (L.schema_idx) {
+        case 0: AC.l_name = c.offs; AC.d_name = c.data; break;
+        case 1: AC.l_desc = c.offs; AC.v_desc = c.valid; AC.d_desc = c.data; break;
+        case 2: AC.l_seq = c.offs; SQ.dst = c.data; break;
+      }
+    }
+  };
+  bind(S.A);
+  fa_lengths_kernel<<<(n + 255) / 256, 256, 0, cs>>>(AC);
+  s->st.kernel_launches++;
+  const std::vector<CountCol> counts = offset_counts(S);
+  if (counts.empty() || (rc = layout_region_b(s, S, counts, false))) return rc;
+  bind(S.A);
+  if (AC.d_name || AC.d_desc) { fa_copy_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(AC); s->st.kernel_launches++; }
+  if (SQ.dst && b1 > b0) { fa_seq_kernel<<<(b1 - s->cur.fa_lo + FQ_TILE - 1) / FQ_TILE - SQ.t0, 256, 0, cs>>>(SQ); s->st.kernel_launches++; }
+  return BAMSCAN_OK;
+}
+
+// BAM and SAM (lines that transcode_sam turned into BAM records): decode_fixed -> scan -> decode_var.  Short records take 8 lanes
+// each, long records (and debug_flags bit 1) a warp.
+static int decode_bam(BamScanStream* s, Slice& S) {
   const BamFile* f = s->f;
   cudaStream_t cs = s->cur.cs;
-  int rc;
-  if ((rc = flush_slice(s))) return rc;
   const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
-  const uint64_t row0 = s->st.rows;
+  int rc;
+  if ((rc = layout_region_a(s, S, n, [](const BamFile&, int32_t c) { return c >= 12 || c == 1 || c == 2 || c == 3 || c == 7 || c == 8; }))) return rc;
+  // scratch: per variable-length tag column, each row's aux field offset in U
+  std::vector<size_t> src_off(S.cols.size(), 0);
+  size_t scratch = 0;
+  for (size_t i = 0; i < S.cols.size(); i++) if (S.cols[i].schema_idx >= 12 && is_var(S.cols[i].kind)) { src_off[i] = scratch; scratch += align_up(4ull * n, 256); }
+  if ((rc = s->d_scratch.ensure(scratch + 256))) return rc;
+  DecodeParams DP{};
+  DP.U = s->cur.U; DP.rec_off = s->cur.recoff + s->cur.pos; DP.n = n; DP.zero_based = f->zero_based; DP.binary_cigar = f->binary_cigar;
+  const size_t n_ref = f->ref_names.size(); DP.n_ref = (int32_t)n_ref;
+  DP.end_zero_span = f->format == FMT_SAM; DP.qual_absent = s->cur.qabs ? s->cur.qabs + s->cur.pos : nullptr;
+  DP.ref_name_off = reinterpret_cast<const uint32_t*>(s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16));
+  DP.ref_names = s->d_refs.as<uint8_t>() + align_up(4 * n_ref + 4, 16) + align_up(4 * (n_ref + 1), 16);
+  s->cur.pos += n;
+  auto bind = [&](uint8_t* A) {
+    DP.err = reinterpret_cast<uint32_t*>(A + S.err_off);
+    DP.n_tags = 0;
+    for (size_t i = 0; i < S.cols.size(); i++) {
+      const ColLayout& L = S.cols[i];
+      const ColPtrs c = col_ptrs(A, L);
+      switch (L.schema_idx) {
+        case 0: DP.l_name = c.offs; DP.d_name = c.data; break;
+        case 1: DP.l_chrom = c.offs; DP.v_chrom = c.valid; DP.d_chrom = c.data; break;
+        case 2: DP.start = c.vals; DP.v_start = c.valid; break;
+        case 3: DP.end = c.vals; DP.v_end = c.valid; break;
+        case 4: DP.flags = c.vals; break;
+        case 5: DP.l_cigar = c.offs; DP.d_cigar = c.data; break;
+        case 6: DP.mapq = c.vals; break;
+        case 7: DP.l_mchrom = c.offs; DP.v_mchrom = c.valid; DP.d_mchrom = c.data; break;
+        case 8: DP.mate_start = c.vals; DP.v_mstart = c.valid; break;
+        case 9: DP.l_seq = c.offs; DP.d_seq = c.data; break;
+        case 10: DP.l_qual = c.offs; DP.d_qual = c.data; break;
+        case 11: DP.tlen = reinterpret_cast<int32_t*>(c.vals); break;
+        default: {
+          TagPlan& T = DP.tags[DP.n_tags++];
+          const std::string& tg = f->fields[L.schema_idx].name;
+          T.tag = tg.size() == 2 ? (uint16_t)((uint8_t)tg[0] | ((uint16_t)(uint8_t)tg[1] << 8)) : 0xffffu;   // names that are not 2 bytes never match (sam_tag_io.rs:58-68)
+          T.kind = L.kind; T.valid = c.valid;
+          if (is_var(L.kind)) { T.lens = c.offs; T.src = reinterpret_cast<uint32_t*>(s->d_scratch.as<uint8_t>() + src_off[i]); T.data = c.data; }
+          else T.values = c.vals;
+        }
+      }
+    }
+  };
+  bind(S.A);
+  if (s->cur.long_records) {
+    CU_TRY(cudaMemsetAsync(S.A, 0, S.region_a, cs));                                     // validity words are OR-ed in
+    decode_fixed_warp_kernel<<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(DP);     // a warp per row, lanes co-operate inside the record
+  }
+  else
+    decode_fixed_kernel<<<(n + 255) / 256, 256, 0, cs>>>(DP);
+  s->st.kernel_launches++;
+  const std::vector<CountCol> counts = offset_counts(S);
+  if (counts.empty() || (rc = layout_region_b(s, S, counts, false))) return rc;
+  bind(S.A);
+  if (s->cur.long_records)
+    decode_var_kernel<32><<<std::min<uint32_t>((n + VAR_WARPS - 1) / VAR_WARPS, 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
+  else
+    decode_var_kernel<8><<<std::min<uint32_t>((n + VAR_WARPS * 4 - 1) / (VAR_WARPS * 4), 148u * 8u * 4u), VAR_WARPS * 32, 0, cs>>>(DP);
+  s->st.kernel_launches++;
+  return BAMSCAN_OK;
+}
+
+// VCF: vcf_fields -> vcf_rows -> scan -> vcf_write (kernels_vcf.cuh).  The count columns are the Utf8 bytes and list elements, and
+// for List<Utf8> also the elements' bytes.
+static int decode_vcf(BamScanStream* s, Slice& S) {
+  const BamFile* f = s->f;
+  cudaStream_t cs = s->cur.cs;
+  const uint32_t n = std::min<uint32_t>(s->cur.rows_per_slice, s->cur.n - s->cur.pos);
   const uint32_t* lines = s->cur.recoff + s->cur.pos;
   s->cur.pos += n;
-  CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
-  const size_t n_dec = s->dec_cols.size();
-  std::vector<ColLayout> cols(n_dec);
-  std::vector<int> info_col(n_dec, -1);           // dec column -> INFO column (key) index
-  ArenaBuilder AB;
-  const size_t bm_bytes = 4ull * ((n + 31) / 32), off_bytes = 4ull * (n + 1), val_bytes = 4ull * n;
-  const size_t err_off = AB.take(64);
-  int n_info = 0;
-  for (size_t i = 0; i < n_dec; i++) {
-    ColLayout& L = cols[i]; L.schema_idx = s->dec_cols[i]; L.kind = f->fields[L.schema_idx].kind;
-    L.has_validity = f->fields[L.schema_idx].nullable;
-    if (L.has_validity) L.validity_off = AB.take(bm_bytes);
-    if (L.kind == HK_Utf8 || L.kind >= HK_ListInt8) L.offsets_off = AB.take(off_bytes);
-    else L.values_off = AB.take(L.kind == HK_Boolean ? bm_bytes : val_bytes);
-    if (L.schema_idx >= 8) info_col[i] = n_info++;
-  }
-  const size_t regionA = AB.pos;
-  // keys: the projected INFO IDs, then END unless it is one of them
+  int rc;
+  if ((rc = layout_region_a(s, S, n, [](const BamFile& file, int32_t c) { return file.fields[c].nullable; }))) return rc;
+  const size_t n_dec = S.cols.size();
+  // keys: the projected INFO IDs (key k is INFO column k), then END unless it is one of them
+  std::vector<int> info_col(n_dec, -1);           // column -> INFO column (key) index
   std::vector<std::string> keys;
-  for (size_t i = 0; i < n_dec; i++) if (info_col[i] >= 0) keys.push_back(f->fields[cols[i].schema_idx].name);
+  for (size_t i = 0; i < n_dec; i++) if (S.cols[i].schema_idx >= 8) { info_col[i] = (int)keys.size(); keys.push_back(f->fields[S.cols[i].schema_idx].name); }
+  const int n_info = (int)keys.size();
   int end_key = (int)(std::find(keys.begin(), keys.end(), std::string("END")) - keys.begin());
   if (end_key == (int)keys.size()) keys.push_back("END");
   // Keys::off and Params::cols hold MAX_INFO + 1 keys (stream_init refuses more projected INFO columns)
@@ -920,116 +946,86 @@ static int decode_slice_vcf(BamScanStream* s, bool* produced) {
   const size_t o_tok = align_up(sizeof(vcf::Row) * n, 256), o_blen = o_tok + align_up(8ull * n * keys.size(), 256);
   size_t scratch = o_blen;
   std::vector<size_t> blen_off(n_dec, 0);
-  for (size_t i = 0; i < n_dec; i++) if (cols[i].kind == HK_ListUtf8) { blen_off[i] = scratch; scratch += align_up(off_bytes, 256); }
+  for (size_t i = 0; i < n_dec; i++) if (S.cols[i].kind == HK_ListUtf8) { blen_off[i] = scratch; scratch += align_up(4ull * (n + 1), 256); }
   if ((rc = s->d_scratch.ensure(scratch + 256))) return rc;
   uint8_t* SCR = s->d_scratch.as<uint8_t>();
-  DeviceBuf& arena = s->d_arena[s->arena_flip];
-  if (arena.cap < regionA && (rc = arena.ensure(regionA + (size_t)s->cur.ubytes * 2))) return rc;
-  // the kernels' view of the arena (rebuilt when the arena grows)
   auto bind = [&](uint8_t* A) {
     P->U = s->cur.U; P->lines = lines; P->n = n; P->zero_based = f->zero_based; P->n_info = n_info;
-    P->rows = reinterpret_cast<vcf::Row*>(SCR); P->err = reinterpret_cast<uint32_t*>(A + err_off);
+    P->rows = reinterpret_cast<vcf::Row*>(SCR); P->err = reinterpret_cast<uint32_t*>(A + S.err_off);
     for (size_t k = 0; k < keys.size(); k++) P->cols[k].tok = reinterpret_cast<uint2*>(SCR + o_tok) + (size_t)k * n;
     for (size_t i = 0; i < n_dec; i++) {
-      const ColLayout& L = cols[i];
-      uint32_t* v = L.has_validity ? reinterpret_cast<uint32_t*>(A + L.validity_off) : nullptr;
-      int32_t* offs = reinterpret_cast<int32_t*>(A + L.offsets_off);
-      uint32_t* vals = reinterpret_cast<uint32_t*>(A + L.values_off);
-      uint8_t* d = L.data_bytes || L.child_len ? A + L.data_off : nullptr;
+      const ColLayout& L = S.cols[i];
+      const ColPtrs c = col_ptrs(A, L);
+      uint8_t* d = L.data_bytes ? c.data : nullptr;     // a fixed column without bytes in the slice (an all-'.' ID) is skipped by vcf_write_kernel
       switch (L.schema_idx) {
-        case 0: P->l_chrom = offs; P->d_chrom = d; break;
-        case 1: P->start = vals; break;
-        case 2: P->end = vals; break;
-        case 3: P->l_id = offs; P->v_id = v; P->d_id = d; break;
-        case 4: P->l_ref = offs; P->d_ref = d; break;
-        case 5: P->l_alt = offs; P->v_alt = v; P->d_alt = d; break;
-        case 6: P->qual = vals; P->v_qual = v; break;
-        case 7: P->l_filter = offs; P->v_filter = v; P->d_filter = d; break;
+        case 0: P->l_chrom = c.offs; P->d_chrom = d; break;
+        case 1: P->start = c.vals; break;
+        case 2: P->end = c.vals; break;
+        case 3: P->l_id = c.offs; P->v_id = c.valid; P->d_id = d; break;
+        case 4: P->l_ref = c.offs; P->d_ref = d; break;
+        case 5: P->l_alt = c.offs; P->v_alt = c.valid; P->d_alt = d; break;
+        case 6: P->qual = c.vals; P->v_qual = c.valid; break;
+        case 7: P->l_filter = c.offs; P->v_filter = c.valid; P->d_filter = d; break;
         default: {
           vcf::InfoCol& C = P->cols[info_col[i]];
-          C.kind = L.kind; C.valid = v;
-          if (L.kind == HK_Utf8 || L.kind >= HK_ListInt8) C.lens = offs; else C.values = vals;
+          C.kind = L.kind; C.valid = c.valid; C.data = c.data;
+          if (is_var(L.kind)) C.lens = c.offs; else C.values = c.vals;
           if (L.kind == HK_ListUtf8) { C.blens = reinterpret_cast<int32_t*>(SCR + blen_off[i]); C.coffs = reinterpret_cast<int32_t*>(A + L.child_offsets_off); }
           if (L.child_validity) C.cvalid = reinterpret_cast<uint32_t*>(A + L.child_validity_off);
-          C.data = A + L.data_off;
         }
       }
     }
   };
-  uint8_t* A = arena.as<uint8_t>();
-  bind(A);
-  CU_TRY(cudaMemsetAsync(A + err_off, 0, 64, cs));
+  bind(S.A);
   CU_TRY(cudaMemsetAsync(SCR + o_tok, 0, 8ull * n * keys.size(), cs));
-  // 8 lanes per line; 32 when the previous chunk's lines averaged above 2 KiB (sam_records_kernel's rule)
-  const bool wide = (f->debug_flags & 2) || s->mean_record_bytes > 2048;
-  if (wide) vcf::vcf_fields_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
+  // 8 lanes per line; 32 for long lines (sam_records_kernel's rule)
+  if (s->cur.long_records) vcf::vcf_fields_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
   else vcf::vcf_fields_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
   vcf::vcf_rows_kernel<<<(n + 255) / 256, 256, 0, cs>>>(*P);
   s->st.kernel_launches += 2;
-  // count columns -> offsets, in launches of up to MAX_SCAN_COLS columns
-  std::vector<int32_t*> scan_cols;
-  std::vector<std::pair<size_t, bool>> scan_owner;     // (dec column, is the List<Utf8> byte column)
+  std::vector<CountCol> counts;
   for (size_t i = 0; i < n_dec; i++) {
-    const ColLayout& L = cols[i];
-    if (!(L.kind == HK_Utf8 || L.kind >= HK_ListInt8)) continue;
-    scan_cols.push_back(reinterpret_cast<int32_t*>(A + L.offsets_off)); scan_owner.push_back({i, false});
-    if (L.kind == HK_ListUtf8) { scan_cols.push_back(reinterpret_cast<int32_t*>(SCR + blen_off[i])); scan_owner.push_back({i, true}); }
+    if (!is_var(S.cols[i].kind)) continue;
+    counts.push_back({reinterpret_cast<int32_t*>(S.A + S.cols[i].offsets_off), i});
+    if (S.cols[i].kind == HK_ListUtf8) counts.push_back({reinterpret_cast<int32_t*>(SCR + blen_off[i]), i});
   }
-  const size_t n_scan = scan_cols.size();
-  uint64_t* h_totals = reinterpret_cast<uint64_t*>(s->h_flags + 16);
-  if (n_scan) {
-    if ((rc = s->d_totals.ensure(8 * n_scan))) return rc;
-    for (size_t k0 = 0; k0 < n_scan; k0 += MAX_SCAN_COLS) {
-      ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = n + 1;
-      for (size_t k = k0; k < std::min(n_scan, k0 + MAX_SCAN_COLS); k++) SC.col[SC.n_cols++] = scan_cols[k];
-      if ((rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>() + k0))) return rc;
-    }
-    publish_kernel<<<1, 256, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, (int)(2 * n_scan));   // [16, 16 + 2 * 229) < 512
-    s->st.kernel_launches++;
-    CU_TRY(cudaEventRecord(s->ev_dflags, cs));
-    CU_TRY(cudaEventSynchronize(s->ev_dflags));
-    CU_TRY(cudaGetLastError());
-    for (size_t k = 0; k < n_scan; k++) {
-      ColLayout& L = cols[scan_owner[k].first];
-      const uint64_t tot = h_totals[k];
-      if (tot > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", f->fields[L.schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
-      if (scan_owner[k].second) { L.data_bytes = tot; L.data_off = AB.take((size_t)tot + 16); continue; }
-      if (L.kind == HK_Utf8) { L.data_bytes = tot; L.data_off = AB.take((size_t)tot + 16); continue; }
-      L.child_len = tot; L.child_validity = true;
-      L.child_validity_off = AB.take(4 * ((tot + 31) / 32));
-      if (L.kind == HK_ListUtf8) L.child_offsets_off = AB.take(4 * (tot + 1));
-      else { L.data_bytes = 4 * tot; L.data_off = AB.take(4 * (size_t)tot + 16); }
-    }
+  if (!counts.empty()) {
+    s->st.kernel_launches++;     // the totals publish: VCF has always counted it, the other formats never have, so both stay comparable
+    if ((rc = layout_region_b(s, S, counts, true))) return rc;
   }
-  if (AB.pos > arena.cap) {
-    // grow, keeping region A
-    DeviceBuf bigger;
-    if ((rc = bigger.ensure(AB.pos))) return rc;
-    CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, regionA, cudaMemcpyDeviceToDevice, cs));
-    CU_TRY(cudaStreamSynchronize(cs));
-    arena.release(); arena = bigger; bigger.p = nullptr; bigger.cap = 0;
-    A = arena.as<uint8_t>();
-  }
-  bind(A);
-  for (const ColLayout& L : cols) if (L.child_validity) CU_TRY(cudaMemsetAsync(A + L.child_validity_off, 0, 4 * ((L.child_len + 31) / 32), cs));
-  if (wide) vcf::vcf_write_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
+  bind(S.A);
+  for (const ColLayout& L : S.cols) if (L.child_validity) CU_TRY(cudaMemsetAsync(S.A + L.child_validity_off, 0, 4 * ((L.child_len + 31) / 32), cs));
+  if (s->cur.long_records) vcf::vcf_write_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
   else vcf::vcf_write_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
   s->st.kernel_launches++;
-  const size_t arena_bytes = AB.pos;
-  s->st.rows += n; s->st.batches++;
-  for (auto& L : cols) {
-    const bool is_var = L.kind == HK_Utf8 || L.kind >= HK_ListInt8;
-    s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var ? off_bytes + L.data_bytes : L.kind == HK_Boolean ? bm_bytes : val_bytes);
-  }
-  if ((rc = hand_off_batch(s, cs, A, cols, n, arena_bytes, err_off, row0, produced))) return rc;
-  CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
-  s->slice_pending = true;
   return BAMSCAN_OK;
 }
 
-// the next slice of the current chunk's rows: VCF has its own decode path
-static int decode_next_slice(BamScanStream* s, bool* produced) {
-  return s->f->format == FMT_VCF ? decode_slice_vcf(s, produced) : decode_slice(s, produced);
+// Decodes the next slice of the current chunk's rows into the arena and queues its hand-off (one batch).  A decode slice is queued
+// without waiting for it; its time (and, for device-resident runs, its error word) is collected when the next slice starts or the
+// partition ends (flush_slice).
+static int decode_slice(BamScanStream* s, bool* produced) {
+  NvtxRange nv("bamscan: decode slice (count, scan, write) + D2H issue");
+  cudaStream_t cs = s->cur.cs;
+  int rc;
+  if ((rc = flush_slice(s))) return rc;
+  CU_TRY(cudaEventRecord(s->ev_dt[0], cs));
+  Slice S;
+  switch (s->f->format) {
+    case FMT_BAM: case FMT_SAM: rc = decode_bam(s, S); break;
+    case FMT_FASTQ: rc = decode_fastq(s, S); break;
+    case FMT_FASTA: rc = decode_fasta(s, S); break;
+    case FMT_VCF: rc = decode_vcf(s, S); break;
+  }
+  if (rc) return rc;
+  const uint32_t n = S.n;
+  const uint64_t row0 = s->st.rows;
+  s->st.rows += n; s->st.batches++;
+  for (const ColLayout& L : S.cols) s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var(L.kind) ? 4ull * (n + 1) + L.data_bytes : fixed_bytes(L.kind, n));
+  if ((rc = hand_off_batch(s, cs, S.A, S.cols, n, S.AB.pos, S.err_off, row0, produced))) return rc;
+  CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
+  s->slice_pending = true;
+  return BAMSCAN_OK;
 }
 
 static int sam_error_to_rc(uint32_t code, unsigned long long rec) {
@@ -1490,7 +1486,7 @@ static int advance(BamScanStream* s, bool* produced) {
   BamFile* f = s->f;
   for (;;) {
     if (s->cur.pos < s->cur.n) {   // rows of the current chunk still to decode
-      int rc = decode_next_slice(s, produced);
+      int rc = decode_slice(s, produced);
       if (!rc) rc = launch_next_chunk_early(s);
       return rc ? rc : 1;
     }
@@ -1539,7 +1535,7 @@ static int advance(BamScanStream* s, bool* produced) {
     else if (s->range_stop) { s->carry_len = 0; s->range_open = false; s->range_idx++; }                      // unmapped tail: another reference began
     // first slice now (its kernels get the whole GPU: decode_slice does not wait for them), then the next chunk's inflate on the
     // other stream -- a persistent kernel that fills the SMs as the decode CTAs drain and overlaps the remaining slices
-    if (s->cur.pos < s->cur.n && (rc = decode_next_slice(s, produced))) return rc;
+    if (s->cur.pos < s->cur.n && (rc = decode_slice(s, produced))) return rc;
     if ((rc = launch_next_chunk_early(s))) return rc;
     return 1;
   }
@@ -1587,10 +1583,9 @@ static void export_batch(const BamScanStream* s, const ReadyBatch& rb, ArrowArra
   for (size_t i = 0; i < n_out; i++) {
     const ColLayout& L = rb.cols[s->out_to_dec[i]];
     ArrowArray* ch = out->children[i];
-    const bool is_list = L.kind >= HK_ListInt8, is_var = L.kind == HK_Utf8 || L.kind == HK_Binary;
     int64_t nulls = L.has_validity ? (on_device ? -1 : count_nulls(H + L.validity_off, rb.row0, rb.nrows)) : 0;
     const void* validity = (L.has_validity && nulls) ? H + L.validity_off : nullptr;
-    if (is_list) {
+    if (L.kind >= HK_ListInt8) {
       NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 2, 1);
       p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off;
       // VCF lists have nullable elements (child validity) and List<Utf8> a child with offsets; the BAM tag lists have neither
@@ -1600,7 +1595,7 @@ static void export_batch(const BamScanStream* s, const ReadyBatch& rb, ArrowArra
       cp->buffers[0] = cnulls ? H + L.child_validity_off : nullptr;
       if (utf8_items) { cp->buffers[1] = H + L.child_offsets_off; cp->buffers[2] = H + L.data_off; }
       else cp->buffers[1] = H + L.data_off;
-    } else if (is_var) {
+    } else if (is_var(L.kind)) {
       NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 3, 0);
       p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off; p->buffers[2] = H + L.data_off;
     } else {
