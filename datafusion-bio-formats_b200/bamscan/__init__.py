@@ -49,7 +49,8 @@ class _Options(C.Structure):
                 ("infer_tag_types", C.c_int32), ("infer_tag_sample_size", C.c_int32),
                 ("n_tag_type_hints", C.c_int32), ("tag_type_hints", C.POINTER(C.c_char_p)),
                 ("device_id", C.c_int32), ("batch_rows", C.c_int32), ("chunk_inflated_bytes", C.c_uint64),
-                ("segment_bytes", C.c_uint32), ("skip_crc", C.c_int32), ("debug_flags", C.c_int32), ("decode_all_tag_fields", C.c_int32)]
+                ("segment_bytes", C.c_uint32), ("skip_crc", C.c_int32), ("debug_flags", C.c_int32), ("decode_all_tag_fields", C.c_int32),
+                ("has_format_fields", C.c_int32), ("n_format_fields", C.c_int32), ("format_fields", C.POINTER(C.c_char_p))]
 
 
 class _Filter(C.Structure):
@@ -849,10 +850,15 @@ class VcfTableProvider(BamTableProvider):
     `scan` with target_partitions > 1 uses BGZF block ranges balanced by compressed bytes (a line belongs to the range that holds its
     first byte); no filter is pushed down and `limit` is not applied, as for FastqTableProvider; everything else is
     BamTableProvider's.  At most 112 INFO columns can be projected in one scan: execute raises BamScanError -5 (unsupported)
-    above that, so a header with more ##INFO fields needs info_fields or a projection."""
+    above that, so a header with more ##INFO fields needs info_fields or a projection.
+
+    format_fields: FORMAT IDs, each a column format_<ID> behind the INFO columns holding one element per sample (header sample
+    order): Number=1 gives List<Int32 / Float32 / Utf8>, any other Number on Integer / Float gives List<List<Int32 / Float32>>;
+    GT stays text.  Unlike info_fields, None (the default) selects NO FORMAT column, and so does [], so a scan without it reads
+    the file exactly as before.  The rules are in bamscan.h (bamscan_open_vcf) and oracle/vcf_format_oracle.py."""
 
     def __init__(self, file_path, info_fields=None, object_storage_options=None, coordinate_system_zero_based=True, *, device_id=0,
-                 batch_rows=0, chunk_inflated_bytes=0, skip_crc=False, debug_flags=0):
+                 batch_rows=0, chunk_inflated_bytes=0, skip_crc=False, debug_flags=0, format_fields=None):
         if object_storage_options is not None:
             raise BamScanError(-5, "remote object storage is out of scope for this build (local files only)")
         L = load_library()
@@ -869,6 +875,11 @@ class VcfTableProvider(BamTableProvider):
         o.chunk_inflated_bytes = chunk_inflated_bytes
         o.skip_crc = int(skip_crc)
         o.debug_flags = debug_flags
+        o.has_format_fields = int(format_fields is not None)
+        self._fmt_arr, self._fmt_enc = _strs(list(format_fields or []))
+        o.n_format_fields = len(format_fields or [])
+        if self._fmt_arr is not None:
+            o.format_fields = self._fmt_arr
         self._h = C.c_void_p()
         _check(L.bamscan_open_vcf(str(file_path).encode(), C.byref(o), C.byref(self._h)))
         self.file_path = str(file_path)

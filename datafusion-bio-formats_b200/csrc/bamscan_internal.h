@@ -18,7 +18,8 @@ enum : int32_t {
   HK_Int32 = 1, HK_UInt32 = 2, HK_Float32 = 3, HK_Utf8 = 4, HK_Binary = 5,
   HK_Boolean = 6,                                             // VCF Flag columns only
   HK_ListInt8 = 10, HK_ListUInt8 = 11, HK_ListInt16 = 12, HK_ListUInt16 = 13, HK_ListInt32 = 14, HK_ListUInt32 = 15, HK_ListFloat32 = 16,
-  HK_ListUtf8 = 17                                            // VCF String / Character lists only
+  HK_ListUtf8 = 17,                                           // VCF String / Character lists only
+  HK_ListListInt32 = 18, HK_ListListFloat32 = 19              // VCF FORMAT columns with Number other than 1: List<List<...>>
 };
 
 struct TagDef { std::string tag; char sam_type; int32_t kind; std::string description; };
@@ -113,6 +114,12 @@ struct BamFile {
   // VCF: the header's ##INFO lines, in header order (Number, Type and Description as written)
   struct VcfInfo { std::string id, number, type, description; };
   std::vector<VcfInfo> vcf_info;
+  // VCF FORMAT: the selected IDs (BamScanOptions.format_fields; empty selects none), the ##FORMAT lines and the sample names (read
+  // only when an ID is selected), and the schema index behind the last INFO column (FORMAT columns follow it)
+  std::vector<std::string> format_fields;
+  std::vector<VcfInfo> vcf_format;
+  std::vector<std::string> vcf_samples;
+  int32_t vcf_info_end = 0;
 };
 
 // genomic_filter.rs:16-32

@@ -21,6 +21,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <functional>
 #include <numeric>
 #include <cstdio>
 #include <cstring>
@@ -38,6 +39,7 @@
 #include "kernels_fasta.cuh"
 #include "kernels_sam.cuh"
 #include "kernels_vcf.cuh"
+#include "kernels_vcf_format.cuh"
 
 namespace bamscan {
 
@@ -192,6 +194,11 @@ struct ColLayout {
   uint64_t child_len = 0;       // list child element count
   bool child_validity = false;  // VCF lists: the child has a validity bitmap (child_validity_off)
   size_t child_validity_off = 0, child_offsets_off = 0;   // List<Utf8>: child_offsets_off holds the child's offsets
+  // VCF FORMAT List<List<...>>: the child is the middle list (child_validity_off, child_offsets_off), the leaves have their own
+  // validity and their values at data_off
+  uint64_t leaf_len = 0;
+  size_t leaf_validity_off = 0;
+  uint64_t elem_bytes = 0;      // VCF FORMAT: the bytes of the element and leaf buffers that data_bytes does not count
 };
 
 struct ChunkPlan { uint32_t b0 = 0, b1 = 0; uint64_t c0 = 0, c1 = 0, u0 = 0, ubytes = 0; bool extension = false; };
@@ -238,6 +245,7 @@ struct BamScanStream {
   uint32_t headroom = HEADROOM, desc_base[2] = {HEADROOM, HEADROOM};
   bool fa_lead_nl = true;     // FASTA: the byte in front of the next chunk is a '\n' (its first byte starts a line)
   bool fa_leading = false;    // FASTA: the range owns the file's first byte and no '>' was found yet
+  int n_format = 0;           // VCF: projected FORMAT columns
   // unique decoded columns
   std::vector<int32_t> dec_cols;          // schema indices, unique
   std::vector<int32_t> out_to_dec;        // projection position -> index into dec_cols
@@ -424,7 +432,11 @@ static int stream_init(BamScanStream* s) {
   }
   if (f->format == FMT_VCF) {
     int n_info = 0;
-    for (int32_t c : s->dec_cols) if (c >= 8) n_info++;          // INFO columns follow the eight fixed ones
+    s->n_format = 0;
+    for (int32_t c : s->dec_cols) {                               // INFO columns follow the eight fixed ones, FORMAT columns them
+      if (c >= f->vcf_info_end) s->n_format++;
+      else if (c >= 8) n_info++;
+    }
     if (n_info > vcf::MAX_INFO) { set_error("more than %d projected INFO columns are not supported by this build", vcf::MAX_INFO); return BAMSCAN_ERR_UNSUPPORTED; }
     return BAMSCAN_OK;
   }
@@ -484,6 +496,7 @@ static uint32_t inflate_wave_members(int device) { return (uint32_t)device_sms(d
 // inflated (Arrow offsets are i32).  Default: one whole inflate wave per chunk (a member takes milliseconds, so a chunk
 // that is not a whole number of waves leaves most of the GPU idle in its last wave); chunk_inflated_bytes overrides it.
 static const uint64_t SLICE_BYTES = 768ull << 20;
+static const uint64_t FMT_SLICE_ELEMS = 1ull << 24;
 static uint64_t chunk_cap_bytes(const BamFile& f) {
   if (f.chunk_bytes) return f.chunk_bytes;
   if (f.format == FMT_SAM) return 512ull << 20;    // SAM: text bytes per chunk (no inflate wave to fill)
@@ -698,11 +711,14 @@ struct Slice {
   size_t err_off = 0, region_a = 0;
   uint8_t* A = nullptr;            // s->d_arena[s->arena_flip]
 };
-struct CountCol { int32_t* counts; size_t col; };   // a count column, scanned in place, and its index in Slice::cols
+struct CountCol { int32_t* counts; size_t col; uint32_t len = 0; };   // a count column, scanned in place, its index in Slice::cols, and
+                                                                      // its entries (0: the slice's rows + 1)
 
 // Region A of an n-row slice, in an arena that holds it (a first sizing guess, grown by layout_region_b), with the error word
-// cleared.  has_validity: the format's rule for which columns carry a validity bitmap.
-static int layout_region_a(BamScanStream* s, Slice& S, uint32_t n, bool (*has_validity)(const BamFile&, int32_t)) {
+// cleared.  has_validity: the format's rule for which columns carry a validity bitmap; more (optional): buffers of a column whose
+// sizes the row count decides besides its validity and offsets or values.
+static int layout_region_a(BamScanStream* s, Slice& S, uint32_t n, bool (*has_validity)(const BamFile&, int32_t),
+                           const std::function<void(ColLayout&)>& more = nullptr) {
   S.n = n;
   S.err_off = S.AB.take(64);
   S.cols.resize(s->dec_cols.size());
@@ -711,6 +727,7 @@ static int layout_region_a(BamScanStream* s, Slice& S, uint32_t n, bool (*has_va
     L.has_validity = has_validity(*s->f, L.schema_idx);
     if (L.has_validity) L.validity_off = S.AB.take(4ull * ((n + 31) / 32));
     if (is_var(L.kind)) L.offsets_off = S.AB.take(4ull * (n + 1)); else L.values_off = S.AB.take(fixed_bytes(L.kind, n));
+    if (more) more(L);
   }
   S.region_a = S.AB.pos;
   DeviceBuf& arena = s->d_arena[s->arena_flip];
@@ -727,30 +744,36 @@ static std::vector<CountCol> offset_counts(const Slice& S) {
   return counts;
 }
 
-// Count columns -> Arrow offsets, in launches of up to MAX_SCAN_COLS columns.  The totals reach the host through the mapped flags
-// page at [16, 16 + 2 * counts) (VCF's 229 at most stay below the decode error words at [512, 516)) with one host sync, and each is
-// held to Arrow's 2^31-1 limit.  Region B then takes per column its data: the total's bytes (Utf8, Binary) or, for a list, the
-// child validity words when list_child_validity (VCF; BAM tag lists have none), then the child values, or for List<Utf8> the
-// child offsets and the bytes the next count column totals.  The arena grows when region B does not fit, keeping region A; the
-// format binds its kernels again afterwards.
-static int layout_region_b(BamScanStream* s, Slice& S, const std::vector<CountCol>& counts, bool list_child_validity) {
+// Count columns -> Arrow offsets, in launches of up to MAX_SCAN_COLS columns of equal length.  The totals reach the host through the
+// mapped flags page at [16, 16 + 2 * counts) (VCF's 229 INFO and 16 FORMAT columns at most stay below the decode error words at
+// [512, 516)) with one host sync, and each is held to Arrow's 2^31-1 limit.  *T: the totals, in the order of counts.
+static int scan_counts(BamScanStream* s, const Slice& S, const std::vector<CountCol>& counts, const uint64_t** T) {
   cudaStream_t cs = s->cur.cs;
   const size_t n_scan = counts.size();
   int rc;
   if ((rc = s->d_totals.ensure(8 * n_scan))) return rc;
-  for (size_t k0 = 0; k0 < n_scan; k0 += MAX_SCAN_COLS) {
-    ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = S.n + 1;
-    for (size_t k = k0; k < std::min(n_scan, k0 + MAX_SCAN_COLS); k++) SC.col[SC.n_cols++] = counts[k].counts;
+  for (size_t k0 = 0; k0 < n_scan;) {
+    ScanCols SC; memset(&SC, 0, sizeof SC); SC.n = counts[k0].len ? counts[k0].len : S.n + 1;
+    size_t k = k0;
+    for (; k < n_scan && k < k0 + MAX_SCAN_COLS && (counts[k].len ? counts[k].len : S.n + 1) == SC.n; k++) SC.col[SC.n_cols++] = counts[k].counts;
     if ((rc = launch_offsets_scan(s, cs, SC, s->d_tiles, s->d_totals.as<uint64_t>() + k0))) return rc;
+    k0 = k;
   }
   publish_kernel<<<1, 256, 0, cs>>>(s->d_totals.as<uint32_t>(), s->d_hflags + 16, (int)(2 * n_scan));
   CU_TRY(cudaEventRecord(s->ev_dflags, cs));
   CU_TRY(cudaEventSynchronize(s->ev_dflags));
   CU_TRY(cudaGetLastError());
-  const uint64_t* T = reinterpret_cast<const uint64_t*>(s->h_flags + 16);
+  *T = reinterpret_cast<const uint64_t*>(s->h_flags + 16);
   for (size_t k = 0; k < n_scan; k++)
-    if (T[k] > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", s->f->fields[S.cols[counts[k].col].schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
-  for (size_t k = 0; k < n_scan; k++) {
+    if ((*T)[k] > 0x7fffffffull) { set_error("column '%s' exceeds 2^31-1 bytes in one batch; lower chunk_inflated_bytes", s->f->fields[S.cols[counts[k].col].schema_idx].name.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
+  return BAMSCAN_OK;
+}
+
+// Region B per count column: the total's bytes (Utf8, Binary) or, for a list, the child validity words when list_child_validity
+// (VCF; BAM tag lists have none), then the child values, or for List<Utf8> the child offsets and the bytes the next count column
+// totals.
+static void layout_counts(Slice& S, const std::vector<CountCol>& counts, const uint64_t* T, bool list_child_validity) {
+  for (size_t k = 0; k < counts.size(); k++) {
     ColLayout& L = S.cols[counts[k].col];
     uint64_t bytes = T[k];
     if (L.kind >= HK_ListInt8) {
@@ -762,16 +785,28 @@ static int layout_region_b(BamScanStream* s, Slice& S, const std::vector<CountCo
     L.data_bytes = bytes;
     L.data_off = S.AB.take((size_t)bytes + 16);
   }
+}
+
+// The arena grows when region B does not fit, keeping region A; the format binds its kernels again afterwards.
+static int fit_region_b(BamScanStream* s, Slice& S) {
   DeviceBuf& arena = s->d_arena[s->arena_flip];
   if (S.AB.pos > arena.cap) {
     DeviceBuf bigger;
-    if ((rc = bigger.ensure(S.AB.pos))) return rc;
-    CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, S.region_a, cudaMemcpyDeviceToDevice, cs));
-    CU_TRY(cudaStreamSynchronize(cs));
+    if (int rc = bigger.ensure(S.AB.pos)) return rc;
+    CU_TRY(cudaMemcpyAsync(bigger.p, arena.p, S.region_a, cudaMemcpyDeviceToDevice, s->cur.cs));
+    CU_TRY(cudaStreamSynchronize(s->cur.cs));
     arena.release(); arena = bigger;
     S.A = arena.as<uint8_t>();
   }
   return BAMSCAN_OK;
+}
+
+// Count columns -> Arrow offsets, then region B laid out behind region A
+static int layout_region_b(BamScanStream* s, Slice& S, const std::vector<CountCol>& counts, bool list_child_validity) {
+  const uint64_t* T = nullptr;
+  if (int rc = scan_counts(s, S, counts, &T)) return rc;
+  layout_counts(S, counts, T, list_child_validity);
+  return fit_region_b(s, S);
 }
 
 // FASTQ: fq_lengths -> scan -> fq_copy.  name, description, sequence and quality_scores (schema 0-3) are Utf8; description is the
@@ -910,7 +945,9 @@ static int decode_bam(BamScanStream* s, Slice& S) {
 }
 
 // VCF: vcf_fields -> vcf_rows -> scan -> vcf_write (kernels_vcf.cuh).  The count columns are the Utf8 bytes and list elements, and
-// for List<Utf8> also the elements' bytes.
+// for List<Utf8> also the elements' bytes.  Projected FORMAT columns add vcf_samples and vcf_values in front of the scan and
+// vcf_fmt_write behind it (kernels_vcf_format.cuh); their count columns are element-level (n * S + 1 entries) and share the
+// scan's host sync.
 static int decode_vcf(BamScanStream* s, Slice& S) {
   const BamFile* f = s->f;
   cudaStream_t cs = s->cur.cs;
@@ -918,12 +955,25 @@ static int decode_vcf(BamScanStream* s, Slice& S) {
   const uint32_t* lines = s->cur.recoff + s->cur.pos;
   s->cur.pos += n;
   int rc;
-  if ((rc = layout_region_a(s, S, n, [](const BamFile& file, int32_t c) { return file.fields[c].nullable; }))) return rc;
+  const int32_t info_end = f->vcf_info_end;
+  const uint32_t n_smp = (uint32_t)f->vcf_samples.size();
+  const uint64_t nel = (uint64_t)n * n_smp;          // FORMAT elements (< 2^31: run_chunk cuts the slices so)
+  // FORMAT columns: besides their outer offsets, region A holds the element validity and the Int32 / Float32 values or the
+  // element counts (-> offsets) of Utf8 and nested columns, all sized by n * S
+  auto fmt_elems = [&](ColLayout& L) {
+    if (L.schema_idx < info_end) return;
+    L.child_validity = true; L.child_len = nel;
+    L.child_validity_off = S.AB.take(4 * ((nel + 31) / 32));
+    L.elem_bytes = (nel + 7) / 8;
+    if (L.kind == HK_ListInt32 || L.kind == HK_ListFloat32) { L.data_bytes = 4 * nel; L.data_off = S.AB.take(4 * nel + 16); }
+    else { L.child_offsets_off = S.AB.take(4 * (nel + 1)); L.elem_bytes += 4 * (nel + 1); }
+  };
+  if ((rc = layout_region_a(s, S, n, [](const BamFile& file, int32_t c) { return file.fields[c].nullable; }, fmt_elems))) return rc;
   const size_t n_dec = S.cols.size();
   // keys: the projected INFO IDs (key k is INFO column k), then END unless it is one of them
   std::vector<int> info_col(n_dec, -1);           // column -> INFO column (key) index
   std::vector<std::string> keys;
-  for (size_t i = 0; i < n_dec; i++) if (S.cols[i].schema_idx >= 8) { info_col[i] = (int)keys.size(); keys.push_back(f->fields[S.cols[i].schema_idx].name); }
+  for (size_t i = 0; i < n_dec; i++) if (S.cols[i].schema_idx >= 8 && S.cols[i].schema_idx < info_end) { info_col[i] = (int)keys.size(); keys.push_back(f->fields[S.cols[i].schema_idx].name); }
   const int n_info = (int)keys.size();
   int end_key = (int)(std::find(keys.begin(), keys.end(), std::string("END")) - keys.begin());
   if (end_key == (int)keys.size()) keys.push_back("END");
@@ -947,9 +997,41 @@ static int decode_vcf(BamScanStream* s, Slice& S) {
   size_t scratch = o_blen;
   std::vector<size_t> blen_off(n_dec, 0);
   for (size_t i = 0; i < n_dec; i++) if (S.cols[i].kind == HK_ListUtf8) { blen_off[i] = scratch; scratch += align_up(4ull * (n + 1), 256); }
+  // FORMAT scratch: the sample starts and the per-line key map
+  const size_t o_samp = align_up(scratch, 256), o_frow = o_samp + align_up(4 * nel, 256);
+  std::vector<size_t> fmt_cols;                   // FORMAT column c -> index into S.cols
+  for (size_t i = 0; i < n_dec; i++) if (S.cols[i].schema_idx >= info_end) fmt_cols.push_back(i);
+  if (!fmt_cols.empty()) scratch = o_frow + sizeof(vcf::FmtRow) * n;
   if ((rc = s->d_scratch.ensure(scratch + 256))) return rc;
   uint8_t* SCR = s->d_scratch.as<uint8_t>();
+  std::unique_ptr<vcf::FormatParams> FP;
+  if (!fmt_cols.empty()) {
+    FP.reset(new vcf::FormatParams());
+    memset(FP.get(), 0, sizeof(vcf::FormatParams));
+    uint32_t blob = 0;
+    for (size_t c = 0; c < fmt_cols.size(); c++) {
+      const std::string id = f->fields[S.cols[fmt_cols[c]].schema_idx].name.substr(7);     // behind "format_"
+      if (blob + id.size() > (size_t)vcf::FMT_BLOB) { set_error("the projected FORMAT IDs exceed %d bytes, which is not supported by this build", vcf::FMT_BLOB); return BAMSCAN_ERR_UNSUPPORTED; }
+      FP->off[c] = (uint16_t)blob;
+      memcpy(FP->blob + blob, id.data(), id.size()); blob += (uint32_t)id.size();
+    }
+    FP->off[fmt_cols.size()] = (uint16_t)blob;
+  }
   auto bind = [&](uint8_t* A) {
+    if (FP) {
+      vcf::FormatParams& F = *FP;
+      F.U = s->cur.U; F.lines = lines; F.rows = reinterpret_cast<const vcf::Row*>(SCR); F.n = n; F.S = n_smp; F.nf = (int32_t)fmt_cols.size();
+      F.samp = reinterpret_cast<uint32_t*>(SCR + o_samp); F.frow = reinterpret_cast<vcf::FmtRow*>(SCR + o_frow);
+      F.err = reinterpret_cast<uint32_t*>(A + S.err_off);
+      for (size_t c = 0; c < fmt_cols.size(); c++) {
+        const ColLayout& L = S.cols[fmt_cols[c]];
+        vcf::FmtCol& C = F.cols[c];
+        C.kind = L.kind; C.offs = reinterpret_cast<int32_t*>(A + L.offsets_off); C.valid = reinterpret_cast<uint32_t*>(A + L.child_validity_off);
+        if (L.kind == HK_ListInt32 || L.kind == HK_ListFloat32) C.values = reinterpret_cast<uint32_t*>(A + L.data_off);
+        else { C.counts = reinterpret_cast<int32_t*>(A + L.child_offsets_off); C.data = L.data_off ? A + L.data_off : nullptr; }
+        if (L.leaf_validity_off) C.lvalid = reinterpret_cast<uint32_t*>(A + L.leaf_validity_off);
+      }
+    }
     P->U = s->cur.U; P->lines = lines; P->n = n; P->zero_based = f->zero_based; P->n_info = n_info;
     P->rows = reinterpret_cast<vcf::Row*>(SCR); P->err = reinterpret_cast<uint32_t*>(A + S.err_off);
     for (size_t k = 0; k < keys.size(); k++) P->cols[k].tok = reinterpret_cast<uint2*>(SCR + o_tok) + (size_t)k * n;
@@ -967,6 +1049,7 @@ static int decode_vcf(BamScanStream* s, Slice& S) {
         case 6: P->qual = c.vals; P->v_qual = c.valid; break;
         case 7: P->l_filter = c.offs; P->v_filter = c.valid; P->d_filter = d; break;
         default: {
+          if (L.schema_idx >= info_end) break;      // (FORMAT: FP)
           vcf::InfoCol& C = P->cols[info_col[i]];
           C.kind = L.kind; C.valid = c.valid; C.data = c.data;
           if (is_var(L.kind)) C.lens = c.offs; else C.values = c.vals;
@@ -983,21 +1066,44 @@ static int decode_vcf(BamScanStream* s, Slice& S) {
   else vcf::vcf_fields_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
   vcf::vcf_rows_kernel<<<(n + 255) / 256, 256, 0, cs>>>(*P);
   s->st.kernel_launches += 2;
+  if (FP) {
+    if (s->cur.long_records) vcf::vcf_samples_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*FP);
+    else vcf::vcf_samples_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*FP);
+    vcf::vcf_values_kernel<<<(uint32_t)((nel + 255) / 256), 256, 0, cs>>>(*FP);
+    s->st.kernel_launches += 2;
+  }
   std::vector<CountCol> counts;
   for (size_t i = 0; i < n_dec; i++) {
-    if (!is_var(S.cols[i].kind)) continue;
+    if (!is_var(S.cols[i].kind) || S.cols[i].schema_idx >= info_end) continue;
     counts.push_back({reinterpret_cast<int32_t*>(S.A + S.cols[i].offsets_off), i});
     if (S.cols[i].kind == HK_ListUtf8) counts.push_back({reinterpret_cast<int32_t*>(SCR + blen_off[i]), i});
   }
+  const size_t n_info_counts = counts.size();
+  for (size_t i : fmt_cols)
+    if (S.cols[i].kind != HK_ListInt32 && S.cols[i].kind != HK_ListFloat32) counts.push_back({reinterpret_cast<int32_t*>(S.A + S.cols[i].child_offsets_off), i, (uint32_t)nel + 1u});
   if (!counts.empty()) {
     s->st.kernel_launches++;     // the totals publish: VCF has always counted it, the other formats never have, so both stay comparable
-    if ((rc = layout_region_b(s, S, counts, true))) return rc;
+    const uint64_t* T = nullptr;
+    if ((rc = scan_counts(s, S, counts, &T))) return rc;
+    layout_counts(S, std::vector<CountCol>(counts.begin(), counts.begin() + n_info_counts), T, true);
+    for (size_t k = n_info_counts; k < counts.size(); k++) {
+      // FORMAT: Utf8 bytes, or the leaves of a nested column (validity, values)
+      ColLayout& L = S.cols[counts[k].col];
+      if (L.kind == HK_ListUtf8) L.data_bytes = T[k];
+      else { L.leaf_len = T[k]; L.leaf_validity_off = S.AB.take(4 * ((T[k] + 31) / 32)); L.elem_bytes += (T[k] + 7) / 8; L.data_bytes = 4 * T[k]; }
+      L.data_off = S.AB.take((size_t)L.data_bytes + 16);
+    }
+    if ((rc = fit_region_b(s, S))) return rc;
   }
   bind(S.A);
-  for (const ColLayout& L : S.cols) if (L.child_validity) CU_TRY(cudaMemsetAsync(S.A + L.child_validity_off, 0, 4 * ((L.child_len + 31) / 32), cs));
+  for (const ColLayout& L : S.cols) {
+    if (L.child_validity && L.schema_idx < info_end) CU_TRY(cudaMemsetAsync(S.A + L.child_validity_off, 0, 4 * ((L.child_len + 31) / 32), cs));
+    if (L.leaf_validity_off) CU_TRY(cudaMemsetAsync(S.A + L.leaf_validity_off, 0, 4 * ((L.leaf_len + 31) / 32), cs));
+  }
   if (s->cur.long_records) vcf::vcf_write_kernel<32><<<(uint32_t)(((uint64_t)n * 32 + 255) / 256), 256, 0, cs>>>(*P);
   else vcf::vcf_write_kernel<8><<<(uint32_t)(((uint64_t)n * 8 + 255) / 256), 256, 0, cs>>>(*P);
   s->st.kernel_launches++;
+  if (FP) { vcf::vcf_fmt_write_kernel<<<(uint32_t)((nel + 255) / 256), 256, 0, cs>>>(*FP); s->st.kernel_launches++; }
   return BAMSCAN_OK;
 }
 
@@ -1021,7 +1127,7 @@ static int decode_slice(BamScanStream* s, bool* produced) {
   const uint32_t n = S.n;
   const uint64_t row0 = s->st.rows;
   s->st.rows += n; s->st.batches++;
-  for (const ColLayout& L : S.cols) s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var(L.kind) ? 4ull * (n + 1) + L.data_bytes : fixed_bytes(L.kind, n));
+  for (const ColLayout& L : S.cols) s->st.arrow_bytes += (L.has_validity ? (n + 7) / 8 : 0) + (is_var(L.kind) ? 4ull * (n + 1) + L.data_bytes : fixed_bytes(L.kind, n)) + L.elem_bytes;
   if ((rc = hand_off_batch(s, cs, S.A, S.cols, n, S.AB.pos, S.err_off, row0, produced))) return rc;
   CU_TRY(cudaEventRecord(s->ev_dt[1], cs));
   s->slice_pending = true;
@@ -1430,6 +1536,9 @@ static int run_chunk(BamScanStream* s, const ChunkPlan& c, const ScanRange& rang
     const uint32_t n_slices = (uint32_t)std::max<uint64_t>(1, (c.ubytes + SLICE_BYTES - 1) / SLICE_BYTES);
     s->cur.U = U_rows; s->cur.recoff = d_recoff; s->cur.n = n; s->cur.pos = 0; s->cur.cs = cs;
     s->cur.rows_per_slice = (n + n_slices - 1) / n_slices;
+    // VCF FORMAT columns: at most FMT_SLICE_ELEMS elements (rows * samples) per slice, which keeps them below 2^31 and bounds the
+    // per-element buffers
+    if (s->n_format) s->cur.rows_per_slice = std::min<uint32_t>(s->cur.rows_per_slice, std::max<uint64_t>(1, FMT_SLICE_ELEMS / f->vcf_samples.size()));
     s->mean_record_bytes = (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)(data_hi - H) / std::max<uint32_t>(n_rec, 1));
     s->cur.long_records = (f->debug_flags & 2) || s->mean_record_bytes > 2048;
     s->cur.ubytes = c.ubytes / n_slices + (H / 4);
@@ -1585,7 +1694,17 @@ static void export_batch(const BamScanStream* s, const ReadyBatch& rb, ArrowArra
     ArrowArray* ch = out->children[i];
     int64_t nulls = L.has_validity ? (on_device ? -1 : count_nulls(H + L.validity_off, rb.row0, rb.nrows)) : 0;
     const void* validity = (L.has_validity && nulls) ? H + L.validity_off : nullptr;
-    if (L.kind >= HK_ListInt8) {
+    if (L.kind == HK_ListListInt32 || L.kind == HK_ListListFloat32) {
+      // VCF FORMAT List<List<...>>: outer offsets; middle validity and offsets; leaf validity and values
+      NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 2, 1);
+      p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off;
+      const int64_t mnulls = on_device ? -1 : count_nulls(H + L.child_validity_off, 0, L.child_len);
+      NodePriv* mp = new_node(ch->children[0], rb.owner, (int64_t)L.child_len, mnulls, 0, 2, 1);
+      mp->buffers[0] = mnulls ? H + L.child_validity_off : nullptr; mp->buffers[1] = H + L.child_offsets_off;
+      const int64_t lnulls = on_device ? -1 : count_nulls(H + L.leaf_validity_off, 0, L.leaf_len);
+      NodePriv* lp = new_node(ch->children[0]->children[0], rb.owner, (int64_t)L.leaf_len, lnulls, 0, 2, 0);
+      lp->buffers[0] = lnulls ? H + L.leaf_validity_off : nullptr; lp->buffers[1] = H + L.data_off;
+    } else if (L.kind >= HK_ListInt8) {
       NodePriv* p = new_node(ch, rb.owner, (int64_t)rb.nrows, nulls, (int64_t)rb.row0, 2, 1);
       p->buffers[0] = validity; p->buffers[1] = H + L.offsets_off;
       // VCF lists have nullable elements (child validity) and List<Utf8> a child with offsets; the BAM tag lists have neither
@@ -1634,6 +1753,10 @@ static int decode_error_to_rc(uint32_t code, uint32_t row, uint64_t row0) {
     case vcf::VCF_ERR_VALUE: set_error("VCF read error: record %llu of the partition (0-based): an INFO value does not parse as its declared type", prow); return BAMSCAN_ERR_SCHEMA;
     case vcf::VCF_ERR_POS0: set_error("VCF read error: record %llu of the partition (0-based): POS 0 (a telomere) is not supported by this build", prow); return BAMSCAN_ERR_UNSUPPORTED;
     case vcf::VCF_ERR_LONG: set_error("VCF read error: record %llu of the partition (0-based): a line longer than %u bytes is not supported", prow, vcf::MAX_LINE); return BAMSCAN_ERR_UNSUPPORTED;
+    case vcf::VCF_ERR_FMT_FIELDS: set_error("VCF read error: record %llu of the partition (0-based): the line does not have 9 + samples fields", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_FMT_DUP: set_error("VCF read error: record %llu of the partition (0-based): a FORMAT key is given twice", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_FMT_MANY: set_error("VCF read error: record %llu of the partition (0-based): a sample has more values than the FORMAT field has keys", prow); return BAMSCAN_ERR_FORMAT;
+    case vcf::VCF_ERR_FMT_VALUE: set_error("VCF read error: record %llu of the partition (0-based): a FORMAT value does not parse as its declared type", prow); return BAMSCAN_ERR_SCHEMA;
     case FA_ERR_TOO_LONG: set_error("FASTA read error: record %llu of the partition (0-based) is larger than %llu bytes, which is not supported", prow, (unsigned long long)FA_MAX_RECORD); return BAMSCAN_ERR_UNSUPPORTED;
   }
   set_error("decode error %u at record %u", code, row);
@@ -1702,6 +1825,8 @@ static int bamscan_open_impl(const char* path, const char* index_path_or_null, c
   f.zero_based = opt.coordinate_system_zero_based != 0; f.binary_cigar = opt.binary_cigar != 0;
   f.has_tag_fields = opt.has_tag_fields != 0;
   for (int i = 0; i < opt.n_tag_fields && opt.tag_fields; i++) f.tag_fields.push_back(opt.tag_fields[i]);
+  if (format == FMT_VCF && opt.has_format_fields)
+    for (int i = 0; i < opt.n_format_fields && opt.format_fields; i++) f.format_fields.push_back(opt.format_fields[i] ? opt.format_fields[i] : "");
   f.batch_rows = opt.batch_rows;
   if (opt.chunk_inflated_bytes) f.chunk_bytes = std::min<uint64_t>(opt.chunk_inflated_bytes, 768ull << 20);   // an explicit size is also the slice size
   if (opt.segment_bytes) { f.seg_bytes = std::max<uint32_t>(256, opt.segment_bytes); f.seg_bytes_set = true; }

@@ -261,10 +261,11 @@ static int infer_tag_types_sam(const BamFile& f, const std::vector<std::string>&
 }
 
 // ---- VCF header ----
-// One ##INFO=<...> line -> *out.  Values may be quoted ("..." with \" and \\ escapes), so a quoted Description may hold ',' '=' '>'.
-// Keys other than ID, Number, Type and Description are skipped.  false: the line does not parse (or lacks ID, Number or Type).
-static bool vcf_info_line(const std::string& line, BamFile::VcfInfo* out) {
-  size_t k = 8;                                   // behind "##INFO=<"
+// One ##INFO=<...> or ##FORMAT=<...> line (prefix: the bytes in front of the first key) -> *out.  Values may be quoted ("..." with
+// \" and \\ escapes), so a quoted Description may hold ',' '=' '>'.  Keys other than ID, Number, Type and Description are skipped.
+// false: the line does not parse (or lacks ID, Number or Type).
+static bool vcf_info_line(const std::string& line, size_t prefix, BamFile::VcfInfo* out) {
+  size_t k = prefix;
   bool has_id = false, has_num = false, has_type = false;
   for (;;) {
     const size_t eq = line.find('=', k);
@@ -313,9 +314,17 @@ static int load_vcf_header(BamFile* f) {
     if (line_no == 0 && line.compare(0, 16, "##fileformat=VCF") != 0) { set_error("%s: not a VCF file (the first line is not ##fileformat=VCF...)", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
     f->text += line; f->text += '\n';
     if (line.compare(0, 2, "##") == 0) {
+      if (line.compare(0, 10, "##FORMAT=<") == 0 && !f->format_fields.empty()) {
+        BamFile::VcfInfo fmt;
+        if (!vcf_info_line(line, 10, &fmt)) { set_error("%s: malformed ##FORMAT header line: %s", f->path.c_str(), line.c_str()); return BAMSCAN_ERR_FORMAT; }
+        for (const auto& o : f->vcf_format)
+          if (o.id == fmt.id) { set_error("%s: FORMAT field '%s' is declared twice in the header", f->path.c_str(), fmt.id.c_str()); return BAMSCAN_ERR_FORMAT; }
+        f->vcf_format.push_back(fmt);
+        continue;
+      }
       if (line.compare(0, 8, "##INFO=<") != 0) continue;
       BamFile::VcfInfo info;
-      if (!vcf_info_line(line, &info)) { set_error("%s: malformed ##INFO header line: %s", f->path.c_str(), line.c_str()); return BAMSCAN_ERR_FORMAT; }
+      if (!vcf_info_line(line, 8, &info)) { set_error("%s: malformed ##INFO header line: %s", f->path.c_str(), line.c_str()); return BAMSCAN_ERR_FORMAT; }
       for (const auto& o : f->vcf_info)
         if (o.id == info.id) { set_error("%s: INFO field '%s' is declared twice in the header", f->path.c_str(), info.id.c_str()); return BAMSCAN_ERR_FORMAT; }
       f->vcf_info.push_back(info);
@@ -323,6 +332,18 @@ static int load_vcf_header(BamFile* f) {
     }
     const size_t n = sizeof kChrom - 1;
     if (line.compare(0, n, kChrom) != 0 || (line.size() > n && line[n] != '\t')) { set_error("%s: VCF header without a #CHROM line", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
+    if (!f->format_fields.empty() && line.size() > n) {
+      // the sample names: the fields behind FORMAT
+      std::vector<std::string> extra;
+      for (size_t a = n + 1;;) {
+        const size_t t = line.find('\t', a);
+        extra.push_back(line.substr(a, t == std::string::npos ? std::string::npos : t - a));
+        if (t == std::string::npos) break;
+        a = t + 1;
+      }
+      if (extra[0] != "FORMAT") { set_error("%s: the #CHROM line has fields behind INFO but the first one is not FORMAT", f->path.c_str()); return BAMSCAN_ERR_FORMAT; }
+      f->vcf_samples.assign(extra.begin() + 1, extra.end());
+    }
     f->first_record_uoff = hs.uoff();
     f->header_ok = true;
     return BAMSCAN_OK;

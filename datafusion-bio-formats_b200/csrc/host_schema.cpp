@@ -262,6 +262,53 @@ int build_vcf_schema(BamFile* f, const BamScanOptions* opt) {
     fd.metadata = {{"bio.vcf.info.number", d->number}, {"bio.vcf.info.type", d->type}, {"bio.vcf.info.description", d->description}};
     f->fields.push_back(fd);
   }
+  f->vcf_info_end = (int32_t)f->fields.size();
+  // FORMAT columns (format_fields; none when empty): format_<ID>, one element per sample
+  const std::vector<std::string>& ff = f->format_fields;
+  if (ff.empty()) return BAMSCAN_OK;
+  if (ff.size() > 16) { set_error("more than 16 FORMAT fields (%zu) are not supported by this build", ff.size()); return BAMSCAN_ERR_UNSUPPORTED; }
+  if (f->vcf_samples.empty()) { set_error("FORMAT field '%s' is selected but the VCF header has no samples", ff[0].c_str()); return BAMSCAN_ERR_SCHEMA; }
+  for (size_t i = 0; i < ff.size(); i++) {
+    const BamFile::VcfInfo* d = nullptr;
+    for (const auto& x : f->vcf_format) if (x.id == ff[i]) { d = &x; break; }
+    if (!d) { set_error("FORMAT field '%s' is not declared in the VCF header", ff[i].c_str()); return BAMSCAN_ERR_SCHEMA; }
+    if (std::find(ff.begin(), ff.begin() + i, ff[i]) != ff.begin() + i) { set_error("FORMAT field '%s' is selected twice", ff[i].c_str()); return BAMSCAN_ERR_SCHEMA; }
+    int32_t kind;
+    if (d->type == "Integer") kind = HK_ListInt32;
+    else if (d->type == "Float") kind = HK_ListFloat32;
+    else if (d->type == "String" || d->type == "Character") kind = HK_ListUtf8;
+    else if (d->type == "Flag") { set_error("FORMAT field '%s' has Type=Flag, which a FORMAT field cannot have", d->id.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    else { set_error("FORMAT field '%s' has the unknown Type '%s'", d->id.c_str(), d->type.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    if (d->number == "0") { set_error("FORMAT field '%s' has Number=0", d->id.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    if (d->number != "1") {
+      if (kind == HK_ListUtf8) { set_error("FORMAT field '%s': Type=%s with Number=%s is not supported by this build", d->id.c_str(), d->type.c_str(), d->number.c_str()); return BAMSCAN_ERR_UNSUPPORTED; }
+      kind = kind == HK_ListInt32 ? HK_ListListInt32 : HK_ListListFloat32;
+    }
+    const std::string name = "format_" + d->id;
+    for (const FieldDef& o : f->fields)
+      if (o.name == name) { set_error("FORMAT field '%s': a column named '%s' exists already", d->id.c_str(), name.c_str()); return BAMSCAN_ERR_SCHEMA; }
+    FieldDef fd{name, kind, false, {}};
+    fd.metadata = {{"bio.vcf.format.number", d->number}, {"bio.vcf.format.type", d->type}, {"bio.vcf.format.description", d->description}};
+    f->fields.push_back(fd);
+  }
+  // the sample names as a JSON array (escapes as Python's json.dumps with ensure_ascii=False)
+  std::string js = "[";
+  for (size_t i = 0; i < f->vcf_samples.size(); i++) {
+    js += i ? ", \"" : "\"";
+    for (unsigned char c : f->vcf_samples[i]) {
+      if (c == '"' || c == '\\') { js += '\\'; js += (char)c; }
+      else if (c == '\n') js += "\\n";
+      else if (c == '\r') js += "\\r";
+      else if (c == '\t') js += "\\t";
+      else if (c == '\b') js += "\\b";
+      else if (c == '\f') js += "\\f";
+      else if (c < 0x20) { char u[8]; snprintf(u, sizeof u, "\\u%04x", c); js += u; }
+      else js += (char)c;
+    }
+    js += '"';
+  }
+  js += "]";
+  f->schema_metadata.push_back({"bio.vcf.samples", js});
   return BAMSCAN_OK;
 }
 
@@ -294,13 +341,14 @@ static const char* kind_format(int32_t kind) {
     case HK_Int32: return "i"; case HK_UInt32: return "I"; case HK_Float32: return "f"; case HK_Utf8: return "u"; case HK_Binary: return "z";
     case HK_Boolean: return "b";
     case HK_ListInt8: case HK_ListUInt8: case HK_ListInt16: case HK_ListUInt16: case HK_ListInt32: case HK_ListUInt32: case HK_ListFloat32:
-    case HK_ListUtf8: return "+l";
+    case HK_ListUtf8: case HK_ListListInt32: case HK_ListListFloat32: return "+l";
   }
   return "n";
 }
 static const char* list_item_format(int32_t kind) {
   switch (kind) { case HK_ListInt8: return "c"; case HK_ListUInt8: return "C"; case HK_ListInt16: return "s"; case HK_ListUInt16: return "S";
-                  case HK_ListInt32: return "i"; case HK_ListUInt32: return "I"; case HK_ListFloat32: return "f"; case HK_ListUtf8: return "u"; }
+                  case HK_ListInt32: return "i"; case HK_ListUInt32: return "I"; case HK_ListFloat32: return "f"; case HK_ListUtf8: return "u";
+                  case HK_ListListInt32: case HK_ListListFloat32: return "+l"; }
   return "n";
 }
 
@@ -323,7 +371,9 @@ int export_schema(const std::vector<FieldDef>& fields, const std::vector<std::pa
     const FieldDef& f = fields[i];
     bool is_list = f.kind >= HK_ListInt8;
     fill_schema_node(out->children[i], kind_format(f.kind), f.name, f.nullable, f.metadata, is_list ? 1 : 0);
-    if (is_list) fill_schema_node(out->children[i]->children[0], list_item_format(f.kind), "item", true, {}, 0);   // tag_registry.rs:17-19
+    const bool nested = f.kind == HK_ListListInt32 || f.kind == HK_ListListFloat32;
+    if (is_list) fill_schema_node(out->children[i]->children[0], list_item_format(f.kind), "item", true, {}, nested ? 1 : 0);   // tag_registry.rs:17-19
+    if (nested) fill_schema_node(out->children[i]->children[0]->children[0], f.kind == HK_ListListInt32 ? "i" : "f", "item", true, {}, 0);
   }
   return BAMSCAN_OK;
 }

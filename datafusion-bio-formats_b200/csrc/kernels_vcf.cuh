@@ -32,7 +32,10 @@ namespace vcf {
 enum VcfErr : uint32_t {
   VCF_ERR_FIELDS = 40 /* fewer than 8 fields */, VCF_ERR_HASH = 41 /* a '#' line or an empty line */, VCF_ERR_POS = 42,
   VCF_ERR_CHROM = 43 /* empty CHROM */, VCF_ERR_REF = 44 /* empty REF */, VCF_ERR_END = 45 /* END below POS */, VCF_ERR_DUP = 46,
-  VCF_ERR_UTF8 = 47, VCF_ERR_QUAL = 48, VCF_ERR_VALUE = 49, VCF_ERR_POS0 = 50, VCF_ERR_LONG = 51
+  VCF_ERR_UTF8 = 47, VCF_ERR_QUAL = 48, VCF_ERR_VALUE = 49, VCF_ERR_POS0 = 50, VCF_ERR_LONG = 51,
+  // FORMAT columns (kernels_vcf_format.cuh): the first three are BAMSCAN_ERR_FORMAT, FMT_VALUE is BAMSCAN_ERR_SCHEMA
+  VCF_ERR_FMT_FIELDS = 52 /* not 9 + samples fields */, VCF_ERR_FMT_DUP = 53 /* a projected FORMAT key given twice */,
+  VCF_ERR_FMT_MANY = 54 /* a sample with more values than keys */, VCF_ERR_FMT_VALUE = 55
 };
 
 constexpr int32_t K_Boolean = 6, K_ListUtf8 = 17;   // (bamscan_internal.h: HK_Boolean, HK_ListUtf8)

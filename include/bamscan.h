@@ -69,6 +69,9 @@ typedef struct BamScanOptions {
   int32_t skip_crc;                       /* 0 (default): verify CRC32 of every BGZF member on the device; 1: skip */
   int32_t debug_flags;                    /* tests only. bit0: poison boundary candidates (exercises the repair path); bit1: force the long-record decode kernels (a warp per record); bit2 / bit3 / bit4: force the warp-per-member / the lane-group / the CTA-per-member inflate kernel (default: the CTA-per-member kernel); bit5: queue the next chunk's inflate behind the current chunk's first decode slice (the two overlap on the GPU; measured +1 % scan rate, -10 % inflate rate); bit6: skip the parallel boundary-repair rounds (every disagreeing seam goes to the sequential repair) */
   int32_t decode_all_tag_fields;          /* 1: reference behaviour (sam_tag_io.rs:42-52): once ANY tag column is projected every tag_fields entry is decoded, so a value that does not fit an UNPROJECTED tag column's type fails the scan; 0 (default): only projected tag columns are decoded */
+  int32_t has_format_fields;              /* VCF only: 0 => format_fields = None, which selects NO FORMAT column (unlike tag_fields / info_fields, where None selects all) */
+  int32_t n_format_fields;
+  const char* const* format_fields;       /* VCF only: FORMAT IDs, one list column per sample each (bamscan_open_vcf) */
 } BamScanOptions;
 
 /* ---- pushed-down predicates (reference: `filters: &[Expr]` of TableProvider::scan, restricted to the
@@ -175,7 +178,23 @@ int bamscan_open_fasta(const char* path, const BamScanOptions* options, BamScanH
  * (BAMSCAN_ERR_SCHEMA), POS 0 and lines over 16 MiB (BAMSCAN_ERR_UNSUPPORTED).  An INFO key given twice in one record is a
  * format error only for the keys the scan looks up (the projected INFO fields and END): other keys are skipped unread, as
  * their values are.  At most 112 INFO columns can be projected in one scan; bamscan_execute refuses more with
- * BAMSCAN_ERR_UNSUPPORTED (a header with more ##INFO fields needs info_fields or a projection).  FORMAT and sample columns are skipped.  bamscan_plan with
+ * BAMSCAN_ERR_UNSUPPORTED (a header with more ##INFO fields needs info_fields or a projection).
+ * FORMAT fields: has_format_fields / n_format_fields / format_fields select FORMAT IDs.  Unlike info_fields, 0 (None) selects NO
+ * FORMAT column, and so does an empty list: such a scan reads the header, the schema and the records exactly as without these
+ * fields.  A selected ID becomes the column format_<ID>, behind the INFO columns in format_fields order: non-nullable, one element
+ * per sample in header sample order (the #CHROM fields behind FORMAT).  Number=1 -> List<Int32 / Float32 / Utf8> (String and
+ * Character; GT is kept as written), any other Number on Integer / Float -> List<List<Int32 / Float32>>; elements and leaves are
+ * nullable.  Field metadata bio.vcf.format.{number,type,description}; schema metadata bio.vcf.samples (a JSON array of the sample
+ * names) when a FORMAT column is selected.  With format_fields non-empty, ##FORMAT lines are parsed as ##INFO lines are and a
+ * malformed one, an ID declared twice, or a first field behind INFO other than FORMAT is BAMSCAN_ERR_FORMAT.  Refused at open with
+ * BAMSCAN_ERR_SCHEMA naming the field: an undeclared or repeated ID, Type=Flag, Number=0, an unknown Type, a column name that
+ * exists already, a header without samples; with BAMSCAN_ERR_UNSUPPORTED: String / Character with Number other than 1, more than
+ * 16 IDs.  When a FORMAT column is projected, each record must have exactly 9 + samples fields (BAMSCAN_ERR_FORMAT otherwise); its
+ * FORMAT field is a ':'-separated key list ('.' or empty: none) whose order may differ per line, and a projected key given twice is
+ * a format error.  A sample's ':'-separated values match the keys by position: missing trailing values, '.', a key the line does
+ * not list, an empty sample and a lone '.' give NULL elements (for nested columns a NULL middle list, and ',' separates leaves,
+ * '.' a NULL leaf); more values than keys is BAMSCAN_ERR_FORMAT; a value that does not parse (an empty number, a ',' in a
+ * Number=1 value) is BAMSCAN_ERR_SCHEMA; a byte of 0x80 or above in a projected text value is BAMSCAN_ERR_FORMAT.  bamscan_plan with
  * BAMSCAN_PARTITION_BLOCK_RANGE balances BGZF block ranges by compressed bytes (a line belongs to the range that holds its first
  * byte); otherwise one partition.  No filter is pushed down, there is no index, describe is refused. */
 int bamscan_open_vcf(const char* path, const BamScanOptions* options, BamScanHandle** out);

@@ -227,19 +227,23 @@ class FastaTableProvider {
 // A provider for BGZF-compressed VCF (bamscan_open_vcf): the eight fixed columns, then one column per selected ##INFO field
 // (info_fields nullopt: all of them, in header order).  scan() with target_partitions > 1 cuts BGZF block ranges balanced by
 // compressed bytes; no filter is pushed down.  At most 112 INFO columns can be projected in one scan (execute throws
-// BAMSCAN_ERR_UNSUPPORTED above that): pass info_fields or a projection for headers with more ##INFO fields.
+// BAMSCAN_ERR_UNSUPPORTED above that): pass info_fields or a projection for headers with more ##INFO fields.  format_fields adds one
+// column format_<ID> per FORMAT ID, one element per sample; unlike info_fields, nullopt (and an empty list) selects none.
 class VcfTableProvider {
  public:
   explicit VcfTableProvider(const std::string& file_path, const std::optional<std::vector<std::string>>& info_fields = std::nullopt,
                             const std::optional<std::string>& object_storage_options = std::nullopt, bool coordinate_system_zero_based = true,
-                            int32_t device_id = 0, int32_t batch_rows = 0) {
+                            int32_t device_id = 0, int32_t batch_rows = 0,
+                            const std::optional<std::vector<std::string>>& format_fields = std::nullopt) {
     if (object_storage_options) throw Error(BAMSCAN_ERR_UNSUPPORTED, "remote object storage is out of scope for this build (local files only)");
-    std::vector<const char*> ids;
+    std::vector<const char*> ids, fmt;
     if (info_fields) for (auto& i : *info_fields) ids.push_back(i.c_str());
+    if (format_fields) for (auto& i : *format_fields) fmt.push_back(i.c_str());
     BamScanOptions o; std::memset(&o, 0, sizeof o);
     o.struct_size = sizeof o; o.device_id = device_id; o.batch_rows = batch_rows;
     o.coordinate_system_zero_based = coordinate_system_zero_based;
     o.has_tag_fields = info_fields.has_value(); o.n_tag_fields = (int32_t)ids.size(); o.tag_fields = ids.empty() ? nullptr : ids.data();
+    o.has_format_fields = format_fields.has_value(); o.n_format_fields = (int32_t)fmt.size(); o.format_fields = fmt.empty() ? nullptr : fmt.data();
     check(bamscan_open_vcf(file_path.c_str(), &o, &h_));
   }
   VcfTableProvider(VcfTableProvider&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }

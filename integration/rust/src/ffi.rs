@@ -35,6 +35,11 @@ pub struct BamScanOptions {
     pub segment_bytes: u32,
     pub skip_crc: i32,
     pub debug_flags: i32,
+    pub decode_all_tag_fields: i32,
+    /// VCF only: 0 => `format_fields` = None, which selects no FORMAT column (unlike `tag_fields`)
+    pub has_format_fields: i32,
+    pub n_format_fields: i32,
+    pub format_fields: *const *const c_char,
 }
 
 #[repr(C)]

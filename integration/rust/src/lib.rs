@@ -102,6 +102,10 @@ impl GpuBamTableProvider {
             segment_bytes: 0,
             skip_crc: 0,
             debug_flags: 0,
+            decode_all_tag_fields: 0,
+            has_format_fields: 0,
+            n_format_fields: 0,
+            format_fields: std::ptr::null(),
         };
         let mut raw = std::ptr::null_mut();
         // index_path = NULL: discover `<file>.bai` / `.csi` next to the file like `discover_bam_index` does
@@ -433,6 +437,10 @@ impl GpuFastaTableProvider {
             segment_bytes: 0,
             skip_crc: 0,
             debug_flags: 0,
+            decode_all_tag_fields: 0,
+            has_format_fields: 0,
+            n_format_fields: 0,
+            format_fields: std::ptr::null(),
         };
         let mut raw = std::ptr::null_mut();
         if unsafe { ffi::bamscan_open_fasta(c_path.as_ptr(), &opts, &mut raw) } != 0 {
@@ -508,7 +516,8 @@ impl TableProvider for GpuFastaTableProvider {
 
 /// A provider for BGZF-compressed VCF (`bamscan_open_vcf`), shaped like the BAM one: chrom, start, end, id, ref, alt, qual and
 /// filter, then one column per selected `##INFO` field (Flag -> Boolean, Number=1 -> Int32 / Float32 / Utf8, any other Number ->
-/// a list of those); FORMAT and sample columns are skipped.  `info_fields` `None` selects every `##INFO` field in header order;
+/// a list of those), then one column `format_<ID>` per selected FORMAT field holding one element per sample (`format_fields`
+/// `None` or empty selects none, unlike `info_fields`; rules in bamscan.h).  `info_fields` `None` selects every `##INFO` field in header order;
 /// at most 112 INFO columns can be projected in one scan (more fail with BAMSCAN_ERR_UNSUPPORTED).  No filter is pushed down
 /// (DataFusion applies them), `limit` is passed on and not applied, and with `target_partitions` > 1 the file is cut into BGZF
 /// block ranges balanced by compressed bytes (a line belongs to the range that holds its first byte).  Scans return
@@ -522,7 +531,7 @@ pub struct GpuVcfTableProvider {
 impl GpuVcfTableProvider {
     /// `object_storage_options` must be `None` (local files only).  `device_id` selects the GPU.
     pub fn new(file_path: String, info_fields: Option<Vec<String>>, object_storage_options: Option<String>, coordinate_system_zero_based: bool,
-               device_id: i32) -> Result<Self> {
+               device_id: i32, format_fields: Option<Vec<String>>) -> Result<Self> {
         if object_storage_options.is_some() {
             return Err(DataFusionError::NotImplemented("remote object storage is out of scope for this build (local files only)".into()));
         }
@@ -530,6 +539,9 @@ impl GpuVcfTableProvider {
         let c_ids: Vec<CString> = info_fields.iter().flatten().map(|s| CString::new(s.as_str())).collect::<std::result::Result<_, _>>()
             .map_err(|e| DataFusionError::Execution(e.to_string()))?;
         let id_ptrs: Vec<*const c_char> = c_ids.iter().map(|c| c.as_ptr()).collect();
+        let c_fmt: Vec<CString> = format_fields.iter().flatten().map(|s| CString::new(s.as_str())).collect::<std::result::Result<_, _>>()
+            .map_err(|e| DataFusionError::Execution(e.to_string()))?;
+        let fmt_ptrs: Vec<*const c_char> = c_fmt.iter().map(|c| c.as_ptr()).collect();
         let opts = ffi::BamScanOptions {
             struct_size: std::mem::size_of::<ffi::BamScanOptions>() as u32,
             coordinate_system_zero_based: coordinate_system_zero_based as i32,
@@ -547,6 +559,10 @@ impl GpuVcfTableProvider {
             segment_bytes: 0,
             skip_crc: 0,
             debug_flags: 0,
+            decode_all_tag_fields: 0,
+            has_format_fields: format_fields.is_some() as i32,
+            n_format_fields: fmt_ptrs.len() as i32,
+            format_fields: if fmt_ptrs.is_empty() { std::ptr::null() } else { fmt_ptrs.as_ptr() },
         };
         let mut raw = std::ptr::null_mut();
         if unsafe { ffi::bamscan_open_vcf(c_path.as_ptr(), &opts, &mut raw) } != 0 {

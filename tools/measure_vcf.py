@@ -6,7 +6,9 @@
 Per input: device-resident CUDA-event time per stage (run_device_resident: ms_inflate, ms_boundary = the newline scan and line
 framing, ms_decode = the VCF kernels), rows/s and inflated GB/s, kernel launches, kernel times by name (torch.profiler, in a run of
 its own), and end to end through the ABI (host batches).  The card's name and power limit are read in the same run.
-usage: python tools/measure_vcf.py [out.md] [sites_records=5000000] [genotype_records=200000]"""
+With a fourth argument, instead: one genotype input of that many records x 2 504 samples carrying FORMAT GT:DP:AD:GQ:PL
+(tests/vcf_format_inputs.py), scanned (a) without FORMAT columns, (b) with format_fields=["GT"] and (c) with all five.
+usage: python tools/measure_vcf.py [out.md] [sites_records=5000000] [genotype_records=200000] [format_records]"""
 import os
 import subprocess
 import sys
@@ -20,6 +22,7 @@ for p in (str(ROOT), str(ROOT / "datafusion-bio-formats_b200"), str(ROOT / "test
 OUT = Path(sys.argv[1]) if len(sys.argv) > 1 else ROOT / "profiles" / "r4_vcf.md"
 SITES = int(sys.argv[2]) if len(sys.argv) > 2 else 5_000_000
 GENOTYPES = int(sys.argv[3]) if len(sys.argv) > 3 else 200_000
+FORMAT_RECORDS = int(sys.argv[4]) if len(sys.argv) > 4 else 0
 
 
 def card():
@@ -42,10 +45,10 @@ def kernel_ms(fn):
     return out
 
 
-def measure(path):
+def measure(path, format_fields=None):
     import bamscan
     rows = {}
-    p = bamscan.VcfTableProvider(str(path))
+    p = bamscan.VcfTableProvider(str(path), format_fields=format_fields)
     plan = p.scan()
     plan.run_device_resident(0, 1)                                   # warm-up (module load, allocations)
     st = plan.run_device_resident(0, 3)
@@ -59,7 +62,7 @@ def measure(path):
     rows["device-resident M rows/s"] = st["rows"] / st["ms_total"] / 1e3
     rows["device-resident inflated GB/s"] = st["inflated_bytes"] / st["ms_total"] / 1e6
     t0 = time.perf_counter()
-    p2 = bamscan.VcfTableProvider(str(path))
+    p2 = bamscan.VcfTableProvider(str(path), format_fields=format_fields)
     n = sum(b.num_rows for b in p2.scan().execute(0))
     t1 = time.perf_counter()
     assert n == st["rows"]
@@ -75,7 +78,45 @@ def measure(path):
     return rows
 
 
+def main_format():
+    from vcf_format_inputs import FIVE, format_text
+    from vcf_inputs import bgzf_parallel
+    info = card()
+    base = Path(os.environ.get("BAMSCAN_BENCH_DIR", tempfile.mkdtemp(prefix="bamscan_vcf_")))
+    base.mkdir(parents=True, exist_ok=True)
+    path = base / "format.vcf.gz"
+    t0 = time.time()
+    text = format_text(FORMAT_RECORDS)
+    path.write_bytes(bgzf_parallel(text))
+    print(f"[format] generated {len(text) / 1e9:.2f} GB text, {path.stat().st_size / 1e9:.2f} GB file in {time.time() - t0:.1f} s", file=sys.stderr)
+    del text
+    cases = {"(a) no FORMAT": None, "(b) GT": ["GT"], "(c) GT DP AD GQ PL": FIVE}
+    results = {}
+    for name, sel in cases.items():
+        results[name] = measure(path, sel)
+        print(f"[{name}] {results[name]}", file=sys.stderr)
+    path.unlink()
+    keys = list(dict.fromkeys(k for r in results.values() for k in r))
+    lines = ["# VCF FORMAT columns on one GPU (`tools/measure_vcf.py`, FORMAT input)", "",
+             f"Card (nvidia-smi name, power limit, max SM clock): **{info}**.", "",
+             f"Input from `tests/vcf_format_inputs.py::format_text`: {FORMAT_RECORDS:,} records x 2 504 samples of FORMAT "
+             "GT:DP:AD:GQ:PL (every seventh line GT:PL:DP), zlib level 1 BGZF members of 0xff00 bytes.", "",
+             "Device-resident times are CUDA events around the whole partition with the compressed file staged in HBM (mean of 3 "
+             "runs after a warm-up); the stage split is of the last run. Kernel times come from a separate run under "
+             "torch.profiler. End to end is `VcfTableProvider.scan().execute(0)` to host Arrow batches of every column.", "",
+             "| | " + " | ".join(cases) + " |", "|---|" + "---:|" * len(cases)]
+    for k in keys:
+        vals = [r.get(k, 0.0) for r in results.values()]
+        fmt = (lambda v: f"{v:,}") if all(isinstance(v, int) for v in vals) else (lambda v: f"{v:,.3f}")
+        lines.append(f"| {k} | " + " | ".join(fmt(v) for v in vals) + " |")
+    OUT.parent.mkdir(parents=True, exist_ok=True)
+    OUT.write_text("\n".join(lines) + "\n")
+    print("\n".join(lines))
+
+
 def main():
+    if FORMAT_RECORDS:
+        return main_format()
     from vcf_inputs import bgzf_parallel, genotypes_text, sites_text
     info = card()
     base = Path(os.environ.get("BAMSCAN_BENCH_DIR", tempfile.mkdtemp(prefix="bamscan_vcf_")))
